@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mode-I frames/s decoded (IQ -> Viterbi) on N B200s, one JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Headline workload (BASELINE.json configs[1]): FIC-only decode of a ~10 000-frame synthetic Mode-I batch per GPU (PRS sync,
@@ -206,6 +206,17 @@ def int_alu_peak_acs(sm_mhz):
     return 148 * 128 * sm_mhz * 1e6 / 4.0
 
 
+def load_sweep_softbits():
+    """tests/golden/sweep_softbits.npz with its soft bits decoded: every soft_<level> is stored as an xz stream of little-endian
+    int16 (16 logical frames x size_cu * 64), which keeps the file under 1 MB; the other arrays are stored as they are."""
+    import lzma
+    g = np.load(os.path.join(ROOT, "tests", "golden", "sweep_softbits.npz"))
+    out = {k: g[k] for k in g.files}
+    for li, (_, _, _, _, cu) in enumerate(SWEEP_PROFILES):
+        out[f"soft_{li}"] = np.frombuffer(lzma.decompress(out[f"soft_{li}"].tobytes()), "<i2").astype(np.int16).reshape(-1, cu * 64)
+    return out
+
+
 def prbs_bits(n):
     """Energy-dispersal sequence x^9 + x^5 + 1, all-ones start (backend.cpp:72-83)."""
     reg = [1] * 9
@@ -225,7 +236,7 @@ def viterbi_sweep(ctx, stream, n_frames, sm_mhz):
     import ctypes
     import torch
     from dabstar_b200 import api
-    gold = np.load(os.path.join(ROOT, "tests", "golden", "sweep_softbits.npz"))
+    gold = load_sweep_softbits()
     out = {"logical_frames_per_level": n_frames, "levels": {}, "input": "reference-generated soft bits (oracle/_ref chain at 12 dB SNR, 16 logical frames per level tiled), resident in HBM",
            "bits_equal_reference": True}
     tot_bits, tot_ms = 0.0, 0.0
@@ -322,6 +333,48 @@ class Timed:
         stages = {k: v[0] for k, v in dp.stage_ms().items() if v[0] > 0}
         msc = list(dp.msc_kernel_ms())
         return ms, stages, msc
+
+
+FRAME_INFO_FIELDS = ("sym0_pos", "start_index", "fbb_sym0", "fbb_data", "fbb_null", "fsync", "phase_cp", "clock_err", "fic_ratio_before", "fic_ratio_after")
+DUMP_RECORDING_BYTES = 40 << 20   # budget of the per-recording arrays; beyond it a seeded subset of the recordings is written
+DUMP_SOFT_FRAMES = 16             # (recording, frame) pairs of soft_bits_sample.npy (14 MB), drawn with a fixed seed
+
+
+def dump_outputs(dp, R, F, out_dir):
+    """Writes what the headline decode returned to its caller for the batch's last run, as float32 / float64 .npy files under
+    out_dir (30 MB at the default sizes, at most 54 MB): for the recordings listed in recordings.npy (all of them unless that
+    would pass the budget) the frame count, the FrameInfo fields of every frame (last axis of frame_info.npy in the order of
+    FRAME_INFO_FIELDS), the FIC CRC flags, the packed FIB bytes and the counters; and the soft bits of a seeded sample of frames
+    (soft_bits_sample_index.npy: recording, frame). Frames a recording did not decode are NaN, so two builds can be compared
+    array for array even where their frame counts differ."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    per_recording = F * (12 * 32 * 4 + len(FRAME_INFO_FIELDS) * 8 + 4 * 4) + 8 * 8 + 8
+    rows = np.arange(R)
+    if R * per_recording > DUMP_RECORDING_BYTES:
+        rows = np.sort(rng.choice(R, max(1, DUMP_RECORDING_BYTES // per_recording), replace=False))
+    res = [dp.result(int(r)) for r in rows]
+    nf = np.array([x.n_frames for x in res], np.float64)
+    n_max = max(1, int(nf.max()))
+    info = np.full((len(rows), n_max, len(FRAME_INFO_FIELDS)), np.nan, np.float64)
+    valid = np.full((len(rows), n_max, 4), np.nan, np.float32)
+    fib = np.full((len(rows), n_max, 12, 32), np.nan, np.float32)
+    for j, (r, x) in enumerate(zip(rows, res)):
+        if not x.n_frames:   # a recording without a decoded frame stays NaN
+            continue
+        info[j, :x.n_frames] = [[getattr(i, k) for k in FRAME_INFO_FIELDS] for i in x.info]
+        valid[j, :x.n_frames] = x.fic_valid
+        fib[j, :x.n_frames] = dp.fib_packed(int(r))
+    pick = np.stack([rng.integers(0, R, DUMP_SOFT_FRAMES), rng.integers(0, F, DUMP_SOFT_FRAMES)], axis=1)
+    soft = np.full((DUMP_SOFT_FRAMES, 75, 3072), np.nan, np.float32)
+    for j, (r, f) in enumerate(pick):
+        if f < dp.n_frames(int(r)):
+            soft[j] = dp.soft_bits(int(r), int(f))
+    arrays = {"recordings": rows.astype(np.float64), "n_frames": nf, "frame_info": info, "fic_valid": valid, "fib_packed": fib,
+              "counters": np.stack([x.counters for x in res]).astype(np.float64), "soft_bits_sample_index": pick.astype(np.float64),
+              "soft_bits_sample": soft}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def replicated_recordings(uniq, copies):
@@ -546,18 +599,12 @@ def native_arm(args, rank, local_rank, world):
     n_samples = LEAD + F * T_F + TAIL
     S_UNIQ = min(8, R)   # recordings with rank-independent seeds: the frames of the shared single stream
 
-    # ---- synthetic recordings in pinned host memory; unique ones up to a time budget, then reused
+    # ---- synthetic recordings in pinned host memory, every one from its own seed: the same arguments give the same input
     host = torch.empty((R, n_samples, 2), dtype=torch.uint8, pin_memory=True)
     hnp = host.numpy()
-    t0 = time.time()
-    unique = 0
     for r in range(R):
-        if time.time() - t0 < args.synth_budget or unique < S_UNIQ:
-            seed = args.seed + r if r < S_UNIQ else args.seed + 7919 * rank + r
-            synth.generate(F, seed=seed, snr_db=args.snr, fmt=synth.FMT_U8, out=hnp[r])
-            unique += 1
-        else:
-            hnp[r] = hnp[S_UNIQ + (r - S_UNIQ) % max(1, unique - S_UNIQ)] if unique > S_UNIQ else hnp[r % unique]
+        seed = args.seed + r if r < S_UNIQ else args.seed + 7919 * rank + r
+        synth.generate(F, seed=seed, snr_db=args.snr, fmt=synth.FMT_U8, out=hnp[r])
     dev = host.cuda(non_blocking=False)
     stream = torch.cuda.Stream()
     ctx = api.Context(local_rank, stream=stream)
@@ -573,9 +620,6 @@ def native_arm(args, rank, local_rank, world):
     with torch.cuda.stream(stream):
         for _ in range(args.warmup):
             dp.run_ptrs(d_ptrs, ns, api.MEM_DEVICE)
-        cnt = np.sum([dp.counters(r) for r in range(R)], axis=0)
-        frames_per_step = int(cnt[6])
-        good_fibs = int(cnt[0])
         # ---- timed: inputs resident in HBM
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         clocks = ClockSampler(local_rank)
@@ -591,6 +635,11 @@ def native_arm(args, rank, local_rank, world):
         clk = clocks.stop()
         ms_total = e0.elapsed_time(e1)
         launches = ctx.kernel_launches - launches0
+        cnt = np.sum([dp.counters(r) for r in range(R)], axis=0)   # of the last timed step
+        frames_per_step = int(cnt[6])
+        good_fibs = int(cnt[0])
+        if args.dump_outputs and rank == 0:
+            dump_outputs(dp, R, F, args.dump_outputs)
         # ---- the same steps again, untimed, for the per-kernel-family CUDA-event times (reading them back after every run costs
         #      host time that is not part of the decode)
         stage_acc = {}
@@ -721,7 +770,7 @@ def native_arm(args, rank, local_rank, world):
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
         "ms_per_step": ms_total / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
-        "data": f"synthetic ({unique} unique recordings per GPU of {R}, random FIB payloads, AWGN {args.snr} dB)",
+        "data": f"synthetic ({R} unique recordings per GPU of {R}, random FIB payloads, AWGN {args.snr} dB)",
         "config": cfg,
         "run": {"frames_per_step_all_gpus": total_frames, "input_bytes_per_gpu": int(R * n_samples * 2),
                 "l2": "inputs (3.9 GB) and intermediates far exceed the 126 MB L2", "window": args.window, "cpus_per_rank": pinned_cpus,
@@ -749,7 +798,6 @@ def main():
     ap.add_argument("--window", type=int, default=128)
     ap.add_argument("--seed", type=int, default=2)
     ap.add_argument("--snr", type=float, default=15.0)
-    ap.add_argument("--synth-budget", type=float, default=45.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-viterbi-sweep", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="only the headline workload (configs[1]) and the Viterbi sweep")
@@ -762,9 +810,12 @@ def main():
     ap.add_argument("--stream-window", type=int, default=9984)
     ap.add_argument("--stream-segment-frames", type=int, default=0, help="single_stream: frames per demapper segment (0 = about 96 segments per window, 32..104 frames)")
     ap.add_argument("--snr-cfo-frames", type=int, default=13)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="native arm only: after the timed headline steps, write what the last step decoded (rank 0) as .npy files to DIR")
     ap.add_argument("--cpu-worker", action="store_true")
     ap.add_argument("--cpu-lib", default="dabo")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the native arm's decoded outputs; --impl reference has none to write")
     if args.cpu_worker:
         return cpu_worker(args)
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)

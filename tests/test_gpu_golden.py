@@ -45,7 +45,7 @@ def test_sweep_soft_bits_of_the_reference_cuda(ctx, viterbi_path):
     reference's Backend output once the energy dispersal is put back; a tiled batch of 2 400 frames takes the
     thread-per-code-word path with its device-written job list, the 16 frames alone the warp-per-code-word kernel."""
     import bench
-    g = load("sweep_softbits.npz")
+    g = bench.load_sweep_softbits()
     assert [tuple(int(x) for x in row) for row in g["profiles"]] == [p[1:] for p in bench.SWEEP_PROFILES]
     for li, (name, sf, lvl, br, cu) in enumerate(bench.SWEEP_PROFILES):
         soft = g[f"soft_{li}"]

@@ -7,6 +7,7 @@ for its Viterbi-only sweep ("on reference-generated soft bits"); tests/test_gpu_
 
 Run in the build container (needs /root/reference for oracle/_ref):  python tools/make_sweep_softbits.py
 De-interleaving follows backend.cpp:131-138: tempX[i] = CIF[c - 16 + map[i & 15]][i]."""
+import lzma
 import os
 import sys
 
@@ -49,7 +50,8 @@ def main():
             bits = res.msc[s.sub_ch_id]       # Backend output: rows from the 17th CIF on, energy dispersal removed
             assert bits.shape[0] == frames.shape[0], (bits.shape, frames.shape)
             assert np.array_equal(bits, rec.msc_truth[j][:bits.shape[0]]), name   # 12 dB: the reference decodes without errors
-            out[f"soft_{len(out) // 2}"] = frames.astype(np.int16)
+            # xz stream of little-endian int16: keeps the file under 1 MB (bench.load_sweep_softbits decodes it)
+            out[f"soft_{len(out) // 2}"] = np.frombuffer(lzma.compress(frames.astype("<i2").tobytes(), preset=9 | lzma.PRESET_EXTREME), np.uint8)
             out[f"bits_{len(out) // 2}"] = np.packbits(bits, axis=1)
             print(name, frames.shape, int(np.abs(frames).max()))
     out["names"] = np.array([p[0] for p in PROFILES])
