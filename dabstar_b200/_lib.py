@@ -62,6 +62,11 @@ class ServiceCompC(ctypes.Structure):
     _fields_ = [("sid", ctypes.c_uint32)] + [(n, ctypes.c_int32) for n in ("comp_index", "tmid", "type", "sub_ch_id", "primary", "ca_flag")]
 
 
+class FftFrameC(ctypes.Structure):
+    _fields_ = [("sym0", ctypes.c_int64), ("eval", ctypes.c_int64)] + [(n, ctypes.c_int32) for n in (
+        "rec", "xslot", "f_sym0", "ph_eval", "f_data", "ph_data", "f_null", "ph_null", "n_syms", "reserved")]
+
+
 # every symbol include/dabstar_b200.h declares: (name, restype)
 EXPORTS = [
     ("dabstar_create", ctypes.c_int), ("dabstar_destroy", None), ("dabstar_last_error", ctypes.c_char_p),
@@ -79,6 +84,7 @@ EXPORTS = [
     ("dabstar_ofdm_state_create", ctypes.c_int), ("dabstar_ofdm_state_destroy", None), ("dabstar_ofdm_state_reset", ctypes.c_int),
     ("dabstar_ofdm_state_get", ctypes.c_int), ("dabstar_ofdm_state_quality", ctypes.c_int), ("dabstar_ofdm_decode_frames", ctypes.c_int),
     ("dabstar_prs_correlate", ctypes.c_int), ("dabstar_estimate_carrier_offset", ctypes.c_int), ("dabstar_cp_correlate", ctypes.c_int),
+    ("dabstar_fft_frames", ctypes.c_int),
     ("dabstar_decoder_create", ctypes.c_int), ("dabstar_decoder_destroy", None), ("dabstar_decoder_set_subchannels", ctypes.c_int),
     ("dabstar_decoder_run", ctypes.c_int), ("dabstar_decoder_n_frames", ctypes.c_int), ("dabstar_decoder_frame_info", ctypes.c_int),
     ("dabstar_decoder_fib_bits", ctypes.c_int), ("dabstar_decoder_fib_packed", ctypes.c_int), ("dabstar_decoder_soft_bits", ctypes.c_int),

@@ -318,6 +318,28 @@ def cp_correlate(frames: np.ndarray, ctx: Context | None = None) -> np.ndarray:
     return out
 
 
+def fft_frames(recordings: list[np.ndarray], fmt: int, frames: list[dict], n_xslots: int, max_ctas_per_sm: int = 0, with_null: bool = False,
+               ctx: Context | None = None):
+    """The decoder's frame FFT (k_fft_frames; with_null: k_fft_null too) over caller-made frame descriptors (see dabstar_fft_frames).
+    recordings: arrays of one format (cf32: complex64[n]; u8: uint8[n, 2]; i16: int16[n, 2]), laid end to end in one buffer.
+    frames: dicts with the fields of dabstar_fft_frame (missing ones are 0). Returns (X complex64[n_xslots, 77, 1536] in nominal
+    carrier order, unwritten rows holding the 0xFF fill bit for bit; null complex64[n_frames, 2048] or None)."""
+    ctx = ctx or default_context()
+    dt = {FMT_CF32: np.complex64, FMT_U8: np.uint8, FMT_I16: np.int16}.get(fmt, np.uint8)
+    recs = [_np(r, dt).reshape(-1) for r in recordings]
+    n_rec = np.array([r.size if fmt == FMT_CF32 else r.size // 2 for r in recs], np.int64)
+    buf = np.concatenate(recs) if recs else np.zeros(1, dt)
+    fr = (_lib.FftFrameC * max(len(frames), 1))(*[_lib.FftFrameC(**f) for f in frames])
+    raw = np.empty((n_xslots, 77, 768, 4), np.float32)
+    null = np.empty((len(frames), 2048), np.complex64) if with_null else None
+    ctx.check(ctx.lib.dabstar_fft_frames(ctx.h, _ptr(buf), int(fmt), _ptr(n_rec), len(recs), fr, len(frames), int(n_xslots), int(max_ctas_per_sm),
+                                         _ptr(raw), _ptr(null) if with_null else None, MEM_HOST), "dabstar_fft_frames")
+    x = np.empty((n_xslots, 77, 768, 2, 2), np.float32)  # [pair][carrier 2p / 2p + 1][re / im]
+    x[..., 0] = raw[..., 0:2]
+    x[..., 1] = raw[..., 2:4]
+    return x.view(np.complex64).reshape(n_xslots, 77, 1536), null
+
+
 class ViterbiSpiral:
     """support/viterbi_spiral/viterbi_spiral.h:20 — deconvolve() over a batch of equally long code words."""
 

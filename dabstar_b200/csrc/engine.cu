@@ -1058,6 +1058,72 @@ extern "C" int dabstar_cp_correlate(dabstar_ctx * ctx, const float * samples, in
   return stage_out_end(ctx, dout, out, sizeof(float2) * (size_t)n, mem);
 }
 
+// Stage tap of k_fft_frames (and k_fft_null) over caller-made frame descriptors: the recordings lie end to end in one buffer, so
+// their base addresses take every alignment a caller's device buffer can have. Every argument is checked before anything is
+// queued: an xslot out of range would be a store outside X.
+extern "C" int dabstar_fft_frames(dabstar_ctx * ctx, const void * samples, int fmt, const int64_t * rec_samples, int n_recs,
+                                  const dabstar_fft_frame * frames, int n_frames, int n_xslots, int max_ctas_per_sm, float * X,
+                                  float * null_fft, int mem)
+{
+  if (!ctx || !samples || !X || n_recs < 0 || n_frames < 0 || n_xslots < 0 || max_ctas_per_sm < 0) return DABSTAR_E_INVALID;
+  if ((n_recs > 0 && !rec_samples) || (n_frames > 0 && !frames)) return DABSTAR_E_INVALID;
+  if (fmt != FMT_CF32 && fmt != FMT_U8 && fmt != FMT_I16) return ctx->fail(DABSTAR_E_INVALID, "unknown sample format %d", fmt);
+  const size_t elem = fmt == FMT_CF32 ? sizeof(float2) : (fmt == FMT_I16 ? 2 * sizeof(int16_t) : 2 * sizeof(uint8_t));
+  long long total = 0;
+  for (int r = 0; r < n_recs; r++)
+  {
+    if (rec_samples[r] < 0) return ctx->fail(DABSTAR_E_INVALID, "recording %d: %lld samples", r, (long long)rec_samples[r]);
+    total += rec_samples[r];
+  }
+  std::vector<FrameDesc> fd((size_t)n_frames);
+  for (int f = 0; f < n_frames; f++)
+  {
+    const dabstar_fft_frame & s = frames[f];
+    if (s.rec < 0 || s.rec >= n_recs) return ctx->fail(DABSTAR_E_INVALID, "frame %d: recording %d of %d", f, s.rec, n_recs);
+    if (s.xslot < 0 || s.xslot >= n_xslots) return ctx->fail(DABSTAR_E_INVALID, "frame %d: X slot %d of %d", f, s.xslot, n_xslots);
+    if (s.n_syms < 0 || s.n_syms > 75) return ctx->fail(DABSTAR_E_INVALID, "frame %d: n_syms %d", f, s.n_syms);
+    for (int hz : { s.f_sym0, s.f_data, s.f_null })
+      if (hz <= -FS || hz >= FS) return ctx->fail(DABSTAR_E_INVALID, "frame %d: %d Hz", f, hz); // (keeps the kernel's 32-bit phase products in range)
+    memset(&fd[f], 0, sizeof(FrameDesc));
+    fd[f].sym0 = s.sym0;
+    fd[f].eval = s.eval;
+    fd[f].rec = s.rec;
+    fd[f].slot = f;
+    fd[f].xslot = s.xslot;
+    fd[f].f_sym0 = s.f_sym0; fd[f].ph_eval = s.ph_eval;
+    fd[f].f_data = s.f_data; fd[f].ph_data = s.ph_data;
+    fd[f].f_null = s.f_null; fd[f].ph_null = s.ph_null;
+    fd[f].n_syms = s.n_syms;
+  }
+  CK(cudaSetDevice(ctx->device));
+  const size_t x_bytes = sizeof(float2) * (size_t)n_xslots * X_ROWS * K_CARR, null_bytes = sizeof(float2) * (size_t)n_frames * T_U;
+  const void * din = samples; void * dX; void * dnull = nullptr;
+  if (total > 0)
+    if (int r = stage_in(ctx, ctx->scratch[0], samples, elem * (size_t)total, mem, &din)) return r;
+  if (int r = stage_out_begin(ctx, ctx->scratch[1], X, x_bytes, mem, &dX)) return r;
+  if (null_fft && n_frames > 0)
+    if (int r = stage_out_begin(ctx, ctx->scratch[4], null_fft, null_bytes, mem, &dnull)) return r;
+  std::vector<RecInput> rin((size_t)n_recs);
+  long long off = 0;
+  for (int r = 0; r < n_recs; off += rec_samples[r], r++) rin[r] = RecInput{ static_cast<const unsigned char *>(din) + elem * (size_t)off, rec_samples[r] };
+  CK(cudaMemsetAsync(dX, 0xFF, x_bytes, ctx->stream));
+  if (n_frames > 0)
+  {
+    CK(ctx->scratch[3].reserve(sizeof(FrameDesc) * fd.size() + sizeof(RecInput) * rin.size() + 64));
+    FrameDesc * dfd = ctx->scratch[3].as<FrameDesc>();
+    RecInput * drin = reinterpret_cast<RecInput *>(dfd + fd.size());
+    UP(dfd, fd.data(), sizeof(FrameDesc) * fd.size());
+    UP(drin, rin.data(), sizeof(RecInput) * rin.size());
+    CK(launch_fft_frames(ctx->stream, ctx->tab, dfd, n_frames, drin, fmt, (float2 *)dX, max_ctas_per_sm, &ctx->launches));
+    if (dnull)
+    {
+      CK(launch_fft_null(ctx->stream, ctx->tab, dfd, n_frames, drin, fmt, (float2 *)dnull, &ctx->launches));
+      if (mem == DABSTAR_MEM_HOST) CK(cudaMemcpyAsync(null_fft, dnull, null_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+  }
+  return stage_out_end(ctx, dX, X, x_bytes, mem);
+}
+
 // ------------------------------------------------------------------------------------------------ whole path
 namespace
 {

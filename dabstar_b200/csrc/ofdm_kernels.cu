@@ -439,6 +439,17 @@ __global__ void __launch_bounds__(FFT_THREADS, 4) k_fft_null(const FrameDesc * _
     const SymbolItem it = symbol_item(fd, rin, X_ROWS - 1);
     float2 v[16];
     load_symbol<FMT>(v, it.iq, it.n_total, it.start, it.f, it.ph, step, tid);
+    if (!(it.start >= 0 && it.start + T_U <= it.n_total))
+    {
+      // zero AFTER the oscillator, as k_fft_frames does: mixing a zero amplitude can give -0, and then a null symbol that lies
+      // past the end of the recording transforms to a row with -0 where row 76 of X has +0
+#pragma unroll
+      for (int n1 = 0; n1 < 16; n1++)
+      {
+        const long long i = it.start + 128 * n1 + tid;
+        if (i < 0 || i >= it.n_total) v[n1] = make_float2(0.0f, 0.0f);
+      }
+    }
     fft2048_to_smem(v, tw, smem, tid);
     for (int i = tid; i < T_U; i += FFT_THREADS) out[(size_t)fi * T_U + i] = smem[fft_nat(i)];
     __syncthreads();

@@ -306,6 +306,32 @@ int  dabstar_fib_parser_components(const dabstar_fib_parser * p, dabstar_service
  * sum_sym sum_{i < 504} x[i + 2048] conj(x[i]); its argument, limited to +-20 degrees, is the fine AFC step (:236-251,366). */
 int dabstar_cp_correlate(dabstar_ctx * ctx, const float * samples, int n, float * out_re_im, int mem);
 
+/* The decoder's own frame FFT (sample conversion, cyclic-prefix removal, integer-Hz oscillator, 2048-point transform and
+ * frequency de-interleaving in one kernel), exposed for tests. samples: n_recs recordings laid end to end in one buffer of
+ * DABSTAR_FMT_* `fmt` (u8 / i16 I,Q pairs or complex floats), recording r holding rec_samples[r] samples; samples outside a
+ * recording count as zero. frames: host array of n_frames descriptors; frame f writes rows 0..n_syms (and the null row 76
+ * when n_syms is 75) of X slot xslot. X: n_xslots x 77 x 1536 complex floats in the demapper's pair layout (re 2p, re 2p+1,
+ * im 2p, im 2p+1), filled with 0xFF bytes before the launch, so rows the kernel does not write keep that pattern.
+ * max_ctas_per_sm: resident CTAs per SM of the launch (0: the launcher's choice). null_fft (may be NULL): n_frames x 2048
+ * complex floats, the natural-order FFT of each frame's null symbol as the TII detector receives it.
+ * Oscillator (sample_reader.cpp:276-281): sample i (0-based) of a symbol read from phase ph is multiplied by
+ * e^{j 2 pi ((ph - f (i + 1)) mod 2048000) / 2048000}. Rejects an out-of-range rec / xslot, n_syms outside 0..75, a frequency
+ * of 2 048 000 Hz or more in magnitude, an unknown format or a negative count with DABSTAR_E_INVALID before launching anything. */
+typedef struct
+{
+  int64_t sym0;             /* sample index within the recording of the first useful sample of symbol 0 */
+  int64_t eval;             /* sample index at which the oscillator stands at ph_eval with f_sym0 */
+  int32_t rec, xslot;       /* recording index, row block of X */
+  int32_t f_sym0, ph_eval;  /* integer Hz and phase of symbol 0 */
+  int32_t f_data, ph_data;  /* ... before the first sample (cyclic prefix) of symbol 1 */
+  int32_t f_null, ph_null;  /* ... before the first sample of the null symbol */
+  int32_t n_syms;           /* data symbols present, 0..75 */
+  int32_t reserved;
+} dabstar_fft_frame;
+int dabstar_fft_frames(dabstar_ctx * ctx, const void * samples, int fmt, const int64_t * rec_samples, int n_recs,
+                       const dabstar_fft_frame * frames, int n_frames, int n_xslots, int max_ctas_per_sm, float * X,
+                       float * null_fft, int mem);
+
 /* ------------------------------------------------------------------------------------------------ whole path */
 typedef struct
 {
