@@ -83,6 +83,7 @@ EXPORTS = [
     ("dabstar_fic_decode", ctypes.c_int), ("dabstar_backend_process", ctypes.c_int),
     ("dabstar_ofdm_state_create", ctypes.c_int), ("dabstar_ofdm_state_destroy", None), ("dabstar_ofdm_state_reset", ctypes.c_int),
     ("dabstar_ofdm_state_get", ctypes.c_int), ("dabstar_ofdm_state_quality", ctypes.c_int), ("dabstar_ofdm_decode_frames", ctypes.c_int),
+    ("dabstar_ofdm_decode_frames_quality", ctypes.c_int),
     ("dabstar_prs_correlate", ctypes.c_int), ("dabstar_estimate_carrier_offset", ctypes.c_int), ("dabstar_cp_correlate", ctypes.c_int),
     ("dabstar_fft_frames", ctypes.c_int),
     ("dabstar_decoder_create", ctypes.c_int), ("dabstar_decoder_destroy", None), ("dabstar_decoder_set_subchannels", ctypes.c_int),
@@ -93,6 +94,7 @@ EXPORTS = [
     ("dabstar_decoder_enable_eti", ctypes.c_int), ("dabstar_decoder_eti_size", ctypes.c_int64), ("dabstar_decoder_eti_copy", ctypes.c_int64),
     ("dabstar_decoder_enable_tii", ctypes.c_int), ("dabstar_decoder_tii_events", ctypes.c_int), ("dabstar_decoder_tii_results", ctypes.c_int),
     ("dabstar_decoder_counters", ctypes.c_int), ("dabstar_decoder_quality", ctypes.c_int), ("dabstar_decoder_last_ms", ctypes.c_double),
+    ("dabstar_decoder_set_frame_quality", ctypes.c_int), ("dabstar_decoder_frame_quality", ctypes.c_int),
     ("dabstar_decoder_stage_ms", ctypes.c_int),
     ("dabstar_decoder_set_segmentation", ctypes.c_int), ("dabstar_decoder_set_streaming", ctypes.c_int), ("dabstar_decoder_consumed", ctypes.c_int64),
     ("dabstar_decoder_state_size", ctypes.c_int64), ("dabstar_decoder_export_state", ctypes.c_int64), ("dabstar_decoder_import_state", ctypes.c_int),

@@ -513,16 +513,23 @@ class OfdmDecoder:
         self.ctx.check(self.ctx.lib.dabstar_ofdm_state_quality(self.ctx.h, self.st, _ptr(out)), "dabstar_ofdm_state_quality")
         return dict(zip(self.QUALITY, (float(v) for v in out)))
 
-    def decode_frames(self, fft: np.ndarray, clock_err: np.ndarray | None = None, null_is_tii: np.ndarray | None = None) -> np.ndarray:
-        """fft: complex64[n, 77, 2048] (symbol 0, symbols 1..75, null). Returns int16[n, 75, 3072]."""
+    def decode_frames(self, fft: np.ndarray, clock_err: np.ndarray | None = None, null_is_tii: np.ndarray | None = None,
+                      quality: bool = False) -> np.ndarray | tuple[np.ndarray, np.ndarray]:
+        """fft: complex64[n, 77, 2048] (symbol 0, symbols 1..75, null). Returns int16[n, 75, 3072]; with quality, also
+        float32[n, 6] in QUALITY order: row f is quality() after frame f's null symbol (sigma_freq_corr 0)."""
         fft = _np(fft, np.complex64).reshape(-1, 77, 2048)
         n = fft.shape[0]
         ce = _np(clock_err if clock_err is not None else np.zeros(n), np.float32)
         tii = _np(null_is_tii if null_is_tii is not None else np.zeros(n), np.uint8)
         soft = np.zeros((n, 75, 3072), np.int16)
-        self.ctx.check(self.ctx.lib.dabstar_ofdm_decode_frames(self.ctx.h, self.st, _ptr(fft), n, _ptr(ce), _ptr(tii), self.soft_bit_type, _ptr(soft), MEM_HOST),
-                       "dabstar_ofdm_decode_frames")
-        return soft
+        if not quality:
+            self.ctx.check(self.ctx.lib.dabstar_ofdm_decode_frames(self.ctx.h, self.st, _ptr(fft), n, _ptr(ce), _ptr(tii), self.soft_bit_type, _ptr(soft), MEM_HOST),
+                           "dabstar_ofdm_decode_frames")
+            return soft
+        q = np.zeros((n, 6), np.float32)
+        self.ctx.check(self.ctx.lib.dabstar_ofdm_decode_frames_quality(self.ctx.h, self.st, _ptr(fft), n, _ptr(ce), _ptr(tii), self.soft_bit_type, _ptr(soft),
+                                                                       MEM_HOST, _ptr(q)), "dabstar_ofdm_decode_frames_quality")
+        return soft, q
 
 
 @dataclass
@@ -734,6 +741,18 @@ class DabProcessor:
         out = np.zeros(6, np.float32)
         self.ctx.check(self.ctx.lib.dabstar_decoder_quality(self.h, recording, _ptr(out)), "dabstar_decoder_quality")
         return dict(zip(OfdmDecoder.QUALITY, (float(v) for v in out)))
+
+    def set_frame_quality(self, on: bool = True):
+        """Capture quality() for every frame of the next runs (see frame_quality); off by default."""
+        self.ctx.check(self.ctx.lib.dabstar_decoder_set_frame_quality(self.h, int(on)), "dabstar_decoder_set_frame_quality")
+
+    def frame_quality(self, recording: int) -> np.ndarray:
+        """float32[n_frames, 6] in OfdmDecoder.QUALITY order: row f is quality() as it would have been had the recording ended
+        after frame f (the last run must have had set_frame_quality on)."""
+        nf = self.n_frames(recording)
+        out = np.zeros((nf, 6), np.float32)
+        self.ctx.check(self.ctx.lib.dabstar_decoder_frame_quality(self.h, recording, _ptr(out), nf), "dabstar_decoder_frame_quality")
+        return out
 
     STAGES = ("time_sync", "prs_corr", "cp_corr", "coarse_afc", "ingest_fft", "demap", "fic_viterbi", "msc_viterbi")
 

@@ -40,6 +40,21 @@ struct OfdmStateDev
 constexpr double POW_ALL_BETA = 3.255208184782532e-06;   // (float)(0.005f / 1536.0f)
 constexpr float POW_ALL_DECAY = 0.9950124713222692f;     // (1 - beta)^1536
 
+// Per-frame signal quality (dabstar_decoder_set_frame_quality). What the capture instance of the demapper keeps of the state
+// after a frame's null symbol (one per frame of a window, by descriptor index) ...
+struct FrameQualSnap
+{
+  float stddev[K_CARR], null_pow[K_CARR], pow_acc[K_CARR];
+  float pow_carry;  // A^G y0 after the frame
+  float mean_value; // mMeanValue: sum |r| of the frame's last symbol / 1536
+  float pad[2];
+};
+// ... and what k_frame_quality reduces it to (one per frame slot); the host forms the dB figures from it (engine.cu)
+struct FrameQual
+{
+  float sum_stddev, sum_null_pow, mean_pow_all, mean_value;
+};
+
 // One serial run of the demapper: consecutive frames of one recording (a whole window, or one SEGMENT of it).
 // Segments (SURVEY 8e, "frame batches with a warm-up prefix"): the per-carrier IIRs of OfdmDecoder run across all frames
 // of a stream, so a segment that does not start where the recording's state was left starts from reset() state `warmup`
@@ -111,10 +126,14 @@ cudaError_t launch_fft_frames(cudaStream_t s, const DeviceTables & t, const Fram
 cudaError_t launch_reorder_frames(cudaStream_t s, const DeviceTables & t, const float2 * fft_nat, int n_frames, float2 * X, unsigned long long * lc);
 // ring: device scratch of demap_ring_bytes(n_work) bytes (exchange of the per-symbol sums between the CTAs of a recording).
 // The frames of one DemapWork must occupy consecutive row blocks (xslot) of X.
+// qsnap: nullptr runs the plain demapper; else the capture instance, which writes a FrameQualSnap per complete frame it writes
+// soft bits for, at qsnap[descriptor index].
 size_t demap_ring_bytes(int n_work);
 cudaError_t launch_demap(cudaStream_t s, const DeviceTables & t, const DemapWork * work, int n_work, const FrameDesc * frames,
                          const uint8_t * null_is_tii, const float2 * X, OfdmStateDev * states, int soft_bit_type, int16_t * soft,
-                         unsigned long long * ring, unsigned long long * lc);
+                         unsigned long long * ring, FrameQualSnap * qsnap, unsigned long long * lc);
+// out[frames[i].slot] = the sums of qsnap[i], for every complete frame i < n_frames
+cudaError_t launch_frame_quality(cudaStream_t s, const FrameDesc * frames, int n_frames, const FrameQualSnap * qsnap, FrameQual * out, unsigned long long * lc);
 cudaError_t launch_cp_corr(cudaStream_t s, const FrameDesc * frames, int n_frames, const RecInput * recs, int fmt, float2 * cp, unsigned long long * lc);
 cudaError_t launch_prs_corr(cudaStream_t s, const DeviceTables & t, const FrameDesc * frames, int n_frames, const RecInput * recs, int fmt,
                             float threshold_first, float threshold_rest, const uint8_t * first_flags, int strongest, int * start_index, unsigned long long * lc);

@@ -1169,11 +1169,17 @@ __device__ int g_demap_ablate;
 #define ABL(bit) false
 #endif
 
-template <int SOFT, int LAG>
+// QUAL: per-frame signal-quality capture (dabstar_decoder_set_frame_quality). After the null symbol of every complete frame
+// whose soft bits it writes, the run stores the frame's FrameQualSnap into qsnap[descriptor index]: the state the host's
+// quality figures are taken from. mMeanValue of that state is the total of the frame's last symbol, which is known only LAG
+// symbols later (emit of d = symbols at the frame's end, the drain, or tot_last). A complete frame is 75 symbols, more than
+// LAG, so at most one snapshot waits for its mMeanValue at any time.
+template <int SOFT, int LAG, bool QUAL>
 __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restrict__ work, const FrameDesc * __restrict__ frames,
                                                       const uint8_t * __restrict__ null_is_tii, const float2 * __restrict__ X,
                                                       const int16_t * __restrict__ rel_of_k, OfdmStateDev * __restrict__ states,
-                                                      int16_t * __restrict__ soft, unsigned long long * __restrict__ ring, unsigned * __restrict__ ticket)
+                                                      int16_t * __restrict__ soft, unsigned long long * __restrict__ ring, unsigned * __restrict__ ticket,
+                                                      FrameQualSnap * __restrict__ qsnap)
 {
   constexpr int STASH = LAG + 1; // stash depth (power of two)
   constexpr int T = DM5_T;
@@ -1285,6 +1291,14 @@ __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restric
   };
   float part_prev = 0.0f; // this thread's |r| sum of symbol g - 1, published (reduced over the warp) one symbol late
   const bool upper = (lane & 16) != 0;
+  int q_wait_g = -1, q_wait = 0; // QUAL: symbol count at the end of the snapshot that waits for its mMeanValue, and its index
+  auto q_mean_value = [&](int d, float total) {
+    if (QUAL && d == q_wait_g)
+    {
+      if (t_rec == 0) qsnap[q_wait].mean_value = total / (float)K_CARR;
+      q_wait_g = -1;
+    }
+  };
 
   for (int fi = 0; fi < wk.n_frames; fi++)
   {
@@ -1327,6 +1341,7 @@ __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restric
         float tot = tot_fast;
         if (d > 0 && !tags_ok && !ABL(1)) tot = dm5_total(my_ring + (size_t)((d - 1) & (DM3_RING - 1)) * DM5_WARPS, pre_used, (unsigned)d, lane);
         if (!ABL(2)) emit(d, orow_ring[(d & (STASH - 1)) * (T >> 5)], tot);
+        q_mean_value(d, tot);
       }
       g++;
       set_reference();
@@ -1340,6 +1355,16 @@ __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restric
       const float2 pa = add2(fma2(xra, xra, mul2(xia, xia)), f2(MIN_POW)), pb = add2(fma2(xrb, xrb, mul2(xib, xib)), f2(MIN_POW));
       sa.null_pow = fma2(add2(pa, neg2(sa.null_pow)), f2(0.05f), sa.null_pow);
       sb.null_pow = fma2(add2(pb, neg2(sb.null_pow)), f2(0.05f), sb.null_pow);
+    }
+    if (QUAL && out_row0 >= 0 && n_syms == 75)
+    {
+      FrameQualSnap & qs = qsnap[wk.desc_first + fi];
+      *reinterpret_cast<float4 *>(qs.stddev + k0) = make_float4(sa.stddev.x, sa.stddev.y, sb.stddev.x, sb.stddev.y);
+      *reinterpret_cast<float4 *>(qs.null_pow + k0) = make_float4(sa.null_pow.x, sa.null_pow.y, sb.null_pow.x, sb.null_pow.y);
+      *reinterpret_cast<float4 *>(qs.pow_acc + k0) = make_float4(pow_a.x, pow_a.y, pow_b.x, pow_b.y);
+      if (t_rec == 0) qs.pow_carry = pow_carry0 * powf(POW_ALL_DECAY, (float)g);
+      q_wait_g = g;
+      q_wait = wk.desc_first + fi;
     }
   }
   cp_async_wait<0>();
@@ -1366,8 +1391,9 @@ __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restric
       if (!ABL(1)) tot = dm5_total(slot, word, (unsigned)d, lane);
     }
     emit(d, orow_ring[(d & (STASH - 1)) * (T >> 5)], tot);
+    q_mean_value(d, tot);
   }
-  if (wk.state_out < 0) return; // a segment that does not end the window: its state is not the recording's
+  if (!QUAL && wk.state_out < 0) return; // a segment that does not end the window: its state is not the recording's
   // mMeanValue after the last symbol, fetched BEFORE anything is stored: with state_out == state_in the other slices of the
   // recording read mean_value when they start, which may be later than this (the launch is not cooperative); whoever can
   // see the last symbol's total has been waited for by it, i.e. all slices have started and read their input state
@@ -1378,6 +1404,11 @@ __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restric
     const unsigned long long * slot = my_ring + (size_t)((g - 1) & (DM3_RING - 1)) * DM5_WARPS;
     if (lane < DM5_WARPS) word = ld_volatile_global_b64(slot + lane);
     if (!ABL(1)) tot_last = dm5_total(slot, word, (unsigned)g, lane);
+  }
+  if (QUAL)
+  {
+    q_mean_value(g, tot_last); // (the last frame's snapshot: its total is tot_last, also when no state is stored)
+    if (wk.state_out < 0) return;
   }
   OfdmStateDev & so = states[wk.state_out];
   *reinterpret_cast<float4 *>(so.integ + k0) = make_float4(sa.integ.x, sa.integ.y, sb.integ.x, sb.integ.y);
@@ -1722,14 +1753,15 @@ cudaError_t launch_reorder_frames(cudaStream_t s, const DeviceTables & t, const 
 // exchange ring of the per-symbol sums (one word per warp of a recording and ring slot) + the ticket counter of k_demap5
 size_t demap_ring_bytes(int n_work) { return sizeof(unsigned long long) * (size_t)std::max(n_work, 1) * DM3_RING * DM5_WARPS + 256; }
 static size_t demap5_smem_bytes(int lag) { return sizeof(float4) * 2 * (size_t)(lag + 1 + DM5_PF) * DM5_T + sizeof(int) * (size_t)(lag + 1) * (DM5_T / 32); }
-template <int LAG> static const void * demap5_fn(int soft_bit_type)
+template <int LAG, bool QUAL> static const void * demap5_fn(int soft_bit_type)
 {
-  return soft_bit_type == 0 ? (const void *)k_demap5<0, LAG> : (soft_bit_type == 1 ? (const void *)k_demap5<1, LAG> : (const void *)k_demap5<2, LAG>);
+  return soft_bit_type == 0 ? (const void *)k_demap5<0, LAG, QUAL> : (soft_bit_type == 1 ? (const void *)k_demap5<1, LAG, QUAL> : (const void *)k_demap5<2, LAG, QUAL>);
 }
+template <int LAG> static const void * demap5_fn(int soft_bit_type, bool qual) { return qual ? demap5_fn<LAG, true>(soft_bit_type) : demap5_fn<LAG, false>(soft_bit_type); }
 
 cudaError_t launch_demap(cudaStream_t s, const DeviceTables & t, const DemapWork * work, int n_work, const FrameDesc * frames,
                          const uint8_t * null_is_tii, const float2 * X, OfdmStateDev * states, int soft_bit_type, int16_t * soft,
-                         unsigned long long * ring, unsigned long long * lc)
+                         unsigned long long * ring, FrameQualSnap * qsnap, unsigned long long * lc)
 {
   if (n_work <= 0) return cudaSuccess;
   if (soft_bit_type < 0 || soft_bit_type > 2) return cudaErrorInvalidValue;
@@ -1742,7 +1774,8 @@ cudaError_t launch_demap(cudaStream_t s, const DeviceTables & t, const DemapWork
   static const int lag_env = getenv("DABSTAR_DEMAP_LAG") ? atoi(getenv("DABSTAR_DEMAP_LAG")) : 0;
   const int grid_ctas = n_work * DM5_SLICES;
   const int lag = lag_env == 3 || lag_env == 7 || lag_env == 15 ? lag_env : (grid_ctas <= 2 * N_SM ? 15 : (grid_ctas <= 3 * N_SM ? 7 : 3));
-  const void * fn = lag == 3 ? demap5_fn<3>(soft_bit_type) : (lag == 15 ? demap5_fn<15>(soft_bit_type) : demap5_fn<7>(soft_bit_type));
+  const bool qual = qsnap != nullptr;
+  const void * fn = lag == 3 ? demap5_fn<3>(soft_bit_type, qual) : (lag == 15 ? demap5_fn<15>(soft_bit_type, qual) : demap5_fn<7>(soft_bit_type, qual));
   const size_t smem = demap5_smem_bytes(lag);
   const LaunchProps lp = launch_props(fn, DM5_T, smem, smem); // opt-in for the dynamic shared memory, once per device
   if (lp.err != cudaSuccess) return lp.err;
@@ -1761,8 +1794,40 @@ cudaError_t launch_demap(cudaStream_t s, const DeviceTables & t, const DemapWork
 #endif
   unsigned * ticket = reinterpret_cast<unsigned *>(reinterpret_cast<unsigned char *>(ring) + demap_ring_bytes(n_work) - 256);
   const int16_t * rel = t.rel_of_k;
-  void * args[] = { (void *)&work, (void *)&frames, (void *)&null_is_tii, (void *)&X, (void *)&rel, (void *)&states, (void *)&soft, (void *)&ring, (void *)&ticket };
+  void * args[] = { (void *)&work, (void *)&frames, (void *)&null_is_tii, (void *)&X, (void *)&rel, (void *)&states, (void *)&soft, (void *)&ring, (void *)&ticket, (void *)&qsnap };
   return cudaLaunchKernel(fn, dim3((unsigned)(n_work * DM5_SLICES)), dim3(DM5_T), args, smem, s);
+}
+
+// The sums of the host's quality_from_state (engine.cu) over one snapshot, in its order and precision: serial float sums over
+// k = 0..1535 and the double weighted sum of mMeanPowerOvrAll from k = 1535 down. The explicit roundings keep nvcc from
+// contracting to FMA, so the figures the host forms from them equal those of the end-of-run state bit for bit.
+__global__ void __launch_bounds__(128) k_frame_quality(const FrameDesc * __restrict__ frames, int n_frames, const FrameQualSnap * __restrict__ qsnap,
+                                                       FrameQual * __restrict__ out)
+{
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_frames || frames[i].n_syms != 75) return; // a cut frame has no snapshot
+  const FrameQualSnap & q = qsnap[i];
+  double acc = 0.0, w = 1.0;
+  for (int k = K_CARR - 1; k >= 0; k--)
+  {
+    acc = __dadd_rn(acc, __dmul_rn(w, (double)q.pow_acc[k]));
+    w = __dmul_rn(w, 1.0 - POW_ALL_BETA);
+  }
+  float sum_noise = 0.0f, sd = 0.0f;
+  for (int k = 0; k < K_CARR; k++)
+  {
+    sum_noise = __fadd_rn(sum_noise, q.null_pow[k]);
+    sd = __fadd_rn(sd, q.stddev[k]);
+  }
+  out[frames[i].slot] = FrameQual{ sd, sum_noise, (float)__dadd_rn((double)q.pow_carry, __dmul_rn(POW_ALL_BETA, acc)), q.mean_value };
+}
+
+cudaError_t launch_frame_quality(cudaStream_t s, const FrameDesc * frames, int n_frames, const FrameQualSnap * qsnap, FrameQual * out, unsigned long long * lc)
+{
+  if (n_frames <= 0) return cudaSuccess;
+  k_frame_quality<<<(n_frames + 127) / 128, 128, 0, s>>>(frames, n_frames, qsnap, out);
+  if (lc) (*lc)++;
+  return cudaGetLastError();
 }
 
 cudaError_t launch_cp_corr(cudaStream_t s, const FrameDesc * frames, int n_frames, const RecInput * recs, int fmt, float2 * cp, unsigned long long * lc)

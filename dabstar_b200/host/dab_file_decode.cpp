@@ -1,6 +1,6 @@
 // dab_file_decode — headless file-input harness: raw interleaved IQ file(s) -> decoded FIC / MSC bits on the GPU.
 //
-//   dab_file_decode [-f u8|i16|cf32] [-x container,bits,LSB|MSB,IQ|QI|I_Only|Q_Only] [-a] [-e]
+//   dab_file_decode [-f u8|i16|cf32] [-x container,bits,LSB|MSB,IQ|QI|I_Only|Q_Only] [-a] [-e] [-q quality.csv]
 //                   [-s subChId,startCU,sizeCU,shortForm,protLevel,bitRate]... [-o prefix] file.iq [file2.iq ...]
 //     -x  XML/UFF sample description (container int8|uint8|int16|int24|int32|float32) for layouts other than the three native ones
 //     -c  containers: every file's header is inspected (RIFF/WAVE .wav / .sdr, XML .uff, else raw u8); samples are converted and
@@ -9,6 +9,8 @@
 //     -t  with -a: TII detection on the null symbols the recording's CIF counter selects (5 per search, threshold 8 dB), and those
 //         null symbols leave the demapper's null power alone, as in the reference with its FIB decoder running
 //     -e  also write the ETI(NI) stream, <prefix><n>.eti (what DABstar's ETI generator writes)
+//     -q  signal quality of every frame as CSV: frame,sym0_pos,mer_db,snr_db,noise_power,fbb_hz (fbb_hz: the baseband frequency
+//         correction of the frame's data symbols); with several files, file n's lines go to <path>.<n>
 //
 // The reference can only play files through its GUI, paced to real time (raw_reader.cpp:153-165); this harness feeds
 // whole files to dabstar::DabProcessor (one reference DabProcessor per file, all files in lock step) and writes
@@ -39,7 +41,7 @@ int main(int argc, char ** argv)
   int fmt = DABSTAR_FMT_U8;
   bool autoCfg = false, eti = false, xml = false, containers = false, tii = false;
   dabstar_sample_format sf{};
-  std::string prefix = "dab_out_";
+  std::string prefix = "dab_out_", qualPath;
   std::vector<dabstar_subch> subch;
   std::vector<const char *> files;
   for (int i = 1; i < argc; i++)
@@ -51,6 +53,7 @@ int main(int argc, char ** argv)
     else if (a == "-t") tii = true;
     else if (a == "-c") { containers = true; fmt = DABSTAR_FMT_CF32; }
     else if (a == "-e") eti = true;
+    else if (a == "-q" && i + 1 < argc) qualPath = argv[++i];
     else if (a == "-x" && i + 1 < argc)
     {
       char cont[16] = { 0 }, order[8] = { 0 }, iq[16] = { 0 };
@@ -107,6 +110,7 @@ int main(int argc, char ** argv)
       else proc.set_audio_channel((int)r, subch);
       if (eti) proc.start_eti_generator((int)r);
     }
+    if (!qualPath.empty()) proc.set_frame_quality(true);
     if (xml && !containers) proc.run_files(ptrs, ns, sf);
     else proc.run(ptrs, ns);
     for (size_t r = 0; r < files.size(); r++)
@@ -153,6 +157,18 @@ int main(int argc, char ** argv)
       {
         const dabstar::SLcdData q = proc.lcd_data((int)r);
         printf("%s: MER %.1f dB, SNR %.1f dB\n", files[r], q.MER, q.SNR);
+      }
+      if (!qualPath.empty())
+      {
+        const std::string path = files.size() > 1 ? qualPath + "." + std::to_string(r) : qualPath;
+        FILE * qf = fopen(path.c_str(), "w");
+        if (!qf) throw std::runtime_error("cannot write " + path);
+        const std::vector<dabstar::SLcdData> lcd = proc.frame_lcd_data((int)r);
+        const std::vector<dabstar_frame_info> info = proc.frame_info((int)r);
+        fprintf(qf, "frame,sym0_pos,mer_db,snr_db,noise_power,fbb_hz\n");
+        for (size_t f = 0; f < lcd.size() && f < info.size(); f++)
+          fprintf(qf, "%zu,%lld,%.4f,%.4f,%.9g,%.3f\n", f, (long long)info[f].sym0_pos, lcd[f].MER, lcd[f].SNR, lcd[f].NoisePower, info[f].fbb_data);
+        fclose(qf);
       }
     }
   }

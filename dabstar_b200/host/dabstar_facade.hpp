@@ -315,11 +315,18 @@ public:
   ~OfdmDecoder() { dabstar_ofdm_state_destroy(mC.get(), mSt); }
   void reset() { mC.check(dabstar_ofdm_state_reset(mC.get(), mSt), "dabstar_ofdm_state_reset"); }
   void set_soft_bit_gen_type(ESoftBitType t) { mType = t; }
-  // iFft: nFrames x 77 x 2048 spectra; oBits: nFrames x 75 x 3072
-  void decode_frames(const cf32 * iFft, int nFrames, const f32 * iClockErr, const u8 * iNullIsTii, i16 * oBits)
+  // iFft: nFrames x 77 x 2048 spectra; oBits: nFrames x 75 x 3072; oQuality (optional): nFrames x SLcdData, lcd_data() after
+  // each frame's null symbol
+  void decode_frames(const cf32 * iFft, int nFrames, const f32 * iClockErr, const u8 * iNullIsTii, i16 * oBits, SLcdData * oQuality = nullptr)
   {
-    mC.check(dabstar_ofdm_decode_frames(mC.get(), mSt, reinterpret_cast<const float *>(iFft), nFrames, iClockErr, iNullIsTii, (int)mType, oBits, DABSTAR_MEM_HOST),
-             "dabstar_ofdm_decode_frames");
+    static_assert(sizeof(SLcdData) == 6 * sizeof(float), "SLcdData is the 6-float record of the C ABI");
+    if (oQuality)
+      mC.check(dabstar_ofdm_decode_frames_quality(mC.get(), mSt, reinterpret_cast<const float *>(iFft), nFrames, iClockErr, iNullIsTii, (int)mType, oBits,
+                                                  DABSTAR_MEM_HOST, reinterpret_cast<float *>(oQuality)),
+               "dabstar_ofdm_decode_frames_quality");
+    else
+      mC.check(dabstar_ofdm_decode_frames(mC.get(), mSt, reinterpret_cast<const float *>(iFft), nFrames, iClockErr, iNullIsTii, (int)mType, oBits, DABSTAR_MEM_HOST),
+               "dabstar_ofdm_decode_frames");
   }
   SLcdData lcd_data() const // what signal_show_lcd_data would carry now
   {
@@ -422,6 +429,16 @@ public:
     float q[6];
     mC.check(dabstar_decoder_quality(mDec, recording, q), "dabstar_decoder_quality");
     return SLcdData{ q[0], q[1], q[2], q[3], q[4], q[5] };
+  }
+  // Capture lcd_data() for every frame of the next runs (frame_lcd_data); off by default.
+  void set_frame_quality(bool on) { mC.check(dabstar_decoder_set_frame_quality(mDec, on ? 1 : 0), "dabstar_decoder_set_frame_quality"); }
+  // One SLcdData per frame of frame_info(): the figures as they stood after that frame's null symbol (the last run must have
+  // captured them). Replaying slot_show_lcd_data from these needs no per-symbol callback.
+  std::vector<SLcdData> frame_lcd_data(int recording) const
+  {
+    std::vector<SLcdData> v((size_t)std::max(0, n_frames(recording)));
+    mC.check(dabstar_decoder_frame_quality(mDec, recording, reinterpret_cast<float *>(v.data()), (int)v.size()), "dabstar_decoder_frame_quality");
+    return v;
   }
   std::vector<dabstar_frame_info> frame_info(int recording) const
   {

@@ -237,6 +237,11 @@ int  dabstar_ofdm_state_quality(dabstar_ctx * ctx, dabstar_ofdm_state * st, floa
 int  dabstar_ofdm_decode_frames(dabstar_ctx * ctx, dabstar_ofdm_state * st, const float * fft, int n_frames,
                                 const float * clock_err, const uint8_t * null_is_tii, int soft_bit_type,
                                 int16_t * soft, int mem);
+/* The same, and quality: n_frames x 6 host floats, row f = what dabstar_ofdm_state_quality returns after frame f's null
+ * symbol (field 5 is 0, as for a bare state). The last row equals dabstar_ofdm_state_quality after the call bit for bit. */
+int  dabstar_ofdm_decode_frames_quality(dabstar_ctx * ctx, dabstar_ofdm_state * st, const float * fft, int n_frames,
+                                        const float * clock_err, const uint8_t * null_is_tii, int soft_bit_type,
+                                        int16_t * soft, int mem, float * quality);
 
 /* PhaseReference::correlate_with_phase_ref_and_find_max_peak (ofdm/phasereference.h:53) for n windows of
  * 2048 complex samples; start_index[i] = peak index or -1. */
@@ -412,6 +417,20 @@ int     dabstar_decoder_tii_results(const dabstar_decoder * dec, int recording, 
 /* dabstar_ofdm_state_quality for a recording's decoder at the end of the last run (the reference shows these figures
  * every 5 frames; mMeanSigmaSqFreqCorr is replayed from the per-frame cyclic-prefix phases). */
 int     dabstar_decoder_quality(const dabstar_decoder * dec, int recording, float out[6]);
+/* The same figures for every frame (row D4 over time): with dabstar_decoder_set_frame_quality(dec, 1) before a run (default off;
+ * applies to all recordings; the demapper then runs its capture instance and keeps 16 bytes per frame on the device),
+ * dabstar_decoder_frame_quality writes up to cap records of 6 floats, in the layout of dabstar_decoder_quality, one per frame
+ * dabstar_decoder_frame_info lists, and returns that frame count. Record f is what dabstar_decoder_quality would return had the
+ * recording ended after frame f: the OFDM state after the frame's null symbol (which updates the noise power only for a plain,
+ * non-TII null symbol). A cut trailing frame is not listed and has no record, but its symbols are demapped, so then the
+ * end-of-run figures are not the last record; otherwise they are, bit for bit. Records follow the soft bits: a window replayed
+ * after verification keeps those of the pass that committed it, self-configuration level 2 those of the final pass, and a
+ * segment's frames carry its warm-started state. With streaming, records cover the frames of the current chunk; fields 0-4
+ * continue across chunks through the imported OFDM state, while field 5 (sqrt(mMeanSigmaSqFreqCorr)) is replayed from the
+ * cyclic-prefix phases of this run's frames only, as dabstar_decoder_quality does, so it starts again at every chunk.
+ * dabstar_decoder_frame_quality returns DABSTAR_E_INVALID when the last run did not capture. */
+int     dabstar_decoder_set_frame_quality(dabstar_decoder * dec, int enable);
+int     dabstar_decoder_frame_quality(const dabstar_decoder * dec, int recording, float * out /* cap x 6 */, int cap);
 /* out[0] good FIBs, [1] time-sync established count, [2] time-sync failures, [3] samples consumed,
  * [4] speculation windows run, [5] windows cut short by verification, [6] frames decoded,
  * [7] frames sent through the FFT/demap/FIC pass (exceeds [6] by replayed and partial frames) */
