@@ -770,7 +770,7 @@ class DabProcessor:
         return a.value, b.value
 
     def heavy_ms(self, with_fic: bool = True) -> float:
-        """Device milliseconds of the FFT + demap (+ FIC) passes of the last run(), one span per window (the chunks overlap)."""
+        """Device milliseconds of the FFT + demap (+ FIC) passes of the last run(), one span per window."""
         return float(self.ctx.lib.dabstar_decoder_heavy_ms(self.h, int(with_fic)))
 
     def soft_bits(self, recording: int, frame: int) -> np.ndarray:

@@ -1289,14 +1289,11 @@ struct dabstar_decoder
   }
   void span_begin(int stage, cudaStream_t s = nullptr) { Span sp{ stage, ev_get(), ev_get() }; cudaEventRecord(sp.a, s ? s : ctx->stream); spans.push_back(sp); }
   void span_end(cudaStream_t s = nullptr) { cudaEventRecord(spans.back().b, s ? s : ctx->stream); stage_launches[spans.back().stage]++; }
-  // FFT + demap + FIC of a window as ONE span (the chunks of a window overlap on two streams: the per-family spans then
-  // cover each other's time, this one is what the stage costs)
+  // per window: FFT + demap + FIC (heavy_spans) and FFT + demap (fft_demap_spans), each as ONE span from the FFT's start to
+  // the last kernel's end (dabstar_decoder_heavy_ms)
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> heavy_spans, fft_demap_spans;
   double heavy_ms = 0, fft_demap_ms = 0;
-  cudaStream_t heavy_stream = nullptr;
-  int state_slots = 0;  // OfdmStateDev slots in d_states: 2 per recording + scratch for the segments of a window
   HostBuf h_dip, h_start, h_cp, h_coarse; // pinned read-back of the control kernels' results (a pageable target makes the copy a blocking, staged one)
-  DevBuf d_descc;       // chunk-major copy of the window's descriptors
 };
 enum { ST_DIP = 0, ST_PRS = 1, ST_CP = 2, ST_COARSE = 3, ST_FFT = 4, ST_DEMAP = 5, ST_FIC = 6, ST_MSC = 7, ST_MSC_GATHER = 8, ST_MSC_TRELLIS = 9 };
 
@@ -1331,11 +1328,6 @@ extern "C" int dabstar_decoder_create(dabstar_ctx * ctx, const dabstar_decoder_c
   CK(cudaEventCreate(&d->ev0));
   CK(cudaEventCreate(&d->ev1));
   CK(cudaStreamCreateWithFlags(&d->copy_stream, cudaStreamNonBlocking));
-  {
-    int lo = 0, hi = 0; // the demapper's stream gets the higher priority: its CTAs are placed before the next chunk's FFT CTAs
-    cudaDeviceGetStreamPriorityRange(&lo, &hi);
-    CK(cudaStreamCreateWithPriority(&d->heavy_stream, cudaStreamNonBlocking, hi));
-  }
   *out = d.release();
   return 0;
 }
@@ -1349,7 +1341,6 @@ extern "C" void dabstar_decoder_destroy(dabstar_decoder * dec)
   for (cudaEvent_t e : dec->ev_pool) cudaEventDestroy(e);
   for (cudaEvent_t e : dec->chunk_ev) cudaEventDestroy(e);
   if (dec->copy_stream) cudaStreamDestroy(dec->copy_stream);
-  if (dec->heavy_stream) cudaStreamDestroy(dec->heavy_stream);
   delete dec;
 }
 
@@ -1737,14 +1728,8 @@ static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, cons
   CK(dec->d_ber.reserve(sizeof(int) * (size_t)dec->total_slots * 8));
   dec->frame_quality_run = dec->frame_quality;
   if (dec->frame_quality) CK(dec->d_fq.reserve(sizeof(FrameQual) * (size_t)dec->total_slots));
-  {
-    // two state buffers per recording + one scratch slot per possible segment of a window
-    long long extra = 0;
-    if (dec->seg_frames > 0) for (int r = 0; r < n_rec; r++) extra += dec->recs[r].slot_cap / dec->seg_frames + 1;
-    dec->state_slots = 2 * n_rec + (int)extra;
-  }
-  CK(dec->d_states.reserve(sizeof(OfdmStateDev) * (size_t)dec->state_slots));
-  if (int e = ofdm_state_init(ctx, dec->d_states.as<OfdmStateDev>(), true, dec->state_slots)) return e;
+  CK(dec->d_states.reserve(sizeof(OfdmStateDev) * 2 * (size_t)n_rec));
+  if (int e = ofdm_state_init(ctx, dec->d_states.as<OfdmStateDev>(), true, 2 * n_rec)) return e;
   for (int r = 0; r < n_rec; r++)
   {
     dabstar_decoder::Resume & rs = dec->resume[r];
@@ -2216,12 +2201,7 @@ static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, cons
     FrameDesc * d_fd = dec->d_desc.as<FrameDesc>();
 
     cudaEvent_t wake_ev = nullptr; // end of the round's last demapper launch
-    // ---- heavy pass: FFT (+ingest, derotation, de-interleave) -> demap -> FIC
-    // The window is cut into `nch` chunks in TIME (the same share of every recording's frames); the FFT of chunk c + 1 runs
-    // on the context's stream while the demapper and the FIC Viterbi of chunk c run on a second stream. The two kernels
-    // have complementary stall profiles and neither fills the SMs (ncu, profiles/): next to each other they share the
-    // issue slots. The FFT launches of an overlapped window keep to `fft_ctas` CTAs per SM so that the demapper's CTAs
-    // find room (k_demap5 takes its work from a ticket counter and needs no co-residency guarantee).
+    // ---- heavy pass: FFT (+ingest, derotation, de-interleave) -> demap -> FIC, one launch of each over the whole window
     CK(dec->d_X.reserve((size_t)x_frame_bytes * (size_t)n_desc));
     FrameQualSnap * d_qsnap = nullptr;
     if (dec->frame_quality)
@@ -2232,45 +2212,11 @@ static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, cons
     if (int e = sync_profiles(ctx)) return e;
     if (int e = reserve_viterbi_ws(ctx, 4 * n_desc, FIC_OUT + 6)) return e;
     {
-      // (read per run: the parity tests switch the chunking on for small windows)
-      const int chunks_env = getenv("DABSTAR_CHUNKS") ? atoi(getenv("DABSTAR_CHUNKS")) : 1;
-      const int fft_ctas_env = getenv("DABSTAR_FFT_OVERLAP_CTAS") ? atoi(getenv("DABSTAR_FFT_OVERLAP_CTAS")) : 2;
-      const int chunk_min_env = getenv("DABSTAR_CHUNK_MIN_FRAMES") ? atoi(getenv("DABSTAR_CHUNK_MIN_FRAMES")) : 1024;
-      // DABSTAR_CHUNK_MODE = 1: the FFT of the whole window first, then the demapper chunk by chunk on the same stream with the
-      // FIC decoder of chunk c on the second stream, next to the demapper of chunk c + 1 (0: FFT of chunk c + 1 next to the
-      // demapper of chunk c, as described above)
-      const bool fic_beside_demap = getenv("DABSTAR_CHUNK_MODE") && atoi(getenv("DABSTAR_CHUNK_MODE")) == 1;
-      const int nch = n_desc >= chunk_min_env ? std::max(1, std::min(chunks_env, 16)) : 1; // small windows (acquisition): one chunk
-      // chunk-major copy of the descriptors: what the FFT and the FIC decoder of a chunk walk (the demapper indexes the
-      // recording-major array, where the frames of a recording and their spectra are consecutive)
-      std::vector<int> chunk_off((size_t)nch + 1, 0);
-      const FrameDesc * d_fdc = d_fd; // one chunk: the recording-major array is the chunk
-      chunk_off[nch] = n_desc;
-      if (nch > 1)
-      {
-        std::vector<FrameDesc> fdc;
-        fdc.reserve((size_t)n_desc);
-        for (int c = 0; c < nch; c++)
-        {
-          chunk_off[c] = (int)fdc.size();
-          for (auto & pl : plans)
-          {
-            const int n = (int)pl.fr.size(), base = dec->recs[pl.rec].w_first_desc;
-            for (int j = (int)((long long)n * c / nch); j < (int)((long long)n * (c + 1) / nch); j++) fdc.push_back(ctl[base + j].desc);
-          }
-        }
-        CK(dec->d_descc.reserve(sizeof(FrameDesc) * (size_t)n_desc + 64));
-        UP(dec->d_descc.p, fdc.data(), sizeof(FrameDesc) * (size_t)n_desc);
-        d_fdc = dec->d_descc.as<FrameDesc>();
-      }
-
-      // demapper runs: (segment of a recording's window) x (chunk). Segment s > 0 starts from reset() state `seg_warmup`
-      // frames early (their spectra are in the window's buffer anyway) and discards those frames' soft bits; a run hands
-      // its state to the segment's next chunk through a scratch slot; the run that ends the window writes the recording's
-      // OTHER state buffer, and the buffers swap when the window is committed: a window that fails verification leaves the
-      // recording's state untouched.
-      std::vector<std::vector<DemapWork>> cw((size_t)nch);
-      int scratch = 2 * n_rec;
+      // demapper runs: one per segment of a recording's window. Segment s > 0 starts from reset() state `seg_warmup` frames
+      // early (their spectra are in the window's buffer anyway) and discards those frames' soft bits; the segment that ends
+      // the window writes the recording's OTHER state buffer, and the buffers swap when the window is committed: a window
+      // that fails verification leaves the recording's state untouched.
+      std::vector<DemapWork> wk;
       for (auto & pl : plans)
       {
         Recording & R = dec->recs[pl.rec];
@@ -2283,28 +2229,10 @@ static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, cons
           const int b = (int)((long long)n * sg / n_seg), e = (int)((long long)n * (sg + 1) / n_seg);
           const int w = sg == 0 ? 0 : std::min(dec->seg_warmup, b);
           const bool from_state = b - w == 0; // reaches back to the window's first frame: continue from the recording's state (exact)
-          const bool last_seg = sg == n_seg - 1;
-          int carry = last_seg ? s_out : -1; // where this segment's state travels from chunk to chunk
           if (sg > 0) R.cnt_warmup += w;
-          for (int c = 0; c < nch; c++)
-          {
-            const int lo = std::max(b - w, (int)((long long)n * c / nch)), hi = std::min(e, (int)((long long)n * (c + 1) / nch));
-            if (lo >= hi) continue;
-            const bool first = lo == b - w, last = hi == e;
-            if (!last && carry < 0)
-            {
-              if (scratch >= dec->state_slots) return ctx->fail(DABSTAR_E_NOMEM, "demapper state slots exhausted (%d)", dec->state_slots);
-              carry = scratch++;
-            }
-            cw[c].push_back({ R.w_first_desc + lo, hi - lo, first ? s_in : carry, last ? (last_seg ? s_out : -1) : carry,
-                              first ? (from_state ? (R.ofdm_reset ? 1 : 0) : 1) : 0, std::max(0, std::min(hi, b) - lo) });
-          }
+          wk.push_back({ R.w_first_desc + b - w, e - b + w, s_in, sg == n_seg - 1 ? s_out : -1, from_state ? (R.ofdm_reset ? 1 : 0) : 1, w });
         }
       }
-      std::vector<DemapWork> wk;
-      std::vector<int> wk_off((size_t)nch + 1, 0);
-      for (int c = 0; c < nch; c++) { wk_off[c] = (int)wk.size(); wk.insert(wk.end(), cw[c].begin(), cw[c].end()); }
-      wk_off[nch] = (int)wk.size();
       CK(dec->d_work.reserve(sizeof(DemapWork) * wk.size() + 64));
       DemapWork * d_wk = dec->d_work.as<DemapWork>();
       UP(d_wk, wk.data(), sizeof(DemapWork) * wk.size());
@@ -2330,74 +2258,30 @@ static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, cons
           d_tii = dec->d_tii_flags.as<uint8_t>();
         }
       }
-      size_t ring_bytes = 0;
-      std::vector<size_t> ring_off((size_t)nch);
-      for (int c = 0; c < nch; c++) { ring_off[c] = ring_bytes; ring_bytes += demap_ring_bytes(wk_off[c + 1] - wk_off[c]); }
-      CK(ctx->demap_ring.reserve(ring_bytes));
+      CK(ctx->demap_ring.reserve(demap_ring_bytes((int)wk.size())));
 
-      cudaStream_t sb = nch > 1 ? dec->heavy_stream : st; // demapper + FIC decoder of a chunk
-      cudaEvent_t h0 = dec->ev_get(), h1 = dec->ev_get(), hd = nullptr;
+      cudaEvent_t h0 = dec->ev_get(), h1 = dec->ev_get(), hd = dec->ev_get();
       CK(cudaEventRecord(h0, st));
-      if (nch > 1 && fic_beside_demap)
-      {
-        dec->span_begin(ST_FFT, st);
-        CK(launch_fft_frames(st, ctx->tab, d_fdc, n_desc, d_rin, fmt, dec->d_X.as<float2>(), 0, &ctx->launches));
-        dec->span_end(st);
-        for (int c = 0; c < nch; c++)
-        {
-          const int n_c = chunk_off[c + 1] - chunk_off[c];
-          dec->span_begin(ST_DEMAP, st);
-          CK(launch_demap(st, ctx->tab, d_wk + wk_off[c], wk_off[c + 1] - wk_off[c], d_fd, d_tii, dec->d_X.as<float2>(), dec->d_states.as<OfdmStateDev>(), dec->cfg.soft_bit_type,
-                          dec->d_soft.as<int16_t>(), reinterpret_cast<unsigned long long *>(ctx->demap_ring.as<unsigned char>() + ring_off[c]), d_qsnap, &ctx->launches));
-          dec->span_end(st);
-          cudaEvent_t ev = dec->ev_get();
-          CK(cudaEventRecord(ev, st));
-          if (c == nch - 1) hd = ev;
-          CK(cudaStreamWaitEvent(sb, ev, 0));
-          dec->span_begin(ST_FIC, sb);
-          CK(launch_viterbi(sb, nullptr, d_fdc + chunk_off[c], 4 * n_c, ctx->d_profiles.as<VitProfile>(), FIC_OUT + 6, dec->d_soft.as<int16_t>(), dec->d_fib.as<uint8_t>(),
-                            ctx->tab.prbs, dec->d_crc.as<uint8_t>(), dec->d_ber.as<int>(), ctx->d_step_tab.as<unsigned>(), ctx->vit_ws.p, ctx->vit_ws.cap, &ctx->launches));
-          dec->span_end(sb);
-        }
-      }
-      else
-      for (int c = 0; c < nch; c++)
-      {
-        const int n_c = chunk_off[c + 1] - chunk_off[c];
-        dec->span_begin(ST_FFT, st);
-        CK(launch_fft_frames(st, ctx->tab, d_fdc + chunk_off[c], n_c, d_rin, fmt, dec->d_X.as<float2>(), nch > 1 ? fft_ctas_env : 0, &ctx->launches));
-        dec->span_end(st);
-        if (nch > 1)
-        {
-          cudaEvent_t ev = dec->ev_get();
-          CK(cudaEventRecord(ev, st));
-          CK(cudaStreamWaitEvent(sb, ev, 0));
-        }
-        dec->span_begin(ST_DEMAP, sb);
-        CK(launch_demap(sb, ctx->tab, d_wk + wk_off[c], wk_off[c + 1] - wk_off[c], d_fd, d_tii, dec->d_X.as<float2>(), dec->d_states.as<OfdmStateDev>(), dec->cfg.soft_bit_type,
-                        dec->d_soft.as<int16_t>(), reinterpret_cast<unsigned long long *>(ctx->demap_ring.as<unsigned char>() + ring_off[c]), d_qsnap, &ctx->launches));
-        dec->span_end(sb);
-        if (c == nch - 1) { hd = dec->ev_get(); CK(cudaEventRecord(hd, sb)); }
-        // the 4 FIC blocks of every frame of the chunk, straight from the descriptors (no job list)
-        dec->span_begin(ST_FIC, sb);
-        CK(launch_viterbi(sb, nullptr, d_fdc + chunk_off[c], 4 * n_c, ctx->d_profiles.as<VitProfile>(), FIC_OUT + 6, dec->d_soft.as<int16_t>(), dec->d_fib.as<uint8_t>(),
-                          ctx->tab.prbs, dec->d_crc.as<uint8_t>(), dec->d_ber.as<int>(), ctx->d_step_tab.as<unsigned>(), ctx->vit_ws.p, ctx->vit_ws.cap, &ctx->launches));
-        dec->span_end(sb);
-      }
+      dec->span_begin(ST_FFT, st);
+      CK(launch_fft_frames(st, ctx->tab, d_fd, n_desc, d_rin, fmt, dec->d_X.as<float2>(), 0, &ctx->launches));
+      dec->span_end(st);
+      dec->span_begin(ST_DEMAP, st);
+      CK(launch_demap(st, ctx->tab, d_wk, (int)wk.size(), d_fd, d_tii, dec->d_X.as<float2>(), dec->d_states.as<OfdmStateDev>(), dec->cfg.soft_bit_type,
+                      dec->d_soft.as<int16_t>(), ctx->demap_ring.as<unsigned long long>(), d_qsnap, &ctx->launches));
+      dec->span_end(st);
+      CK(cudaEventRecord(hd, st));
+      // the 4 FIC blocks of every frame of the window, straight from the descriptors (no job list)
+      dec->span_begin(ST_FIC, st);
+      CK(launch_viterbi(st, nullptr, d_fd, 4 * n_desc, ctx->d_profiles.as<VitProfile>(), FIC_OUT + 6, dec->d_soft.as<int16_t>(), dec->d_fib.as<uint8_t>(),
+                        ctx->tab.prbs, dec->d_crc.as<uint8_t>(), dec->d_ber.as<int>(), ctx->d_step_tab.as<unsigned>(), ctx->vit_ws.p, ctx->vit_ws.cap, &ctx->launches));
+      dec->span_end(st);
       if (d_qsnap)
       {
         // every frame's snapshot is in: reduce them into the per-slot records (a rolled-back frame's slot is written again
         // by the window that commits it, as its soft bits are)
-        cudaStream_t qs = nch > 1 && fic_beside_demap ? st : sb;
-        dec->span_begin(ST_DEMAP, qs);
-        CK(launch_frame_quality(qs, d_fd, n_desc, d_qsnap, dec->d_fq.as<FrameQual>(), &ctx->launches));
-        dec->span_end(qs);
-      }
-      if (nch > 1)
-      {
-        cudaEvent_t ev = dec->ev_get();
-        CK(cudaEventRecord(ev, sb));
-        CK(cudaStreamWaitEvent(st, ev, 0));
+        dec->span_begin(ST_DEMAP, st);
+        CK(launch_frame_quality(st, d_fd, n_desc, d_qsnap, dec->d_fq.as<FrameQual>(), &ctx->launches));
+        dec->span_end(st);
       }
       CK(cudaEventRecord(h1, st));
       dec->heavy_spans.push_back({ h0, h1 });

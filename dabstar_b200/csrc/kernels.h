@@ -120,7 +120,8 @@ cudaError_t launch_dabplus(cudaStream_t s, const uint8_t * frames, int bit_rate,
 // ofdm_kernels.cu
 cudaError_t launch_init_ref_arg(cudaStream_t s, const DeviceTables & t, unsigned long long * lc);
 cudaError_t launch_fft_batch(cudaStream_t s, const DeviceTables & t, const float2 * in, float2 * out, int n, int sign, unsigned long long * lc);
-// max_ctas_per_sm > 0: size the persistent grid for at most that many resident CTAs per SM (leaves room for a kernel running next to it)
+// max_ctas_per_sm > 0: size the persistent grid for at most that many resident CTAs per SM (0: as many as fit); lets a caller
+// run the kernel at a launch shape other than the decoder's, e.g. one CTA per SM
 cudaError_t launch_fft_frames(cudaStream_t s, const DeviceTables & t, const FrameDesc * frames, int n_frames, const RecInput * recs, int fmt,
                               float2 * X, int max_ctas_per_sm, unsigned long long * lc);
 cudaError_t launch_reorder_frames(cudaStream_t s, const DeviceTables & t, const float2 * fft_nat, int n_frames, float2 * X, unsigned long long * lc);

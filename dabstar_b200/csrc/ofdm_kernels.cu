@@ -1159,16 +1159,6 @@ __device__ __forceinline__ float dm5_total(const unsigned long long * slot, unsi
   return v;
 }
 
-// Measurement builds only (-DDABSTAR_ABLATE, never shipped: the results are wrong): parts of the demapper switched off through
-// DABSTAR_DEMAP_ABLATE to see what each costs. 1: no waiting on the ring, 2: no soft-bit output, 4: no spectrum row loads,
-// 8: no publishing of the partial sums.
-#ifdef DABSTAR_ABLATE
-__device__ int g_demap_ablate;
-#define ABL(bit) ((abl & (bit)) != 0)
-#else
-#define ABL(bit) false
-#endif
-
 // QUAL: per-frame signal-quality capture (dabstar_decoder_set_frame_quality). After the null symbol of every complete frame
 // whose soft bits it writes, the run stores the frame's FrameQualSnap into qsnap[descriptor index]: the state the host's
 // quality figures are taken from. mMeanValue of that state is the total of the frame's last symbol, which is known only LAG
@@ -1189,9 +1179,6 @@ __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restric
   __shared__ unsigned s_ticket;
   if (threadIdx.x == 0) s_ticket = atomicAdd(ticket, 1u);
   __syncthreads();
-#ifdef DABSTAR_ABLATE
-  const int abl = g_demap_ablate;
-#endif
   float4 * stash = dm5_smem;
   float4 * rowbuf = dm5_smem + STASH * T * 2;
   int * orow_ring = reinterpret_cast<int *>(rowbuf + DM5_PF * T * 2) + (threadIdx.x >> 5);
@@ -1271,7 +1258,7 @@ __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restric
     const unsigned slot = (unsigned)((q & (DM5_PF - 1)) * T);
     cur_a = rowbuf[(slot + tid) * 2];
     cur_b = rowbuf[(slot + tid) * 2 + 1];
-    if (q + DM5_PF < total_rows && !ABL(4))
+    if (q + DM5_PF < total_rows)
     {
       cp_async16(rowbuf_addr + slot * 32u, rows + (size_t)(q + DM5_PF) * DM3_ROW4);
       cp_async16(rowbuf_addr + slot * 32u + 16u, rows + (size_t)(q + DM5_PF) * DM3_ROW4 + 1);
@@ -1320,7 +1307,7 @@ __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restric
       const float b_in = lane < DM5_WARPS ? __uint_as_float((unsigned)pre) : 0.0f;
       const bool tags_ok = __all_sync(0xffffffffu, lane >= DM5_WARPS || (unsigned)(pre >> 32) == (unsigned)d);
       const unsigned long long pre_used = pre;
-      if (d >= 0 && lane < DM5_WARPS && !ABL(1)) pre = ld_volatile_global_b64(my_ring + (size_t)(d & (DM3_RING - 1)) * DM5_WARPS + lane);
+      if (d >= 0 && lane < DM5_WARPS) pre = ld_volatile_global_b64(my_ring + (size_t)(d & (DM3_RING - 1)) * DM5_WARPS + lane);
       float v = (upper ? b_in : part_prev) + __shfl_xor_sync(0xffffffffu, upper ? part_prev : b_in, 16);
 #pragma unroll
       for (int o = 8; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -1333,14 +1320,14 @@ __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restric
       stash[((g & (STASH - 1)) * T + tid) * 2 + 1] = make_float4(b_re.x, b_re.y, b_im.x, b_im.y);
       if (lane == 0) orow_ring[(g & (STASH - 1)) * (T >> 5)] = out_row0 + (sym - 1);
       __syncwarp();
-      if (lane == 0 && g > 0 && !ABL(8))
+      if (lane == 0 && g > 0)
         st_volatile_global_b64(my_ring + (size_t)((g - 1) & (DM3_RING - 1)) * DM5_WARPS + gw,
                                ((unsigned long long)(unsigned)g << 32) | (unsigned long long)__float_as_uint(v));
       if (d >= 0)
       {
         float tot = tot_fast;
-        if (d > 0 && !tags_ok && !ABL(1)) tot = dm5_total(my_ring + (size_t)((d - 1) & (DM3_RING - 1)) * DM5_WARPS, pre_used, (unsigned)d, lane);
-        if (!ABL(2)) emit(d, orow_ring[(d & (STASH - 1)) * (T >> 5)], tot);
+        if (d > 0 && !tags_ok) tot = dm5_total(my_ring + (size_t)((d - 1) & (DM3_RING - 1)) * DM5_WARPS, pre_used, (unsigned)d, lane);
+        emit(d, orow_ring[(d & (STASH - 1)) * (T >> 5)], tot);
         q_mean_value(d, tot);
       }
       g++;
@@ -1388,7 +1375,7 @@ __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restric
       const unsigned long long * slot = my_ring + (size_t)((d - 1) & (DM3_RING - 1)) * DM5_WARPS;
       unsigned long long word = 0;
       if (lane < DM5_WARPS) word = ld_volatile_global_b64(slot + lane);
-      if (!ABL(1)) tot = dm5_total(slot, word, (unsigned)d, lane);
+      tot = dm5_total(slot, word, (unsigned)d, lane);
     }
     emit(d, orow_ring[(d & (STASH - 1)) * (T >> 5)], tot);
     q_mean_value(d, tot);
@@ -1403,7 +1390,7 @@ __global__ void __launch_bounds__(DM5_T, 4) k_demap5(const DemapWork * __restric
     unsigned long long word = 0;
     const unsigned long long * slot = my_ring + (size_t)((g - 1) & (DM3_RING - 1)) * DM5_WARPS;
     if (lane < DM5_WARPS) word = ld_volatile_global_b64(slot + lane);
-    if (!ABL(1)) tot_last = dm5_total(slot, word, (unsigned)g, lane);
+    tot_last = dm5_total(slot, word, (unsigned)g, lane);
   }
   if (QUAL)
   {
@@ -1737,7 +1724,6 @@ cudaError_t launch_fft_frames(cudaStream_t s, const DeviceTables & t, const Fram
     const LaunchProps lp = launch_props((const void *)k_fft_frames<FMT>, FFT_THREADS, stage, stage); // per device: resident CTAs per SM of this instantiation
     int per_sm = lp.err == cudaSuccess && lp.ctas_per_sm > 0 ? lp.ctas_per_sm : 4;
     if (max_ctas_per_sm > 0) per_sm = std::min(per_sm, max_ctas_per_sm);
-    if (const char * ev = getenv("DABSTAR_FFT_CTAS")) per_sm = std::max(1, std::min(per_sm, atoi(ev))); // A/B switch: resident CTAs per SM
     k_fft_frames<FMT><<<std::min(n_items, lp.n_sm * per_sm), FFT_THREADS, stage, s>>>(frames, n_items, recs, t.w2048, t.fft_slot_w, t.fft_slot_r, X);
   });
 }
@@ -1781,17 +1767,6 @@ cudaError_t launch_demap(cudaStream_t s, const DeviceTables & t, const DemapWork
   if (lp.err != cudaSuccess) return lp.err;
   cudaError_t e = cudaMemsetAsync(ring, 0, demap_ring_bytes(n_work), s); // ring tags and the ticket counter
   if (e != cudaSuccess) return e;
-#ifdef DABSTAR_ABLATE
-  {
-    // the first DABSTAR_DEMAP_ABLATE_AFTER launches run complete (their soft bits stay in the buffers: the control flow of the
-    // later, ablated runs over the same input does not change)
-    static int n_launch = 0;
-    const int after = getenv("DABSTAR_DEMAP_ABLATE_AFTER") ? atoi(getenv("DABSTAR_DEMAP_ABLATE_AFTER")) : 0;
-    const int abl = (getenv("DABSTAR_DEMAP_ABLATE") && n_launch++ >= after) ? atoi(getenv("DABSTAR_DEMAP_ABLATE")) : 0;
-    e = cudaMemcpyToSymbolAsync(g_demap_ablate, &abl, sizeof(int), 0, cudaMemcpyHostToDevice, s);
-    if (e != cudaSuccess) return e;
-  }
-#endif
   unsigned * ticket = reinterpret_cast<unsigned *>(reinterpret_cast<unsigned char *>(ring) + demap_ring_bytes(n_work) - 256);
   const int16_t * rel = t.rel_of_k;
   void * args[] = { (void *)&work, (void *)&frames, (void *)&null_is_tii, (void *)&X, (void *)&rel, (void *)&states, (void *)&soft, (void *)&ring, (void *)&ticket, (void *)&qsnap };

@@ -469,8 +469,8 @@ int     dabstar_decoder_import_state(dabstar_decoder * dec, int recording, const
 
 /* Device time of the last dabstar_decoder_run in milliseconds (CUDA events on the context's stream). */
 double  dabstar_decoder_last_ms(const dabstar_decoder * dec);
-/* Device time of the FFT + demap + FIC passes of the last run taken as ONE span per window (the chunks of a window run the
- * FFT of chunk c + 1 next to the demapper of chunk c on two streams, so the per-family times below overlap). */
+/* Device time of the FFT + demap + FIC passes of the last run taken as ONE span per window, from the start of the window's
+ * FFT to the end of its last kernel (unlike the per-family times below, it includes the gaps between the launches). */
 double  dabstar_decoder_heavy_ms(const dabstar_decoder * dec, int with_fic /* 0: first FFT launch to last demap launch of a window */);
 /* Device time and launch count per kernel family of the last run (CUDA events around every launch):
  * [0] time sync [1] PRS correlation [2] CP correlation [3] coarse AFC [4] ingest+FFT [5] demap [6] FIC Viterbi [7] MSC Viterbi */

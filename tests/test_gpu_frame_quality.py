@@ -320,19 +320,6 @@ def test_tap_rows_against_oracle_and_state_quality(ctx, oracle):
 
 # ------------------------------------------------------------------------------------------------ GPU: determinism
 @pytest.mark.gpu
-def test_chunked_fft_demap_path(ctx, monkeypatch):
-    """DABSTAR_CHUNKS=4 (FFT of chunk c + 1 beside the demapper of chunk c, the state handed between chunks): records as without."""
-    iqs = [synth.generate(12, seed=80 + i, snr_db=12.0 + 2 * i, cfo_hz=500.0 * i, fmt=synth.FMT_U8).iq for i in range(6)]
-    want = gpu(ctx, iqs)
-    monkeypatch.setenv("DABSTAR_CHUNKS", "4")
-    monkeypatch.setenv("DABSTAR_CHUNK_MIN_FRAMES", "4")
-    got = gpu(ctx, iqs)
-    for r in range(len(iqs)):
-        assert got.n_frames(r) == want.n_frames(r) >= 11
-        assert np.array_equal(got.frame_quality(r).view(np.uint32), want.frame_quality(r).view(np.uint32)), r
-
-
-@pytest.mark.gpu
 def test_cut_windows(ctx):
     """max_window 4 against 128 on recordings whose FIC fails (low SNR, a lost time sync): windows are cut by verification and
     replayed, and each frame keeps the record of the pass that committed it."""
