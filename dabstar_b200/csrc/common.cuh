@@ -71,7 +71,7 @@ __host__ __device__ inline float2 csub_j(float2 a, float2 b) { return make_float
 __host__ __device__ inline float2 cadd_j(float2 a, float2 b) { return make_float2(a.x - b.y, a.y + b.x); }
 #endif
 
-// One frame of one recording as the kernels see it. Built on the host by the control loop (engine.cu),
+// One frame of one recording as the kernels see it. Built on the host by the control loop (decoder.cu),
 // which restates DabProcessor's AFC/clock bookkeeping (main/dab_processor.cpp:191-265).
 // Oscillator convention (ofdm/sample_reader.cpp:276-281): for every sample read, phase = (phase - f) mod FS
 // first, then out = v * e^{j 2 pi phase / FS}. ph_* is the phase BEFORE the first sample of the segment.

@@ -70,7 +70,7 @@ struct BackendJobRange
   int pad;
 };
 
-// CIF read by de-interleaver row m of a job (see VitJob::skip_plus1 and engine.cu, ETI section)
+// CIF read by de-interleaver row m of a job (see VitJob::skip_plus1 and decoder.cu, ETI section)
 __host__ __device__ inline int vit_row_cif(int cif_first, int skip_plus1, int m)
 {
   int cif = cif_first + m;

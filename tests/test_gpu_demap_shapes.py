@@ -88,7 +88,7 @@ def replay(oracle, fft, clock_err, segments, soft_bit_type):
 
 
 def engine_segments(windows, seg_frames, seg_warmup):
-    """The engine's demapper runs over a recording's windows (engine.cu, heavy pass: 'demapper runs'), as replay segments.
+    """The engine's demapper runs over a recording's windows (decoder.cu, heavy pass: 'demapper runs'), as replay segments.
 
     A window of n >= 2 seg_frames frames is cut into n_seg = n // seg_frames segments; segment sg covers [b, e) with
     b = n sg / n_seg and starts w = min(warm-up, b) frames early (w = 0 for sg = 0). A segment that reaches back to the window's
