@@ -144,6 +144,16 @@ static int stage_out_end(dabstar_ctx * ctx, const void * dev, void * dst, size_t
   CK(cudaStreamSynchronize(ctx->stream));
   return 0;
 }
+// Frame descriptors and the recordings they index, uploaded back to back into scratch[3]; returns the device copies.
+static int upload_frames(dabstar_ctx * ctx, const std::vector<FrameDesc> & fd, const std::vector<RecInput> & rin, FrameDesc ** dfd, RecInput ** drin)
+{
+  CK(ctx->scratch[3].reserve(sizeof(FrameDesc) * fd.size() + sizeof(RecInput) * rin.size() + 64));
+  *dfd = ctx->scratch[3].as<FrameDesc>();
+  *drin = reinterpret_cast<RecInput *>(*dfd + fd.size());
+  UP(*dfd, fd.data(), sizeof(FrameDesc) * fd.size());
+  UP(*drin, rin.data(), sizeof(RecInput) * rin.size());
+  return 0;
+}
 
 // ------------------------------------------------------------------------------------------------ context
 extern "C" int dabstar_abi_version(void) { return DABSTAR_ABI_VERSION; }
@@ -887,7 +897,13 @@ extern "C" int dabstar_prs_correlate(dabstar_ctx * ctx, const float * samples, i
   const void * din; void * dout;
   if (int r = stage_in(ctx, ctx->scratch[0], samples, sizeof(float2) * T_U * (size_t)n, mem, &din)) return r;
   if (int r = stage_out_begin(ctx, ctx->scratch[1], start_index, sizeof(int32_t) * (size_t)n, mem, &dout)) return r;
-  CK(launch_prs_corr_raw(ctx->stream, ctx->tab, (const float2 *)din, n, threshold, strongest_peak, (int *)dout, &ctx->launches));
+  // window i = samples [2048 i, 2048 i + 2048) of recording 0; every other field is zero, so there is no oscillator
+  // (f_sym0 = ph_eval = 0) and the decoder's kernel correlates the samples as given
+  std::vector<FrameDesc> fd((size_t)n);
+  for (int i = 0; i < n; i++) fd[i].eval = (long long)i * T_U;
+  FrameDesc * dfd; RecInput * drin;
+  if (int r = upload_frames(ctx, fd, { RecInput{ din, (long long)T_U * n } }, &dfd, &drin)) return r;
+  CK(launch_prs_corr(ctx->stream, ctx->tab, dfd, n, drin, FMT_CF32, threshold, threshold, nullptr, strongest_peak, (int *)dout, &ctx->launches));
   return stage_out_end(ctx, dout, start_index, sizeof(int32_t) * (size_t)n, mem);
 }
 
@@ -922,12 +938,8 @@ extern "C" int dabstar_cp_correlate(dabstar_ctx * ctx, const float * samples, in
     fd[f].sym0 = (long long)f * per - T_U; // the kernel's symbol 1 starts T_u after sym0
     fd[f].n_syms = 75;
   }
-  const RecInput rin{ din, per * n };
-  CK(ctx->scratch[3].reserve(sizeof(FrameDesc) * fd.size() + sizeof(RecInput) + 64));
-  FrameDesc * dfd = ctx->scratch[3].as<FrameDesc>();
-  RecInput * drin = reinterpret_cast<RecInput *>(dfd + fd.size());
-  UP(dfd, fd.data(), sizeof(FrameDesc) * fd.size());
-  UP(drin, &rin, sizeof(rin));
+  FrameDesc * dfd; RecInput * drin;
+  if (int r = upload_frames(ctx, fd, { RecInput{ din, per * n } }, &dfd, &drin)) return r;
   CK(launch_cp_corr(ctx->stream, dfd, n, drin, FMT_CF32, (float2 *)dout, &ctx->launches));
   return stage_out_end(ctx, dout, out, sizeof(float2) * (size_t)n, mem);
 }
@@ -983,11 +995,8 @@ extern "C" int dabstar_fft_frames(dabstar_ctx * ctx, const void * samples, int f
   CK(cudaMemsetAsync(dX, 0xFF, x_bytes, ctx->stream));
   if (n_frames > 0)
   {
-    CK(ctx->scratch[3].reserve(sizeof(FrameDesc) * fd.size() + sizeof(RecInput) * rin.size() + 64));
-    FrameDesc * dfd = ctx->scratch[3].as<FrameDesc>();
-    RecInput * drin = reinterpret_cast<RecInput *>(dfd + fd.size());
-    UP(dfd, fd.data(), sizeof(FrameDesc) * fd.size());
-    UP(drin, rin.data(), sizeof(RecInput) * rin.size());
+    FrameDesc * dfd; RecInput * drin;
+    if (int r = upload_frames(ctx, fd, rin, &dfd, &drin)) return r;
     CK(launch_fft_frames(ctx->stream, ctx->tab, dfd, n_frames, drin, fmt, (float2 *)dX, max_ctas_per_sm, &ctx->launches));
     if (dnull)
     {

@@ -138,8 +138,6 @@ cudaError_t launch_frame_quality(cudaStream_t s, const FrameDesc * frames, int n
 cudaError_t launch_cp_corr(cudaStream_t s, const FrameDesc * frames, int n_frames, const RecInput * recs, int fmt, float2 * cp, unsigned long long * lc);
 cudaError_t launch_prs_corr(cudaStream_t s, const DeviceTables & t, const FrameDesc * frames, int n_frames, const RecInput * recs, int fmt,
                             float threshold_first, float threshold_rest, const uint8_t * first_flags, int strongest, int * start_index, unsigned long long * lc);
-cudaError_t launch_prs_corr_raw(cudaStream_t s, const DeviceTables & t, const float2 * samples, int n, float threshold, int strongest,
-                                int * start_index, unsigned long long * lc);
 cudaError_t launch_coarse_afc(cudaStream_t s, const DeviceTables & t, const FrameDesc * frames, int n_frames, const RecInput * recs, int fmt,
                               int * offset_hz, unsigned long long * lc);
 cudaError_t launch_coarse_afc_raw(cudaStream_t s, const DeviceTables & t, const float2 * fft_nat, int n, int * offset_hz, unsigned long long * lc);

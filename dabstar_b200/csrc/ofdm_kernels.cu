@@ -576,29 +576,6 @@ __global__ void __launch_bounds__(FFT_THREADS, 4) k_prs_corr(const FrameDesc * _
   }
 }
 
-__global__ void __launch_bounds__(FFT_THREADS, 4) k_prs_corr_raw(const float2 * __restrict__ samples, int n, const float2 * __restrict__ w2048,
-                                                                 const float2 * __restrict__ prs, float threshold, int strongest,
-                                                                 int * __restrict__ start_index)
-{
-  __shared__ float2 smem[FFT_SMEM_F2];
-  __shared__ float red[4];
-  __shared__ int result;
-  const int tid = threadIdx.x;
-  __shared__ float2 tw2s[FFT_TW2_F2];
-  FftTwiddles tw;
-  fft_load_twiddles(tw, w2048, tw2s, tid);
-  __syncthreads();
-  for (int it = blockIdx.x; it < n; it += gridDim.x)
-  {
-    float2 v[16];
-#pragma unroll
-    for (int n1 = 0; n1 < 16; n1++) v[n1] = samples[(size_t)it * T_U + 128 * n1 + tid];
-    prs_correlate_cta(v, tw, prs, threshold, strongest, smem, red, &result, tid);
-    if (tid == 0) start_index[it] = result;
-    __syncthreads();
-  }
-}
-
 // ------------------------------------------------------------------------------------------------ coarse AFC (S3)
 // smem holds the natural-order spectrum of symbol 0 on entry.
 __device__ void coarse_afc_cta(const FftTwiddles & tw, const float2 * __restrict__ ref_arg_conj, float2 * smem, float * magw, int * result, int tid)
@@ -1832,15 +1809,6 @@ cudaError_t launch_prs_corr(cudaStream_t s, const DeviceTables & t, const FrameD
   return dispatch_fmt(fmt, [&](auto F) {
     k_prs_corr<decltype(F)::value><<<fft_grid(n_frames), FFT_THREADS, 0, s>>>(frames, n_frames, recs, t.w2048, t.prs, threshold_first, threshold_rest, first_flags, strongest, start_index);
   });
-}
-
-cudaError_t launch_prs_corr_raw(cudaStream_t s, const DeviceTables & t, const float2 * samples, int n, float threshold, int strongest,
-                                int * start_index, unsigned long long * lc)
-{
-  if (n <= 0) return cudaSuccess;
-  k_prs_corr_raw<<<fft_grid(n), FFT_THREADS, 0, s>>>(samples, n, t.w2048, t.prs, threshold, strongest, start_index);
-  if (lc) (*lc)++;
-  return cudaGetLastError();
 }
 
 cudaError_t launch_coarse_afc(cudaStream_t s, const DeviceTables & t, const FrameDesc * frames, int n_frames, const RecInput * recs, int fmt,
