@@ -99,6 +99,9 @@ EXPORTS = [
     ("dabstar_decoder_set_segmentation", ctypes.c_int), ("dabstar_decoder_set_streaming", ctypes.c_int), ("dabstar_decoder_consumed", ctypes.c_int64),
     ("dabstar_decoder_state_size", ctypes.c_int64), ("dabstar_decoder_export_state", ctypes.c_int64), ("dabstar_decoder_import_state", ctypes.c_int),
     ("dabstar_decoder_warmup_frames", ctypes.c_int64), ("dabstar_decoder_heavy_ms", ctypes.c_double), ("dabstar_decoder_msc_kernel_ms", ctypes.c_int),
+    ("dabstar_decoder_components", ctypes.c_int), ("dabstar_decoder_set_dabplus", ctypes.c_int), ("dabstar_decoder_superframes", ctypes.c_int),
+    ("dabstar_decoder_superframe_payload", ctypes.c_int64), ("dabstar_decoder_dabplus_ms", ctypes.c_double),
+    ("dabstar_decoder_dabplus_windows", ctypes.c_int),
 ]
 
 _lib = None

@@ -591,6 +591,43 @@ class DabProcessor:
         self.ctx.check(self.ctx.lib.dabstar_decoder_ensemble(self.h, recording, ctypes.byref(e)), "dabstar_decoder_ensemble")
         return e
 
+    def components(self, recording: int) -> list[ServiceComponent]:
+        """FIG 0/2 service components of a self-configured recording as the FIB parser holds them after the last run()."""
+        n = self.ctx.check(self.ctx.lib.dabstar_decoder_components(self.h, recording, None, 0), "dabstar_decoder_components")
+        arr = (_lib.ServiceCompC * max(n, 1))()
+        self.ctx.lib.dabstar_decoder_components(self.h, recording, arr, n)
+        return [ServiceComponent(a.sid, a.comp_index, a.tmid, a.type, a.sub_ch_id, a.primary, a.ca_flag) for a in arr[:n]]
+
+    def set_dabplus(self, recording: int, sub_ch_id: int = -1, enable: bool = True):
+        """Mp4Processor behind the sub-channel's Backend: the next runs find, repair and dissect its DAB+ super-frames on the device
+        (see superframes()). sub_ch_id -1: every sub-channel the recording's own FIG 0/2 lists as DAB+ (needs set_auto_config)."""
+        self.ctx.check(self.ctx.lib.dabstar_decoder_set_dabplus(self.h, recording, int(sub_ch_id), int(enable)), "dabstar_decoder_set_dabplus")
+
+    def superframes(self, recording: int, sub_ch_id: int):
+        """(records, payload uint8[n, 110 * bit_rate / 8]) of the super-frames Mp4Processor attempted in the last run, as
+        Mp4Processor.add_frames returns them for the sub-channel's logical frames; Mp4Processor.access_units cuts the AUs."""
+        lib = self.ctx.lib
+        n = self.ctx.check(lib.dabstar_decoder_superframes(self.h, recording, int(sub_ch_id), None, 0), "dabstar_decoder_superframes")
+        rec = (_lib.SuperFrameC * max(n, 1))()
+        lib.dabstar_decoder_superframes(self.h, recording, int(sub_ch_id), rec, n)
+        bit_rate = next(s.bit_rate for s in self.sub_channels(recording) if s.sub_ch_id == sub_ch_id)
+        pay = np.zeros((n, 110 * (bit_rate // 8)), np.uint8)
+        if n:
+            lib.dabstar_decoder_superframe_payload(self.h, recording, int(sub_ch_id), _ptr(pay), ctypes.c_int64(pay.size))
+        return list(rec[:n]), pay
+
+    def dabplus_ms(self) -> tuple[float, int]:
+        """(device milliseconds, walk / decode rounds) of the last run's DAB+ pass."""
+        r = ctypes.c_int(0)
+        ms = float(self.ctx.lib.dabstar_decoder_dabplus_ms(self.h, ctypes.byref(r)))
+        return ms, r.value
+
+    def dabplus_windows(self) -> tuple[int, int]:
+        """(windows Fire-code checked, windows decoded) by the last run's DAB+ pass."""
+        out = np.zeros(2, np.int64)
+        self.ctx.check(self.ctx.lib.dabstar_decoder_dabplus_windows(self.h, _ptr(out)), "dabstar_decoder_dabplus_windows")
+        return int(out[0]), int(out[1])
+
     def start_eti_generator(self, recording: int, cif_count_hi: int = 0, cif_count_lo: int = 0):
         """DabProcessor::start_eti_generator (dab_processor.cpp:529-546): the next run also produces the ETI(NI) stream of
         this recording with every sub-channel set through set_audio_channel; see eti()."""

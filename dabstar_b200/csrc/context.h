@@ -53,6 +53,27 @@ struct HostBuf
   template <typename T> T * as() const { return static_cast<T *>(p); }
 };
 
+// The DAB+ outer code over a table of streams (run_dabplus): device work buffers, and the result in pinned host memory
+struct DabplusPass
+{
+  std::vector<dab::DabplusStream> streams; // the caller sets src (device, packed frames), bit_rate and n_frames
+  // results of the last run_dabplus: per stream the attempted super-frames' records and decoded bytes, in stream order
+  std::vector<int> n_out;
+  const dab::SuperFrameRec * rec = nullptr; // sum(n_out) records ...
+  const uint8_t * payload = nullptr;        // ... and their super-frames (stream i's at streams[i].out_pay0)
+  long long scanned = 0, decoded = 0;       // windows whose raw header was checked / that went through Reed-Solomon
+  int rounds = 0;                           // walks (a walk that lists nothing new ends the pass)
+  double ms = 0;                            // device time of the pass
+  DevBuf d_streams, d_state, d_att, d_meta, d_list, d_slot, d_ler, d_rec, d_pay, d_out;
+  HostBuf h_meta, h_out;
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  ~DabplusPass()
+  {
+    if (ev0) cudaEventDestroy(ev0);
+    if (ev1) cudaEventDestroy(ev1);
+  }
+};
+
 struct dabstar_ctx
 {
   int device = 0;
@@ -73,6 +94,7 @@ struct dabstar_ctx
   DevBuf demap_ring;    // exchange ring of the sliced demapper
   DevBuf vit_ws;        // symbols + decision words of the thread-per-code-word Viterbi
   DevBuf d_gf, d_fc_syn; // DAB+ outer code: GF(2^8) / Fire code tables (built on first use)
+  DabplusPass dabplus;   // dabstar_dabplus_decode's pass
   HostBuf arena;        // pinned staging of small uploads; reused after every stream synchronisation
   size_t arena_off = 0;
   std::unique_ptr<dab::HostPool> pool; // host threads of the per-recording control loops (created by the first decoder run)
@@ -125,6 +147,21 @@ int upload_begin(dabstar_ctx * ctx, size_t bytes, unsigned char ** stage);
 int upload_commit(dabstar_ctx * ctx, void * dst, const unsigned char * stage, size_t bytes);
 #define UP(dst, src, bytes) do { if (int r_ = upload(ctx, (dst), (src), (bytes))) return r_; } while (0)
 #define SYNC() do { if (int r_ = sync_stream(ctx)) return r_; } while (0)
+
+// The super-frames Mp4Processor attempts in every stream of p.streams, decoded on the device (dabplus_kernels.cu): scan the
+// Fire code of every window, then alternate walk and decode until a walk lists no window without an outcome (one small
+// read-back per round), then compact the attempted windows in stream order and copy them to p.h_out. Runs on `s`.
+int run_dabplus(dabstar_ctx * ctx, cudaStream_t s, DabplusPass & p);
+inline dabstar_superframe superframe_public(const dab::SuperFrameRec & r)
+{
+  dabstar_superframe o;
+  o.first_frame = r.first_frame; o.ok = r.ok; o.rs_errors = r.rs_errors; o.rs_corrections = r.rs_corrections; o.fc_corrected = r.fc_corrected;
+  o.dac_rate = r.dac_rate; o.sbr_flag = r.sbr_flag; o.aac_channel_mode = r.aac_channel_mode; o.ps_flag = r.ps_flag; o.mpeg_surround = r.mpeg_surround;
+  o.num_aus = r.num_aus;
+  for (int i = 0; i < 7; i++) o.au_start[i] = r.au_start[i];
+  for (int i = 0; i < 6; i++) o.au_state[i] = r.au_state[i];
+  return o;
+}
 
 int get_profile(dabstar_ctx * ctx, int short_form, int bit_rate, int prot_level);
 int sync_profiles(dabstar_ctx * ctx);

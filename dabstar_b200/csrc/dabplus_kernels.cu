@@ -6,12 +6,16 @@
 //
 // The reference walks the logical frames of a sub-channel one by one: a five-frame window is tested with the Fire code,
 // decoded (bit_rate / 8 interleaved code words), dissected into access units, and the outcome decides where the next
-// window starts. That dependency is broken by decoding EVERY five-frame window (n_frames - 4 of them, one thread per
-// code word) and replaying the small synchronisation state machine on the host over the per-window outcomes. The
-// Reed-Solomon decoder restates the reference's own sequence (Horner syndromes with its zero shortcut, its
-// Berlekamp-Massey variant, Chien search, Forney with the same early exits), because the corrected bytes are handed on
-// whatever the decoder returns: uncorrectable words leave with whatever corrections were applied before the decoder gave up.
+// window starts. That dependency is handled by speculation, as the decoder handles frame positions: the walk of the
+// synchronisation state machine (dabplus.cuh) runs on the device, one thread per stream, taking every window it has no
+// outcome for as a success; only the windows it attempts are decoded, and walk and decode alternate until a walk attempts
+// nothing new (engine.cu: run_dabplus). A stream keeps its five-frame stride through single failures, so the first walk is
+// final unless synchronisation runs out. The Reed-Solomon decoder restates the reference's own sequence (Horner syndromes
+// with its zero shortcut, its Berlekamp-Massey variant, Chien search, Forney with the same early exits), because the
+// corrected bytes are handed on whatever the decoder returns: uncorrectable words leave with whatever corrections were
+// applied before the decoder gave up.
 #include "kernels.h"
+#include "dabplus.cuh"
 
 #include <cstring>
 #include <vector>
@@ -26,6 +30,7 @@ struct GfTables
 {
   uint8_t exp[256], log[256]; // log[0] = 255 stands for log(0), exp[255] = 0
   uint16_t fc[256];           // Fire code CRC table, polynomial 0x782f
+  uint8_t mulr[10][256];      // mulr[r][x] = x alpha^r (syndrome Horner steps)
 };
 
 __host__ __device__ inline int gf_modnn(int x)
@@ -134,56 +139,120 @@ __device__ int rs_correct(const GfTables & t, const uint8_t (&syn)[RS_ROOTS], ui
   return root_count;
 }
 
-// thread = (window w, code word j): gather with the super-frame interleave, decode, scatter the 110 data bytes
-__global__ void __launch_bounds__(128) k_dabplus_rs(const uint8_t * __restrict__ frames, int num_bytes, int rs_dims, int n_windows, const GfTables * __restrict__ tabs,
+__device__ inline void load_tables(GfTables & t, const GfTables * __restrict__ tabs)
+{
+  for (int i = threadIdx.x; i < (int)(sizeof(GfTables) / 4); i += blockDim.x) reinterpret_cast<unsigned *>(&t)[i] = reinterpret_cast<const unsigned *>(tabs)[i];
+  __syncthreads();
+}
+
+// the stream whose range [key(s), key(s + 1)) holds i: the last s with key(s) <= i (streams with an empty range share the key of the next)
+template <typename K> __device__ inline int find_stream(const DabplusStream * __restrict__ st, int n, long long i, K key)
+{
+  int lo = 0, hi = n - 1;
+  while (lo < hi)
+  {
+    const int mid = (lo + hi + 1) >> 1;
+    if (key(st[mid]) <= i) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// thread = window of any stream: the Fire code on its raw header
+__global__ void __launch_bounds__(128) k_dabplus_scan(const DabplusStream * __restrict__ st, int n_streams, long long n_windows, const GfTables * __restrict__ tabs,
+                                                      uint8_t * __restrict__ state)
+{
+  __shared__ GfTables t;
+  load_tables(t, tabs);
+  const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= n_windows) return;
+  const DabplusStream & s = st[find_stream(st, n_streams, g, [](const DabplusStream & x) { return x.win0; })];
+  const uint8_t * raw = s.src + (size_t)(g - s.win0) * 3 * s.bit_rate;
+  state[g] = fire_crc(t, raw) == 0 ? SF_PRE_OK : 0;
+}
+
+// thread = stream: the processor's walk over what is known; attempted windows without an outcome are appended to the decode list
+__global__ void __launch_bounds__(128) k_dabplus_walk(const DabplusStream * __restrict__ st, int n_streams, const uint8_t * __restrict__ state, int * __restrict__ att,
+                                                      DabplusMeta * __restrict__ meta, int * __restrict__ att_n, DabplusEntry * __restrict__ list, int * __restrict__ slot)
+{
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_streams) return;
+  const DabplusStream & s = st[i];
+  const uint8_t * sw = state + s.win0;
+  int * a = att + s.att0;
+  const int n = superframe_walk(sw, s.n_frames, a);
+  att_n[i] = n;
+  int todo = 0;
+  for (int k = 0; k < n; k++) todo += (sw[a[k]] & SF_DECODED) ? 0 : 1;
+  if (todo == 0) return;
+  const long long sf_bytes = 110LL * (s.bit_rate / 8);
+  unsigned long long e = atomicAdd(&meta->entries, (unsigned long long)todo);
+  unsigned long long b = atomicAdd(&meta->bytes, (unsigned long long)todo * sf_bytes);
+  for (int k = 0; k < n; k++)
+  {
+    if (sw[a[k]] & SF_DECODED) continue;
+    list[e] = DabplusEntry{ b, i, a[k] };
+    slot[s.win0 + a[k]] = (int)e;
+    e++;
+    b += sf_bytes;
+  }
+}
+
+// thread = (listed window, code word j < 24): gather with the super-frame interleave, decode, scatter the 110 data bytes
+__global__ void __launch_bounds__(128) k_dabplus_rs(const DabplusStream * __restrict__ st, const DabplusEntry * __restrict__ list, int n_list, const GfTables * __restrict__ tabs,
                                                     uint8_t * __restrict__ payload, int8_t * __restrict__ ler)
 {
   __shared__ GfTables t;
-  for (int i = threadIdx.x; i < (int)(sizeof(GfTables) / 4); i += blockDim.x) reinterpret_cast<unsigned *>(&t)[i] = reinterpret_cast<const unsigned *>(tabs)[i];
-  __syncthreads();
+  load_tables(t, tabs);
   const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (id >= (long long)n_windows * rs_dims) return;
-  const int w = (int)(id / rs_dims), j = (int)(id - (long long)w * rs_dims);
-  const uint8_t * in = frames + (size_t)w * num_bytes + j;            // byte k of the code word at in[k * rs_dims]
-  uint8_t * out = payload + (size_t)w * RS_DATA * rs_dims + j;        // mOutVec[j + k * rs_dims]
-  // Horner for the ten roots alpha^0..alpha^9 in one pass; the 135 leading zeros leave every accumulator at zero
-  unsigned s[RS_ROOTS];
+  if (id >= (long long)n_list * DABPLUS_MAX_RS_DIMS) return;
+  const int e = (int)(id / DABPLUS_MAX_RS_DIMS), j = (int)(id - (long long)e * DABPLUS_MAX_RS_DIMS);
+  const DabplusEntry le = list[e];
+  const DabplusStream & s = st[le.stream];
+  const int rs_dims = s.bit_rate / 8;
+  if (j >= rs_dims) return;
+  const uint8_t * in = s.src + (size_t)le.window * 3 * s.bit_rate + j; // byte k of the code word at in[k * rs_dims]
+  uint8_t * out = payload + le.pay_off + j;                            // mOutVec[j + k * rs_dims]
+  // Horner for the ten roots alpha^0..alpha^9 in one pass; the 135 leading zeros leave every accumulator at zero.
+  // mulr[r][x] = x alpha^r (mulr[r][0] = 0) is the reference's  s == 0 ? d : d ^ exp[modnn(log[s] + r)]  in one lookup.
+  unsigned s_[RS_ROOTS];
 #pragma unroll
-  for (int r = 0; r < RS_ROOTS; r++) s[r] = 0;
+  for (int r = 0; r < RS_ROOTS; r++) s_[r] = 0;
   for (int k = 0; k < RS_LEN; k++)
   {
     const unsigned d = in[(size_t)k * rs_dims];
     if (k < RS_DATA) out[(size_t)k * rs_dims] = (uint8_t)d;
 #pragma unroll
-    for (int r = 0; r < RS_ROOTS; r++) s[r] = s[r] == 0 ? d : (d ^ t.exp[gf_modnn(t.log[s[r]] + r)]);
+    for (int r = 0; r < RS_ROOTS; r++) s_[r] = d ^ t.mulr[r][s_[r]];
   }
   uint8_t syn[RS_ROOTS];
   unsigned any = 0;
 #pragma unroll
-  for (int r = 0; r < RS_ROOTS; r++) { syn[r] = (uint8_t)s[r]; any |= s[r]; }
+  for (int r = 0; r < RS_ROOTS; r++) { syn[r] = (uint8_t)s_[r]; any |= s_[r]; }
   ler[id] = any == 0 ? (int8_t)0 : (int8_t)rs_correct(t, syn, out, rs_dims);
 }
 
-// thread = window: Fire code on the raw and on the decoded super-frame header, header fields, access-unit CRCs
-__global__ void __launch_bounds__(128) k_dabplus_check(const uint8_t * __restrict__ frames, int num_bytes, int rs_dims, int n_windows, const GfTables * __restrict__ tabs,
+// thread = listed window: Fire code on the raw and on the decoded super-frame header, header fields, access-unit CRCs
+__global__ void __launch_bounds__(128) k_dabplus_check(const DabplusStream * __restrict__ st, const DabplusEntry * __restrict__ list, int n_list, const GfTables * __restrict__ tabs,
                                                        const uint16_t * __restrict__ fc_syn, uint8_t * __restrict__ payload, const int8_t * __restrict__ ler,
-                                                       SuperFrameRec * __restrict__ rec)
+                                                       SuperFrameRec * __restrict__ rec, uint8_t * __restrict__ state)
 {
   __shared__ GfTables t;
-  for (int i = threadIdx.x; i < (int)(sizeof(GfTables) / 4); i += blockDim.x) reinterpret_cast<unsigned *>(&t)[i] = reinterpret_cast<const unsigned *>(tabs)[i];
-  __syncthreads();
-  const int w = blockIdx.x * blockDim.x + threadIdx.x;
-  if (w >= n_windows) return;
+  load_tables(t, tabs);
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= n_list) return;
+  const DabplusEntry le = list[e];
+  const DabplusStream & s = st[le.stream];
+  const int rs_dims = s.bit_rate / 8, w = le.window;
   SuperFrameRec r;
   memset(&r, 0, sizeof(r));
   r.first_frame = w;
-  const uint8_t * raw = frames + (size_t)w * num_bytes;
-  uint8_t * o = payload + (size_t)w * RS_DATA * rs_dims;
+  const uint8_t * raw = s.src + (size_t)w * 3 * s.bit_rate;
+  uint8_t * o = payload + le.pay_off;
   const int sf_bytes = RS_DATA * rs_dims;
   r.pre_ok = fire_crc(t, raw) == 0;                       // FirecodeChecker::check on the undecoded block (mp4processor.cpp:133)
   for (int j = 0; j < rs_dims; j++)
   {
-    const int l = ler[(size_t)w * rs_dims + j];
+    const int l = ler[(size_t)e * DABPLUS_MAX_RS_DIMS + j];
     if (l < 0) r.rs_errors++; else r.rs_corrections += l;
   }
   // check_and_correct_6bits on the decoded header (firecode_checker.cpp:166-184)
@@ -235,7 +304,25 @@ __global__ void __launch_bounds__(128) k_dabplus_check(const uint8_t * __restric
       r.au_state[u] = crc == (((unsigned)o[a[u] + len] << 8) | o[a[u] + len + 1]) ? 1 : 2;
     }
   }
-  rec[w] = r;
+  rec[e] = r;
+  state[s.win0 + w] |= (uint8_t)(SF_DECODED | (ok ? SF_OK : 0));
+}
+
+// block = output record: the attempted windows' records and super-frames in stream order
+__global__ void __launch_bounds__(128) k_dabplus_compact(const DabplusStream * __restrict__ st, int n_streams, const int * __restrict__ att, const int * __restrict__ slot,
+                                                         const DabplusEntry * __restrict__ list, const SuperFrameRec * __restrict__ rec, const uint8_t * __restrict__ payload,
+                                                         SuperFrameRec * __restrict__ out_rec, uint8_t * __restrict__ out_pay)
+{
+  const long long k = blockIdx.x;
+  const int si = find_stream(st, n_streams, k, [](const DabplusStream & x) { return x.out_rec0; });
+  const DabplusStream & s = st[si];
+  const int i = (int)(k - s.out_rec0);
+  const int e = slot[s.win0 + att[s.att0 + i]];
+  const int sf_bytes = RS_DATA * (s.bit_rate / 8);
+  const uint8_t * src = payload + list[e].pay_off;
+  uint8_t * dst = out_pay + s.out_pay0 + (long long)i * sf_bytes;
+  for (int b = threadIdx.x; b < sf_bytes; b += blockDim.x) dst[b] = src[b];
+  if (threadIdx.x == 0) out_rec[k] = rec[e];
 }
 } // namespace
 
@@ -263,6 +350,8 @@ void dabplus_host_tables(std::vector<uint8_t> & gf_blob, std::vector<uint16_t> &
     for (int j = 0; j < 8; j++) crc = (crc & 0x8000u) ? ((crc << 1) ^ 0x782fu) : (crc << 1);
     t.fc[i] = (uint16_t)crc;
   }
+  for (int r = 0; r < RS_ROOTS; r++)
+    for (int x = 0; x < 256; x++) t.mulr[r][x] = x == 0 ? 0 : t.exp[gf_modnn(t.log[x] + r)];
   gf_blob.resize(sizeof(t));
   memcpy(gf_blob.data(), &t, sizeof(t));
   // burst patterns of up to 6 bits, grouped by the bit shifts they are tried at
@@ -287,15 +376,41 @@ void dabplus_host_tables(std::vector<uint8_t> & gf_blob, std::vector<uint16_t> &
       }
 }
 
-cudaError_t launch_dabplus(cudaStream_t s, const uint8_t * frames, int bit_rate, int n_frames, const void * gf_tables, const uint16_t * fc_syn,
-                           uint8_t * payload, int8_t * ler, SuperFrameRec * rec, unsigned long long * lc)
+cudaError_t launch_dabplus_scan(cudaStream_t s, const DabplusStream * st, int n_streams, long long n_windows, const void * gf_tables, uint8_t * state, unsigned long long * lc)
 {
-  const int n_windows = n_frames - 4, rs_dims = bit_rate / 8, num_bytes = 3 * bit_rate;
   if (n_windows <= 0) return cudaSuccess;
-  const long long words = (long long)n_windows * rs_dims;
-  k_dabplus_rs<<<(unsigned)((words + 127) / 128), 128, 0, s>>>(frames, num_bytes, rs_dims, n_windows, static_cast<const GfTables *>(gf_tables), payload, ler);
-  k_dabplus_check<<<(n_windows + 127) / 128, 128, 0, s>>>(frames, num_bytes, rs_dims, n_windows, static_cast<const GfTables *>(gf_tables), fc_syn, payload, ler, rec);
+  k_dabplus_scan<<<(unsigned)((n_windows + 127) / 128), 128, 0, s>>>(st, n_streams, n_windows, static_cast<const GfTables *>(gf_tables), state);
+  if (lc) (*lc)++;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_dabplus_walk(cudaStream_t s, const DabplusStream * st, int n_streams, const uint8_t * state, int * att, DabplusMeta * meta, int * att_n,
+                                DabplusEntry * list, int * slot, unsigned long long * lc)
+{
+  if (n_streams <= 0) return cudaSuccess;
+  k_dabplus_walk<<<(n_streams + 127) / 128, 128, 0, s>>>(st, n_streams, state, att, meta, att_n, list, slot);
+  if (lc) (*lc)++;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_dabplus_decode(cudaStream_t s, const DabplusStream * st, const DabplusEntry * list, int n_list, const void * gf_tables, const uint16_t * fc_syn,
+                                  uint8_t * payload, int8_t * ler, SuperFrameRec * rec, uint8_t * state, unsigned long long * lc)
+{
+  if (n_list <= 0) return cudaSuccess;
+  const GfTables * t = static_cast<const GfTables *>(gf_tables);
+  const long long words = (long long)n_list * DABPLUS_MAX_RS_DIMS;
+  k_dabplus_rs<<<(unsigned)((words + 127) / 128), 128, 0, s>>>(st, list, n_list, t, payload, ler);
+  k_dabplus_check<<<(n_list + 127) / 128, 128, 0, s>>>(st, list, n_list, t, fc_syn, payload, ler, rec, state);
   if (lc) (*lc) += 2;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_dabplus_compact(cudaStream_t s, const DabplusStream * st, int n_streams, long long n_out, const int * att, const int * slot, const DabplusEntry * list,
+                                   const SuperFrameRec * rec, const uint8_t * payload, SuperFrameRec * out_rec, uint8_t * out_pay, unsigned long long * lc)
+{
+  if (n_out <= 0) return cudaSuccess;
+  k_dabplus_compact<<<(unsigned)n_out, 128, 0, s>>>(st, n_streams, att, slot, list, rec, payload, out_rec, out_pay);
+  if (lc) (*lc)++;
   return cudaGetLastError();
 }
 } // namespace dab

@@ -47,6 +47,9 @@ struct Recording
     std::vector<uint8_t> tii_flags; // ... per frame, as known from the previous pass over this recording (see dabstar_decoder_run)
     bool eti_on = false;       // EtiGenerator running from the first frame of the run (DabProcessor::start_eti_generator)
     int eti_cif_hi = 0, eti_cif_lo = 0; // IFibDecoder::get_cif_count(hi, lo) as the generator samples it at symbol 4
+    std::vector<int> dabplus_ids; // sub-channels whose logical frames go through the DAB+ outer code (dabstar_decoder_set_dabplus)
+    bool dabplus_all = false;     // ... and every sub-channel the recording's own FIG 0/2 lists as DAB+
+    bool dabplus() const { return dabplus_all || !dabplus_ids.empty(); }
   } cfg;
   // input
   const void * d_iq = nullptr;
@@ -86,6 +89,9 @@ struct Recording
   std::vector<int> sync_frames;      // n_slots at every successful time sync (mTiiDetector.reset(), dab_processor.cpp:150-152)
   std::vector<int> cif_hi_f, cif_lo_f; // auto_cfg: CIF counter as the FIB decoder holds it after each frame's FIC (-1: none yet)
   dabstar_ensemble_info ens{};
+  std::vector<dabstar_service_comp> comps; // auto_cfg: FIG 0/2 service components as the FIB parser holds them after the run
+  struct DabplusOut { int sub_ch_id, bit_rate, n; long long rec0, pay0; }; // a DAB+-decoded sub-channel: its records / bytes in dec->dabplus
+  std::vector<DabplusOut> dabplus_out;
   long long cnt_good_fibs = 0, cnt_sync_ok = 0, cnt_sync_fail = 0, cnt_windows = 0, cnt_cut = 0, cnt_heavy = 0, cnt_warmup = 0;
   // window scratch
   int w_first_desc = 0;
@@ -222,6 +228,7 @@ struct dabstar_decoder
   std::vector<Span> spans;
   std::vector<cudaEvent_t> ev_pool;
   size_t ev_used = 0;
+  DabplusPass dabplus; // the DAB+ outer code of the last run (Recording::dabplus_out)
   double stage_ms[10] = { 0 };   // [8], [9]: the MSC pass split into its gather and trellis kernels (VitSpanHook)
   long long stage_launches[10] = { 0 };
   cudaEvent_t ev_get()
@@ -328,6 +335,45 @@ extern "C" int dabstar_decoder_ensemble(const dabstar_decoder * dec, int recordi
 {
   if (!dec || !out || recording < 0 || recording >= (int)dec->recs.size()) return DABSTAR_E_INVALID;
   *out = dec->recs[recording].ens;
+  return 0;
+}
+extern "C" int dabstar_decoder_components(const dabstar_decoder * dec, int recording, dabstar_service_comp * out, int cap)
+{
+  if (!dec || recording < 0 || recording >= (int)dec->recs.size() || cap < 0 || (!out && cap > 0)) return DABSTAR_E_INVALID;
+  const Recording & R = dec->recs[recording];
+  if (!R.cfg.auto_cfg) return dec->ctx->fail(DABSTAR_E_INVALID, "components: recording %d is not self-configured", recording);
+  for (int i = 0; i < (int)R.comps.size() && i < cap; i++) out[i] = R.comps[i];
+  return (int)R.comps.size();
+}
+extern "C" int dabstar_decoder_set_dabplus(dabstar_decoder * dec, int recording, int sub_ch_id, int enable)
+{
+  if (!dec || recording < 0 || recording >= (int)dec->recs.size()) return DABSTAR_E_INVALID;
+  dabstar_ctx * ctx = dec->ctx;
+  Recording::Cfg & c = dec->recs[recording].cfg;
+  if (sub_ch_id < -1 || sub_ch_id > 63) return ctx->fail(DABSTAR_E_INVALID, "DAB+: sub-channel id %d", sub_ch_id);
+  if (enable && dec->streaming) return ctx->fail(DABSTAR_E_UNSUPPORTED, "DAB+ super-frames across stream chunks are not supported");
+  std::vector<int> & ids = c.dabplus_ids;
+  if (!enable)
+  {
+    if (sub_ch_id == -1) c.dabplus_all = false;
+    else ids.erase(std::remove(ids.begin(), ids.end(), sub_ch_id), ids.end());
+    return 0;
+  }
+  if (sub_ch_id == -1)
+  {
+    if (!c.auto_cfg) return ctx->fail(DABSTAR_E_INVALID, "DAB+: sub-channel -1 (the recording's own FIG 0/2) needs self-configuration");
+    c.dabplus_all = true;
+    return 0;
+  }
+  if (!c.auto_cfg) // with self-configuration the sub-channel is looked up in the run's FIC
+  {
+    const MscOut * m = nullptr;
+    for (const MscOut & x : c.msc) if (x.sc.sub_ch_id == sub_ch_id) m = &x;
+    if (!m) return ctx->fail(DABSTAR_E_INVALID, "DAB+: recording %d has no sub-channel %d", recording, sub_ch_id);
+    if (m->sc.bit_rate < 8 || m->sc.bit_rate > 192 || m->sc.bit_rate % 8)
+      return ctx->fail(DABSTAR_E_INVALID, "DAB+: sub-channel %d has %d kbit/s (a multiple of 8 in 8..192 is needed)", sub_ch_id, m->sc.bit_rate);
+  }
+  if (std::find(ids.begin(), ids.end(), sub_ch_id) == ids.end()) ids.push_back(sub_ch_id);
   return 0;
 }
 extern "C" int dabstar_decoder_enable_eti(dabstar_decoder * dec, int recording, int enable, int cif_count_hi, int cif_count_lo)
@@ -674,6 +720,7 @@ struct Run
       R.d_iq = rin[r].iq;
       R.n = rin[r].n;
       const dabstar_decoder::Resume & rs = dec->resume[r];
+      if ((dec->streaming || rs.on) && R.cfg.dabplus()) return ctx->fail(DABSTAR_E_UNSUPPORTED, "recording %d: DAB+ super-frames across stream chunks are not supported", r);
       if (rs.on)
       {
         if (R.cfg.eti_on || R.cfg.auto_cfg || R.cfg.tii.on) return ctx->fail(DABSTAR_E_UNSUPPORTED, "stream continuation with ETI / self-configuration / TII is not supported");
@@ -1382,6 +1429,8 @@ struct Run
         R.ens = e;
       }
       for (int f = n_f; f <= R.n_slots; f++) { R.cif_hi_f[f] = f > 0 ? R.cif_hi_f[f - 1] : -1; R.cif_lo_f[f] = f > 0 ? R.cif_lo_f[f - 1] : -1; }
+      R.comps.resize((size_t)std::max(0, dabstar_fib_parser_components(fp, nullptr, 0)));
+      dabstar_fib_parser_components(fp, R.comps.data(), (int)R.comps.size());
       dabstar_fib_parser_destroy(fp);
     }
     return sync_profiles(ctx);
@@ -1559,12 +1608,15 @@ struct Run
       CK(cudaStreamWaitEvent(dec->copy_stream, ev, 0));
       CK(cudaMemcpyAsync(dec->h_mscp.as<uint8_t>() + g.bit_base / 8, dec->d_mscpacked.as<uint8_t>() + g.bit_base / 8, (size_t)(g.bits / 8), cudaMemcpyDeviceToHost, dec->copy_stream));
     }
-    {
-      cudaEvent_t ev = dec->ev_get();
-      CK(cudaEventRecord(ev, dec->copy_stream));
-      CK(cudaStreamWaitEvent(st, ev, 0)); // the run's final synchronisation of `st` covers the copies
-    }
     tr("msc enqueued");
+    return 0;
+  }
+  // the run's final synchronisation of `st` covers the payload copies of the MSC pass
+  int join_copies()
+  {
+    cudaEvent_t ev = dec->ev_get();
+    CK(cudaEventRecord(ev, dec->copy_stream));
+    CK(cudaStreamWaitEvent(st, ev, 0));
     return 0;
   }
   // ---- ETI: every sub-channel of every CIF through EtiGenerator's own de-interleaver (eti_generator.cpp:90-204)
@@ -1691,6 +1743,47 @@ struct Run
 };
 } // namespace
 
+// ---- DAB+: Mp4Processor (mp4processor.cpp:95-334) behind every selected sub-channel's Backend, on the packed MSC payload the
+// MSC pass left on the device (run_dabplus, one stream per recording and sub-channel). Record first_frame counts the logical
+// frames of the sub-channel's output of the run, as dabstar_decoder_msc_copy lists them.
+static int dabplus_phase(dabstar_decoder * dec)
+{
+  dabstar_ctx * ctx = dec->ctx;
+  DabplusPass & p = dec->dabplus;
+  p.streams.clear();
+  std::vector<std::pair<int, const MscOut *>> owner;
+  for (int r = 0; r < (int)dec->recs.size(); r++)
+  {
+    Recording & R = dec->recs[r];
+    R.dabplus_out.clear();
+    if (!R.cfg.dabplus()) continue;
+    for (const MscOut & m : R.cfg.msc)
+    {
+      bool on = std::find(R.cfg.dabplus_ids.begin(), R.cfg.dabplus_ids.end(), m.sc.sub_ch_id) != R.cfg.dabplus_ids.end();
+      if (R.cfg.dabplus_all && R.cfg.auto_cfg)
+        for (const dabstar_service_comp & c : R.comps) on = on || (c.tmid == 0 && c.type == 63 && c.sub_ch_id == m.sc.sub_ch_id);
+      const int br = m.sc.bit_rate;
+      if (!on || br < 8 || br > 192 || br % 8) continue;
+      p.streams.push_back(DabplusStream{ dec->d_mscpacked.as<uint8_t>() + m.out_off / 8, br, (int)(m.out_len / (24 * br)), 0, 0, 0, 0 });
+      owner.push_back({ r, &m });
+    }
+  }
+  if (p.streams.empty()) return 0;
+  if (int e = run_dabplus(ctx, ctx->stream, p)) return e;
+  for (size_t i = 0; i < owner.size(); i++)
+  {
+    const MscOut & m = *owner[i].second;
+    dec->recs[owner[i].first].dabplus_out.push_back({ m.sc.sub_ch_id, m.sc.bit_rate, p.n_out[i], p.streams[i].out_rec0, p.streams[i].out_pay0 });
+  }
+  return 0;
+}
+// With self-configuration level 2 the recordings may be decoded again (dabstar_decoder_run): the DAB+ pass then runs once, after the final pass.
+static bool dabplus_after_passes(const dabstar_decoder * dec)
+{
+  for (const Recording & R : dec->recs) if (R.cfg.auto_cfg && R.cfg.tii_nulls) return true;
+  return false;
+}
+
 static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, const int64_t * n_samples, int mem)
 {
   if (!dec || !iq || !n_samples) return DABSTAR_E_INVALID;
@@ -1721,7 +1814,12 @@ static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, cons
   if (int e = run.self_configure()) return e;
   if (int e = run.tii_pass()) return e;
   if (!dec->cfg.scan_mode)
+  {
     if (int e = run.msc_pass()) return e;
+    if (!dabplus_after_passes(dec))
+      if (int e = dabplus_phase(dec)) return e; // on `st`, beside the MSC payload copies
+    if (int e = run.join_copies()) return e;
+  }
   std::vector<EtiRef> eti_refs;
   if (int e = run.eti_jobs(eti_refs)) return e;
   run.tr("rounds done");
@@ -1737,7 +1835,10 @@ static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, cons
 extern "C" int dabstar_decoder_run(dabstar_decoder * dec, const void * const * iq, const int64_t * n_samples, int mem)
 {
   if (!dec || !iq || !n_samples) return DABSTAR_E_INVALID;
-  for (auto & R : dec->recs) R.cfg.tii_flags.clear();
+  for (auto & R : dec->recs) { R.cfg.tii_flags.clear(); R.dabplus_out.clear(); }
+  dec->dabplus.ms = 0;
+  dec->dabplus.rounds = 0;
+  dec->dabplus.scanned = dec->dabplus.decoded = 0;
   int rc = decoder_run_pass(dec, iq, n_samples, mem);
   double total_ms = dec->last_ms;
   for (int pass = 1; rc == 0 && pass <= 3; pass++)
@@ -1761,6 +1862,11 @@ extern "C" int dabstar_decoder_run(dabstar_decoder * dec, const void * const * i
     for (size_t r = 0; r < dec->recs.size(); r++) dptr[r] = dec->recs[r].d_iq;
     rc = decoder_run_pass(dec, dptr.data(), n_samples, DABSTAR_MEM_DEVICE);
     total_ms += dec->last_ms;
+  }
+  if (rc == 0 && !dec->cfg.scan_mode && dabplus_after_passes(dec))
+  {
+    rc = dabplus_phase(dec);
+    total_ms += dec->dabplus.ms;
   }
   dec->last_ms = total_ms;
   return rc;
@@ -1840,6 +1946,44 @@ extern "C" int64_t dabstar_decoder_msc_copy(const dabstar_decoder * dec, int rec
   }
   for (int64_t i = 8 * whole; i < n; i++) out[i] = (uint8_t)((p[i >> 3] >> (7 - (i & 7))) & 1u);
   return n;
+}
+static const Recording::DabplusOut * find_dabplus(const dabstar_decoder * dec, int recording, int sub_ch_id)
+{
+  if (!dec || recording < 0 || recording >= (int)dec->recs.size()) return nullptr;
+  for (const auto & d : dec->recs[recording].dabplus_out) if (d.sub_ch_id == sub_ch_id) return &d;
+  return nullptr;
+}
+extern "C" int dabstar_decoder_superframes(const dabstar_decoder * dec, int recording, int sub_ch_id, dabstar_superframe * out, int cap)
+{
+  if (!dec || cap < 0 || (!out && cap > 0)) return DABSTAR_E_INVALID;
+  const Recording::DabplusOut * d = find_dabplus(dec, recording, sub_ch_id);
+  if (!d) return dec->ctx->fail(DABSTAR_E_INVALID, "superframes: recording %d sub-channel %d was not DAB+-decoded in the last run", recording, sub_ch_id);
+  for (int i = 0; i < d->n && i < cap; i++) out[i] = superframe_public(dec->dabplus.rec[d->rec0 + i]);
+  return d->n;
+}
+extern "C" int64_t dabstar_decoder_superframe_payload(const dabstar_decoder * dec, int recording, int sub_ch_id, uint8_t * out, int64_t cap)
+{
+  if (!dec || cap < 0) return DABSTAR_E_INVALID;
+  const Recording::DabplusOut * d = find_dabplus(dec, recording, sub_ch_id);
+  if (!d) return dec->ctx->fail(DABSTAR_E_INVALID, "superframe_payload: recording %d sub-channel %d was not DAB+-decoded in the last run", recording, sub_ch_id);
+  const int64_t total = (int64_t)d->n * 110 * (d->bit_rate / 8);
+  if (!out) return total;
+  const int64_t n = std::min(cap, total);
+  if (n > 0) memcpy(out, dec->dabplus.payload + d->pay0, (size_t)n);
+  return n;
+}
+extern "C" double dabstar_decoder_dabplus_ms(const dabstar_decoder * dec, int * rounds)
+{
+  if (!dec) return 0.0;
+  if (rounds) *rounds = dec->dabplus.rounds;
+  return dec->dabplus.ms;
+}
+extern "C" int dabstar_decoder_dabplus_windows(const dabstar_decoder * dec, int64_t out[2])
+{
+  if (!dec || !out) return DABSTAR_E_INVALID;
+  out[0] = dec->dabplus.scanned;
+  out[1] = dec->dabplus.decoded;
+  return 0;
 }
 extern "C" int64_t dabstar_decoder_msc_packed(const dabstar_decoder * dec, int recording, int sub_ch_id, uint8_t * out, int64_t cap)
 {

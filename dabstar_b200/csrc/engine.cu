@@ -496,14 +496,21 @@ extern "C" int64_t dabstar_resample_linear(dabstar_ctx * ctx, const float * in, 
 }
 
 // ------------------------------------------------------------------------------------------------ DAB+ outer code (next row f2)
-extern "C" int dabstar_dabplus_decode(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, dabstar_superframe * out, int cap,
-                                      uint8_t * payload, int mem)
+// Grows a device buffer of which the first `used` bytes are live, keeping them.
+static int reserve_keep(dabstar_ctx * ctx, cudaStream_t s, DevBuf & b, size_t used, size_t bytes)
 {
-  if (!ctx || (!frame_bits && n_frames > 0) || n_frames < 0 || cap < 0 || (cap > 0 && !out)) return DABSTAR_E_INVALID;
-  if (bit_rate < 8 || bit_rate > 192 || bit_rate % 8) return ctx->fail(DABSTAR_E_INVALID, "DAB+ bit rate %d", bit_rate);
-  const int n_windows = n_frames - 4;
-  if (n_windows <= 0) return 0;
-  CK(cudaSetDevice(ctx->device));
+  if (bytes <= b.cap) return 0;
+  DevBuf n;
+  CK(n.reserve(std::max(bytes, 2 * b.cap)));
+  if (used) CK(cudaMemcpyAsync(n.p, b.p, used, cudaMemcpyDeviceToDevice, s));
+  CK(cudaStreamSynchronize(s)); // the old buffer is freed below
+  std::swap(b.p, n.p);
+  std::swap(b.cap, n.cap);
+  return 0;
+}
+
+int run_dabplus(dabstar_ctx * ctx, cudaStream_t s, DabplusPass & p)
+{
   if (!ctx->d_gf.p)
   {
     std::vector<uint8_t> gf;
@@ -511,54 +518,120 @@ extern "C" int dabstar_dabplus_decode(dabstar_ctx * ctx, const uint8_t * frame_b
     dabplus_host_tables(gf, syn);
     CK(ctx->d_gf.reserve(gf.size()));
     CK(ctx->d_fc_syn.reserve(sizeof(uint16_t) * syn.size()));
-    CK(cudaMemcpyAsync(ctx->d_gf.p, gf.data(), gf.size(), cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaMemcpyAsync(ctx->d_fc_syn.p, syn.data(), sizeof(uint16_t) * syn.size(), cudaMemcpyHostToDevice, ctx->stream));
-    SYNC();
+    CK(cudaMemcpy(ctx->d_gf.p, gf.data(), gf.size(), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(ctx->d_fc_syn.p, syn.data(), sizeof(uint16_t) * syn.size(), cudaMemcpyHostToDevice));
   }
-  const int rs_dims = bit_rate / 8, sf_bytes = 110 * rs_dims;
+  if (!p.ev0) { CK(cudaEventCreate(&p.ev0)); CK(cudaEventCreate(&p.ev1)); }
+  const int ns = (int)p.streams.size();
+  long long n_win = 0, est_entries = 0, est_bytes = 0;
+  for (DabplusStream & st : p.streams)
+  {
+    const long long nw = std::max(0, st.n_frames - 4), sf = 110LL * (st.bit_rate / 8);
+    st.win0 = n_win;
+    st.att0 = n_win;
+    n_win += nw;
+    est_entries += st.n_frames / 5 + (nw > 0 ? 2 : 0); // a clean stream, plus room for a few extra attempts
+    est_bytes += (st.n_frames / 5 + (nw > 0 ? 2 : 0)) * sf;
+  }
+  p.n_out.assign((size_t)ns, 0);
+  p.scanned = n_win;
+  p.decoded = 0;
+  p.rounds = 0;
+  p.ms = 0;
+  p.rec = nullptr;
+  p.payload = nullptr;
+  if (n_win == 0) return 0;
+  CK(cudaEventRecord(p.ev0, s));
+  CK(p.d_streams.reserve(sizeof(DabplusStream) * (size_t)ns));
+  CK(p.d_state.reserve((size_t)n_win));
+  CK(p.d_slot.reserve(sizeof(int) * (size_t)n_win));
+  CK(p.d_list.reserve(sizeof(DabplusEntry) * (size_t)n_win)); // every window is listed at most once
+  CK(p.d_att.reserve(sizeof(int) * (size_t)n_win));
+  const size_t meta_bytes = sizeof(DabplusMeta) + sizeof(int) * (size_t)ns;
+  CK(p.d_meta.reserve(meta_bytes));
+  CK(p.h_meta.reserve(meta_bytes));
+  CK(p.d_rec.reserve(sizeof(SuperFrameRec) * (size_t)est_entries));
+  CK(p.d_pay.reserve((size_t)est_bytes));
+  DabplusStream * d_st = p.d_streams.as<DabplusStream>();
+  DabplusMeta * d_meta = p.d_meta.as<DabplusMeta>();
+  int * d_att_n = reinterpret_cast<int *>(d_meta + 1);
+  CK(cudaMemcpyAsync(d_st, p.streams.data(), sizeof(DabplusStream) * (size_t)ns, cudaMemcpyHostToDevice, s));
+  CK(cudaMemsetAsync(d_meta, 0, sizeof(DabplusMeta), s));
+  CK(launch_dabplus_scan(s, d_st, ns, n_win, ctx->d_gf.p, p.d_state.as<uint8_t>(), &ctx->launches));
+  DabplusMeta done{ 0, 0 };
+  const DabplusMeta * h_meta = p.h_meta.as<DabplusMeta>();
+  while (true)
+  {
+    CK(launch_dabplus_walk(s, d_st, ns, p.d_state.as<uint8_t>(), p.d_att.as<int>(), d_meta, d_att_n, p.d_list.as<DabplusEntry>(), p.d_slot.as<int>(), &ctx->launches));
+    CK(cudaMemcpyAsync(p.h_meta.p, d_meta, meta_bytes, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    p.rounds++;
+    const DabplusMeta now = *h_meta;
+    const int n_new = (int)(now.entries - done.entries);
+    if (n_new == 0) break;
+    if (int r = reserve_keep(ctx, s, p.d_rec, sizeof(SuperFrameRec) * done.entries, sizeof(SuperFrameRec) * now.entries)) return r;
+    if (int r = reserve_keep(ctx, s, p.d_pay, (size_t)done.bytes, (size_t)now.bytes)) return r;
+    CK(p.d_ler.reserve((size_t)n_new * DABPLUS_MAX_RS_DIMS));
+    CK(launch_dabplus_decode(s, d_st, p.d_list.as<DabplusEntry>() + done.entries, n_new, ctx->d_gf.p, ctx->d_fc_syn.as<uint16_t>(), p.d_pay.as<uint8_t>(),
+                             p.d_ler.as<int8_t>(), p.d_rec.as<SuperFrameRec>() + done.entries, p.d_state.as<uint8_t>(), &ctx->launches));
+    p.decoded += n_new;
+    done = now;
+  }
+  // the last walk's attempts are final: compact them in stream order
+  const int * att_n = reinterpret_cast<const int *>(h_meta + 1);
+  long long n_rec = 0, n_bytes = 0;
+  for (int i = 0; i < ns; i++)
+  {
+    DabplusStream & st = p.streams[(size_t)i];
+    p.n_out[(size_t)i] = att_n[i];
+    st.out_rec0 = n_rec;
+    st.out_pay0 = n_bytes;
+    n_rec += att_n[i];
+    n_bytes += (long long)att_n[i] * 110 * (st.bit_rate / 8);
+  }
+  const size_t rec_bytes = sizeof(SuperFrameRec) * (size_t)n_rec, out_bytes = rec_bytes + (size_t)n_bytes;
+  if (n_rec > 0)
+  {
+    CK(p.d_out.reserve(out_bytes));
+    CK(p.h_out.reserve(out_bytes));
+    CK(cudaMemcpyAsync(d_st, p.streams.data(), sizeof(DabplusStream) * (size_t)ns, cudaMemcpyHostToDevice, s));
+    CK(launch_dabplus_compact(s, d_st, ns, n_rec, p.d_att.as<int>(), p.d_slot.as<int>(), p.d_list.as<DabplusEntry>(), p.d_rec.as<SuperFrameRec>(), p.d_pay.as<uint8_t>(),
+                              p.d_out.as<SuperFrameRec>(), p.d_out.as<uint8_t>() + rec_bytes, &ctx->launches));
+    CK(cudaMemcpyAsync(p.h_out.p, p.d_out.p, out_bytes, cudaMemcpyDeviceToHost, s));
+    p.rec = p.h_out.as<SuperFrameRec>();
+    p.payload = p.h_out.as<uint8_t>() + rec_bytes;
+  }
+  CK(cudaEventRecord(p.ev1, s));
+  CK(cudaStreamSynchronize(s));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, p.ev0, p.ev1));
+  p.ms = ms;
+  return 0;
+}
+
+extern "C" int dabstar_dabplus_decode(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, dabstar_superframe * out, int cap,
+                                      uint8_t * payload, int mem)
+{
+  if (!ctx || (!frame_bits && n_frames > 0) || n_frames < 0 || cap < 0 || (cap > 0 && !out)) return DABSTAR_E_INVALID;
+  if (bit_rate < 8 || bit_rate > 192 || bit_rate % 8) return ctx->fail(DABSTAR_E_INVALID, "DAB+ bit rate %d", bit_rate);
+  if (n_frames < 5) return 0;
+  CK(cudaSetDevice(ctx->device));
   const size_t n_bits = (size_t)n_frames * 24 * bit_rate;
   const void * dbits;
   if (int r = stage_in(ctx, ctx->scratch[0], frame_bits, n_bits, mem, &dbits)) return r;
-  CK(ctx->scratch[1].reserve(n_bits / 8));                                   // packed frames
-  CK(ctx->scratch[2].reserve((size_t)n_windows * sf_bytes));                 // decoded super-frame of every window
-  CK(ctx->scratch[3].reserve((size_t)n_windows * rs_dims));                  // Reed-Solomon return codes
-  CK(ctx->scratch[4].reserve(sizeof(SuperFrameRec) * (size_t)n_windows));
+  CK(ctx->scratch[1].reserve(n_bits / 8)); // packed frames
   CK(launch_pack_bits(ctx->stream, (const uint8_t *)dbits, ctx->scratch[1].as<uint8_t>(), (long long)(n_bits / 8), &ctx->launches));
-  CK(launch_dabplus(ctx->stream, ctx->scratch[1].as<uint8_t>(), bit_rate, n_frames, ctx->d_gf.p, ctx->d_fc_syn.as<uint16_t>(), ctx->scratch[2].as<uint8_t>(),
-                    ctx->scratch[3].as<int8_t>(), ctx->scratch[4].as<SuperFrameRec>(), &ctx->launches));
-  std::vector<SuperFrameRec> rec((size_t)n_windows);
-  CK(cudaMemcpyAsync(rec.data(), ctx->scratch[4].p, sizeof(SuperFrameRec) * rec.size(), cudaMemcpyDeviceToHost, ctx->stream));
-  SYNC();
-  // Mp4Processor::add_to_frame (mp4processor.cpp:95-180): which windows the processor attempts, given every window's outcome
-  int in_buf = 0, sync = 0, n_out = 0;
-  for (int f = 0; f < n_frames; f++)
+  DabplusPass & p = ctx->dabplus;
+  p.streams.assign(1, DabplusStream{ ctx->scratch[1].as<uint8_t>(), bit_rate, n_frames, 0, 0, 0, 0 });
+  if (int r = run_dabplus(ctx, ctx->stream, p)) return r;
+  ctx->arena_off = 0;
+  const int n_out = p.n_out[0], sf_bytes = 110 * (bit_rate / 8), n_copy = std::min(n_out, cap);
+  for (int i = 0; i < n_copy; i++) out[i] = superframe_public(p.rec[i]);
+  if (payload && n_copy > 0)
   {
-    if (++in_buf < 5) continue;
-    const int w = f - 4;
-    if (sync == 0)
-    {
-      if (rec[w].pre_ok) sync = 4;
-      else { in_buf = 4; continue; }
-    }
-    in_buf = 0;
-    if (rec[w].ok) sync = 4;
-    else if (--sync == 0) in_buf = 4;
-    if (n_out < cap)
-    {
-      const SuperFrameRec & r = rec[w];
-      dabstar_superframe & o = out[n_out];
-      o.first_frame = r.first_frame; o.ok = r.ok; o.rs_errors = r.rs_errors; o.rs_corrections = r.rs_corrections; o.fc_corrected = r.fc_corrected;
-      o.dac_rate = r.dac_rate; o.sbr_flag = r.sbr_flag; o.aac_channel_mode = r.aac_channel_mode; o.ps_flag = r.ps_flag; o.mpeg_surround = r.mpeg_surround;
-      o.num_aus = r.num_aus;
-      for (int i = 0; i < 7; i++) o.au_start[i] = r.au_start[i];
-      for (int i = 0; i < 6; i++) o.au_state[i] = r.au_state[i];
-      if (payload)
-        CK(cudaMemcpyAsync(payload + (size_t)n_out * sf_bytes, ctx->scratch[2].as<uint8_t>() + (size_t)w * sf_bytes, (size_t)sf_bytes,
-                           mem == DABSTAR_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, ctx->stream));
-    }
-    n_out++;
+    if (mem == DABSTAR_MEM_HOST) memcpy(payload, p.payload, (size_t)n_copy * sf_bytes);
+    else CK(cudaMemcpy(payload, p.payload, (size_t)n_copy * sf_bytes, cudaMemcpyHostToDevice));
   }
-  SYNC();
   return n_out;
 }
 

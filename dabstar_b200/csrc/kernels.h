@@ -105,17 +105,45 @@ cudaError_t launch_linear_jobs(cudaStream_t stream, VitJob * jobs, int n, long l
 cudaError_t launch_expand_backend_jobs(cudaStream_t stream, const BackendJobRange * ranges, int n_ranges, VitJob * jobs, unsigned long long * launch_counter);
 cudaError_t launch_pack_bits(cudaStream_t stream, const uint8_t * bits, uint8_t * out, long long n_bytes, unsigned long long * launch_counter);
 
-// dabplus_kernels.cu: one record per five-frame window of a DAB+ sub-channel
+// dabplus_kernels.cu: the DAB+ outer code over a table of streams (one DAB+ sub-channel of one recording each)
 struct SuperFrameRec
 {
   int first_frame, pre_ok, ok, rs_errors, rs_corrections, fc_corrected;
   int dac_rate, sbr_flag, aac_channel_mode, ps_flag, mpeg_surround;
   int num_aus, au_start[7], au_state[6];
 };
+constexpr int DABPLUS_MAX_RS_DIMS = 24; // code words per super-frame at 192 kbit/s
+struct DabplusStream
+{
+  const uint8_t * src;     // n_frames logical frames of 3 * bit_rate packed bytes
+  int bit_rate, n_frames;
+  long long win0;          // first of its n_frames - 4 windows (none below 5 frames) in the pass's per-window arrays
+  long long att0;          // first of its n_frames - 4 slots of attempted windows (as win0)
+  long long out_rec0;      // first output record (filled once the walk has converged)
+  long long out_pay0;      // byte offset of its first output super-frame
+};
+struct DabplusEntry        // a window listed for decoding
+{
+  unsigned long long pay_off; // its decoded super-frame: 110 * bit_rate / 8 bytes at this offset
+  int stream, window;
+};
+struct DabplusMeta         // running totals of the listed windows and their super-frame bytes
+{
+  unsigned long long entries, bytes;
+};
 void dabplus_host_tables(std::vector<uint8_t> & gf_blob, std::vector<uint16_t> & fc_syn);
-// frames: n_frames x 3*bit_rate packed bytes; payload: (n_frames-4) x 110*(bit_rate/8); ler: (n_frames-4) x bit_rate/8; rec: n_frames-4
-cudaError_t launch_dabplus(cudaStream_t s, const uint8_t * frames, int bit_rate, int n_frames, const void * gf_tables, const uint16_t * fc_syn,
-                           uint8_t * payload, int8_t * ler, SuperFrameRec * rec, unsigned long long * lc);
+// state: one byte per window (dabplus.cuh: SF_*), filled with SF_PRE_OK
+cudaError_t launch_dabplus_scan(cudaStream_t s, const DabplusStream * st, int n_streams, long long n_windows, const void * gf_tables, uint8_t * state, unsigned long long * lc);
+// att_n[i]: windows stream i attempts, listed at att[att0 ..]; those not decoded yet are appended to list at meta->entries, and
+// slot[window] = their list index
+cudaError_t launch_dabplus_walk(cudaStream_t s, const DabplusStream * st, int n_streams, const uint8_t * state, int * att, DabplusMeta * meta, int * att_n,
+                                DabplusEntry * list, int * slot, unsigned long long * lc);
+// the n_list windows at list: rec[i] for list[i], payload at list[i].pay_off, SF_DECODED / SF_OK into state; ler: n_list x 24 bytes
+cudaError_t launch_dabplus_decode(cudaStream_t s, const DabplusStream * st, const DabplusEntry * list, int n_list, const void * gf_tables, const uint16_t * fc_syn,
+                                  uint8_t * payload, int8_t * ler, SuperFrameRec * rec, uint8_t * state, unsigned long long * lc);
+// the attempted windows' records and super-frames, n_out of them, in stream order from out_rec0 / out_pay0
+cudaError_t launch_dabplus_compact(cudaStream_t s, const DabplusStream * st, int n_streams, long long n_out, const int * att, const int * slot, const DabplusEntry * list,
+                                   const SuperFrameRec * rec, const uint8_t * payload, SuperFrameRec * out_rec, uint8_t * out_pay, unsigned long long * lc);
 
 // ofdm_kernels.cu
 cudaError_t launch_init_ref_arg(cudaStream_t s, const DeviceTables & t, unsigned long long * lc);

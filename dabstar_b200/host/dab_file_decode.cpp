@@ -9,6 +9,10 @@
 //     -t  with -a: TII detection on the null symbols the recording's CIF counter selects (5 per search, threshold 8 dB), and those
 //         null symbols leave the demapper's null power alone, as in the reference with its FIB decoder running
 //     -e  also write the ETI(NI) stream, <prefix><n>.eti (what DABstar's ETI generator writes)
+//     -d  all|id[,id...]: DAB+ super-frames of those sub-channels (all: what the recording's FIG 0/2 lists as DAB+, needs -a),
+//         found, repaired and cut into access units on the GPU; prints per sub-channel super-frames attempted / ok, RS corrections /
+//         failures and access units good / bad; with -o, <prefix><n>.subch<id>.aus holds every CRC-good AU after its 2-byte
+//         big-endian length
 //     -q  signal quality of every frame as CSV: frame,sym0_pos,mer_db,snr_db,noise_power,fbb_hz (fbb_hz: the baseband frequency
 //         correction of the frame's data symbols); with several files, file n's lines go to <path>.<n>
 //
@@ -41,14 +45,16 @@ int main(int argc, char ** argv)
   int fmt = DABSTAR_FMT_U8;
   bool autoCfg = false, eti = false, xml = false, containers = false, tii = false;
   dabstar_sample_format sf{};
-  std::string prefix = "dab_out_", qualPath;
+  std::string prefix = "dab_out_", qualPath, dabplus;
+  bool prefixSet = false;
   std::vector<dabstar_subch> subch;
   std::vector<const char *> files;
   for (int i = 1; i < argc; i++)
   {
     const std::string a = argv[i];
     if (a == "-f" && i + 1 < argc) { const std::string v = argv[++i]; fmt = v == "i16" ? DABSTAR_FMT_I16 : (v == "cf32" ? DABSTAR_FMT_CF32 : DABSTAR_FMT_U8); }
-    else if (a == "-o" && i + 1 < argc) prefix = argv[++i];
+    else if (a == "-o" && i + 1 < argc) { prefix = argv[++i]; prefixSet = true; }
+    else if (a == "-d" && i + 1 < argc) dabplus = argv[++i];
     else if (a == "-a") autoCfg = true;
     else if (a == "-t") tii = true;
     else if (a == "-c") { containers = true; fmt = DABSTAR_FMT_CF32; }
@@ -109,6 +115,14 @@ int main(int argc, char ** argv)
       if (autoCfg && tii) proc.set_tii_processing((int)r, true);
       else proc.set_audio_channel((int)r, subch);
       if (eti) proc.start_eti_generator((int)r);
+      if (dabplus == "all") proc.set_dabplus((int)r, -1);
+      else if (!dabplus.empty())
+        for (size_t p = 0; p <= dabplus.size();)
+        {
+          const size_t q = std::min(dabplus.find(',', p), dabplus.size());
+          proc.set_dabplus((int)r, atoi(dabplus.substr(p, q - p).c_str()));
+          p = q + 1;
+        }
     }
     if (!qualPath.empty()) proc.set_frame_quality(true);
     if (xml && !containers) proc.run_files(ptrs, ns, sf);
@@ -148,6 +162,27 @@ int main(int argc, char ** argv)
       if (fic) fclose(fic);
       for (FILE * o : outs) if (o) fclose(o);
       printf("%s: %d frames, %ld good FIBs, %.2f ms device time\n", files[r], proc.n_frames((int)r), fibs, proc.last_ms());
+      for (const auto & s : proc.sub_channels((int)r))
+      {
+        if (dabplus.empty() || !proc.dabplus_decoded((int)r, s.sub_ch_id)) continue;
+        long good = 0, bad = 0;
+        FILE * af = prefixSet ? fopen((prefix + std::to_string(r) + ".subch" + std::to_string(s.sub_ch_id) + ".aus").c_str(), "wb") : nullptr;
+        const std::vector<dabstar_superframe> sfs = proc.superframes((int)r, s.sub_ch_id, [&](const dabstar::u8 * au, int len, const dabstar_superframe &) {
+          good++;
+          if (af) { fputc((len >> 8) & 0xff, af); fputc(len & 0xff, af); fwrite(au, 1, (size_t)len, af); }
+        });
+        if (af) fclose(af);
+        long ok = 0, corr = 0, fail = 0;
+        for (const auto & x : sfs)
+        {
+          ok += x.ok ? 1 : 0;
+          corr += x.rs_corrections;
+          fail += x.rs_errors;
+          for (int u = 0; x.ok && u < x.num_aus; u++) bad += x.au_state[u] != 1 ? 1 : 0;
+        }
+        printf("%s: DAB+ sub-channel %d: %zu super-frames attempted, %ld ok, %ld RS corrections, %ld RS failures, %ld AUs good, %ld bad\n", files[r], s.sub_ch_id,
+               sfs.size(), ok, corr, fail, good, bad);
+      }
       if (autoCfg && tii)
         for (const auto & ev : proc.tii_events((int)r))
           for (const auto & id : ev.transmitterIds)

@@ -397,6 +397,38 @@ public:
     mC.check(dabstar_decoder_enable_eti(mDec, recording, 1, cifCountHi, cifCountLo), "dabstar_decoder_enable_eti");
   }
   void stop_eti_generator(int recording) { mC.check(dabstar_decoder_enable_eti(mDec, recording, 0, 0, 0), "dabstar_decoder_enable_eti"); }
+  // Mp4Processor behind the sub-channel's Backend (backend_driver.cpp:38-59) in the next runs, on the device; subChId -1: every
+  // sub-channel the recording's own FIG 0/2 lists as DAB+ (needs set_auto_config)
+  void set_dabplus(int recording, int subChId = -1, bool on = true)
+  {
+    mC.check(dabstar_decoder_set_dabplus(mDec, recording, subChId, on ? 1 : 0), "dabstar_decoder_set_dabplus");
+  }
+  bool dabplus_decoded(int recording, int subChId) const { return dabstar_decoder_superframes(mDec, recording, subChId, nullptr, 0) >= 0; }
+  // the super-frames Mp4Processor attempted in the last run; every CRC-good access unit of an accepted one goes to sink, in order
+  std::vector<dabstar_superframe> superframes(int recording, int subChId, const Mp4Processor::AuSink & sink = nullptr) const
+  {
+    const int n = mC.check(dabstar_decoder_superframes(mDec, recording, subChId, nullptr, 0), "dabstar_decoder_superframes");
+    std::vector<dabstar_superframe> rec((size_t)n);
+    if (n > 0) dabstar_decoder_superframes(mDec, recording, subChId, rec.data(), n);
+    if (sink && n > 0)
+    {
+      std::vector<u8> pay((size_t)dabstar_decoder_superframe_payload(mDec, recording, subChId, nullptr, 0));
+      dabstar_decoder_superframe_payload(mDec, recording, subChId, pay.data(), (int64_t)pay.size());
+      const size_t sf = pay.size() / (size_t)n;
+      for (int i = 0; i < n; i++)
+        if (rec[i].ok)
+          for (int u = 0; u < rec[i].num_aus; u++)
+            if (rec[i].au_state[u] == 1) sink(&pay[(size_t)i * sf + rec[i].au_start[u]], rec[i].au_start[u + 1] - rec[i].au_start[u] - 2, rec[i]);
+    }
+    return rec;
+  }
+  // FIG 0/2 service components of a self-configured recording after the last run
+  std::vector<dabstar_service_comp> components(int recording) const
+  {
+    std::vector<dabstar_service_comp> v((size_t)mC.check(dabstar_decoder_components(mDec, recording, nullptr, 0), "dabstar_decoder_components"));
+    if (!v.empty()) dabstar_decoder_components(mDec, recording, v.data(), (int)v.size());
+    return v;
+  }
   std::vector<u8> eti(int recording) const
   {
     std::vector<u8> v((size_t)std::max<int64_t>(0, dabstar_decoder_eti_size(mDec, recording)));

@@ -39,6 +39,8 @@ typedef struct
   int32_t  eid;           /* ensemble identifier for fig_mode 1 */
   int32_t  tii_main;      /* fig_mode 1: transmitter identification sent in the null symbol after every frame whose CIF counter has */
   int32_t  tii_sub;       /*   (count & 7) >= 4 (EN 300 401 clause 14.8): main id 0..69 (pattern), sub id 0..23 (comb); -1: no TII */
+  const uint8_t * const * msc_payload; /* NULL, or n_subch pointers: the logical frames sub-channel s carries, n_frames*4*24*bitRate bits
+                                          (one per byte, transmit order), or NULL for random bits (drawn as if no payload were given) */
 } dabsynth_cfg;
 
 /* ---------------------------------------------------------------------------------------------- rng */
@@ -400,11 +402,17 @@ int dabsynth_generate(const dabsynth_cfg * c, void * out_iq, uint8_t * fib_truth
     {
       uint8_t * info = (uint8_t *)malloc((size_t)nbits);
       uint8_t * mother = (uint8_t *)malloc((size_t)(4 * (nbits + 6)));
-      rng_t r = rng_make(c->seed, 0x1000 + (uint64_t)s, (uint64_t)q);
-      for (int i = 0; i < nbits; i += 64)
+      const uint8_t * given = c->msc_payload ? c->msc_payload[s] : NULL;
+      if (given)
+        for (int i = 0; i < nbits; i++) info[i] = given[(size_t)q * nbits + i] & 1u;
+      else
       {
-        uint64_t w = rng_next(&r);
-        for (int b = 0; b < 64 && i + b < nbits; b++) info[i + b] = (uint8_t)((w >> b) & 1u);
+        rng_t r = rng_make(c->seed, 0x1000 + (uint64_t)s, (uint64_t)q);
+        for (int i = 0; i < nbits; i += 64)
+        {
+          uint64_t w = rng_next(&r);
+          for (int b = 0; b < 64 && i + b < nbits; b++) info[i + b] = (uint8_t)((w >> b) & 1u);
+        }
       }
       if (msc_truth && msc_truth[s]) memcpy(msc_truth[s] + (size_t)q * nbits, info, (size_t)nbits);
       for (int i = 0; i < nbits; i++) info[i] ^= g_prbs[i];

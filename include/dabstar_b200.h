@@ -397,6 +397,26 @@ int     dabstar_decoder_set_auto_config(dabstar_decoder * dec, int recording, in
 /* sub-channels of the last run (as set, or as discovered); returns the count */
 int     dabstar_decoder_subchannels(const dabstar_decoder * dec, int recording, dabstar_subch * out, int cap);
 int     dabstar_decoder_ensemble(const dabstar_decoder * dec, int recording, dabstar_ensemble_info * out);
+/* FIG 0/2 service components of a self-configured recording as the FIB parser holds them at the end of the run (what tells a
+ * DAB+ sub-channel, TMId 0 / ASCTy 63, from an MPEG layer II one); returns the count (E_INVALID: not self-configured) */
+int     dabstar_decoder_components(const dabstar_decoder * dec, int recording, dabstar_service_comp * out, int cap);
+/* DAB+ outer code inside the run: Mp4Processor::add_to_frame behind BackendDriver (backend_driver.cpp:38-59) for the chosen
+ * sub-channels, on the device, on the run's own MSC payload (see dabstar_dabplus_decode). sub_ch_id -1: every sub-channel the
+ * recording's own FIG 0/2 lists as DAB+ (TMId 0, ASCTy 63; needs auto-config). An explicit id must name a sub-channel set with
+ * dabstar_decoder_set_subchannels whose bit rate is a multiple of 8 in 8..192 (with auto-config it is looked up in the run's
+ * own FIC). enable = 0 deselects it. scan_mode decodes no MSC and so no super-frames; streaming is not supported
+ * (DABSTAR_E_UNSUPPORTED). */
+int     dabstar_decoder_set_dabplus(dabstar_decoder * dec, int recording, int sub_ch_id, int enable);
+/* records of the super-frames the processor attempted in the last run, in stream order, exactly as dabstar_dabplus_decode
+ * returns them for dabstar_decoder_msc_copy's bits of that sub-channel; returns the count (E_INVALID: not DAB+-decoded) */
+int     dabstar_decoder_superframes(const dabstar_decoder * dec, int recording, int sub_ch_id, dabstar_superframe * out, int cap);
+/* their decoded super-frames, 110 * (bit_rate / 8) bytes each; returns bytes written (out NULL: the bytes there are) */
+int64_t dabstar_decoder_superframe_payload(const dabstar_decoder * dec, int recording, int sub_ch_id, uint8_t * out, int64_t cap);
+/* device time of the last run's DAB+ pass; *rounds (may be NULL): its walk / decode rounds */
+double  dabstar_decoder_dabplus_ms(const dabstar_decoder * dec, int * rounds);
+/* windows (five-frame candidates) of the last run's DAB+ pass: out[0] whose raw header was Fire-code checked, out[1] that went
+ * through Reed-Solomon (the processor attempts about one in five of a synchronised stream) */
+int     dabstar_decoder_dabplus_windows(const dabstar_decoder * dec, int64_t out[2]);
 /* EtiGenerator (eti_handler/eti_generator.h:56-66: start_eti_generator before run / process_block per symbol): every
  * sub-channel set with dabstar_decoder_set_subchannels is decoded for every CIF through the generator's own whole-CIF
  * de-interleaver (first frame with its 17th CIF; its start-up bookkeeping, which loses the 16th CIF, is reproduced) and
