@@ -54,6 +54,11 @@ class SuperFrameC(ctypes.Structure):
                                               "aac_channel_mode", "ps_flag", "mpeg_surround", "num_aus")] + [("au_start", ctypes.c_int32 * 7), ("au_state", ctypes.c_int32 * 6)]
 
 
+class Mp2FrameC(ctypes.Structure):
+    _fields_ = [("first_frame", ctypes.c_int32), ("n_frames", ctypes.c_int32), ("status", ctypes.c_int32), ("header", ctypes.c_uint32),
+                ("crc_stored", ctypes.c_int32), ("crc_computed", ctypes.c_int32)]
+
+
 class EnsembleInfoC(ctypes.Structure):
     _fields_ = [(n, ctypes.c_int32) for n in ("eid", "change_flags", "alarm", "cif_count_hi", "cif_count_lo", "n_subch", "n_components", "restarts")]
 
@@ -102,6 +107,8 @@ EXPORTS = [
     ("dabstar_decoder_components", ctypes.c_int), ("dabstar_decoder_set_dabplus", ctypes.c_int), ("dabstar_decoder_superframes", ctypes.c_int),
     ("dabstar_decoder_superframe_payload", ctypes.c_int64), ("dabstar_decoder_dabplus_ms", ctypes.c_double),
     ("dabstar_decoder_dabplus_windows", ctypes.c_int),
+    ("dabstar_mp2_frames", ctypes.c_int), ("dabstar_decoder_set_mp2", ctypes.c_int), ("dabstar_decoder_mp2_frames", ctypes.c_int),
+    ("dabstar_decoder_mp2_payload", ctypes.c_int64), ("dabstar_decoder_mp2_ms", ctypes.c_double),
 ]
 
 _lib = None

@@ -85,6 +85,44 @@ class Mp4Processor:
         return [payload_row[rec.au_start[u]:rec.au_start[u + 1] - 2].tobytes() for u in range(rec.num_aus) if rec.au_state[u] == 1]
 
 
+MP2_OK, MP2_NO_HEADER, MP2_MISMATCH, MP2_CRC_ERROR, MP2_CUT = 0, 1, 2, 3, 4
+
+
+class Mp2Processor:
+    """MPEG layer II audio frames of a run of logical frames of one DAB (MP2) sub-channel: header and CRC of every audio-frame slot
+    checked on the GPU (include/dabstar_b200.h, dabstar_mp2_frames). PCM decoding stays a CPU consumer of the frames."""
+
+    def __init__(self, bit_rate: int, ctx: "Context | None" = None):
+        self.ctx = ctx or default_context()
+        self.bit_rate = int(bit_rate)
+
+    def add_frames(self, frame_bits: np.ndarray):
+        """frame_bits: uint8[n_frames, 24*bit_rate] (one bit per byte). Returns (records, payload uint8[bytes]): one record per slot,
+        and the OK frames' bytes concatenated in record order."""
+        b = _np(frame_bits, np.uint8).reshape(-1, 24 * self.bit_rate)
+        n = b.shape[0]
+        cap = max(n, 1)
+        rec = (_lib.Mp2FrameC * cap)()
+        pay = np.zeros(cap * 3 * self.bit_rate, np.uint8)
+        m = self.ctx.check(self.ctx.lib.dabstar_mp2_frames(self.ctx.h, _ptr(b), self.bit_rate, n, rec, cap, _ptr(pay), MEM_HOST), "dabstar_mp2_frames")
+        recs = list(rec[:m])
+        return recs, pay[:Mp2Processor.payload_size(recs, self.bit_rate)]
+
+    @staticmethod
+    def payload_size(records, bit_rate: int) -> int:
+        return sum(3 * bit_rate * r.n_frames for r in records if r.status == MP2_OK)
+
+    @staticmethod
+    def frames(records, payload: np.ndarray, bit_rate: int):
+        """Yields (record, frame bytes) for the OK records: the payload cut into its audio frames."""
+        o = 0
+        for r in records:
+            if r.status == MP2_OK:
+                n = 3 * bit_rate * r.n_frames
+                yield r, payload[o:o + n].tobytes()
+                o += n
+
+
 @dataclass
 class ServiceComponent:
     sid: int
@@ -627,6 +665,29 @@ class DabProcessor:
         out = np.zeros(2, np.int64)
         self.ctx.check(self.ctx.lib.dabstar_decoder_dabplus_windows(self.h, _ptr(out)), "dabstar_decoder_dabplus_windows")
         return int(out[0]), int(out[1])
+
+    def set_mp2(self, recording: int, sub_ch_id: int = -1, enable: bool = True):
+        """MPEG layer II audio frames of the sub-channel: the next runs check the header and CRC of every audio-frame slot on the
+        device (see mp2_frames()). sub_ch_id -1: every sub-channel the recording's own FIG 0/2 lists as MPEG layer II (TMId 0,
+        ASCTy 0; needs set_auto_config)."""
+        self.ctx.check(self.ctx.lib.dabstar_decoder_set_mp2(self.h, recording, int(sub_ch_id), int(enable)), "dabstar_decoder_set_mp2")
+
+    def mp2_frames(self, recording: int, sub_ch_id: int):
+        """(records, payload uint8[bytes]) of the last run's audio-frame slots, as Mp2Processor.add_frames returns them for the
+        sub-channel's logical frames; Mp2Processor.frames cuts the payload into the OK frames."""
+        lib = self.ctx.lib
+        n = self.ctx.check(lib.dabstar_decoder_mp2_frames(self.h, recording, int(sub_ch_id), None, 0), "dabstar_decoder_mp2_frames")
+        rec = (_lib.Mp2FrameC * max(n, 1))()
+        lib.dabstar_decoder_mp2_frames(self.h, recording, int(sub_ch_id), rec, n)
+        size = int(self.ctx.check(lib.dabstar_decoder_mp2_payload(self.h, recording, int(sub_ch_id), None, ctypes.c_int64(0)), "dabstar_decoder_mp2_payload"))
+        pay = np.zeros(size, np.uint8)
+        if size:
+            lib.dabstar_decoder_mp2_payload(self.h, recording, int(sub_ch_id), _ptr(pay), ctypes.c_int64(size))
+        return list(rec[:n]), pay
+
+    def mp2_ms(self) -> float:
+        """Device milliseconds of the last run's MP2 pass."""
+        return float(self.ctx.lib.dabstar_decoder_mp2_ms(self.h))
 
     def start_eti_generator(self, recording: int, cif_count_hi: int = 0, cif_count_lo: int = 0):
         """DabProcessor::start_eti_generator (dab_processor.cpp:529-546): the next run also produces the ETI(NI) stream of

@@ -74,6 +74,26 @@ struct DabplusPass
   }
 };
 
+// MPEG layer II audio frames over a table of streams (run_mp2): device work buffers, and the result in pinned host memory
+struct Mp2Pass
+{
+  std::vector<dab::Mp2Stream> streams; // the caller sets src (device, packed frames), bit_rate and n_frames
+  // results of the last run_mp2: per stream its records and the bytes of its OK frames, in stream order
+  std::vector<dab::Mp2Count> n_out;
+  const dab::Mp2Rec * rec = nullptr; // sum(n_out.recs) records (stream i's from streams[i].out_rec0) ...
+  const uint8_t * payload = nullptr; // ... and the OK frames' bytes (stream i's at streams[i].out_pay0)
+  long long slots = 0;               // logical frames classified
+  double ms = 0;                     // device time of the pass
+  DevBuf d_streams, d_cls, d_crc, d_hdr, d_stage, d_stage_off, d_cnt, d_out;
+  HostBuf h_cnt, h_out;
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  ~Mp2Pass()
+  {
+    if (ev0) cudaEventDestroy(ev0);
+    if (ev1) cudaEventDestroy(ev1);
+  }
+};
+
 struct dabstar_ctx
 {
   int device = 0;
@@ -95,6 +115,7 @@ struct dabstar_ctx
   DevBuf vit_ws;        // symbols + decision words of the thread-per-code-word Viterbi
   DevBuf d_gf, d_fc_syn; // DAB+ outer code: GF(2^8) / Fire code tables (built on first use)
   DabplusPass dabplus;   // dabstar_dabplus_decode's pass
+  Mp2Pass mp2;           // dabstar_mp2_frames's pass
   HostBuf arena;        // pinned staging of small uploads; reused after every stream synchronisation
   size_t arena_off = 0;
   std::unique_ptr<dab::HostPool> pool; // host threads of the per-recording control loops (created by the first decoder run)
@@ -160,6 +181,17 @@ inline dabstar_superframe superframe_public(const dab::SuperFrameRec & r)
   o.num_aus = r.num_aus;
   for (int i = 0; i < 7; i++) o.au_start[i] = r.au_start[i];
   for (int i = 0; i < 6; i++) o.au_state[i] = r.au_state[i];
+  return o;
+}
+
+// The audio-frame slots of every stream of p.streams, on the device (mp2_kernels.cu): classify every logical frame, walk each
+// stream (one read-back of the per-stream counts), then compact the records and OK frames in stream order and copy them to
+// p.h_out. Runs on `s`.
+int run_mp2(dabstar_ctx * ctx, cudaStream_t s, Mp2Pass & p);
+inline dabstar_mp2_frame mp2_public(const dab::Mp2Rec & r)
+{
+  dabstar_mp2_frame o;
+  o.first_frame = r.first_frame; o.n_frames = r.n_frames; o.status = r.status; o.header = r.header; o.crc_stored = r.crc_stored; o.crc_computed = r.crc_computed;
   return o;
 }
 

@@ -16,6 +16,7 @@
 // applied before the decoder gave up.
 #include "kernels.h"
 #include "dabplus.cuh"
+#include "stream_search.cuh"
 
 #include <cstring>
 #include <vector>
@@ -143,18 +144,6 @@ __device__ inline void load_tables(GfTables & t, const GfTables * __restrict__ t
 {
   for (int i = threadIdx.x; i < (int)(sizeof(GfTables) / 4); i += blockDim.x) reinterpret_cast<unsigned *>(&t)[i] = reinterpret_cast<const unsigned *>(tabs)[i];
   __syncthreads();
-}
-
-// the stream whose range [key(s), key(s + 1)) holds i: the last s with key(s) <= i (streams with an empty range share the key of the next)
-template <typename K> __device__ inline int find_stream(const DabplusStream * __restrict__ st, int n, long long i, K key)
-{
-  int lo = 0, hi = n - 1;
-  while (lo < hi)
-  {
-    const int mid = (lo + hi + 1) >> 1;
-    if (key(st[mid]) <= i) lo = mid; else hi = mid - 1;
-  }
-  return lo;
 }
 
 // thread = window of any stream: the Fire code on its raw header

@@ -50,6 +50,9 @@ struct Recording
     std::vector<int> dabplus_ids; // sub-channels whose logical frames go through the DAB+ outer code (dabstar_decoder_set_dabplus)
     bool dabplus_all = false;     // ... and every sub-channel the recording's own FIG 0/2 lists as DAB+
     bool dabplus() const { return dabplus_all || !dabplus_ids.empty(); }
+    std::vector<int> mp2_ids; // sub-channels whose logical frames go through the MPEG layer II frame check (dabstar_decoder_set_mp2)
+    bool mp2_all = false;     // ... and every sub-channel the recording's own FIG 0/2 lists as MPEG layer II
+    bool mp2() const { return mp2_all || !mp2_ids.empty(); }
   } cfg;
   // input
   const void * d_iq = nullptr;
@@ -90,8 +93,9 @@ struct Recording
   std::vector<int> cif_hi_f, cif_lo_f; // auto_cfg: CIF counter as the FIB decoder holds it after each frame's FIC (-1: none yet)
   dabstar_ensemble_info ens{};
   std::vector<dabstar_service_comp> comps; // auto_cfg: FIG 0/2 service components as the FIB parser holds them after the run
-  struct DabplusOut { int sub_ch_id, bit_rate, n; long long rec0, pay0; }; // a DAB+-decoded sub-channel: its records / bytes in dec->dabplus
-  std::vector<DabplusOut> dabplus_out;
+  // an audio-decoded sub-channel: its n records from rec0 and pay_bytes bytes from pay0 in the pass's result (dec->dabplus / dec->mp2)
+  struct AudioOut { int sub_ch_id, bit_rate, n; long long rec0, pay0, pay_bytes; };
+  std::vector<AudioOut> dabplus_out, mp2_out;
   long long cnt_good_fibs = 0, cnt_sync_ok = 0, cnt_sync_fail = 0, cnt_windows = 0, cnt_cut = 0, cnt_heavy = 0, cnt_warmup = 0;
   // window scratch
   int w_first_desc = 0;
@@ -229,6 +233,7 @@ struct dabstar_decoder
   std::vector<cudaEvent_t> ev_pool;
   size_t ev_used = 0;
   DabplusPass dabplus; // the DAB+ outer code of the last run (Recording::dabplus_out)
+  Mp2Pass mp2;         // the MPEG layer II frames of the last run (Recording::mp2_out)
   double stage_ms[10] = { 0 };   // [8], [9]: the MSC pass split into its gather and trellis kernels (VitSpanHook)
   long long stage_launches[10] = { 0 };
   cudaEvent_t ev_get()
@@ -345,36 +350,51 @@ extern "C" int dabstar_decoder_components(const dabstar_decoder * dec, int recor
   for (int i = 0; i < (int)R.comps.size() && i < cap; i++) out[i] = R.comps[i];
   return (int)R.comps.size();
 }
-extern "C" int dabstar_decoder_set_dabplus(dabstar_decoder * dec, int recording, int sub_ch_id, int enable)
+// The two audio passes after the MSC pass: DAB+ super-frames (ASCTy 63) and MPEG layer II frames (ASCTy 0)
+enum AudioKind { AUDIO_DABPLUS, AUDIO_MP2 };
+static bool dabplus_rate_ok(int bit_rate) { return bit_rate >= 8 && bit_rate <= 192 && bit_rate % 8 == 0; }
+static bool audio_rate_ok(AudioKind k, int bit_rate) { return k == AUDIO_MP2 ? mp2_rate_ok(bit_rate) : dabplus_rate_ok(bit_rate); }
+static int set_audio(dabstar_decoder * dec, int recording, int sub_ch_id, int enable, AudioKind kind)
 {
   if (!dec || recording < 0 || recording >= (int)dec->recs.size()) return DABSTAR_E_INVALID;
   dabstar_ctx * ctx = dec->ctx;
   Recording::Cfg & c = dec->recs[recording].cfg;
-  if (sub_ch_id < -1 || sub_ch_id > 63) return ctx->fail(DABSTAR_E_INVALID, "DAB+: sub-channel id %d", sub_ch_id);
-  if (enable && dec->streaming) return ctx->fail(DABSTAR_E_UNSUPPORTED, "DAB+ super-frames across stream chunks are not supported");
-  std::vector<int> & ids = c.dabplus_ids;
+  const char * what = kind == AUDIO_MP2 ? "MP2" : "DAB+";
+  if (sub_ch_id < -1 || sub_ch_id > 63) return ctx->fail(DABSTAR_E_INVALID, "%s: sub-channel id %d", what, sub_ch_id);
+  if (enable && dec->streaming)
+    return ctx->fail(DABSTAR_E_UNSUPPORTED, "%s across stream chunks are not supported", kind == AUDIO_MP2 ? "MPEG audio frames" : "DAB+ super-frames");
+  std::vector<int> & ids = kind == AUDIO_MP2 ? c.mp2_ids : c.dabplus_ids;
+  bool & all = kind == AUDIO_MP2 ? c.mp2_all : c.dabplus_all;
   if (!enable)
   {
-    if (sub_ch_id == -1) c.dabplus_all = false;
+    if (sub_ch_id == -1) all = false;
     else ids.erase(std::remove(ids.begin(), ids.end(), sub_ch_id), ids.end());
     return 0;
   }
   if (sub_ch_id == -1)
   {
-    if (!c.auto_cfg) return ctx->fail(DABSTAR_E_INVALID, "DAB+: sub-channel -1 (the recording's own FIG 0/2) needs self-configuration");
-    c.dabplus_all = true;
+    if (!c.auto_cfg) return ctx->fail(DABSTAR_E_INVALID, "%s: sub-channel -1 (the recording's own FIG 0/2) needs self-configuration", what);
+    all = true;
     return 0;
   }
   if (!c.auto_cfg) // with self-configuration the sub-channel is looked up in the run's FIC
   {
     const MscOut * m = nullptr;
     for (const MscOut & x : c.msc) if (x.sc.sub_ch_id == sub_ch_id) m = &x;
-    if (!m) return ctx->fail(DABSTAR_E_INVALID, "DAB+: recording %d has no sub-channel %d", recording, sub_ch_id);
-    if (m->sc.bit_rate < 8 || m->sc.bit_rate > 192 || m->sc.bit_rate % 8)
-      return ctx->fail(DABSTAR_E_INVALID, "DAB+: sub-channel %d has %d kbit/s (a multiple of 8 in 8..192 is needed)", sub_ch_id, m->sc.bit_rate);
+    if (!m) return ctx->fail(DABSTAR_E_INVALID, "%s: recording %d has no sub-channel %d", what, recording, sub_ch_id);
+    if (!audio_rate_ok(kind, m->sc.bit_rate)) return ctx->fail(DABSTAR_E_INVALID, "%s: sub-channel %d has %d kbit/s, which %s", what, sub_ch_id, m->sc.bit_rate,
+                                                               kind == AUDIO_MP2 ? "no layer II frame has" : "is not a multiple of 8 in 8..192");
   }
   if (std::find(ids.begin(), ids.end(), sub_ch_id) == ids.end()) ids.push_back(sub_ch_id);
   return 0;
+}
+extern "C" int dabstar_decoder_set_dabplus(dabstar_decoder * dec, int recording, int sub_ch_id, int enable)
+{
+  return set_audio(dec, recording, sub_ch_id, enable, AUDIO_DABPLUS);
+}
+extern "C" int dabstar_decoder_set_mp2(dabstar_decoder * dec, int recording, int sub_ch_id, int enable)
+{
+  return set_audio(dec, recording, sub_ch_id, enable, AUDIO_MP2);
 }
 extern "C" int dabstar_decoder_enable_eti(dabstar_decoder * dec, int recording, int enable, int cif_count_hi, int cif_count_lo)
 {
@@ -720,7 +740,8 @@ struct Run
       R.d_iq = rin[r].iq;
       R.n = rin[r].n;
       const dabstar_decoder::Resume & rs = dec->resume[r];
-      if ((dec->streaming || rs.on) && R.cfg.dabplus()) return ctx->fail(DABSTAR_E_UNSUPPORTED, "recording %d: DAB+ super-frames across stream chunks are not supported", r);
+      if ((dec->streaming || rs.on) && (R.cfg.dabplus() || R.cfg.mp2()))
+        return ctx->fail(DABSTAR_E_UNSUPPORTED, "recording %d: DAB+ super-frames / MPEG audio frames across stream chunks are not supported", r);
       if (rs.on)
       {
         if (R.cfg.eti_on || R.cfg.auto_cfg || R.cfg.tii.on) return ctx->fail(DABSTAR_E_UNSUPPORTED, "stream continuation with ETI / self-configuration / TII is not supported");
@@ -1743,42 +1764,66 @@ struct Run
 };
 } // namespace
 
-// ---- DAB+: Mp4Processor (mp4processor.cpp:95-334) behind every selected sub-channel's Backend, on the packed MSC payload the
-// MSC pass left on the device (run_dabplus, one stream per recording and sub-channel). Record first_frame counts the logical
-// frames of the sub-channel's output of the run, as dabstar_decoder_msc_copy lists them.
-static int dabplus_phase(dabstar_decoder * dec)
+// ---- audio: the outer code behind every selected sub-channel's Backend, on the packed MSC payload the MSC pass left on the
+// device, one stream per recording and sub-channel and kind: DAB+ super-frames (Mp4Processor, mp4processor.cpp:95-334;
+// run_dabplus) and MPEG layer II frames (run_mp2). A sub-channel may be selected for both; the passes read the same payload.
+// Record first_frame counts the logical frames of the sub-channel's output of the run, as dabstar_decoder_msc_copy lists them.
+static int audio_phase(dabstar_decoder * dec)
 {
   dabstar_ctx * ctx = dec->ctx;
-  DabplusPass & p = dec->dabplus;
-  p.streams.clear();
-  std::vector<std::pair<int, const MscOut *>> owner;
+  DabplusPass & dp = dec->dabplus;
+  Mp2Pass & mp = dec->mp2;
+  dp.streams.clear();
+  mp.streams.clear();
+  std::vector<std::pair<int, const MscOut *>> owner[2];
   for (int r = 0; r < (int)dec->recs.size(); r++)
   {
     Recording & R = dec->recs[r];
     R.dabplus_out.clear();
-    if (!R.cfg.dabplus()) continue;
+    R.mp2_out.clear();
+    if (!R.cfg.dabplus() && !R.cfg.mp2()) continue;
     for (const MscOut & m : R.cfg.msc)
     {
-      bool on = std::find(R.cfg.dabplus_ids.begin(), R.cfg.dabplus_ids.end(), m.sc.sub_ch_id) != R.cfg.dabplus_ids.end();
-      if (R.cfg.dabplus_all && R.cfg.auto_cfg)
-        for (const dabstar_service_comp & c : R.comps) on = on || (c.tmid == 0 && c.type == 63 && c.sub_ch_id == m.sc.sub_ch_id);
-      const int br = m.sc.bit_rate;
-      if (!on || br < 8 || br > 192 || br % 8) continue;
-      p.streams.push_back(DabplusStream{ dec->d_mscpacked.as<uint8_t>() + m.out_off / 8, br, (int)(m.out_len / (24 * br)), 0, 0, 0, 0 });
-      owner.push_back({ r, &m });
+      const int id = m.sc.sub_ch_id, br = m.sc.bit_rate, n = (int)(m.out_len / (24 * br));
+      const uint8_t * src = dec->d_mscpacked.as<uint8_t>() + m.out_off / 8;
+      for (AudioKind k : { AUDIO_DABPLUS, AUDIO_MP2 })
+      {
+        const std::vector<int> & ids = k == AUDIO_MP2 ? R.cfg.mp2_ids : R.cfg.dabplus_ids;
+        bool on = std::find(ids.begin(), ids.end(), id) != ids.end();
+        if ((k == AUDIO_MP2 ? R.cfg.mp2_all : R.cfg.dabplus_all) && R.cfg.auto_cfg)
+          for (const dabstar_service_comp & c : R.comps) on = on || (c.tmid == 0 && c.type == (k == AUDIO_MP2 ? 0 : 63) && c.sub_ch_id == id);
+        if (!on || !audio_rate_ok(k, br)) continue;
+        if (k == AUDIO_MP2) mp.streams.push_back(Mp2Stream{ src, br, n, 0, 0, 0 });
+        else dp.streams.push_back(DabplusStream{ src, br, n, 0, 0, 0, 0 });
+        owner[k].push_back({ r, &m });
+      }
     }
   }
-  if (p.streams.empty()) return 0;
-  if (int e = run_dabplus(ctx, ctx->stream, p)) return e;
-  for (size_t i = 0; i < owner.size(); i++)
+  if (!dp.streams.empty())
   {
-    const MscOut & m = *owner[i].second;
-    dec->recs[owner[i].first].dabplus_out.push_back({ m.sc.sub_ch_id, m.sc.bit_rate, p.n_out[i], p.streams[i].out_rec0, p.streams[i].out_pay0 });
+    if (int e = run_dabplus(ctx, ctx->stream, dp)) return e;
+    for (size_t i = 0; i < owner[AUDIO_DABPLUS].size(); i++)
+    {
+      const MscOut & m = *owner[AUDIO_DABPLUS][i].second;
+      const int n = dp.n_out[i];
+      dec->recs[owner[AUDIO_DABPLUS][i].first].dabplus_out.push_back({ m.sc.sub_ch_id, m.sc.bit_rate, n, dp.streams[i].out_rec0, dp.streams[i].out_pay0,
+                                                                      (long long)n * 110 * (m.sc.bit_rate / 8) });
+    }
+  }
+  if (!mp.streams.empty())
+  {
+    if (int e = run_mp2(ctx, ctx->stream, mp)) return e;
+    for (size_t i = 0; i < owner[AUDIO_MP2].size(); i++)
+    {
+      const MscOut & m = *owner[AUDIO_MP2][i].second;
+      dec->recs[owner[AUDIO_MP2][i].first].mp2_out.push_back({ m.sc.sub_ch_id, m.sc.bit_rate, (int)mp.n_out[i].recs, mp.streams[i].out_rec0, mp.streams[i].out_pay0,
+                                                              mp.n_out[i].bytes });
+    }
   }
   return 0;
 }
-// With self-configuration level 2 the recordings may be decoded again (dabstar_decoder_run): the DAB+ pass then runs once, after the final pass.
-static bool dabplus_after_passes(const dabstar_decoder * dec)
+// With self-configuration level 2 the recordings may be decoded again (dabstar_decoder_run): the audio phase then runs once, after the final pass.
+static bool audio_after_passes(const dabstar_decoder * dec)
 {
   for (const Recording & R : dec->recs) if (R.cfg.auto_cfg && R.cfg.tii_nulls) return true;
   return false;
@@ -1816,8 +1861,8 @@ static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, cons
   if (!dec->cfg.scan_mode)
   {
     if (int e = run.msc_pass()) return e;
-    if (!dabplus_after_passes(dec))
-      if (int e = dabplus_phase(dec)) return e; // on `st`, beside the MSC payload copies
+    if (!audio_after_passes(dec))
+      if (int e = audio_phase(dec)) return e; // on `st`, beside the MSC payload copies
     if (int e = run.join_copies()) return e;
   }
   std::vector<EtiRef> eti_refs;
@@ -1835,10 +1880,12 @@ static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, cons
 extern "C" int dabstar_decoder_run(dabstar_decoder * dec, const void * const * iq, const int64_t * n_samples, int mem)
 {
   if (!dec || !iq || !n_samples) return DABSTAR_E_INVALID;
-  for (auto & R : dec->recs) { R.cfg.tii_flags.clear(); R.dabplus_out.clear(); }
+  for (auto & R : dec->recs) { R.cfg.tii_flags.clear(); R.dabplus_out.clear(); R.mp2_out.clear(); }
   dec->dabplus.ms = 0;
   dec->dabplus.rounds = 0;
   dec->dabplus.scanned = dec->dabplus.decoded = 0;
+  dec->mp2.ms = 0;
+  dec->mp2.slots = 0;
   int rc = decoder_run_pass(dec, iq, n_samples, mem);
   double total_ms = dec->last_ms;
   for (int pass = 1; rc == 0 && pass <= 3; pass++)
@@ -1863,10 +1910,10 @@ extern "C" int dabstar_decoder_run(dabstar_decoder * dec, const void * const * i
     rc = decoder_run_pass(dec, dptr.data(), n_samples, DABSTAR_MEM_DEVICE);
     total_ms += dec->last_ms;
   }
-  if (rc == 0 && !dec->cfg.scan_mode && dabplus_after_passes(dec))
+  if (rc == 0 && !dec->cfg.scan_mode && audio_after_passes(dec))
   {
-    rc = dabplus_phase(dec);
-    total_ms += dec->dabplus.ms;
+    rc = audio_phase(dec);
+    total_ms += dec->dabplus.ms + dec->mp2.ms;
   }
   dec->last_ms = total_ms;
   return rc;
@@ -1947,16 +1994,17 @@ extern "C" int64_t dabstar_decoder_msc_copy(const dabstar_decoder * dec, int rec
   for (int64_t i = 8 * whole; i < n; i++) out[i] = (uint8_t)((p[i >> 3] >> (7 - (i & 7))) & 1u);
   return n;
 }
-static const Recording::DabplusOut * find_dabplus(const dabstar_decoder * dec, int recording, int sub_ch_id)
+static const Recording::AudioOut * find_audio(const dabstar_decoder * dec, int recording, int sub_ch_id, AudioKind kind)
 {
   if (!dec || recording < 0 || recording >= (int)dec->recs.size()) return nullptr;
-  for (const auto & d : dec->recs[recording].dabplus_out) if (d.sub_ch_id == sub_ch_id) return &d;
+  const Recording & R = dec->recs[recording];
+  for (const auto & d : kind == AUDIO_MP2 ? R.mp2_out : R.dabplus_out) if (d.sub_ch_id == sub_ch_id) return &d;
   return nullptr;
 }
 extern "C" int dabstar_decoder_superframes(const dabstar_decoder * dec, int recording, int sub_ch_id, dabstar_superframe * out, int cap)
 {
   if (!dec || cap < 0 || (!out && cap > 0)) return DABSTAR_E_INVALID;
-  const Recording::DabplusOut * d = find_dabplus(dec, recording, sub_ch_id);
+  const Recording::AudioOut * d = find_audio(dec, recording, sub_ch_id, AUDIO_DABPLUS);
   if (!d) return dec->ctx->fail(DABSTAR_E_INVALID, "superframes: recording %d sub-channel %d was not DAB+-decoded in the last run", recording, sub_ch_id);
   for (int i = 0; i < d->n && i < cap; i++) out[i] = superframe_public(dec->dabplus.rec[d->rec0 + i]);
   return d->n;
@@ -1964,11 +2012,10 @@ extern "C" int dabstar_decoder_superframes(const dabstar_decoder * dec, int reco
 extern "C" int64_t dabstar_decoder_superframe_payload(const dabstar_decoder * dec, int recording, int sub_ch_id, uint8_t * out, int64_t cap)
 {
   if (!dec || cap < 0) return DABSTAR_E_INVALID;
-  const Recording::DabplusOut * d = find_dabplus(dec, recording, sub_ch_id);
+  const Recording::AudioOut * d = find_audio(dec, recording, sub_ch_id, AUDIO_DABPLUS);
   if (!d) return dec->ctx->fail(DABSTAR_E_INVALID, "superframe_payload: recording %d sub-channel %d was not DAB+-decoded in the last run", recording, sub_ch_id);
-  const int64_t total = (int64_t)d->n * 110 * (d->bit_rate / 8);
-  if (!out) return total;
-  const int64_t n = std::min(cap, total);
+  if (!out) return d->pay_bytes;
+  const int64_t n = std::min(cap, (int64_t)d->pay_bytes);
   if (n > 0) memcpy(out, dec->dabplus.payload + d->pay0, (size_t)n);
   return n;
 }
@@ -1977,6 +2024,28 @@ extern "C" double dabstar_decoder_dabplus_ms(const dabstar_decoder * dec, int * 
   if (!dec) return 0.0;
   if (rounds) *rounds = dec->dabplus.rounds;
   return dec->dabplus.ms;
+}
+extern "C" int dabstar_decoder_mp2_frames(const dabstar_decoder * dec, int recording, int sub_ch_id, dabstar_mp2_frame * out, int cap)
+{
+  if (!dec || cap < 0 || (!out && cap > 0)) return DABSTAR_E_INVALID;
+  const Recording::AudioOut * d = find_audio(dec, recording, sub_ch_id, AUDIO_MP2);
+  if (!d) return dec->ctx->fail(DABSTAR_E_INVALID, "mp2_frames: recording %d sub-channel %d was not MP2-decoded in the last run", recording, sub_ch_id);
+  for (int i = 0; i < d->n && i < cap; i++) out[i] = mp2_public(dec->mp2.rec[d->rec0 + i]);
+  return d->n;
+}
+extern "C" int64_t dabstar_decoder_mp2_payload(const dabstar_decoder * dec, int recording, int sub_ch_id, uint8_t * out, int64_t cap)
+{
+  if (!dec || cap < 0) return DABSTAR_E_INVALID;
+  const Recording::AudioOut * d = find_audio(dec, recording, sub_ch_id, AUDIO_MP2);
+  if (!d) return dec->ctx->fail(DABSTAR_E_INVALID, "mp2_payload: recording %d sub-channel %d was not MP2-decoded in the last run", recording, sub_ch_id);
+  if (!out) return d->pay_bytes;
+  const int64_t n = std::min(cap, (int64_t)d->pay_bytes);
+  if (n > 0) memcpy(out, dec->mp2.payload + d->pay0, (size_t)n);
+  return n;
+}
+extern "C" double dabstar_decoder_mp2_ms(const dabstar_decoder * dec)
+{
+  return dec ? dec->mp2.ms : 0.0;
 }
 extern "C" int dabstar_decoder_dabplus_windows(const dabstar_decoder * dec, int64_t out[2])
 {

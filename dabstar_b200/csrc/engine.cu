@@ -635,6 +635,97 @@ extern "C" int dabstar_dabplus_decode(dabstar_ctx * ctx, const uint8_t * frame_b
   return n_out;
 }
 
+// ------------------------------------------------------------------------------------------------ MPEG layer II audio frames
+int run_mp2(dabstar_ctx * ctx, cudaStream_t s, Mp2Pass & p)
+{
+  if (!p.ev0) { CK(cudaEventCreate(&p.ev0)); CK(cudaEventCreate(&p.ev1)); }
+  const int ns = (int)p.streams.size();
+  long long n_slots = 0;
+  for (Mp2Stream & st : p.streams)
+  {
+    st.slot0 = n_slots;
+    n_slots += st.n_frames;
+  }
+  p.n_out.assign((size_t)ns, Mp2Count{ 0, 0 });
+  p.slots = n_slots;
+  p.ms = 0;
+  p.rec = nullptr;
+  p.payload = nullptr;
+  if (n_slots == 0) return 0;
+  CK(cudaEventRecord(p.ev0, s));
+  CK(p.d_streams.reserve(sizeof(Mp2Stream) * (size_t)ns));
+  CK(p.d_cls.reserve((size_t)n_slots));
+  CK(p.d_crc.reserve(sizeof(int2) * (size_t)n_slots));
+  CK(p.d_hdr.reserve(sizeof(uint32_t) * (size_t)n_slots));
+  CK(p.d_stage.reserve(sizeof(Mp2Rec) * (size_t)n_slots)); // a stream has at most one record per logical frame
+  CK(p.d_stage_off.reserve(sizeof(long long) * (size_t)n_slots));
+  CK(p.d_cnt.reserve(sizeof(Mp2Count) * (size_t)ns));
+  CK(p.h_cnt.reserve(sizeof(Mp2Count) * (size_t)ns));
+  Mp2Stream * d_st = p.d_streams.as<Mp2Stream>();
+  CK(cudaMemcpyAsync(d_st, p.streams.data(), sizeof(Mp2Stream) * (size_t)ns, cudaMemcpyHostToDevice, s));
+  CK(launch_mp2_scan(s, d_st, ns, n_slots, p.d_cls.as<uint8_t>(), p.d_crc.as<int2>(), p.d_hdr.as<uint32_t>(), &ctx->launches));
+  CK(launch_mp2_walk(s, d_st, ns, p.d_cls.as<uint8_t>(), p.d_crc.as<int2>(), p.d_hdr.as<uint32_t>(), p.d_stage.as<Mp2Rec>(), p.d_stage_off.as<long long>(),
+                     p.d_cnt.as<Mp2Count>(), &ctx->launches));
+  CK(cudaMemcpyAsync(p.h_cnt.p, p.d_cnt.p, sizeof(Mp2Count) * (size_t)ns, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  const Mp2Count * cnt = p.h_cnt.as<Mp2Count>();
+  long long n_rec = 0, n_bytes = 0;
+  for (int i = 0; i < ns; i++)
+  {
+    Mp2Stream & st = p.streams[(size_t)i];
+    p.n_out[(size_t)i] = cnt[i];
+    st.out_rec0 = n_rec;
+    st.out_pay0 = n_bytes;
+    n_rec += cnt[i].recs;
+    n_bytes += cnt[i].bytes;
+  }
+  const size_t rec_bytes = sizeof(Mp2Rec) * (size_t)n_rec, out_bytes = rec_bytes + (size_t)n_bytes;
+  CK(p.d_out.reserve(out_bytes));
+  CK(p.h_out.reserve(out_bytes));
+  CK(cudaMemcpyAsync(d_st, p.streams.data(), sizeof(Mp2Stream) * (size_t)ns, cudaMemcpyHostToDevice, s));
+  CK(launch_mp2_compact(s, d_st, ns, n_rec, p.d_stage.as<Mp2Rec>(), p.d_stage_off.as<long long>(), p.d_out.as<Mp2Rec>(), p.d_out.as<uint8_t>() + rec_bytes, &ctx->launches));
+  CK(cudaMemcpyAsync(p.h_out.p, p.d_out.p, out_bytes, cudaMemcpyDeviceToHost, s));
+  p.rec = p.h_out.as<Mp2Rec>();
+  p.payload = p.h_out.as<uint8_t>() + rec_bytes;
+  CK(cudaEventRecord(p.ev1, s));
+  CK(cudaStreamSynchronize(s));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, p.ev0, p.ev1));
+  p.ms = ms;
+  return 0;
+}
+
+extern "C" int dabstar_mp2_frames(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, dabstar_mp2_frame * out, int cap,
+                                  uint8_t * payload, int mem)
+{
+  if (!ctx || (!frame_bits && n_frames > 0) || n_frames < 0 || cap < 0 || (cap > 0 && !out)) return DABSTAR_E_INVALID;
+  if (!mp2_rate_ok(bit_rate)) return ctx->fail(DABSTAR_E_INVALID, "MP2: %d kbit/s is not a layer II bit rate", bit_rate);
+  if (n_frames == 0) return 0;
+  CK(cudaSetDevice(ctx->device));
+  const size_t n_bits = (size_t)n_frames * 24 * bit_rate;
+  const void * dbits;
+  if (int r = stage_in(ctx, ctx->scratch[0], frame_bits, n_bits, mem, &dbits)) return r;
+  CK(ctx->scratch[1].reserve(n_bits / 8)); // packed frames
+  CK(launch_pack_bits(ctx->stream, (const uint8_t *)dbits, ctx->scratch[1].as<uint8_t>(), (long long)(n_bits / 8), &ctx->launches));
+  Mp2Pass & p = ctx->mp2;
+  p.streams.assign(1, Mp2Stream{ ctx->scratch[1].as<uint8_t>(), bit_rate, n_frames, 0, 0, 0 });
+  if (int r = run_mp2(ctx, ctx->stream, p)) return r;
+  ctx->arena_off = 0;
+  const int n_out = (int)p.n_out[0].recs, n_copy = std::min(n_out, cap);
+  size_t bytes = 0;
+  for (int i = 0; i < n_copy; i++)
+  {
+    out[i] = mp2_public(p.rec[i]);
+    if (p.rec[i].status == MP2_OK) bytes += (size_t)p.rec[i].n_frames * 3 * bit_rate;
+  }
+  if (payload && bytes > 0)
+  {
+    if (mem == DABSTAR_MEM_HOST) memcpy(payload, p.payload, bytes);
+    else CK(cudaMemcpy(payload, p.payload, bytes, cudaMemcpyHostToDevice));
+  }
+  return n_out;
+}
+
 // ------------------------------------------------------------------------------------------------ stage taps
 extern "C" int dabstar_fft2048(dabstar_ctx * ctx, const float * in, float * out, int n, int sign, int mem)
 {

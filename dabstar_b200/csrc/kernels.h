@@ -2,6 +2,7 @@
 #pragma once
 #include "common.cuh"
 #include "viterbi.cuh"
+#include "mp2.cuh"
 
 #include <vector>
 
@@ -144,6 +145,28 @@ cudaError_t launch_dabplus_decode(cudaStream_t s, const DabplusStream * st, cons
 // the attempted windows' records and super-frames, n_out of them, in stream order from out_rec0 / out_pay0
 cudaError_t launch_dabplus_compact(cudaStream_t s, const DabplusStream * st, int n_streams, long long n_out, const int * att, const int * slot, const DabplusEntry * list,
                                    const SuperFrameRec * rec, const uint8_t * payload, SuperFrameRec * out_rec, uint8_t * out_pay, unsigned long long * lc);
+
+// mp2_kernels.cu: MPEG layer II audio frames over a table of streams (one MP2 sub-channel of one recording each; mp2.cuh)
+struct Mp2Stream
+{
+  const uint8_t * src;     // n_frames logical frames of 3 * bit_rate packed bytes
+  int bit_rate, n_frames;
+  long long slot0;         // first of its n_frames entries in the pass's per-slot arrays (classes, CRCs, staged records)
+  long long out_rec0;      // first output record (set from the walk's counts)
+  long long out_pay0;      // byte offset of its first OK frame in the output payload
+};
+struct Mp2Count            // per stream, from the walk: records, and bytes of its OK frames
+{
+  long long recs, bytes;
+};
+// cls: class byte per slot (mp2.cuh: status | MP2_LSF), crc: (stored, computed) per slot, hdr: the slot's first 32 bits
+cudaError_t launch_mp2_scan(cudaStream_t s, const Mp2Stream * st, int n_streams, long long n_slots, uint8_t * cls, int2 * crc, uint32_t * hdr, unsigned long long * lc);
+// the walk of every stream (a block each): its records at stage[slot0 ..], the byte offset of each OK one inside the stream's
+// payload at stage_off[slot0 ..] (-1 for the others), and its totals in cnt
+cudaError_t launch_mp2_walk(cudaStream_t s, const Mp2Stream * st, int n_streams, const uint8_t * cls, const int2 * crc, const uint32_t * hdr, Mp2Rec * stage,
+                            long long * stage_off, Mp2Count * cnt, unsigned long long * lc);
+cudaError_t launch_mp2_compact(cudaStream_t s, const Mp2Stream * st, int n_streams, long long n_out, const Mp2Rec * stage, const long long * stage_off,
+                               Mp2Rec * out_rec, uint8_t * out_pay, unsigned long long * lc);
 
 // ofdm_kernels.cu
 cudaError_t launch_init_ref_arg(cudaStream_t s, const DeviceTables & t, unsigned long long * lc);

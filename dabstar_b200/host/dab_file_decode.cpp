@@ -13,6 +13,9 @@
 //         found, repaired and cut into access units on the GPU; prints per sub-channel super-frames attempted / ok, RS corrections /
 //         failures and access units good / bad; with -o, <prefix><n>.subch<id>.aus holds every CRC-good AU after its 2-byte
 //         big-endian length
+//     -m  all|id[,id...]: MPEG layer II audio frames of those sub-channels (all: what the recording's FIG 0/2 lists as MPEG layer
+//         II, needs -a), header- and CRC-checked on the GPU; prints per sub-channel the audio-frame slots per status; with -o,
+//         <prefix><n>.subch<id>.mp2 holds the OK frames (an MPEG audio elementary stream)
 //     -q  signal quality of every frame as CSV: frame,sym0_pos,mer_db,snr_db,noise_power,fbb_hz (fbb_hz: the baseband frequency
 //         correction of the frame's data symbols); with several files, file n's lines go to <path>.<n>
 //
@@ -45,7 +48,7 @@ int main(int argc, char ** argv)
   int fmt = DABSTAR_FMT_U8;
   bool autoCfg = false, eti = false, xml = false, containers = false, tii = false;
   dabstar_sample_format sf{};
-  std::string prefix = "dab_out_", qualPath, dabplus;
+  std::string prefix = "dab_out_", qualPath, dabplus, mp2;
   bool prefixSet = false;
   std::vector<dabstar_subch> subch;
   std::vector<const char *> files;
@@ -55,6 +58,7 @@ int main(int argc, char ** argv)
     if (a == "-f" && i + 1 < argc) { const std::string v = argv[++i]; fmt = v == "i16" ? DABSTAR_FMT_I16 : (v == "cf32" ? DABSTAR_FMT_CF32 : DABSTAR_FMT_U8); }
     else if (a == "-o" && i + 1 < argc) { prefix = argv[++i]; prefixSet = true; }
     else if (a == "-d" && i + 1 < argc) dabplus = argv[++i];
+    else if (a == "-m" && i + 1 < argc) mp2 = argv[++i];
     else if (a == "-a") autoCfg = true;
     else if (a == "-t") tii = true;
     else if (a == "-c") { containers = true; fmt = DABSTAR_FMT_CF32; }
@@ -115,14 +119,19 @@ int main(int argc, char ** argv)
       if (autoCfg && tii) proc.set_tii_processing((int)r, true);
       else proc.set_audio_channel((int)r, subch);
       if (eti) proc.start_eti_generator((int)r);
-      if (dabplus == "all") proc.set_dabplus((int)r, -1);
-      else if (!dabplus.empty())
-        for (size_t p = 0; p <= dabplus.size();)
-        {
-          const size_t q = std::min(dabplus.find(',', p), dabplus.size());
-          proc.set_dabplus((int)r, atoi(dabplus.substr(p, q - p).c_str()));
-          p = q + 1;
-        }
+      for (const bool isMp2 : { false, true })
+      {
+        const std::string & sel = isMp2 ? mp2 : dabplus;
+        auto set = [&](int id) { if (isMp2) proc.set_mp2((int)r, id); else proc.set_dabplus((int)r, id); };
+        if (sel == "all") set(-1);
+        else if (!sel.empty())
+          for (size_t p = 0; p <= sel.size();)
+          {
+            const size_t q = std::min(sel.find(',', p), sel.size());
+            set(atoi(sel.substr(p, q - p).c_str()));
+            p = q + 1;
+          }
+      }
     }
     if (!qualPath.empty()) proc.set_frame_quality(true);
     if (xml && !containers) proc.run_files(ptrs, ns, sf);
@@ -182,6 +191,19 @@ int main(int argc, char ** argv)
         }
         printf("%s: DAB+ sub-channel %d: %zu super-frames attempted, %ld ok, %ld RS corrections, %ld RS failures, %ld AUs good, %ld bad\n", files[r], s.sub_ch_id,
                sfs.size(), ok, corr, fail, good, bad);
+      }
+      for (const auto & s : proc.sub_channels((int)r))
+      {
+        if (mp2.empty() || !proc.mp2_decoded((int)r, s.sub_ch_id)) continue;
+        FILE * mf = prefixSet ? fopen((prefix + std::to_string(r) + ".subch" + std::to_string(s.sub_ch_id) + ".mp2").c_str(), "wb") : nullptr;
+        const std::vector<dabstar_mp2_frame> fr = proc.mp2_frames((int)r, s.sub_ch_id, [&](const dabstar::u8 * f, int len, const dabstar_mp2_frame &) {
+          if (mf) fwrite(f, 1, (size_t)len, mf);
+        });
+        if (mf) fclose(mf);
+        long cnt[5] = { 0 };
+        for (const auto & x : fr) if (x.status >= 0 && x.status < 5) cnt[x.status]++;
+        printf("%s: MP2 sub-channel %d: %zu slots, %ld ok, %ld no header, %ld mismatch, %ld CRC errors, %ld cut\n", files[r], s.sub_ch_id, fr.size(), cnt[0], cnt[1],
+               cnt[2], cnt[3], cnt[4]);
       }
       if (autoCfg && tii)
         for (const auto & ev : proc.tii_events((int)r))

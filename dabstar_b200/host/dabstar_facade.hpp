@@ -216,6 +216,42 @@ private:
   long mSeen = 0;
 };
 
+// MPEG layer II audio frames of one DAB (MP2) sub-channel: header and CRC-16 of every audio-frame slot, on the device
+// (dabstar_mp2_frames). Batch granular; an MP2 decoder stays a CPU consumer of the OK frames handed to the sink.
+class Mp2Processor
+{
+public:
+  using FrameSink = std::function<void(const u8 * frame, int len, const dabstar_mp2_frame & rec)>;
+  Mp2Processor(Context & c, int bitRate, FrameSink sink = nullptr) : mC(c), mBitRate(bitRate), mSink(std::move(sink)) {}
+  // iBits: nFrames x 24*bitRate bytes (one bit each). Returns one record per audio-frame slot.
+  std::vector<dabstar_mp2_frame> add_frames(const u8 * iBits, int nFrames)
+  {
+    std::vector<dabstar_mp2_frame> rec((size_t)std::max(nFrames, 1));
+    std::vector<u8> pay(rec.size() * 3 * (size_t)mBitRate);
+    const int n = mC.check(dabstar_mp2_frames(mC.get(), iBits, mBitRate, nFrames, rec.data(), (int)rec.size(), pay.data(), DABSTAR_MEM_HOST), "dabstar_mp2_frames");
+    rec.resize((size_t)n);
+    if (mSink) deliver(rec, pay.data(), mBitRate, mSink);
+    return rec;
+  }
+  // the OK frames of records, whose bytes follow one another in payload
+  static void deliver(const std::vector<dabstar_mp2_frame> & rec, const u8 * payload, int bitRate, const FrameSink & sink)
+  {
+    size_t o = 0;
+    for (const auto & r : rec)
+      if (r.status == 0)
+      {
+        const int len = 3 * bitRate * r.n_frames;
+        sink(payload + o, len, r);
+        o += (size_t)len;
+      }
+  }
+
+private:
+  Context & mC;
+  int mBitRate;
+  FrameSink mSink;
+};
+
 // backend/audio/mp4processor.h: the DAB+ outer code of one sub-channel (super-frame sync, RS(120,110), Fire code, AU CRCs).
 // Batch granular: add_frames takes a run of FrameProcessor::add_to_frame payloads; the AAC decoder stays a CPU consumer.
 class Mp4Processor
@@ -419,6 +455,30 @@ public:
         if (rec[i].ok)
           for (int u = 0; u < rec[i].num_aus; u++)
             if (rec[i].au_state[u] == 1) sink(&pay[(size_t)i * sf + rec[i].au_start[u]], rec[i].au_start[u + 1] - rec[i].au_start[u] - 2, rec[i]);
+    }
+    return rec;
+  }
+  // MPEG layer II audio frames of the sub-channel in the next runs, on the device; subChId -1: every sub-channel the recording's
+  // own FIG 0/2 lists as MPEG layer II (needs set_auto_config)
+  void set_mp2(int recording, int subChId = -1, bool on = true)
+  {
+    mC.check(dabstar_decoder_set_mp2(mDec, recording, subChId, on ? 1 : 0), "dabstar_decoder_set_mp2");
+  }
+  bool mp2_decoded(int recording, int subChId) const { return dabstar_decoder_mp2_frames(mDec, recording, subChId, nullptr, 0) >= 0; }
+  // the last run's audio-frame slots; every OK frame goes to sink, in order
+  std::vector<dabstar_mp2_frame> mp2_frames(int recording, int subChId, const Mp2Processor::FrameSink & sink = nullptr) const
+  {
+    const int n = mC.check(dabstar_decoder_mp2_frames(mDec, recording, subChId, nullptr, 0), "dabstar_decoder_mp2_frames");
+    std::vector<dabstar_mp2_frame> rec((size_t)n);
+    if (n > 0) dabstar_decoder_mp2_frames(mDec, recording, subChId, rec.data(), n);
+    if (sink && n > 0)
+    {
+      std::vector<u8> pay((size_t)dabstar_decoder_mp2_payload(mDec, recording, subChId, nullptr, 0));
+      dabstar_decoder_mp2_payload(mDec, recording, subChId, pay.data(), (int64_t)pay.size());
+      int bitRate = 0;
+      for (const auto & s : sub_channels(recording)) if (s.sub_ch_id == subChId) bitRate = s.bit_rate;
+      if (bitRate <= 0) throw std::runtime_error("mp2_frames: sub-channel " + std::to_string(subChId) + " is not in the recording's sub-channel list");
+      Mp2Processor::deliver(rec, pay.data(), bitRate, sink);
     }
     return rec;
   }

@@ -274,6 +274,34 @@ typedef struct
 int dabstar_dabplus_decode(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, dabstar_superframe * out, int cap,
                            uint8_t * payload, int mem);
 
+/* ------------------------------------------------------------------------------------------------ MPEG layer II audio frames */
+/* The audio frames of a run of logical frames of one DAB (MP2) sub-channel (TMId 0, ASCTy 0), checked on the device. A DAB audio
+ * frame starts at the first bit of a logical frame and lasts 24 ms at 48 kHz (MPEG-1, one logical frame of 3 * bit_rate bytes) or
+ * 48 ms at 24 kHz (MPEG-2 LSF, two logical frames; ETSI EN 300 401 clause 7). Every slot is classified from its 32-bit header
+ * (ISO/IEC 11172-3 2.4.1.3) and its CRC-16 (x^16 + x^15 + x^2 + 1, preset 0xFFFF, over header bits 16-31, the bit allocation
+ * and the SCFSI; 11172-3 2.4.3.1, allocation tables 11172-3 Annex B Table B.2a / B.2c and 13818-3 Table B.1). Status:
+ *   0 OK         valid header, CRC matches
+ *   1 NO_HEADER  syncword != 0xFFF, layer != II or protection_bit = 1
+ *   2 MISMATCH   sampling_frequency != 01 (48 kHz / 24 kHz), bitrate_index 0 or 15, or the header's rate != the sub-channel's
+ *   3 CRC_ERROR  valid header, CRC mismatch
+ *   4 CUT        a 24 kHz frame whose second logical frame lies past the end of the run
+ * An OK 24 kHz frame is one record covering logical frames i and i + 1; every other slot is a one-frame record. PCM decoding,
+ * PAD and the DAB scale-factor CRC are left to the consumer. */
+typedef struct
+{
+  int32_t first_frame;  /* index of the slot's first logical frame */
+  int32_t n_frames;     /* logical frames it covers: 2 for an OK 24 kHz frame, else 1 */
+  int32_t status;       /* 0..4, above */
+  uint32_t header;      /* the slot's first 32 bits, as read */
+  int32_t crc_stored, crc_computed; /* crc_check and the CRC over the protected bits; -1 where not reached */
+} dabstar_mp2_frame;
+/* frame_bits: n_frames x 24*bit_rate bytes, one bit each (dabstar_decoder_msc_copy). out: one record per slot, in stream order
+ * (at most cap are written); payload (may be NULL; room for n_frames * 3 * bit_rate bytes): the bytes of the OK frames among
+ * those records, concatenated in record order. bit_rate must be a layer II rate (MPEG-1 32..384 or LSF 8..160 kbit/s).
+ * Returns the number of records or <0. */
+int dabstar_mp2_frames(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, dabstar_mp2_frame * out, int cap,
+                       uint8_t * payload, int mem);
+
 /* ------------------------------------------------------------------------------------------------ multiplex configuration (FIG 0/0, 0/1, 0/2) */
 /* The part of FibDecoder the decode path depends on (decoder/fib_decoder.cpp:59-106 process_FIB,
  * fib_decoder_fig0.cpp:89-113 FIG 0/0, :142-227 FIG 0/1, :229-290 FIG 0/2, fib_table.h:51 short-form table): which
@@ -417,6 +445,21 @@ double  dabstar_decoder_dabplus_ms(const dabstar_decoder * dec, int * rounds);
 /* windows (five-frame candidates) of the last run's DAB+ pass: out[0] whose raw header was Fire-code checked, out[1] that went
  * through Reed-Solomon (the processor attempts about one in five of a synchronised stream) */
 int     dabstar_decoder_dabplus_windows(const dabstar_decoder * dec, int64_t out[2]);
+/* MPEG layer II audio frames inside the run (see dabstar_mp2_frames) for the chosen sub-channels, on the device, on the run's own
+ * MSC payload. sub_ch_id -1: every sub-channel the recording's own FIG 0/2 lists as MPEG layer II (TMId 0, ASCTy 0; needs
+ * auto-config). An explicit id must name a sub-channel set with dabstar_decoder_set_subchannels whose bit rate is a layer II rate
+ * (with auto-config it is looked up in the run's own FIC). enable = 0 deselects it. A sub-channel may be selected for DAB+ as
+ * well; both passes read the same payload. scan_mode decodes no MSC and so no frames; streaming is not supported
+ * (DABSTAR_E_UNSUPPORTED: a 48 ms frame can straddle two chunks). */
+int     dabstar_decoder_set_mp2(dabstar_decoder * dec, int recording, int sub_ch_id, int enable);
+/* records of the last run's audio-frame slots, exactly as dabstar_mp2_frames returns them for dabstar_decoder_msc_copy's bits of
+ * that sub-channel; returns the count (E_INVALID: not MP2-decoded in the last run) */
+int     dabstar_decoder_mp2_frames(const dabstar_decoder * dec, int recording, int sub_ch_id, dabstar_mp2_frame * out, int cap);
+/* the OK frames' bytes in record order (a playable MPEG audio elementary stream); returns bytes written (out NULL: the bytes
+ * there are). A damaged frame can be read from dabstar_decoder_msc_packed at first_frame * 3 * bit_rate. */
+int64_t dabstar_decoder_mp2_payload(const dabstar_decoder * dec, int recording, int sub_ch_id, uint8_t * out, int64_t cap);
+/* device time of the last run's MP2 pass */
+double  dabstar_decoder_mp2_ms(const dabstar_decoder * dec);
 /* EtiGenerator (eti_handler/eti_generator.h:56-66: start_eti_generator before run / process_block per symbol): every
  * sub-channel set with dabstar_decoder_set_subchannels is decoded for every CIF through the generator's own whole-CIF
  * de-interleaver (first frame with its 17th CIF; its start-up bookkeeping, which loses the 16th CIF, is reproduced) and
