@@ -575,8 +575,6 @@ void restore(Recording & r, const CtlSnapshot & s)
 
 namespace
 {
-bool trace_on() { static const bool on = getenv("DABSTAR_TRACE") != nullptr; return on; } // per-round progress on stderr (debug aid)
-
 // The window of one recording in a round, grown by the layout passes
 struct Plan
 {
@@ -612,6 +610,7 @@ struct Run
   const int n_rec, fmt;
   const bool host_in;
   const float thr0;
+  const bool trace = getenv("DABSTAR_TRACE") != nullptr; // per-round progress on stderr (debug aid), read once per run
   // X budget: bound the frames of one round so the window spectrum buffer stays below ~12 GB
   const long long x_frame_bytes = (long long)sizeof(float2) * X_ROWS * K_CARR;
   const long long max_round_frames;
@@ -639,7 +638,7 @@ struct Run
   double elapsed_ms() const { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_run0).count(); }
   void tr(const char * what) const
   {
-    if (trace_on()) fprintf(stderr, "[dabstar]   %-28s t=%.3f ms\n", what, elapsed_ms());
+    if (trace) fprintf(stderr, "[dabstar]   %-28s t=%.3f ms\n", what, elapsed_ms());
   }
   // the decode stream must not read samples at or beyond `upto` before their chunk has landed
   cudaError_t need_upto(long long upto)
@@ -931,7 +930,7 @@ struct Run
       long long window_end = 0;
       const int n_tail = lay_out_tail(resident, window_end);
       if (n_tail == 0) break;
-      if (trace_on()) fprintf(stderr, "[dabstar]     pass: %d tail frames\n", n_tail);
+      if (trace) fprintf(stderr, "[dabstar]     pass: %d tail frames\n", n_tail);
       tr("  tail laid out");
       CK(need_upto(window_end));
       CK(dec->d_desc.reserve(sizeof(FrameDesc) * (size_t)n_tail + (size_t)n_tail + 64));
@@ -1201,7 +1200,7 @@ struct Run
         o[base + j] = pl.fr[(size_t)j].desc;
       }
     });
-    if (trace_on())
+    if (trace)
       fprintf(stderr, "[dabstar] round %lld t=%.3f ms: %zu recordings, %d frames, chunks resident %d/%d waited %d\n", dec->cnt_rounds,
               elapsed_ms(), plans.size(), n_desc, dec->chunks_done, dec->n_chunks, dec->chunks_waited);
     return upload_commit(ctx, dec->d_desc.p, desc_stage, sizeof(FrameDesc) * (size_t)n_desc);
@@ -1713,7 +1712,7 @@ struct Run
     }
     CK(cudaEventRecord(dec->ev1, st));
     SYNC();
-    if (trace_on()) fprintf(stderr, "[dabstar] run done t=%.3f ms\n", elapsed_ms());
+    if (trace) fprintf(stderr, "[dabstar] run done t=%.3f ms\n", elapsed_ms());
     // ETI(NI) frames: header, FIC of the frame the CIF belongs to, the streams, EOF and TIST, padding (eti_generator.cpp:163-199)
     for (const EtiRef & er : eti_refs)
     {

@@ -1733,8 +1733,10 @@ cudaError_t launch_demap(cudaStream_t s, const DeviceTables & t, const DemapWork
   // symbols between a symbol's arithmetic and the write of its soft bits: the stash is (lag + 1) x 4 KB of shared memory per
   // CTA, so a shorter lag trades waiting on the slowest warp of a run against resident CTAs per SM (2 / 3 / 4 at lag 15 / 7 /
   // 3). Measured (profiles/README.md): 288 CTAs (96 recordings) 5.57 / 5.61 / 7.07 ms, 576 CTAs (192 segments) - / 7.83 / 6.08 ms:
-  // the longest lag whose residency still holds the whole grid. DABSTAR_DEMAP_LAG = 3 | 7 | 15 overrides (A/B switch).
-  static const int lag_env = getenv("DABSTAR_DEMAP_LAG") ? atoi(getenv("DABSTAR_DEMAP_LAG")) : 0;
+  // the longest lag whose residency still holds the whole grid. DABSTAR_DEMAP_LAG = 3 | 7 | 15 overrides (read per launch: A/B
+  // measurements, and the tests that pin every lag)
+  const char * ev = getenv("DABSTAR_DEMAP_LAG");
+  const int lag_env = ev ? atoi(ev) : 0;
   const int grid_ctas = n_work * DM5_SLICES;
   const int lag = lag_env == 3 || lag_env == 7 || lag_env == 15 ? lag_env : (grid_ctas <= 2 * N_SM ? 15 : (grid_ctas <= 3 * N_SM ? 7 : 3));
   const bool qual = qsnap != nullptr;

@@ -14,21 +14,16 @@ own template instance with its own stash depth, output-row ring and drain loop, 
   frame, against the oracle chain; all copies of a source and the source decoded alone bit identical;
 * the segmented decode of a 400-frame recording against the replay of the engine's own segment layout, frame by frame.
 
-The lag is read from DABSTAR_DEMAP_LAG once per process, so each configuration runs in a fresh process (demap_worker.py).
+The lag is read from DABSTAR_DEMAP_LAG on every launch: each configuration runs here under demap_support.forced_lag.
 """
 from __future__ import annotations
-
-import os
-import shutil
-import subprocess
-import sys
-from collections import Counter
 
 import numpy as np
 import pytest
 
-import demap_worker as W
-from dabstar_b200 import synth
+import demap_support as S
+from dabstar_b200 import api, synth
+from demap_support import N_LONG, engine_segments
 
 LAGS = (3, 7, 15)
 N_SM, CTAS_PER_RUN = 148, 3
@@ -39,73 +34,12 @@ QUALITY = ("mer_db", "snr_db", "mean_value", "mean_power_overall", "noise_power"
 
 # ------------------------------------------------------------------------------------------------ oracle replay model
 def replay(oracle, fft, clock_err, segments, soft_bit_type):
-    """Soft bits of the kept frames of `segments`, decoded by the oracle's OfdmDecoder from the given spectra.
-
-    fft(f): complex64[77, 2048] of frame f (symbol 0, symbols 1..75, null symbol), clock_err[f] its clock error;
-    segments: [(first, last, warmup, parent)]: frames first..last are decoded, the soft bits of first + warmup..last are kept;
-    parent -1 starts from a fresh (reset) decoder, parent j >= 0 continues from the state after segment j (which ends at
-    frame first - 1 and comes earlier in the list).
-    The chain passes its CP phase as phase_corr; that only feeds the frequency-correction statistics, not the soft bits (the
-    self-check pins it), so 0 is passed. Returns {frame: int16[75, 3072]}."""
-
-    def run(h, seg, out):
-        first, last, warmup, _ = seg
-        for f in range(first, last + 1):
-            x = fft(f)
-            soft = np.zeros((75, 3072), np.int16)
-            oracle.ofdm_store_reference(h, x[0])
-            for s in range(1, 76):
-                soft[s - 1] = oracle.ofdm_decode_symbol(h, x[s], s, 0.0, float(clock_err[f]))
-            oracle.ofdm_store_null(h, x[76])
-            if out is not None and f >= first + warmup:
-                out[f] = soft
-
-    def state_after(j):
-        """A new decoder in the state after segment j (replayed again from its own start)."""
-        p = segments[j][3]
-        h = oracle.ofdm_new(soft_bit_type) if p < 0 else state_after(p)
-        run(h, segments[j], None)
-        return h
-
-    children = Counter(s[3] for s in segments if s[3] >= 0)
-    kept, out = {}, {}
-    for i, seg in enumerate(segments):
-        p = seg[3]
-        assert p < i and (p < 0 or segments[p][1] == seg[0] - 1), (i, seg)
-        if p < 0:
-            h = oracle.ofdm_new(soft_bit_type)
-        else:
-            children[p] -= 1
-            h = kept.pop(p) if children[p] == 0 else state_after(p)
-        run(h, seg, out)
-        if children[i] > 0:
-            kept[i] = h
-        else:
-            oracle.ofdm_free(h)
-    for h in kept.values():
-        oracle.ofdm_free(h)
+    """Soft bits of the kept frames of `segments`, decoded by the oracle's OfdmDecoder from the given spectra
+    (demap_support.replay_segments; the self-checks below pin that the CP phase it passes as 0 does not move them).
+    Returns {frame: int16[75, 3072]}."""
+    out = {}
+    S.replay_segments(oracle, fft, clock_err, segments, soft_bit_type, lambda f, h, soft: out.__setitem__(f, soft))
     return out
-
-
-def engine_segments(windows, seg_frames, seg_warmup):
-    """The engine's demapper runs over a recording's windows (decoder.cu, heavy pass: 'demapper runs'), as replay segments.
-
-    A window of n >= 2 seg_frames frames is cut into n_seg = n // seg_frames segments; segment sg covers [b, e) with
-    b = n sg / n_seg and starts w = min(warm-up, b) frames early (w = 0 for sg = 0). A segment that reaches back to the window's
-    first frame continues from the recording's state (reset() in the first window after the time sync), the others start
-    from reset() and discard their w warm-up frames; the window's last segment hands its state to the next window.
-    Returns (segments, sum of w)."""
-    segs, f0, total_w, prev = [], 0, 0, -1
-    for n in windows:
-        n_seg = n // seg_frames if seg_frames > 0 and n >= 2 * seg_frames else 1
-        for sg in range(n_seg):
-            b, e = n * sg // n_seg, n * (sg + 1) // n_seg
-            w = 0 if sg == 0 else min(seg_warmup, b)
-            total_w += w
-            segs.append((f0 + b - w, f0 + e - 1, w, prev if b - w == 0 else -1))
-        prev = len(segs) - 1
-        f0 += n
-    return segs, total_w
 
 
 def _chain_with_taps(oracle, iq, soft_bit_type=0):
@@ -117,7 +51,7 @@ def test_replay_reproduces_the_chain(oracle, soft_bit_type, cut):
     """Replaying the chain's own FFT rows and clock errors through one unsegmented run gives the chain's soft bits bit for bit
     (cut: the recording ends 10 data symbols into its last frame; the chain drops that frame, the complete ones stay exact)."""
     rec = synth.generate(7, seed=30 + soft_bit_type, snr_db=18.0, cfo_hz=1500.0, fmt=synth.FMT_U8)
-    iq = rec.iq[:W.LEAD + 6 * synth.T_FRAME + 2656 + 2552 + 10 * 2552 + 1000] if cut else rec.iq
+    iq = rec.iq[:S.LEAD + 6 * synth.T_FRAME + 2656 + 2552 + 10 * 2552 + 1000] if cut else rec.iq
     r = _chain_with_taps(oracle, iq, soft_bit_type)
     assert r.n_frames == (6 if cut else 7)
     ce = [i.clock_err for i in r.info]
@@ -154,23 +88,6 @@ def test_engine_segment_layout():
     assert engine_segments([5, 7], 4, 2) == ([(0, 4, 0, -1), (5, 11, 0, 0)], 0)  # windows < 2 segments: one run each
 
 
-# ------------------------------------------------------------------------------------------------ worker processes
-def run_worker(mode, lag, out_dir, inputs=None, timeout=900):
-    """demap_worker.py MODE in a fresh process with DABSTAR_DEMAP_LAG = lag (None: the launcher's choice) and DABSTAR_TRACE."""
-    os.makedirs(out_dir, exist_ok=True)
-    if inputs is not None:
-        np.savez(os.path.join(out_dir, "in.npz"), **inputs)
-    env = dict(os.environ, DABSTAR_TRACE="1")
-    env.pop("DABSTAR_DEMAP_LAG", None)
-    if lag is not None:
-        env["DABSTAR_DEMAP_LAG"] = str(lag)
-    flags = (["-s"] if sys.flags.no_user_site else []) + (["-E"] if sys.flags.ignore_environment else [])
-    r = subprocess.run([sys.executable] + flags + [W.__file__, mode, str(out_dir), str(out_dir)], env=env, capture_output=True,
-                       text=True, timeout=timeout)
-    assert r.returncode == 0, f"worker {mode} lag {lag} exited {r.returncode}:\n{r.stderr[-4000:]}"
-    return dict(np.load(os.path.join(out_dir, "out.npz")))
-
-
 def _check_soft(got, want, where):
     """Soft bits of one frame against the oracle: <= 1e-4 of them more than one LSB apart (the parity bar), and <= 1 % apart at
     all. The float arithmetic differs from the oracle's only in its last bits, so a value truncates to another integer rarely;
@@ -178,13 +95,6 @@ def _check_soft(got, want, where):
     d = np.abs(np.asarray(got).astype(np.int32) - np.asarray(want).astype(np.int32))
     beyond, differ = float((d > 1).mean()), float((d > 0).mean())
     assert beyond <= 1e-4 and differ <= 1e-2, (where, f"beyond 1 LSB {beyond:.2e}, differing {differ:.2e}, max {d.max()}")
-
-
-@pytest.fixture(scope="module")
-def work_dir(tmp_path_factory):
-    d = tmp_path_factory.mktemp("demap_shapes")
-    yield d
-    shutil.rmtree(d, ignore_errors=True)  # the soft-bit dumps are some hundred MB
 
 
 # ------------------------------------------------------------------------------------------------ B: the tap at every lag
@@ -201,14 +111,35 @@ def tap_inputs(oracle):
     return fft, ce
 
 
+def tap_outputs(ctx, fft, ce, tii) -> dict:
+    """OfdmDecoder.decode_frames for soft_bit_type 0 / 1 / 2: the six frames with their TII flags, a one-frame call, and the
+    six frames as a continuation over two calls on the same state; soft bits, state vectors and (six frames) quality."""
+    out = {}
+    for st in (0, 1, 2):
+        dec = api.OfdmDecoder(st, ctx)
+        out[f"full_soft_{st}"] = dec.decode_frames(fft, ce, tii)
+        out[f"full_state_{st}"] = np.concatenate([dec.state(w) for w in range(6)])
+        out[f"full_quality_{st}"] = np.array([dec.quality()[k] for k in api.OfdmDecoder.QUALITY], np.float32)
+        dec = api.OfdmDecoder(st, ctx)
+        out[f"one_soft_{st}"] = dec.decode_frames(fft[:1], ce[:1])
+        out[f"one_state_{st}"] = np.concatenate([dec.state(w) for w in range(6)])
+        dec = api.OfdmDecoder(st, ctx)
+        a = dec.decode_frames(fft[:3], ce[:3], tii[:3])
+        b = dec.decode_frames(fft[3:], ce[3:], tii[3:])
+        out[f"cont_soft_{st}"] = np.concatenate([a, b])
+        out[f"cont_state_{st}"] = np.concatenate([dec.state(w) for w in range(6)])
+    return out
+
+
 @pytest.fixture(scope="module")
-def tap_runs(tap_inputs, work_dir):
+def tap_runs(ctx, tap_inputs):
     cache = {}
 
     def get(lag):
         if lag not in cache:
             fft, ce = tap_inputs
-            cache[lag] = run_worker("tap", lag, work_dir / f"tap{lag}", dict(fft=fft, clock_err=ce, tii=TAP_TII), timeout=600)
+            with S.forced_lag(lag):
+                cache[lag] = tap_outputs(ctx, fft, ce, TAP_TII)
         return cache[lag]
     return get
 
@@ -290,24 +221,68 @@ def test_tap_lags_bit_identical(tap_runs, soft_bit_type):
 def batch_want(oracle):
     """The oracle chain of each of the 32 sources (soft_bit_type 0)."""
     want = []
-    for i in range(W.N_SRC):
-        iq, k = W.batch_source(i)
+    for i in range(S.N_SRC):
+        iq, k = S.batch_source(i)
         want.append((oracle.chain_run(oracle.to_cf32(iq), scan_mode=1, tap_soft=True), k))
     yield want
     for r, _ in want:
         r.close()
 
 
+def batch_outputs(ctx) -> dict:
+    """DabProcessor over the 256 copies of the batch sources (traced), then every source decoded alone (traced)."""
+    srcs = [S.batch_source(i)[0] for i in range(S.N_SRC)]
+    dp, rounds, dev = S.decode_batch(ctx, srcs, 0, trace=True)
+    out = S.batch_results(dp)
+    out["rounds"] = rounds
+    # soft bits of the first copy of every source; a digest per frame of every copy
+    soft = np.zeros((S.N_SRC, S.F_MAX, 75, 3072), np.int16)
+    dig = np.zeros((S.N_COPIES, S.F_MAX, 32), np.uint8)
+    for r in range(S.N_COPIES):
+        s = S.soft_of(dp, r)
+        for f in range(s.shape[0]):
+            dig[r, f] = S.digest(s[f])
+        if r < S.N_SRC:
+            soft[r, :s.shape[0]] = s
+    out["digest"] = dig
+    out["soft"] = soft
+    del dp, dev
+    # every source decoded alone: its digests, its result and its own rounds; its soft bits where a frame differs from the batch
+    single = [[] for _ in range(6)]
+    diff_at, diff_soft = [], []
+    import torch
+    for i in range(S.N_SRC):
+        t = torch.from_numpy(srcs[i]).cuda()
+        dp1 = api.DabProcessor(1, input_format=api.FMT_U8, scan_mode=True, ctx=ctx)
+        rounds1 = S.traced(lambda: dp1.run_ptrs([t.data_ptr()], [t.shape[0]], api.MEM_DEVICE))
+        s = S.soft_of(dp1, 0)
+        d = np.zeros((S.F_MAX, 32), np.uint8)
+        for f in range(s.shape[0]):
+            d[f] = S.digest(s[f])
+            if not np.array_equal(d[f], dig[i, f]):
+                diff_at.append((i, f))
+                diff_soft.append(s[f] - soft[i, f])
+        ra = S.result_arrays(dp1, 0)
+        starts = np.zeros(S.F_MAX, np.uint8)  # frames that begin a window of this decode
+        starts[np.cumsum(np.concatenate([[0], rounds1[:, 1]]))[:-1].clip(max=S.F_MAX - 1)] = 1
+        for lst, v in zip(single, (d, ra["n_frames"], ra["pos"], ra["fbb"], ra["fic_valid"], starts)):
+            lst.append(v)
+    for name, lst in zip(("digest", "n_frames", "pos", "fbb", "fic_valid", "window_start"), single):
+        out["single_" + name] = np.stack(lst)
+    # (source, frame) where the lone decode differs from the batch, and the difference (lone - batch)
+    out["single_diff_at"] = np.array(diff_at, np.int64).reshape(-1, 2)
+    out["single_diff"] = np.array(diff_soft, np.int16).reshape(-1, 75, 3072)
+    return out
+
+
 @pytest.fixture(scope="module")
-def batch_runs(work_dir):
+def batch_runs(ctx):
     cache = {}
 
     def get(lag):
         if lag not in cache:
-            d = work_dir / f"batch{lag}"
-            out = run_worker("batch", lag, d, timeout=1200)
-            out["soft"] = np.load(d / "soft.npy", mmap_mode="r")
-            cache[lag] = out
+            with S.forced_lag(lag):
+                cache[lag] = batch_outputs(ctx)
         return cache[lag]
     return get
 
@@ -318,7 +293,7 @@ def _check_copy_against_chain(got, r, want, k, soft=None):
     both) and through the last complete frame, whose trailing rows the drain writes when the cut frame holds fewer than LAG
     symbols."""
     n = int(got["n_frames"][r])
-    assert n == want.n_frames == W.N_FULL, (r, n, want.n_frames)
+    assert n == want.n_frames == S.N_FULL, (r, n, want.n_frames)
     assert [tuple(p) for p in got["pos"][r, :n]] == [(i.sym0_pos, i.start_index) for i in want.info], r
     assert [(round(float(a)), round(float(b))) for a, b in got["fbb"][r, :n]] == [(round(i.fbb_data), round(i.fbb_null)) for i in want.info], r
     assert np.array_equal(got["fic_valid"][r, :n], want.fic_valid), r
@@ -339,13 +314,13 @@ def test_batch_past_one_wave(batch_runs, batch_want, lag):
     are bit identical to each other and to the source decoded alone."""
     out = batch_runs(lag)
     rounds = out["rounds"]
-    heavy = rounds[rounds[:, 0] == W.N_COPIES]
+    heavy = rounds[rounds[:, 0] == S.N_COPIES]
     assert heavy.shape[0] >= 1, rounds   # a heavy round ran every recording in one demapper launch
-    assert W.N_COPIES * CTAS_PER_RUN > RESIDENT[lag]
-    for r in range(W.N_COPIES):
-        s = r % W.N_SRC
+    assert S.N_COPIES * CTAS_PER_RUN > RESIDENT[lag]
+    for r in range(S.N_COPIES):
+        s = r % S.N_SRC
         want, k = batch_want[s]
-        _check_copy_against_chain(out, r, want, k, out["soft"][s] if r < W.N_SRC else None)
+        _check_copy_against_chain(out, r, want, k, out["soft"][s] if r < S.N_SRC else None)
         assert np.array_equal(out["digest"][r], out["digest"][s]), (r, s)
         for key in ("n_frames", "pos", "fbb", "fic_valid", "fib", "counters"):
             assert np.array_equal(out[key][r], out[key][s]), (r, key)
@@ -354,7 +329,7 @@ def test_batch_past_one_wave(batch_runs, batch_want, lag):
     for (s, f), d in zip(out["single_diff_at"], out["single_diff"]):
         assert out["single_window_start"][s, f] and np.abs(d[1:]).max() == 0 and np.abs(d[0]).max() <= 1, (s, f)
     differing = {(int(s), int(f)) for s, f in out["single_diff_at"]}
-    for s in range(W.N_SRC):
+    for s in range(S.N_SRC):
         for f in range(int(out["n_frames"][s])):
             if (s, f) not in differing:
                 assert np.array_equal(out["single_digest"][s, f], out["digest"][s, f]), (s, f)
@@ -377,27 +352,36 @@ def test_batch_lags_bit_identical(batch_runs):
 def test_batch_soft_bit_types(ctx, oracle, soft_bit_type):
     """soft_bit_type 1 and 2 through DabProcessor: the 256-recording batch with the launcher's own lag choice (3 for 768
     CTAs) against chain_run with the same soft-bit type."""
-    srcs = [W.batch_source(i) for i in range(W.N_SRC)]
-    dp, _, dev = W.decode_batch(ctx, [s for s, _ in srcs], soft_bit_type)
-    got = W.batch_results(dp)
+    srcs = [S.batch_source(i) for i in range(S.N_SRC)]
+    dp, _, dev = S.decode_batch(ctx, [s for s, _ in srcs], soft_bit_type)
+    got = S.batch_results(dp)
     for s, (iq, k) in enumerate(srcs):
         want = oracle.chain_run(oracle.to_cf32(iq), scan_mode=1, soft_bit_type=soft_bit_type, tap_soft=True)
-        soft = W.soft_of(dp, s)
-        for r in range(s, W.N_COPIES, W.N_SRC):
+        soft = S.soft_of(dp, s)
+        for r in range(s, S.N_COPIES, S.N_SRC):
             _check_copy_against_chain(got, r, want, k, soft if r == s else None)
             if r != s:
-                assert np.array_equal(W.soft_of(dp, r), soft), r
+                assert np.array_equal(S.soft_of(dp, r), soft), r
         want.close()
     del dp, dev
 
 
 # ------------------------------------------------------------------------------------------------ D: segmented decode
-N_LONG = 400
+def segment_outputs(ctx, seg_frames, warmup, max_window) -> dict:
+    """DabProcessor with set_segmentation over segment_recording() (traced): result, rounds, warm-up frames, soft bits."""
+    iq = S.segment_recording()
+    dp = api.DabProcessor(1, input_format=api.FMT_U8, scan_mode=True, max_window=max_window, ctx=ctx)
+    dp.set_segmentation(seg_frames, warmup)
+    rounds = S.traced(lambda: dp.run([iq]))
+    res = dp.result(0)
+    return dict(n_frames=res.n_frames, pos=np.array([(i.sym0_pos, i.start_index) for i in res.info], np.int64).reshape(-1, 2),
+                fic_valid=res.fic_valid, rounds=rounds, warmup_frames=dp.warmup_frames(0),
+                soft=S.soft_of(dp, 0))
 
 
 @pytest.fixture(scope="module")
 def long_chain(oracle):
-    r = _chain_with_taps(oracle, W.segment_recording())
+    r = _chain_with_taps(oracle, S.segment_recording())
     assert r.n_frames == N_LONG
     yield r
     r.close()
@@ -405,16 +389,16 @@ def long_chain(oracle):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("seg_frames,warmup,lag,max_window", [(48, 4, 15, 200), (48, 18, 15, 200), (2, 4, 3, 512)])
-def test_segmented_decode_matches_exact_model(oracle, long_chain, work_dir, seg_frames, warmup, lag, max_window):
+def test_segmented_decode_matches_exact_model(ctx, oracle, long_chain, seg_frames, warmup, lag, max_window):
     """set_segmentation over a clean 400-frame recording, frame by frame against the oracle replay of the engine's own layout:
     the windows from the round trace, each cut into segments that warm up from reset() or continue the recording's state.
     Every frame within one LSB on <= 1e-4 of its soft bits, and warmup_frames() the sum of the warm-ups. (2, 4) is ~200
     segments in one launch: ~600 CTAs at lag 3, past one wave. With windows of at most 200 frames the last window starts from
     a state adapted over 200 frames, far from reset(): a segment that continued from it instead of warming up from reset()
     would not match."""
-    d = work_dir / f"seg{seg_frames}_{warmup}"
-    out = run_worker("segments", lag, d, dict(segment_frames=seg_frames, warmup=warmup, max_window=max_window), timeout=900)
-    soft = np.load(d / "soft.npy", mmap_mode="r")
+    with S.forced_lag(lag):
+        out = segment_outputs(ctx, seg_frames, warmup, max_window)
+    soft = out["soft"]
     rounds = out["rounds"]
     assert (rounds[:, 0] == 1).all() and rounds[:, 1].sum() == int(out["n_frames"]) == N_LONG, rounds  # no replayed window
     windows = [int(n) for n in rounds[:, 1]]

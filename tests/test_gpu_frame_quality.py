@@ -15,24 +15,18 @@ and precision of the host's quality_from_state, so:
   oracle and its per-carrier form on the GPU (DESIGN.md section 8, row D4): equal up to float rounding, not bit for bit;
 * field 5 is replayed on the host from the frames' cyclic-prefix phases: bit for bit the float recurrence below.
 
-The CPU tests pin the oracle's records themselves. Forced demapper lags and traced segment layouts run in fresh processes
-(frame_quality_worker.py).
+The CPU tests pin the oracle's records themselves. Forced demapper lags and traced segment layouts use demap_support.
 """
 from __future__ import annotations
 
 import ctypes
-import os
-import subprocess
-import sys
-from collections import Counter
 
 import numpy as np
 import pytest
 
-import demap_worker as W
-import frame_quality_worker as FW
+import demap_support as S
 from dabstar_b200 import api, synth
-from test_gpu_demap_shapes import N_LONG, engine_segments
+from demap_support import N_LONG, engine_segments
 
 T_U, T_S, T_N = 2048, 2552, 2656
 LEAD = 60000
@@ -331,100 +325,96 @@ def test_cut_windows(ctx):
         assert np.array_equal(small.frame_quality(r).view(np.uint32), big.frame_quality(r).view(np.uint32)), r
 
 
-def run_worker(mode, lag, out_dir, inputs=None, timeout=900):
-    """frame_quality_worker.py MODE in a fresh process with DABSTAR_DEMAP_LAG = lag (None: the launcher's choice)."""
-    os.makedirs(out_dir, exist_ok=True)
-    if inputs is not None:
-        np.savez(os.path.join(out_dir, "in.npz"), **inputs)
-    env = dict(os.environ, DABSTAR_TRACE="1")
-    env.pop("DABSTAR_DEMAP_LAG", None)
-    if lag is not None:
-        env["DABSTAR_DEMAP_LAG"] = str(lag)
-    flags = (["-s"] if sys.flags.no_user_site else []) + (["-E"] if sys.flags.ignore_environment else [])
-    r = subprocess.run([sys.executable] + flags + [FW.__file__, mode, str(out_dir), str(out_dir)], env=env, capture_output=True,
-                       text=True, timeout=timeout)
-    assert r.returncode == 0, f"worker {mode} lag {lag} exited {r.returncode}:\n{r.stderr[-4000:]}"
-    return dict(np.load(os.path.join(out_dir, "out.npz")))
+def quality_records(dp, r: int, n_max: int) -> np.ndarray:
+    """frame_quality of recording r padded with NaN to n_max rows."""
+    q = dp.frame_quality(r)
+    out = np.full((n_max, 6), np.nan, np.float32)
+    out[:q.shape[0]] = q
+    return out
+
+
+def batch_quality(ctx) -> dict:
+    """Records of the 256 copies of the batch sources in one DabProcessor (traced), then of every source decoded alone."""
+    srcs = [S.batch_source(i)[0] for i in range(S.N_SRC)]
+    dp, rounds, dev = S.decode_batch(ctx, srcs, 0, trace=True, frame_quality=True)
+    out = dict(rounds=rounds,
+               n_frames=np.array([dp.n_frames(r) for r in range(S.N_COPIES)], np.int64),
+               quality=np.stack([quality_records(dp, r, S.F_MAX) for r in range(S.N_COPIES)]))
+    del dp, dev
+    single_n, single_q = [], []
+    for i in range(S.N_SRC):
+        dp1 = gpu(ctx, [srcs[i]])
+        single_n.append(dp1.n_frames(0))
+        single_q.append(quality_records(dp1, 0, S.F_MAX))
+    out["single_n_frames"] = np.array(single_n, np.int64)
+    out["single_quality"] = np.stack(single_q)
+    return out
 
 
 @pytest.mark.gpu
-def test_batch_every_lag_bit_identical(oracle, tmp_path):
+def test_batch_every_lag_bit_identical(ctx, oracle):
     """256 recordings (768 demapper CTAs, past one wave at every lag), every one ending inside a cut frame: at lag 3 / 7 / 15
     every copy's records equal its source decoded alone and the other lags' bit for bit, and the oracle chain's."""
-    outs = {lag: run_worker("batch", lag, tmp_path / f"lag{lag}") for lag in LAGS}
+    outs = {}
+    for lag in LAGS:
+        with S.forced_lag(lag):
+            outs[lag] = batch_quality(ctx)
     ref = outs[LAGS[0]]
     n = ref["single_n_frames"]
-    assert (n == W.N_FULL).all()
+    assert (n == S.N_FULL).all()
     for lag, o in outs.items():
-        assert o["rounds"][0, 0] == W.N_COPIES
-        assert np.array_equal(o["n_frames"], np.tile(n, W.N_COPIES // W.N_SRC)), lag
+        assert o["rounds"][0, 0] == S.N_COPIES
+        assert np.array_equal(o["n_frames"], np.tile(n, S.N_COPIES // S.N_SRC)), lag
         q = o["quality"].view(np.uint32)
-        for c in range(W.N_COPIES):
-            assert np.array_equal(q[c], o["single_quality"][c % W.N_SRC].view(np.uint32)), (lag, c)
+        for c in range(S.N_COPIES):
+            assert np.array_equal(q[c], o["single_quality"][c % S.N_SRC].view(np.uint32)), (lag, c)
         assert np.array_equal(o["single_quality"].view(np.uint32), ref["single_quality"].view(np.uint32)), lag
-    for i in range(0, W.N_SRC, 4):
-        r = chain(oracle, W.batch_source(i)[0])
-        assert r.n_frames == W.N_FULL
-        check_records(ref["single_quality"][i, :W.N_FULL], chain_records(oracle, r), f"source {i}")
+    for i in range(0, S.N_SRC, 4):
+        r = chain(oracle, S.batch_source(i)[0])
+        assert r.n_frames == S.N_FULL
+        check_records(ref["single_quality"][i, :S.N_FULL], chain_records(oracle, r), f"source {i}")
         r.close()
 
 
 # ------------------------------------------------------------------------------------------------ GPU: segments, streaming, TII
 @pytest.fixture(scope="module")
 def long_chain(oracle):
-    r = oracle.chain_run(oracle.to_cf32(W.segment_recording()), scan_mode=1, tap_fft=True)
+    r = oracle.chain_run(oracle.to_cf32(S.segment_recording()), scan_mode=1, tap_fft=True)
     assert r.n_frames == N_LONG
     yield r
     r.close()
 
 
 def replay_quality(oracle, r, segments):
-    """Records of the kept frames of `segments` (as test_gpu_demap_shapes.replay: (first, last, warmup, parent)), from the
+    """Records of the kept frames of `segments` (demap_support.replay_segments: (first, last, warmup, parent)), from the
     chain's FFT rows and clock errors; field 5 from the chain's CP phases."""
     out = {}
-
-    def run(h, seg, keep):
-        first, last, warmup, _ = seg
-        for f in range(first, last + 1):
-            x = r.fft(f)
-            oracle.ofdm_store_reference(h, x[0])
-            for s in range(1, 76):
-                oracle.ofdm_decode_symbol(h, x[s], s, 0.0, float(r.info[f].clock_err))
-            oracle.ofdm_store_null(h, x[76])
-            if keep and f >= first + warmup:
-                out[f] = oracle_quality(oracle, h)
-
-    def state_after(j):
-        p = segments[j][3]
-        h = oracle.ofdm_new(0) if p < 0 else state_after(p)
-        run(h, segments[j], False)
-        return h
-
-    children = Counter(s[3] for s in segments if s[3] >= 0)
-    kept = {}
-    for i, seg in enumerate(segments):
-        p = seg[3]
-        if p < 0:
-            h = oracle.ofdm_new(0)
-        else:
-            children[p] -= 1
-            h = kept.pop(p) if children[p] == 0 else state_after(p)
-        run(h, seg, True)
-        if children[i] > 0:
-            kept[i] = h
-        else:
-            oracle.ofdm_free(h)
+    S.replay_segments(oracle, r.fft, [i.clock_err for i in r.info], segments, 0,
+                      lambda f, h, soft: out.__setitem__(f, oracle_quality(oracle, h)))
     q = np.stack([out[f] for f in range(len(out))])
     q[:, 5] = sigma_replay([i.phase_cp for i in r.info])
     return q
 
 
+def segment_quality(ctx, seg_frames, warmup, max_window) -> dict:
+    """DabProcessor with set_segmentation and set_frame_quality over segment_recording() (traced)."""
+    dp = api.DabProcessor(1, input_format=api.FMT_U8, scan_mode=True, max_window=max_window, ctx=ctx)
+    dp.set_segmentation(seg_frames, warmup)
+    dp.set_frame_quality(True)
+    rounds = S.traced(lambda: dp.run([S.segment_recording()]))
+    res = dp.result(0)
+    return dict(rounds=rounds, warmup_frames=dp.warmup_frames(0), quality=dp.frame_quality(0),
+                pos=np.array([(i.sym0_pos, i.start_index) for i in res.info], np.int64).reshape(-1, 2),
+                phase_cp=np.array([i.phase_cp for i in res.info], np.float32))
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("seg_frames,warmup,lag,max_window", [(48, 4, 15, 200), (48, 18, 15, 200), (2, 4, 3, 512)])
-def test_segmented_records_match_replay(oracle, long_chain, tmp_path, seg_frames, warmup, lag, max_window):
+def test_segmented_records_match_replay(ctx, oracle, long_chain, seg_frames, warmup, lag, max_window):
     """set_segmentation over 400 frames: every record against the oracle replaying the engine's own segment layout (segments
     that warm up from reset() carry that state, as their soft bits do). (2, 4) is ~600 CTAs at lag 3, past one wave."""
-    out = run_worker("segments", lag, tmp_path, dict(segment_frames=seg_frames, warmup=warmup, max_window=max_window))
+    with S.forced_lag(lag):
+        out = segment_quality(ctx, seg_frames, warmup, max_window)
     rounds = out["rounds"]
     assert (rounds[:, 0] == 1).all() and rounds[:, 1].sum() == N_LONG, rounds
     segs, total_w = engine_segments([int(n) for n in rounds[:, 1]], seg_frames, warmup)
