@@ -59,6 +59,22 @@ class Mp2FrameC(ctypes.Structure):
                 ("crc_stored", ctypes.c_int32), ("crc_computed", ctypes.c_int32)]
 
 
+class DataGroupC(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_int32) for n in ("first_frame", "last_frame", "n_packets", "status", "extension_flag", "crc_flag", "segment_flag",
+                                              "user_access_flag", "type", "continuity", "repetition", "extension", "segment_last", "segment_number",
+                                              "transport_id", "length_indicator", "crc_stored", "crc_computed", "length", "data_start", "data_length",
+                                              "reserved")] + [("offset", ctypes.c_int64)]
+
+
+class PacketStatsC(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_int64) for n in ("packets", "crc_errors", "bad_length", "cut", "padding", "command", "other_address", "continuity_breaks",
+                                              "abandoned", "dropped")] + [("groups", ctypes.c_int64 * 5)]
+
+
+class PacketCompC(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_int32) for n in ("scid", "sub_ch_id", "packet_address", "dscty", "dg_flag", "ca_org")]
+
+
 class EnsembleInfoC(ctypes.Structure):
     _fields_ = [(n, ctypes.c_int32) for n in ("eid", "change_flags", "alarm", "cif_count_hi", "cif_count_lo", "n_subch", "n_components", "restarts")]
 
@@ -109,6 +125,9 @@ EXPORTS = [
     ("dabstar_decoder_dabplus_windows", ctypes.c_int),
     ("dabstar_mp2_frames", ctypes.c_int), ("dabstar_decoder_set_mp2", ctypes.c_int), ("dabstar_decoder_mp2_frames", ctypes.c_int),
     ("dabstar_decoder_mp2_payload", ctypes.c_int64), ("dabstar_decoder_mp2_ms", ctypes.c_double),
+    ("dabstar_packet_groups", ctypes.c_int), ("dabstar_fib_parser_packet_components", ctypes.c_int), ("dabstar_decoder_set_packet", ctypes.c_int),
+    ("dabstar_decoder_data_groups", ctypes.c_int), ("dabstar_decoder_data_group_payload", ctypes.c_int64), ("dabstar_decoder_packet_stats", ctypes.c_int),
+    ("dabstar_decoder_packet_ms", ctypes.c_double), ("dabstar_decoder_packet_components", ctypes.c_int),
 ]
 
 _lib = None

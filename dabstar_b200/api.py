@@ -123,6 +123,55 @@ class Mp2Processor:
                 o += n
 
 
+DG_OK, DG_NO_CRC, DG_CRC_ERROR, DG_MALFORMED, DG_RAW = 0, 1, 2, 3, 4
+
+
+class PacketProcessor:
+    """Packet-mode data groups of one address of a run of logical frames of one packet-mode sub-channel: packets parsed and
+    CRC-checked, data groups assembled and (DG flag 0) their MSC data group headers and CRCs checked on the GPU
+    (include/dabstar_b200.h, dabstar_packet_groups). MOT, EPG and the other data-service decoders stay CPU consumers of the groups."""
+
+    def __init__(self, bit_rate: int, address: int, ctx: "Context | None" = None, dg_flag: int = 0):
+        self.ctx = ctx or default_context()
+        self.bit_rate = int(bit_rate)
+        self.address = int(address)
+        self.dg_flag = int(dg_flag)
+
+    def add_frames(self, frame_bits: np.ndarray):
+        """frame_bits: uint8[n_frames, 24*bit_rate] (one bit per byte). Returns (records, payload uint8[bytes]): one record per data
+        group, and the groups' bytes concatenated in record order."""
+        b = _np(frame_bits, np.uint8).reshape(-1, 24 * self.bit_rate)
+        n = b.shape[0]
+        cap = max(n * (self.bit_rate // 8), 1)
+        rec = (_lib.DataGroupC * cap)()
+        pay = np.zeros(max(n * 3 * self.bit_rate, 1), np.uint8)
+        m = self.ctx.check(self.ctx.lib.dabstar_packet_groups(self.ctx.h, _ptr(b), self.bit_rate, n, self.address, self.dg_flag, rec, cap, _ptr(pay), MEM_HOST),
+                           "dabstar_packet_groups")
+        recs = list(rec[:m])
+        return recs, pay[:sum(r.length for r in recs)]
+
+    @staticmethod
+    def groups(records, payload: np.ndarray):
+        """Yields (record, group bytes, data field bytes)."""
+        for r in records:
+            g = payload[r.offset:r.offset + r.length].tobytes()
+            yield r, g, g[r.data_start:r.data_start + r.data_length]
+
+
+@dataclass
+class PacketComponent:
+    scid: int
+    sub_ch_id: int
+    packet_address: int
+    dscty: int
+    dg_flag: int
+    ca_org: int
+
+
+def _packet_components(arr, n) -> list[PacketComponent]:
+    return [PacketComponent(a.scid, a.sub_ch_id, a.packet_address, a.dscty, a.dg_flag, a.ca_org) for a in arr[:n]]
+
+
 @dataclass
 class ServiceComponent:
     sid: int
@@ -135,7 +184,8 @@ class ServiceComponent:
 
 
 class FibParser:
-    """FibDecoder::process_FIB for FIG 0/0, 0/1, 0/2 (fib_decoder.cpp:59-106, fib_decoder_fig0.cpp:89-290): host code, no device."""
+    """FibDecoder::process_FIB for FIG 0/0, 0/1, 0/2 (fib_decoder.cpp:59-106, fib_decoder_fig0.cpp:89-290), and FIG 0/3 from ETSI EN 300 401
+    clause 6.3.2: host code, no device."""
 
     def __init__(self):
         self.lib = _lib.load()
@@ -178,6 +228,13 @@ class FibParser:
         arr = (_lib.ServiceCompC * max(n, 1))()
         self.lib.dabstar_fib_parser_components(self.h, arr, n)
         return [ServiceComponent(a.sid, a.comp_index, a.tmid, a.type, a.sub_ch_id, a.primary, a.ca_flag) for a in arr[:n]]
+
+    def packet_components(self) -> list[PacketComponent]:
+        """FIG 0/3: where each packet-mode component (SCId) is carried, in order of first appearance."""
+        n = self.lib.dabstar_fib_parser_packet_components(self.h, None, 0)
+        arr = (_lib.PacketCompC * max(n, 1))()
+        self.lib.dabstar_fib_parser_packet_components(self.h, arr, n)
+        return _packet_components(arr, n)
 
 
 class Context:
@@ -688,6 +745,45 @@ class DabProcessor:
     def mp2_ms(self) -> float:
         """Device milliseconds of the last run's MP2 pass."""
         return float(self.ctx.lib.dabstar_decoder_mp2_ms(self.h))
+
+    def set_packet(self, recording: int, sub_ch_id: int = -1, address: int = 0, enable: bool = True):
+        """Packet-mode data groups of (sub-channel, address): the next runs parse the sub-channel's packets and assemble the address's
+        data groups on the device (see data_groups()). sub_ch_id -1: every packet-mode component the recording's own FIG 0/2 and
+        FIG 0/3 describe, with their addresses and DG flags (needs set_auto_config; address ignored). An explicit selection takes
+        its DG flag from the run's own FIG 0/3 when self-configured, else 0 (MSC data groups)."""
+        self.ctx.check(self.ctx.lib.dabstar_decoder_set_packet(self.h, recording, int(sub_ch_id), int(address), int(enable)), "dabstar_decoder_set_packet")
+
+    def data_groups(self, recording: int, sub_ch_id: int, address: int):
+        """(records, payload uint8[bytes]) of the last run's data groups of the stream, as PacketProcessor.add_frames returns them
+        for the sub-channel's logical frames; PacketProcessor.groups cuts the payload into the groups."""
+        lib = self.ctx.lib
+        n = self.ctx.check(lib.dabstar_decoder_data_groups(self.h, recording, int(sub_ch_id), int(address), None, 0), "dabstar_decoder_data_groups")
+        rec = (_lib.DataGroupC * max(n, 1))()
+        lib.dabstar_decoder_data_groups(self.h, recording, int(sub_ch_id), int(address), rec, n)
+        size = int(self.ctx.check(lib.dabstar_decoder_data_group_payload(self.h, recording, int(sub_ch_id), int(address), None, ctypes.c_int64(0)),
+                                  "dabstar_decoder_data_group_payload"))
+        pay = np.zeros(max(size, 1), np.uint8)
+        if size:
+            lib.dabstar_decoder_data_group_payload(self.h, recording, int(sub_ch_id), int(address), _ptr(pay), ctypes.c_int64(size))
+        return list(rec[:n]), pay[:size]
+
+    def packet_stats(self, recording: int, sub_ch_id: int, address: int) -> _lib.PacketStatsC:
+        """Counters of the stream in the last run: packets by class, padding, command and other-address packets, continuity breaks,
+        abandoned groups, dropped packets and groups by status."""
+        st = _lib.PacketStatsC()
+        self.ctx.check(self.ctx.lib.dabstar_decoder_packet_stats(self.h, recording, int(sub_ch_id), int(address), ctypes.byref(st)), "dabstar_decoder_packet_stats")
+        return st
+
+    def packet_ms(self) -> float:
+        """Device milliseconds of the last run's packet pass."""
+        return float(self.ctx.lib.dabstar_decoder_packet_ms(self.h))
+
+    def packet_components(self, recording: int) -> list[PacketComponent]:
+        """FIG 0/3 packet-mode components of a self-configured recording as the FIB parser holds them after the last run()."""
+        n = self.ctx.check(self.ctx.lib.dabstar_decoder_packet_components(self.h, recording, None, 0), "dabstar_decoder_packet_components")
+        arr = (_lib.PacketCompC * max(n, 1))()
+        self.ctx.lib.dabstar_decoder_packet_components(self.h, recording, arr, n)
+        return _packet_components(arr, n)
 
     def start_eti_generator(self, recording: int, cif_count_hi: int = 0, cif_count_lo: int = 0):
         """DabProcessor::start_eti_generator (dab_processor.cpp:529-546): the next run also produces the ETI(NI) stream of

@@ -94,6 +94,28 @@ struct Mp2Pass
   }
 };
 
+// Packet-mode data groups over a table of sub-channels and (sub-channel, address) streams (run_packet): device work buffers, and
+// the result in pinned host memory
+struct PacketPass
+{
+  std::vector<dab::PacketSub> subs;       // the caller sets src (device, packed frames), bit_rate and n_frames
+  std::vector<dab::PacketStream> streams; // ... and sub, address and dg_flag
+  // results of the last run_packet: per stream its counters, records and group bytes, in stream order
+  std::vector<dab::PacketCount> n_out;
+  const dab::DgRec * rec = nullptr;       // sum(n_out.groups) records (stream i's from streams[i].out_rec0) ...
+  const uint8_t * payload = nullptr;      // ... and the groups' bytes (stream i's at streams[i].out_pay0)
+  long long slots = 0;                    // packet slots parsed
+  double ms = 0;                          // device time of the pass
+  DevBuf d_subs, d_streams, d_slots, d_stage, d_cnt, d_out;
+  HostBuf h_cnt, h_out;
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  ~PacketPass()
+  {
+    if (ev0) cudaEventDestroy(ev0);
+    if (ev1) cudaEventDestroy(ev1);
+  }
+};
+
 struct dabstar_ctx
 {
   int device = 0;
@@ -116,6 +138,7 @@ struct dabstar_ctx
   DevBuf d_gf, d_fc_syn; // DAB+ outer code: GF(2^8) / Fire code tables (built on first use)
   DabplusPass dabplus;   // dabstar_dabplus_decode's pass
   Mp2Pass mp2;           // dabstar_mp2_frames's pass
+  PacketPass packet;     // dabstar_packet_groups's pass
   HostBuf arena;        // pinned staging of small uploads; reused after every stream synchronisation
   size_t arena_off = 0;
   std::unique_ptr<dab::HostPool> pool; // host threads of the per-recording control loops (created by the first decoder run)
@@ -192,6 +215,28 @@ inline dabstar_mp2_frame mp2_public(const dab::Mp2Rec & r)
 {
   dabstar_mp2_frame o;
   o.first_frame = r.first_frame; o.n_frames = r.n_frames; o.status = r.status; o.header = r.header; o.crc_stored = r.crc_stored; o.crc_computed = r.crc_computed;
+  return o;
+}
+
+// The data groups of every stream of p.streams, on the device (packet_kernels.cu): parse every logical frame's packets once per
+// sub-channel, walk each stream (one read-back of the per-stream counters), then compact the records and group bytes in stream
+// order and copy them to p.h_out. Runs on `s`.
+int run_packet(dabstar_ctx * ctx, cudaStream_t s, PacketPass & p);
+inline dabstar_data_group data_group_public(const dab::DgRec & r)
+{
+  static_assert(sizeof(dab::DgRec) == sizeof(dabstar_data_group), "DgRec mirrors dabstar_data_group");
+  dabstar_data_group o;
+  memcpy(&o, &r, sizeof o);
+  return o;
+}
+// the counters of a stream; the groups by status are counted from its n records
+inline dabstar_packet_stats packet_stats_public(const dab::PacketCount & c, const dab::DgRec * rec, long long n)
+{
+  dabstar_packet_stats o{};
+  o.packets = c.packets; o.crc_errors = c.crc_errors; o.bad_length = c.bad_length; o.cut = c.cut; o.padding = c.padding; o.command = c.command;
+  o.other_address = c.other_address; o.continuity_breaks = c.continuity_breaks; o.abandoned = c.abandoned; o.dropped = c.dropped;
+  for (long long i = 0; i < n; i++)
+    if (rec[i].status >= 0 && rec[i].status < 5) o.groups[rec[i].status]++;
   return o;
 }
 

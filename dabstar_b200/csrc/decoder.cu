@@ -53,6 +53,10 @@ struct Recording
     std::vector<int> mp2_ids; // sub-channels whose logical frames go through the MPEG layer II frame check (dabstar_decoder_set_mp2)
     bool mp2_all = false;     // ... and every sub-channel the recording's own FIG 0/2 lists as MPEG layer II
     bool mp2() const { return mp2_all || !mp2_ids.empty(); }
+    struct PacketSel { int sub_ch_id, address; };
+    std::vector<PacketSel> packet_sel; // (sub-channel, address) streams whose data groups are assembled (dabstar_decoder_set_packet)
+    bool packet_all = false;           // ... and every packet-mode component the recording's own FIG 0/2 and 0/3 describe
+    bool packet() const { return packet_all || !packet_sel.empty(); }
   } cfg;
   // input
   const void * d_iq = nullptr;
@@ -96,6 +100,10 @@ struct Recording
   // an audio-decoded sub-channel: its n records from rec0 and pay_bytes bytes from pay0 in the pass's result (dec->dabplus / dec->mp2)
   struct AudioOut { int sub_ch_id, bit_rate, n; long long rec0, pay0, pay_bytes; };
   std::vector<AudioOut> dabplus_out, mp2_out;
+  std::vector<dabstar_packet_comp> pcomps; // auto_cfg: FIG 0/3 packet-mode components as the FIB parser holds them after the run
+  // a packet-decoded stream: its n records from rec0 and pay_bytes bytes from pay0 in dec->packet's result, and its counters
+  struct PacketOut { int sub_ch_id, address, dg_flag, n; long long rec0, pay0, pay_bytes; dabstar_packet_stats stats; };
+  std::vector<PacketOut> packet_out;
   long long cnt_good_fibs = 0, cnt_sync_ok = 0, cnt_sync_fail = 0, cnt_windows = 0, cnt_cut = 0, cnt_heavy = 0, cnt_warmup = 0;
   // window scratch
   int w_first_desc = 0;
@@ -234,6 +242,7 @@ struct dabstar_decoder
   size_t ev_used = 0;
   DabplusPass dabplus; // the DAB+ outer code of the last run (Recording::dabplus_out)
   Mp2Pass mp2;         // the MPEG layer II frames of the last run (Recording::mp2_out)
+  PacketPass packet;   // the packet-mode data groups of the last run (Recording::packet_out)
   double stage_ms[10] = { 0 };   // [8], [9]: the MSC pass split into its gather and trellis kernels (VitSpanHook)
   long long stage_launches[10] = { 0 };
   cudaEvent_t ev_get()
@@ -395,6 +404,37 @@ extern "C" int dabstar_decoder_set_dabplus(dabstar_decoder * dec, int recording,
 extern "C" int dabstar_decoder_set_mp2(dabstar_decoder * dec, int recording, int sub_ch_id, int enable)
 {
   return set_audio(dec, recording, sub_ch_id, enable, AUDIO_MP2);
+}
+extern "C" int dabstar_decoder_set_packet(dabstar_decoder * dec, int recording, int sub_ch_id, int address, int enable)
+{
+  if (!dec || recording < 0 || recording >= (int)dec->recs.size()) return DABSTAR_E_INVALID;
+  dabstar_ctx * ctx = dec->ctx;
+  Recording::Cfg & c = dec->recs[recording].cfg;
+  if (sub_ch_id < -1 || sub_ch_id > 63) return ctx->fail(DABSTAR_E_INVALID, "packet mode: sub-channel id %d", sub_ch_id);
+  if (sub_ch_id >= 0 && (address < 1 || address > 1023)) return ctx->fail(DABSTAR_E_INVALID, "packet mode: address %d is not 1..1023", address);
+  if (enable && dec->streaming) return ctx->fail(DABSTAR_E_UNSUPPORTED, "packet-mode data groups across stream chunks are not supported");
+  auto same = [&](const Recording::Cfg::PacketSel & x) { return x.sub_ch_id == sub_ch_id && x.address == address; };
+  if (!enable)
+  {
+    if (sub_ch_id == -1) c.packet_all = false;
+    else c.packet_sel.erase(std::remove_if(c.packet_sel.begin(), c.packet_sel.end(), same), c.packet_sel.end());
+    return 0;
+  }
+  if (sub_ch_id == -1)
+  {
+    if (!c.auto_cfg) return ctx->fail(DABSTAR_E_INVALID, "packet mode: sub-channel -1 (the recording's own FIG 0/2 and 0/3) needs self-configuration");
+    c.packet_all = true;
+    return 0;
+  }
+  if (!c.auto_cfg) // with self-configuration the sub-channel is looked up in the run's FIC
+  {
+    const MscOut * m = nullptr;
+    for (const MscOut & x : c.msc) if (x.sc.sub_ch_id == sub_ch_id) m = &x;
+    if (!m) return ctx->fail(DABSTAR_E_INVALID, "packet mode: recording %d has no sub-channel %d", recording, sub_ch_id);
+    if (m->sc.bit_rate < 8 || m->sc.bit_rate % 8) return ctx->fail(DABSTAR_E_INVALID, "packet mode: sub-channel %d has %d kbit/s, not a multiple of 8", sub_ch_id, m->sc.bit_rate);
+  }
+  if (std::find_if(c.packet_sel.begin(), c.packet_sel.end(), same) == c.packet_sel.end()) c.packet_sel.push_back({ sub_ch_id, address });
+  return 0;
 }
 extern "C" int dabstar_decoder_enable_eti(dabstar_decoder * dec, int recording, int enable, int cif_count_hi, int cif_count_lo)
 {
@@ -741,6 +781,8 @@ struct Run
       const dabstar_decoder::Resume & rs = dec->resume[r];
       if ((dec->streaming || rs.on) && (R.cfg.dabplus() || R.cfg.mp2()))
         return ctx->fail(DABSTAR_E_UNSUPPORTED, "recording %d: DAB+ super-frames / MPEG audio frames across stream chunks are not supported", r);
+      if ((dec->streaming || rs.on) && R.cfg.packet())
+        return ctx->fail(DABSTAR_E_UNSUPPORTED, "recording %d: packet-mode data groups across stream chunks are not supported", r);
       if (rs.on)
       {
         if (R.cfg.eti_on || R.cfg.auto_cfg || R.cfg.tii.on) return ctx->fail(DABSTAR_E_UNSUPPORTED, "stream continuation with ETI / self-configuration / TII is not supported");
@@ -1451,6 +1493,8 @@ struct Run
       for (int f = n_f; f <= R.n_slots; f++) { R.cif_hi_f[f] = f > 0 ? R.cif_hi_f[f - 1] : -1; R.cif_lo_f[f] = f > 0 ? R.cif_lo_f[f - 1] : -1; }
       R.comps.resize((size_t)std::max(0, dabstar_fib_parser_components(fp, nullptr, 0)));
       dabstar_fib_parser_components(fp, R.comps.data(), (int)R.comps.size());
+      R.pcomps.resize((size_t)std::max(0, dabstar_fib_parser_packet_components(fp, nullptr, 0)));
+      dabstar_fib_parser_packet_components(fp, R.pcomps.data(), (int)R.pcomps.size());
       dabstar_fib_parser_destroy(fp);
     }
     return sync_profiles(ctx);
@@ -1763,6 +1807,64 @@ struct Run
 };
 } // namespace
 
+// ---- packet mode: the data groups of every selected (sub-channel, address) stream on the same packed MSC payload (run_packet).
+// Each selected sub-channel's packets are parsed once; first_frame / last_frame count its logical frames as msc_copy lists them.
+static int packet_phase(dabstar_decoder * dec)
+{
+  dabstar_ctx * ctx = dec->ctx;
+  PacketPass & pp = dec->packet;
+  pp.subs.clear();
+  pp.streams.clear();
+  std::vector<std::pair<int, int>> owner; // (recording, sub-channel) of every stream
+  for (int r = 0; r < (int)dec->recs.size(); r++)
+  {
+    Recording & R = dec->recs[r];
+    R.packet_out.clear();
+    if (!R.cfg.packet()) continue;
+    for (const MscOut & m : R.cfg.msc)
+    {
+      const int id = m.sc.sub_ch_id, br = m.sc.bit_rate;
+      if (br < 8 || br % 8) continue;
+      // the (address, DG flag) pairs chosen on this sub-channel: explicit ones (DG flag from the run's FIG 0/3 when it lists the
+      // pair, else 0), then the FIG 0/2 TMId 3 components FIG 0/3 puts here
+      std::vector<std::pair<int, int>> sel;
+      auto fig03 = [&](int address) {
+        for (const dabstar_packet_comp & p : R.pcomps) if (p.sub_ch_id == id && p.packet_address == address) return p.dg_flag;
+        return 0;
+      };
+      auto add = [&](int address, int dg) {
+        for (const auto & x : sel) if (x.first == address) return;
+        sel.push_back({ address, dg });
+      };
+      for (const Recording::Cfg::PacketSel & x : R.cfg.packet_sel)
+        if (x.sub_ch_id == id) add(x.address, R.cfg.auto_cfg ? fig03(x.address) : 0);
+      if (R.cfg.packet_all && R.cfg.auto_cfg)
+        for (const dabstar_service_comp & c : R.comps)
+          if (c.tmid == 3)
+            for (const dabstar_packet_comp & p : R.pcomps)
+              if (p.scid == c.type && p.sub_ch_id == id && p.packet_address >= 1) add(p.packet_address, p.dg_flag);
+      if (sel.empty()) continue;
+      const int sub = (int)pp.subs.size();
+      pp.subs.push_back(PacketSub{ dec->d_mscpacked.as<uint8_t>() + m.out_off / 8, br, (int)(m.out_len / (24 * br)), 0, 0 });
+      for (const auto & x : sel)
+      {
+        pp.streams.push_back(PacketStream{ sub, x.first, x.second, 0, 0, 0 });
+        owner.push_back({ r, id });
+      }
+    }
+  }
+  if (pp.streams.empty()) return 0;
+  if (int e = run_packet(ctx, ctx->stream, pp)) return e;
+  for (size_t i = 0; i < pp.streams.size(); i++)
+  {
+    const PacketStream & st = pp.streams[i];
+    const PacketCount & c = pp.n_out[i];
+    dec->recs[owner[i].first].packet_out.push_back({ owner[i].second, st.address, st.dg_flag, (int)c.groups, st.out_rec0, st.out_pay0, c.bytes,
+                             packet_stats_public(c, pp.rec + st.out_rec0, c.groups) });
+  }
+  return 0;
+}
+
 // ---- audio: the outer code behind every selected sub-channel's Backend, on the packed MSC payload the MSC pass left on the
 // device, one stream per recording and sub-channel and kind: DAB+ super-frames (Mp4Processor, mp4processor.cpp:95-334;
 // run_dabplus) and MPEG layer II frames (run_mp2). A sub-channel may be selected for both; the passes read the same payload.
@@ -1819,7 +1921,7 @@ static int audio_phase(dabstar_decoder * dec)
                                                               mp.n_out[i].bytes });
     }
   }
-  return 0;
+  return packet_phase(dec);
 }
 // With self-configuration level 2 the recordings may be decoded again (dabstar_decoder_run): the audio phase then runs once, after the final pass.
 static bool audio_after_passes(const dabstar_decoder * dec)
@@ -1879,12 +1981,14 @@ static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, cons
 extern "C" int dabstar_decoder_run(dabstar_decoder * dec, const void * const * iq, const int64_t * n_samples, int mem)
 {
   if (!dec || !iq || !n_samples) return DABSTAR_E_INVALID;
-  for (auto & R : dec->recs) { R.cfg.tii_flags.clear(); R.dabplus_out.clear(); R.mp2_out.clear(); }
+  for (auto & R : dec->recs) { R.cfg.tii_flags.clear(); R.dabplus_out.clear(); R.mp2_out.clear(); R.packet_out.clear(); }
   dec->dabplus.ms = 0;
   dec->dabplus.rounds = 0;
   dec->dabplus.scanned = dec->dabplus.decoded = 0;
   dec->mp2.ms = 0;
   dec->mp2.slots = 0;
+  dec->packet.ms = 0;
+  dec->packet.slots = 0;
   int rc = decoder_run_pass(dec, iq, n_samples, mem);
   double total_ms = dec->last_ms;
   for (int pass = 1; rc == 0 && pass <= 3; pass++)
@@ -1912,7 +2016,7 @@ extern "C" int dabstar_decoder_run(dabstar_decoder * dec, const void * const * i
   if (rc == 0 && !dec->cfg.scan_mode && audio_after_passes(dec))
   {
     rc = audio_phase(dec);
-    total_ms += dec->dabplus.ms + dec->mp2.ms;
+    total_ms += dec->dabplus.ms + dec->mp2.ms + dec->packet.ms;
   }
   dec->last_ms = total_ms;
   return rc;
@@ -2045,6 +2149,50 @@ extern "C" int64_t dabstar_decoder_mp2_payload(const dabstar_decoder * dec, int 
 extern "C" double dabstar_decoder_mp2_ms(const dabstar_decoder * dec)
 {
   return dec ? dec->mp2.ms : 0.0;
+}
+static const Recording::PacketOut * find_packet(const dabstar_decoder * dec, int recording, int sub_ch_id, int address)
+{
+  if (!dec || recording < 0 || recording >= (int)dec->recs.size()) return nullptr;
+  for (const auto & d : dec->recs[recording].packet_out) if (d.sub_ch_id == sub_ch_id && d.address == address) return &d;
+  return nullptr;
+}
+extern "C" int dabstar_decoder_data_groups(const dabstar_decoder * dec, int recording, int sub_ch_id, int address, dabstar_data_group * out, int cap)
+{
+  if (!dec || cap < 0 || (!out && cap > 0)) return DABSTAR_E_INVALID;
+  const Recording::PacketOut * d = find_packet(dec, recording, sub_ch_id, address);
+  if (!d) return dec->ctx->fail(DABSTAR_E_INVALID, "data_groups: recording %d sub-channel %d address %d was not packet-decoded in the last run", recording, sub_ch_id, address);
+  for (int i = 0; i < d->n && i < cap; i++) out[i] = data_group_public(dec->packet.rec[d->rec0 + i]);
+  return d->n;
+}
+extern "C" int64_t dabstar_decoder_data_group_payload(const dabstar_decoder * dec, int recording, int sub_ch_id, int address, uint8_t * out, int64_t cap)
+{
+  if (!dec || cap < 0) return DABSTAR_E_INVALID;
+  const Recording::PacketOut * d = find_packet(dec, recording, sub_ch_id, address);
+  if (!d) return dec->ctx->fail(DABSTAR_E_INVALID, "data_group_payload: recording %d sub-channel %d address %d was not packet-decoded in the last run", recording, sub_ch_id, address);
+  if (!out) return d->pay_bytes;
+  const int64_t n = std::min(cap, (int64_t)d->pay_bytes);
+  if (n > 0) memcpy(out, dec->packet.payload + d->pay0, (size_t)n);
+  return n;
+}
+extern "C" int dabstar_decoder_packet_stats(const dabstar_decoder * dec, int recording, int sub_ch_id, int address, dabstar_packet_stats * out)
+{
+  if (!dec || !out) return DABSTAR_E_INVALID;
+  const Recording::PacketOut * d = find_packet(dec, recording, sub_ch_id, address);
+  if (!d) return dec->ctx->fail(DABSTAR_E_INVALID, "packet_stats: recording %d sub-channel %d address %d was not packet-decoded in the last run", recording, sub_ch_id, address);
+  *out = d->stats;
+  return 0;
+}
+extern "C" double dabstar_decoder_packet_ms(const dabstar_decoder * dec)
+{
+  return dec ? dec->packet.ms : 0.0;
+}
+extern "C" int dabstar_decoder_packet_components(const dabstar_decoder * dec, int recording, dabstar_packet_comp * out, int cap)
+{
+  if (!dec || recording < 0 || recording >= (int)dec->recs.size() || cap < 0 || (!out && cap > 0)) return DABSTAR_E_INVALID;
+  const Recording & R = dec->recs[recording];
+  if (!R.cfg.auto_cfg) return dec->ctx->fail(DABSTAR_E_INVALID, "packet_components: recording %d is not self-configured", recording);
+  for (int i = 0; i < (int)R.pcomps.size() && i < cap; i++) out[i] = R.pcomps[i];
+  return (int)R.pcomps.size();
 }
 extern "C" int dabstar_decoder_dabplus_windows(const dabstar_decoder * dec, int64_t out[2])
 {

@@ -726,6 +726,107 @@ extern "C" int dabstar_mp2_frames(dabstar_ctx * ctx, const uint8_t * frame_bits,
   return n_out;
 }
 
+// ------------------------------------------------------------------------------------------------ packet-mode data groups
+int run_packet(dabstar_ctx * ctx, cudaStream_t s, PacketPass & p)
+{
+  if (!p.ev0) { CK(cudaEventCreate(&p.ev0)); CK(cudaEventCreate(&p.ev1)); }
+  const int nsub = (int)p.subs.size(), ns = (int)p.streams.size();
+  long long n_frames = 0, n_slots = 0, n_stage = 0;
+  for (PacketSub & sb : p.subs)
+  {
+    sb.frame0 = n_frames;
+    sb.slot0 = n_slots;
+    n_frames += sb.n_frames;
+    n_slots += (long long)sb.n_frames * (sb.bit_rate / 8);
+  }
+  for (PacketStream & st : p.streams)
+  {
+    const PacketSub & sb = p.subs[(size_t)st.sub];
+    st.stage0 = n_stage;
+    n_stage += (long long)sb.n_frames * (sb.bit_rate / 8); // a stream has at most one group per packet slot
+  }
+  p.n_out.assign((size_t)ns, PacketCount{});
+  p.slots = n_slots;
+  p.ms = 0;
+  p.rec = nullptr;
+  p.payload = nullptr;
+  if (n_slots == 0 || ns == 0) return 0;
+  CK(cudaEventRecord(p.ev0, s));
+  CK(p.d_subs.reserve(sizeof(PacketSub) * (size_t)nsub));
+  CK(p.d_streams.reserve(sizeof(PacketStream) * (size_t)ns));
+  CK(p.d_slots.reserve(sizeof(PacketSlot) * (size_t)n_slots));
+  CK(p.d_stage.reserve(sizeof(PacketStage) * (size_t)n_stage));
+  CK(p.d_cnt.reserve(sizeof(PacketCount) * (size_t)ns));
+  CK(p.h_cnt.reserve(sizeof(PacketCount) * (size_t)ns));
+  PacketSub * d_sub = p.d_subs.as<PacketSub>();
+  PacketStream * d_st = p.d_streams.as<PacketStream>();
+  CK(cudaMemcpyAsync(d_sub, p.subs.data(), sizeof(PacketSub) * (size_t)nsub, cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(d_st, p.streams.data(), sizeof(PacketStream) * (size_t)ns, cudaMemcpyHostToDevice, s));
+  CK(launch_packet_scan(s, d_sub, nsub, n_frames, p.d_slots.as<PacketSlot>(), &ctx->launches));
+  CK(launch_packet_walk(s, d_sub, d_st, ns, p.d_slots.as<PacketSlot>(), p.d_stage.as<PacketStage>(), p.d_cnt.as<PacketCount>(), &ctx->launches));
+  CK(cudaMemcpyAsync(p.h_cnt.p, p.d_cnt.p, sizeof(PacketCount) * (size_t)ns, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  const PacketCount * cnt = p.h_cnt.as<PacketCount>();
+  long long n_rec = 0, n_bytes = 0;
+  for (int i = 0; i < ns; i++)
+  {
+    PacketStream & st = p.streams[(size_t)i];
+    p.n_out[(size_t)i] = cnt[i];
+    st.out_rec0 = n_rec;
+    st.out_pay0 = n_bytes;
+    n_rec += cnt[i].groups;
+    n_bytes += cnt[i].bytes;
+  }
+  const size_t rec_bytes = sizeof(DgRec) * (size_t)n_rec, out_bytes = rec_bytes + (size_t)n_bytes;
+  CK(p.d_out.reserve(out_bytes));
+  CK(p.h_out.reserve(out_bytes));
+  CK(cudaMemcpyAsync(d_st, p.streams.data(), sizeof(PacketStream) * (size_t)ns, cudaMemcpyHostToDevice, s));
+  CK(launch_packet_compact(s, d_sub, d_st, ns, n_rec, p.d_slots.as<PacketSlot>(), p.d_stage.as<PacketStage>(), p.d_out.as<DgRec>(), p.d_out.as<uint8_t>() + rec_bytes,
+                           &ctx->launches));
+  if (out_bytes > 0) CK(cudaMemcpyAsync(p.h_out.p, p.d_out.p, out_bytes, cudaMemcpyDeviceToHost, s));
+  p.rec = p.h_out.as<DgRec>();
+  p.payload = p.h_out.as<uint8_t>() + rec_bytes;
+  CK(cudaEventRecord(p.ev1, s));
+  CK(cudaStreamSynchronize(s));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, p.ev0, p.ev1));
+  p.ms = ms;
+  return 0;
+}
+
+extern "C" int dabstar_packet_groups(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, int address, int dg_flag, dabstar_data_group * out,
+                                     int cap, uint8_t * payload, int mem)
+{
+  if (!ctx || (!frame_bits && n_frames > 0) || n_frames < 0 || cap < 0 || (cap > 0 && !out)) return DABSTAR_E_INVALID;
+  if (bit_rate < 8 || bit_rate % 8) return ctx->fail(DABSTAR_E_INVALID, "packet mode: bit rate %d is not a multiple of 8", bit_rate);
+  if (address < 1 || address > 1023) return ctx->fail(DABSTAR_E_INVALID, "packet mode: address %d is not 1..1023", address);
+  if (n_frames == 0) return 0;
+  CK(cudaSetDevice(ctx->device));
+  const size_t n_bits = (size_t)n_frames * 24 * bit_rate;
+  const void * dbits;
+  if (int r = stage_in(ctx, ctx->scratch[0], frame_bits, n_bits, mem, &dbits)) return r;
+  CK(ctx->scratch[1].reserve(n_bits / 8)); // packed frames
+  CK(launch_pack_bits(ctx->stream, (const uint8_t *)dbits, ctx->scratch[1].as<uint8_t>(), (long long)(n_bits / 8), &ctx->launches));
+  PacketPass & p = ctx->packet;
+  p.subs.assign(1, PacketSub{ ctx->scratch[1].as<uint8_t>(), bit_rate, n_frames, 0, 0 });
+  p.streams.assign(1, PacketStream{ 0, address, dg_flag ? 1 : 0, 0, 0, 0 });
+  if (int r = run_packet(ctx, ctx->stream, p)) return r;
+  ctx->arena_off = 0;
+  const int n_out = (int)p.n_out[0].groups, n_copy = std::min(n_out, cap);
+  size_t bytes = 0;
+  for (int i = 0; i < n_copy; i++)
+  {
+    out[i] = data_group_public(p.rec[i]);
+    bytes += (size_t)p.rec[i].length;
+  }
+  if (payload && bytes > 0)
+  {
+    if (mem == DABSTAR_MEM_HOST) memcpy(payload, p.payload, bytes);
+    else CK(cudaMemcpy(payload, p.payload, bytes, cudaMemcpyHostToDevice));
+  }
+  return n_out;
+}
+
 // ------------------------------------------------------------------------------------------------ stage taps
 extern "C" int dabstar_fft2048(dabstar_ctx * ctx, const float * in, float * out, int n, int sign, int mem)
 {

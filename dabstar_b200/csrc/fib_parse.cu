@@ -1,4 +1,4 @@
-// fib_parse.cu — host-side multiplex configuration parser: FIG 0/0, 0/1, 0/2 out of CRC-good FIBs.
+// fib_parse.cu — host-side multiplex configuration parser: FIG 0/0, 0/1, 0/2, 0/3 out of CRC-good FIBs.
 //
 // The minimal part of the reference's FibDecoder the decode path itself depends on (SURVEY.md section 8f.1):
 //   FibDecoder::process_FIB            decoder/fib_decoder.cpp:59-106       FIG walk inside one FIB
@@ -7,8 +7,10 @@
 //   FibDecoder::_subprocess_Fig0s2     decoder/fib_decoder_fig0.cpp:229-290 service -> sub-channel binding
 //   cProtLevelTable                    decoder/fib_table.h:51               EN 300 401 table 8 (short-form index)
 // It feeds MscHandler::set_channel (which sub-channels exist, where, how protected) and EtiGenerator (CIF counter,
-// sub-channel list). Labels, packet mode, announcements, the "next configuration" database and the GUI timers of the
-// reference's decoder are not part of it. Only the current configuration (C/N = 0) is collected.
+// sub-channel list). FIG 0/3 (EN 300 401 clause 6.3.2: where a packet-mode component is carried) is read from the standard; it
+// feeds the packet pass's self-configuration only and never restarts the parser. Labels, announcements, the "next
+// configuration" database and the GUI timers of the reference's decoder are not part of it. Only the current configuration
+// (C/N = 0) is collected.
 // Plain host C++ (no device code); lives in a .cu file so that the one nvcc command of build.py picks it up.
 #include "dabstar_b200.h"
 
@@ -55,10 +57,11 @@ struct dabstar_fib_parser
   bool have_ens = false;
   std::vector<dabstar_subch> subch;          // in order of first appearance (FibConfigFig0::Fig0s1_BasicSubChannelOrganizationVec)
   std::vector<dabstar_service_comp> comps;   // (SId, component index) in order of first appearance
+  std::vector<dabstar_packet_comp> pcomps;   // FIG 0/3, by SCId in order of first appearance
   int prev_change = 0;
   int restarts = 0;
 
-  void restart() { subch.clear(); comps.clear(); restarts++; }   // FibDecoder::_restart_fib_decoding: collected content is untrustworthy
+  void restart() { subch.clear(); comps.clear(); pcomps.clear(); restarts++; }   // FibDecoder::_restart_fib_decoding: collected content is untrustworthy
 
   // returns bytes used, -1 to abandon the FIB, or -2 to abandon this FIG: an entry that would cross the end of the FIG
   // (fig_bits = its length in bits) is not read - a CRC-good but malformed FIG must not make the parser read past the FIB
@@ -130,6 +133,26 @@ struct dabstar_fib_parser
     return o / 8;
   }
 
+  // FIG 0/3: SCId (12), Rfa (3), CAOrg flag, DG flag, Rfu, DSCTy (6), SubChId (6), packet address (10), CAOrg (16) if flagged
+  int fig0s3(const uint8_t * d, int off_bytes, int fig_bits)
+  {
+    const int o = off_bytes * 8;
+    if (o + 40 > fig_bits) return -2;
+    const int ca = (int)bits(d, o + 15, 1), len = ca ? 56 : 40;
+    if (o + len > fig_bits) return -2;
+    dabstar_packet_comp pc{};
+    pc.scid = (int)bits(d, o, 12);
+    pc.dg_flag = (int)bits(d, o + 16, 1);
+    pc.dscty = (int)bits(d, o + 18, 6);
+    pc.sub_ch_id = (int)bits(d, o + 24, 6);
+    pc.packet_address = (int)bits(d, o + 30, 10);
+    pc.ca_org = ca ? (int)bits(d, o + 40, 16) : -1;
+    bool known = false;
+    for (const dabstar_packet_comp & e : pcomps) if (e.scid == pc.scid) known = true;
+    if (!known) pcomps.push_back(pc);
+    return (o + len) / 8;
+  }
+
   void push(const uint8_t * fib) // 256 bits, one per byte; the caller has checked the CRC
   {
     int processed = 0;
@@ -151,6 +174,11 @@ struct dabstar_fib_parser
           ens.cif_count_lo = (int)bits(d, 40, 8);
           have_ens = true;
           prev_change = ens.change_flags;
+        }
+        else if (cn == 0 && ext == 3)
+        {
+          int used = 2;
+          while (used < len + 1 && (used = fig0s3(d, used, 8 * (len + 1))) >= 0) {}
         }
         else if (cn == 0 && (ext == 1 || ext == 2))
         {
@@ -205,4 +233,11 @@ extern "C" int dabstar_fib_parser_components(const dabstar_fib_parser * p, dabst
   const int n = (int)p->comps.size() < cap ? (int)p->comps.size() : cap;
   for (int i = 0; i < n; i++) out[i] = p->comps[i];
   return (int)p->comps.size();
+}
+extern "C" int dabstar_fib_parser_packet_components(const dabstar_fib_parser * p, dabstar_packet_comp * out, int cap)
+{
+  if (!p || (!out && cap > 0)) return DABSTAR_E_INVALID;
+  const int n = (int)p->pcomps.size() < cap ? (int)p->pcomps.size() : cap;
+  for (int i = 0; i < n; i++) out[i] = p->pcomps[i];
+  return (int)p->pcomps.size();
 }

@@ -3,6 +3,7 @@
 #include "common.cuh"
 #include "viterbi.cuh"
 #include "mp2.cuh"
+#include "packet.cuh"
 
 #include <vector>
 
@@ -167,6 +168,52 @@ cudaError_t launch_mp2_walk(cudaStream_t s, const Mp2Stream * st, int n_streams,
                             long long * stage_off, Mp2Count * cnt, unsigned long long * lc);
 cudaError_t launch_mp2_compact(cudaStream_t s, const Mp2Stream * st, int n_streams, long long n_out, const Mp2Rec * stage, const long long * stage_off,
                                Mp2Rec * out_rec, uint8_t * out_pay, unsigned long long * lc);
+
+// packet_kernels.cu: packet-mode data groups over a table of streams (packet.cuh). The packets of a sub-channel (one packet-mode
+// sub-channel of one recording) are parsed once; a stream is one address of one such sub-channel.
+struct PacketSub
+{
+  const uint8_t * src;     // n_frames logical frames of 3 * bit_rate packed bytes
+  int bit_rate, n_frames;
+  long long frame0;        // first of its logical frames in the pass's frame index space
+  long long slot0;         // first of its n_frames * bit_rate / 8 packet slots
+};
+struct PacketStream
+{
+  int sub, address, dg_flag;
+  long long stage0;        // first of its staged groups (room for one per slot of its sub-channel)
+  long long out_rec0;      // first output record (set from the walk's counts)
+  long long out_pay0;      // byte offset of its first group in the output payload
+};
+struct PacketCount         // per stream, from the walk
+{
+  long long groups, bytes; // groups emitted and their useful bytes
+  long long packets;       // CRC-good data packets with the stream's address
+  long long crc_errors, bad_length, cut; // packets of the sub-channel in those classes
+  long long padding, command, other_address, continuity_breaks, abandoned, dropped;
+};
+struct PacketStage         // a group found by the walk: its first and last packet slot of the sub-channel
+{
+  int start, end, n_packets, bytes;
+  long long off;           // byte offset inside the stream's payload
+};
+struct DgRec               // layout of dabstar_data_group
+{
+  int32_t first_frame, last_frame, n_packets, status;
+  int32_t extension_flag, crc_flag, segment_flag, user_access_flag;
+  int32_t type, continuity, repetition, extension;
+  int32_t segment_last, segment_number, transport_id, length_indicator;
+  int32_t crc_stored, crc_computed, length, data_start, data_length, reserved;
+  int64_t offset;
+};
+// every frame's packets: slots[sub.slot0 + frame * bit_rate / 8 + k] (packet.cuh: packet_frame)
+cudaError_t launch_packet_scan(cudaStream_t s, const PacketSub * sub, int n_subs, long long n_frames, PacketSlot * slots, unsigned long long * lc);
+// the walk of every stream (a block each): its groups at stage[stage0 ..] and its counters in cnt
+cudaError_t launch_packet_walk(cudaStream_t s, const PacketSub * sub, const PacketStream * st, int n_streams, const PacketSlot * slots, PacketStage * stage,
+                               PacketCount * cnt, unsigned long long * lc);
+// the groups' records and useful data, n_out of them, in stream order from out_rec0 / out_pay0; the MSC data group headers parsed
+cudaError_t launch_packet_compact(cudaStream_t s, const PacketSub * sub, const PacketStream * st, int n_streams, long long n_out, const PacketSlot * slots,
+                                  const PacketStage * stage, DgRec * out_rec, uint8_t * out_pay, unsigned long long * lc);
 
 // ofdm_kernels.cu
 cudaError_t launch_init_ref_arg(cudaStream_t s, const DeviceTables & t, unsigned long long * lc);

@@ -8,6 +8,7 @@
 // for one copy to the host (engine.cu: run_mp2).
 #include "kernels.h"
 #include "stream_search.cuh"
+#include "block_scan.cuh"
 
 namespace dab
 {
@@ -27,47 +28,10 @@ __global__ void __launch_bounds__(128) k_mp2_scan(const Mp2Stream * __restrict__
   hdr[g] = r.header;
 }
 
-// Block-wide exclusive scan of one value per thread (blockDim.x a multiple of 32): op(a, b) combines an earlier a with a later b;
-// *total (may be null) gets the combination of all values. sh: 32 entries of shared memory.
-__device__ inline unsigned shfl_up(unsigned v, int d) { return __shfl_up_sync(0xffffffffu, v, d); }
-__device__ inline Mp2Count shfl_up(Mp2Count v, int d) { return Mp2Count{ __shfl_up_sync(0xffffffffu, v.recs, d), __shfl_up_sync(0xffffffffu, v.bytes, d) }; }
-template <typename T, typename Op> __device__ T block_exclusive_scan(T v, T id, Op op, T * sh, T * total)
-{
-  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  T x = v;
-  for (int d = 1; d < 32; d <<= 1)
-  {
-    const T y = shfl_up(x, d);
-    if (lane >= d) x = op(y, x);
-  }
-  if (lane == 31) sh[w] = x;
-  __syncthreads();
-  if (w == 0)
-  {
-    T t = lane < nw ? sh[lane] : id;
-    for (int d = 1; d < 32; d <<= 1)
-    {
-      const T y = shfl_up(t, d);
-      if (lane >= d) t = op(y, t);
-    }
-    sh[lane] = t;
-  }
-  __syncthreads();
-  T before = shfl_up(x, 1);
-  if (lane == 0) before = id;
-  const T r = op(w > 0 ? sh[w - 1] : id, before);
-  if (total) *total = sh[nw - 1];
-  __syncthreads(); // sh is reused by the next scan
-  return r;
-}
-
-// The walk as a scan over 2-state maps. A slot is in state 0 (it starts a record) or 1 (it is the second half of an OK 24 kHz
-// frame); slot 0 is in state 0. A slot in state 1 hands state 0 to the next; one in state 0 hands on 1 exactly when
-// mp2_walk_step makes its record span two logical frames. A map of a run of slots holds in bit s the state after the run when
-// it is entered in state s; maps compose, so the entry state of every chunk of slots comes from a block-wide scan.
+// The walk as a scan over 2-state maps (block_scan.cuh). A slot is in state 0 (it starts a record) or 1 (it is the second half
+// of an OK 24 kHz frame); slot 0 is in state 0. A slot in state 1 hands state 0 to the next; one in state 0 hands on 1 exactly
+// when mp2_walk_step makes its record span two logical frames.
 constexpr int MP2_WALK_THREADS = 256;
-constexpr unsigned MAP_IDENTITY = 2u; // 0 -> 0, 1 -> 1
-__device__ inline unsigned map_then(unsigned a, unsigned b) { return ((b >> (a & 1u)) & 1u) | (((b >> ((a >> 1) & 1u)) & 1u) << 1); } // b after a
 __device__ inline unsigned next_state(const uint8_t * cls, int i, int n, unsigned state)
 {
   int status;

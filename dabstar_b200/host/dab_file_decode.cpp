@@ -16,6 +16,9 @@
 //     -m  all|id[,id...]: MPEG layer II audio frames of those sub-channels (all: what the recording's FIG 0/2 lists as MPEG layer
 //         II, needs -a), header- and CRC-checked on the GPU; prints per sub-channel the audio-frame slots per status; with -o,
 //         <prefix><n>.subch<id>.mp2 holds the OK frames (an MPEG audio elementary stream)
+//     -p  all|id:address[,id:address...]: packet-mode data groups of those (sub-channel, address) streams (all: every packet-mode
+//         component of the recording's FIG 0/2 and 0/3, needs -a), packets and groups checked on the GPU; prints per stream the
+//         packet and group counters; with -o, <prefix><n>.subch<id>.addr<address>.dg holds the groups' bytes in order
 //     -q  signal quality of every frame as CSV: frame,sym0_pos,mer_db,snr_db,noise_power,fbb_hz (fbb_hz: the baseband frequency
 //         correction of the frame's data symbols); with several files, file n's lines go to <path>.<n>
 //
@@ -48,7 +51,7 @@ int main(int argc, char ** argv)
   int fmt = DABSTAR_FMT_U8;
   bool autoCfg = false, eti = false, xml = false, containers = false, tii = false;
   dabstar_sample_format sf{};
-  std::string prefix = "dab_out_", qualPath, dabplus, mp2;
+  std::string prefix = "dab_out_", qualPath, dabplus, mp2, packet;
   bool prefixSet = false;
   std::vector<dabstar_subch> subch;
   std::vector<const char *> files;
@@ -59,6 +62,7 @@ int main(int argc, char ** argv)
     else if (a == "-o" && i + 1 < argc) { prefix = argv[++i]; prefixSet = true; }
     else if (a == "-d" && i + 1 < argc) dabplus = argv[++i];
     else if (a == "-m" && i + 1 < argc) mp2 = argv[++i];
+    else if (a == "-p" && i + 1 < argc) packet = argv[++i];
     else if (a == "-a") autoCfg = true;
     else if (a == "-t") tii = true;
     else if (a == "-c") { containers = true; fmt = DABSTAR_FMT_CF32; }
@@ -133,6 +137,21 @@ int main(int argc, char ** argv)
           }
       }
     }
+    std::vector<std::pair<int, int>> streams; // -p id:address list
+    for (size_t p = 0; packet != "all" && p < packet.size();)
+    {
+      const size_t q = std::min(packet.find(',', p), packet.size());
+      const std::string item = packet.substr(p, q - p);
+      const size_t c = item.find(':');
+      if (c == std::string::npos) throw std::runtime_error("-p: expected id:address, got " + item);
+      streams.push_back({ atoi(item.substr(0, c).c_str()), atoi(item.substr(c + 1).c_str()) });
+      p = q + 1;
+    }
+    for (size_t r = 0; r < files.size(); r++)
+    {
+      if (packet == "all") proc.set_packet((int)r, -1);
+      for (const auto & x : streams) proc.set_packet((int)r, x.first, x.second);
+    }
     if (!qualPath.empty()) proc.set_frame_quality(true);
     if (xml && !containers) proc.run_files(ptrs, ns, sf);
     else proc.run(ptrs, ns);
@@ -204,6 +223,27 @@ int main(int argc, char ** argv)
         for (const auto & x : fr) if (x.status >= 0 && x.status < 5) cnt[x.status]++;
         printf("%s: MP2 sub-channel %d: %zu slots, %ld ok, %ld no header, %ld mismatch, %ld CRC errors, %ld cut\n", files[r], s.sub_ch_id, fr.size(), cnt[0], cnt[1],
                cnt[2], cnt[3], cnt[4]);
+      }
+      std::vector<std::pair<int, int>> decoded = streams;
+      if (packet == "all")
+        for (const auto & c : proc.packet_components((int)r)) decoded.push_back({ c.sub_ch_id, c.packet_address });
+      for (size_t k = 0; k < decoded.size(); k++)
+      {
+        const int id = decoded[k].first, addr = decoded[k].second;
+        bool seen = false;
+        for (size_t j = 0; j < k; j++) seen = seen || decoded[j] == decoded[k];
+        if (seen || !proc.packet_decoded((int)r, id, addr)) continue;
+        FILE * df = prefixSet ? fopen((prefix + std::to_string(r) + ".subch" + std::to_string(id) + ".addr" + std::to_string(addr) + ".dg").c_str(), "wb") : nullptr;
+        const std::vector<dabstar_data_group> gr = proc.data_groups((int)r, id, addr, [&](const dabstar::u8 * g, int len, const dabstar_data_group &) {
+          if (df) fwrite(g, 1, (size_t)len, df);
+        });
+        if (df) fclose(df);
+        const dabstar_packet_stats st = proc.packet_stats((int)r, id, addr);
+        printf("%s: packet sub-channel %d address %d: %zu groups, %lld ok, %lld no CRC, %lld CRC errors, %lld malformed, %lld raw; %lld packets, %lld CRC errors, "
+               "%lld bad length, %lld cut, %lld padding, %lld command, %lld other address, %lld continuity breaks, %lld abandoned, %lld dropped\n",
+               files[r], id, addr, gr.size(), (long long)st.groups[0], (long long)st.groups[1], (long long)st.groups[2], (long long)st.groups[3], (long long)st.groups[4],
+               (long long)st.packets, (long long)st.crc_errors, (long long)st.bad_length, (long long)st.cut, (long long)st.padding, (long long)st.command,
+               (long long)st.other_address, (long long)st.continuity_breaks, (long long)st.abandoned, (long long)st.dropped);
       }
       if (autoCfg && tii)
         for (const auto & ev : proc.tii_events((int)r))

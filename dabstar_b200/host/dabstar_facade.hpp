@@ -216,6 +216,37 @@ private:
   long mSeen = 0;
 };
 
+// Packet-mode data groups of one address of one packet-mode sub-channel: packets CRC-checked, groups assembled and (DG flag 0)
+// their MSC data group headers and CRCs checked on the device (dabstar_packet_groups). Batch granular; MOT, EPG and the other
+// data-service decoders stay CPU consumers of the groups handed to the sink.
+class PacketProcessor
+{
+public:
+  using GroupSink = std::function<void(const u8 * group, int len, const dabstar_data_group & rec)>;
+  PacketProcessor(Context & c, int bitRate, int address, int dgFlag = 0, GroupSink sink = nullptr)
+    : mC(c), mBitRate(bitRate), mAddress(address), mDgFlag(dgFlag), mSink(std::move(sink)) {}
+  // iBits: nFrames x 24*bitRate bytes (one bit each). Returns one record per data group.
+  std::vector<dabstar_data_group> add_frames(const u8 * iBits, int nFrames)
+  {
+    std::vector<dabstar_data_group> rec((size_t)std::max(nFrames * (mBitRate / 8), 1));
+    std::vector<u8> pay((size_t)std::max(nFrames, 1) * 3 * (size_t)mBitRate);
+    const int n = mC.check(dabstar_packet_groups(mC.get(), iBits, mBitRate, nFrames, mAddress, mDgFlag, rec.data(), (int)rec.size(), pay.data(), DABSTAR_MEM_HOST),
+                           "dabstar_packet_groups");
+    rec.resize((size_t)n);
+    if (mSink) deliver(rec, pay.data(), mSink);
+    return rec;
+  }
+  static void deliver(const std::vector<dabstar_data_group> & rec, const u8 * payload, const GroupSink & sink)
+  {
+    for (const auto & r : rec) sink(payload + r.offset, r.length, r);
+  }
+
+private:
+  Context & mC;
+  int mBitRate, mAddress, mDgFlag;
+  GroupSink mSink;
+};
+
 // MPEG layer II audio frames of one DAB (MP2) sub-channel: header and CRC-16 of every audio-frame slot, on the device
 // (dabstar_mp2_frames). Batch granular; an MP2 decoder stays a CPU consumer of the OK frames handed to the sink.
 class Mp2Processor
@@ -481,6 +512,40 @@ public:
       Mp2Processor::deliver(rec, pay.data(), bitRate, sink);
     }
     return rec;
+  }
+  // packet-mode data groups of (sub-channel, address) in the next runs, on the device; subChId -1: every packet-mode component of
+  // the recording's own FIG 0/2 and 0/3 (needs set_auto_config; address ignored)
+  void set_packet(int recording, int subChId = -1, int address = 0, bool on = true)
+  {
+    mC.check(dabstar_decoder_set_packet(mDec, recording, subChId, address, on ? 1 : 0), "dabstar_decoder_set_packet");
+  }
+  bool packet_decoded(int recording, int subChId, int address) const { return dabstar_decoder_data_groups(mDec, recording, subChId, address, nullptr, 0) >= 0; }
+  // the last run's data groups of the stream; every group goes to sink, in order
+  std::vector<dabstar_data_group> data_groups(int recording, int subChId, int address, const PacketProcessor::GroupSink & sink = nullptr) const
+  {
+    const int n = mC.check(dabstar_decoder_data_groups(mDec, recording, subChId, address, nullptr, 0), "dabstar_decoder_data_groups");
+    std::vector<dabstar_data_group> rec((size_t)n);
+    if (n > 0) dabstar_decoder_data_groups(mDec, recording, subChId, address, rec.data(), n);
+    if (sink && n > 0)
+    {
+      std::vector<u8> pay((size_t)dabstar_decoder_data_group_payload(mDec, recording, subChId, address, nullptr, 0));
+      dabstar_decoder_data_group_payload(mDec, recording, subChId, address, pay.data(), (int64_t)pay.size());
+      PacketProcessor::deliver(rec, pay.data(), sink);
+    }
+    return rec;
+  }
+  dabstar_packet_stats packet_stats(int recording, int subChId, int address) const
+  {
+    dabstar_packet_stats st{};
+    mC.check(dabstar_decoder_packet_stats(mDec, recording, subChId, address, &st), "dabstar_decoder_packet_stats");
+    return st;
+  }
+  // FIG 0/3 packet-mode components of a self-configured recording after the last run
+  std::vector<dabstar_packet_comp> packet_components(int recording) const
+  {
+    std::vector<dabstar_packet_comp> v((size_t)mC.check(dabstar_decoder_packet_components(mDec, recording, nullptr, 0), "dabstar_decoder_packet_components"));
+    if (!v.empty()) dabstar_decoder_packet_components(mDec, recording, v.data(), (int)v.size());
+    return v;
   }
   // FIG 0/2 service components of a self-configured recording after the last run
   std::vector<dabstar_service_comp> components(int recording) const

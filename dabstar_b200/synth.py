@@ -39,7 +39,7 @@ class _Cfg(ctypes.Structure):
                 ("snr_db", ctypes.c_float), ("cfo_hz", ctypes.c_float), ("rms", ctypes.c_float),
                 ("lead_samples", ctypes.c_int32), ("tail_samples", ctypes.c_int32), ("n_subch", ctypes.c_int32),
                 ("subch", ctypes.c_void_p), ("fig_mode", ctypes.c_int32), ("eid", ctypes.c_int32), ("tii_main", ctypes.c_int32), ("tii_sub", ctypes.c_int32),
-                ("msc_payload", ctypes.c_void_p)]
+                ("msc_payload", ctypes.c_void_p), ("n_packet", ctypes.c_int32), ("packet", ctypes.c_void_p)]
 
 
 @dataclass
@@ -67,14 +67,18 @@ def _load():
 
 def generate(n_frames: int, seed: int = 1, snr_db: float = 20.0, cfo_hz: float = 0.0, subch: list[SubChannel] | None = None,
              fmt: int = FMT_U8, rms: float = 0.25, lead_samples: int = 60000, tail_samples: int = 4096, out: np.ndarray | None = None,
-             fig_mode: int = 0, eid: int = 0x1234, tii: tuple[int, int] | None = None, msc_payload: list | None = None) -> Recording:
+             fig_mode: int = 0, eid: int = 0x1234, tii: tuple[int, int] | None = None, msc_payload: list | None = None,
+             packet: list | None = None) -> Recording:
     """Synthesise `n_frames` Mode-I transmission frames. `lead_samples` of noise-like filler precede the first
     null symbol (the reference spends 40 960 samples on its level estimate before it searches the null).
     fig_mode 1: the FIC carries the ensemble's multiplex configuration (FIG 0/0 with a running CIF counter, FIG 0/1, FIG 0/2)
     instead of random FIB payloads. tii = (main id, sub id): with fig_mode 1 the null symbol after every frame whose CIF counter has
     (count & 7) >= 4 carries that transmitter identification.
     msc_payload: per sub-channel None (random bits) or the logical frames it carries, uint8[4 * n_frames, 24 * bit_rate] bits
-    (e.g. DAB+ super-frames from tests/helpers.dabplus_superframe); the other sub-channels draw what they draw without it."""
+    (e.g. DAB+ super-frames from tests/helpers.dabplus_superframe); the other sub-channels draw what they draw without it.
+    packet: with fig_mode 1, [(sub_ch_id, scid, address, dscty, dg_flag), ...]: each listed sub-channel carries no programme service;
+    each entry becomes a data service with one packet-mode (TMId 3) component in FIG 0/2 and a FIG 0/3 entry. Without it every
+    output is what it is without the argument."""
     lib = _load()
     subch = subch or []
     tab = subch_table(subch)
@@ -85,8 +89,9 @@ def generate(n_frames: int, seed: int = 1, snr_db: float = 20.0, cfo_hz: float =
         for p, s in zip(msc_payload, subch):
             keep.append(None if p is None else np.ascontiguousarray(p, np.uint8).reshape(4 * n_frames, 24 * s.bit_rate))
         pay = (ctypes.c_void_p * max(len(subch), 1))(*[None if k is None else k.ctypes.data for k in keep])
+    ptab = np.ascontiguousarray(np.array(packet or [], np.int32).reshape(-1, 5))
     cfg = _Cfg(n_frames, fmt, seed, snr_db, cfo_hz, rms, lead_samples, tail_samples, len(subch), tab.ctypes.data, fig_mode, eid, tii[0] if tii else -1, tii[1] if tii else -1,
-               ctypes.cast(pay, ctypes.c_void_p) if pay is not None else None)
+               ctypes.cast(pay, ctypes.c_void_p) if pay is not None else None, len(ptab), ptab.ctypes.data if len(ptab) else None)
     n = lib.dabsynth_num_samples(ctypes.byref(cfg))
     if out is None:
         out = np.empty(n, np.complex64) if fmt == FMT_CF32 else np.empty((n, 2), np.uint8 if fmt == FMT_U8 else np.int16)

@@ -41,6 +41,9 @@ typedef struct
   int32_t  tii_sub;       /*   (count & 7) >= 4 (EN 300 401 clause 14.8): main id 0..69 (pattern), sub id 0..23 (comb); -1: no TII */
   const uint8_t * const * msc_payload; /* NULL, or n_subch pointers: the logical frames sub-channel s carries, n_frames*4*24*bitRate bits
                                           (one per byte, transmit order), or NULL for random bits (drawn as if no payload were given) */
+  int32_t  n_packet;      /* fig_mode 1: packet-mode components (0: none, and the FIC is what it is without them) */
+  const int32_t * packet; /*   n_packet x 5: subChId, SCId, packet address, DSCTy, DG flag. A listed sub-channel carries no programme
+                               service; each entry becomes a data service with one TMId 3 component (FIG 0/2, P/D 1) and a FIG 0/3 entry */
 } dabsynth_cfg;
 
 /* ---------------------------------------------------------------------------------------------- rng */
@@ -351,14 +354,21 @@ static int build_mci(const dabsynth_cfg * c, int f, fic_writer * w)
       }
     }
   }
-  /* FIG 0/2: one programme service with one stream-audio component per sub-channel */
+  /* FIG 0/2: one programme service with one stream-audio component per sub-channel that carries no packet-mode component */
+  int prog[c->n_subch > 0 ? c->n_subch : 1], n_prog = 0;
+  for (int j = 0; j < c->n_subch; j++)
+  {
+    int packet = 0;
+    for (int e = 0; e < c->n_packet; e++) packet |= c->packet[5 * e] == c->subch[7 * j];
+    if (!packet) prog[n_prog++] = j;
+  }
   i = 0;
-  while (i < c->n_subch)
+  while (i < n_prog)
   {
     int room = 30 - w->used;
     if (room < 2 + 5) room = 30;
     int n = (room - 2) / 5;
-    if (n > c->n_subch - i) n = c->n_subch - i;
+    if (n > n_prog - i) n = n_prog - i;
     p = ficw_reserve(w, 2 + 5 * n);
     if (!p || n == 0) return -1;
     p[0] = (uint8_t)((0 << 5) | (1 + 5 * n));
@@ -366,13 +376,52 @@ static int build_mci(const dabsynth_cfg * c, int f, fic_writer * w)
     uint8_t * q = p + 2;
     for (int k = 0; k < n; k++, i++, q += 5)
     {
-      const int32_t * s = c->subch + 7 * i;
+      const int32_t * s = c->subch + 7 * prog[i];
       const int sid = 0xD000 + s[0];
       q[0] = (uint8_t)(sid >> 8); q[1] = (uint8_t)sid;
       q[2] = 1;                                         /* local flag 0, CAId 0, one component */
       const int ascty = s[3] ? 0 : 63;                  /* UEP: MPEG layer II, EEP: DAB+ */
       q[3] = (uint8_t)((0 << 6) | ascty);               /* TMId 0 (stream audio) */
       q[4] = (uint8_t)((s[0] << 2) | (1 << 1) | 0);     /* SubChId, primary, no CA */
+    }
+  }
+  /* FIG 0/2 (P/D 1): one data service with one packet-mode component (TMId 3) per packet entry; then FIG 0/3 (clause 6.3.2)
+     tells where each SCId is carried */
+  for (int part = 0; part < 2; part++)
+  {
+    const int size = part == 0 ? 7 : 5;
+    i = 0;
+    while (i < c->n_packet)
+    {
+      int room = 30 - w->used;
+      if (room < 2 + size) room = 30;
+      int n = (room - 2) / size;
+      if (n > c->n_packet - i) n = c->n_packet - i;
+      p = ficw_reserve(w, 2 + size * n);
+      if (!p || n == 0) return -1;
+      p[0] = (uint8_t)((0 << 5) | (1 + size * n));
+      p[1] = part == 0 ? (uint8_t)((1 << 5) | 2) : 3;   /* C/N 0, OE 0, P/D 1, extension 2 / P/D 0, extension 3 */
+      uint8_t * q = p + 2;
+      for (int k = 0; k < n; k++, i++, q += size)
+      {
+        const int32_t * e = c->packet + 5 * i;          /* subChId, SCId, address, DSCTy, DG flag */
+        if (part == 0)
+        {
+          const uint32_t sid = 0xE1D00000u | (uint32_t)(e[1] & 0xfff);
+          q[0] = (uint8_t)(sid >> 24); q[1] = (uint8_t)(sid >> 16); q[2] = (uint8_t)(sid >> 8); q[3] = (uint8_t)sid;
+          q[4] = 1;                                     /* local flag 0, CAId 0, one component */
+          q[5] = (uint8_t)((3 << 6) | ((e[1] >> 6) & 63)); /* TMId 3, SCId */
+          q[6] = (uint8_t)(((e[1] & 63) << 2) | (1 << 1) | 0); /* primary, no CA */
+        }
+        else
+        {
+          q[0] = (uint8_t)(e[1] >> 4);
+          q[1] = (uint8_t)((e[1] & 15) << 4);           /* Rfa 0, CAOrg flag 0 */
+          q[2] = (uint8_t)(((e[4] & 1) << 7) | (e[3] & 63)); /* DG flag, Rfu 0, DSCTy */
+          q[3] = (uint8_t)((e[0] << 2) | ((e[2] >> 8) & 3));
+          q[4] = (uint8_t)(e[2] & 0xff);
+        }
+      }
     }
   }
   ficw_finish(w);

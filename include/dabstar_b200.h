@@ -302,6 +302,55 @@ typedef struct
 int dabstar_mp2_frames(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, dabstar_mp2_frame * out, int cap,
                        uint8_t * payload, int mem);
 
+/* ------------------------------------------------------------------------------------------------ packet-mode data */
+/* The data groups of one address of a run of logical frames of one packet-mode sub-channel (TMId 3), on the device (ETSI EN 300 401
+ * clause 5.3.2 packets, 5.3.3 MSC data groups). Packets of 24, 48, 72 or 96 bytes (length in their first two bits) tile each
+ * logical frame of 3 * bit_rate bytes; each carries a 24-bit header (length, continuity index, first / last flags, 10-bit address,
+ * command flag, useful data length) and a CRC-16 over header and data field (x^16 + x^12 + x^5 + 1, preset 0xFFFF, complemented:
+ * the FIB CRC). A packet is OK, a CRC error, of bad length (useful data length > packet length - 5) or cut (it would run past the
+ * end of the logical frame; the rest of that frame is skipped). Address 0 is padding; command packets are counted, not assembled.
+ * The CRC-good data packets of the address are assembled in stream order: a packet continues the previous one when its
+ * continuity index is the previous one's plus 1 (mod 4); first opens a group (abandoning an open one), single is a group of its
+ * own, intermediate keeps an open group only if it continues it, last closes an open group it continues into a record. Any
+ * other packet abandons the open group or, without one, is dropped. With DG flag 0 the group is an MSC data group: its header,
+ * session header and CRC are parsed and checked (status below); with DG flag 1 it is a RAW record. Packet-mode FEC (FIG 0/14,
+ * RS(204,188)) is not applied: sub-channels that use it are decoded without the outer code. */
+enum { DABSTAR_DG_OK = 0, DABSTAR_DG_NO_CRC = 1, DABSTAR_DG_CRC_ERROR = 2, DABSTAR_DG_MALFORMED = 3, DABSTAR_DG_RAW = 4 };
+typedef struct
+{
+  int32_t first_frame, last_frame; /* logical frames of the group's first and last packet */
+  int32_t n_packets;
+  int32_t status;                  /* DABSTAR_DG_*: OK (CRC good), NO_CRC (CRC flag 0), CRC_ERROR, MALFORMED (headers do not fit), RAW */
+  int32_t extension_flag, crc_flag, segment_flag, user_access_flag; /* data group header; -1 for RAW / where not reached */
+  int32_t type, continuity, repetition;
+  int32_t extension;               /* extension field, -1 if absent */
+  int32_t segment_last, segment_number; /* segment field, -1 if absent */
+  int32_t transport_id, length_indicator; /* user access field, -1 if absent */
+  int32_t crc_stored, crc_computed;     /* data group CRC, -1 if absent */
+  int32_t length;                  /* bytes of the group (the useful data of its packets) */
+  int32_t data_start, data_length; /* data field inside the group (RAW: the whole group) */
+  int32_t reserved;
+  int64_t offset;                  /* first byte of the group in the stream's payload */
+} dabstar_data_group;
+/* frame_bits: n_frames x 24*bit_rate bytes, one bit each (dabstar_decoder_msc_copy); bit_rate a multiple of 8; address 1..1023.
+ * out: one record per data group, in stream order (at most cap are written); payload (may be NULL; room for n_frames * 3 *
+ * bit_rate bytes): the groups' bytes, concatenated in record order. Returns the number of records or <0. */
+int dabstar_packet_groups(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, int address, int dg_flag, dabstar_data_group * out,
+                          int cap, uint8_t * payload, int mem);
+/* per (sub-channel, address) counters of a run */
+typedef struct
+{
+  int64_t packets;            /* CRC-good data packets with the address */
+  int64_t crc_errors, bad_length, cut; /* packets of the sub-channel in these classes */
+  int64_t padding;            /* CRC-good packets with address 0 */
+  int64_t command;            /* CRC-good command packets with the address */
+  int64_t other_address;      /* CRC-good packets with another non-zero address */
+  int64_t continuity_breaks;  /* packets of the address that do not continue the previous one */
+  int64_t abandoned;          /* open groups given up */
+  int64_t dropped;            /* intermediate / last packets without an open group */
+  int64_t groups[5];          /* groups by status (DABSTAR_DG_*) */
+} dabstar_packet_stats;
+
 /* ------------------------------------------------------------------------------------------------ multiplex configuration (FIG 0/0, 0/1, 0/2) */
 /* The part of FibDecoder the decode path depends on (decoder/fib_decoder.cpp:59-106 process_FIB,
  * fib_decoder_fig0.cpp:89-113 FIG 0/0, :142-227 FIG 0/1, :229-290 FIG 0/2, fib_table.h:51 short-form table): which
@@ -333,6 +382,15 @@ int  dabstar_fib_parser_ensemble(const dabstar_fib_parser * p, dabstar_ensemble_
 /* sub-channels in order of first appearance (start_frame = 0); returns the total count */
 int  dabstar_fib_parser_subchannels(const dabstar_fib_parser * p, dabstar_subch * out, int cap);
 int  dabstar_fib_parser_components(const dabstar_fib_parser * p, dabstar_service_comp * out, int cap);
+/* FIG 0/3 (EN 300 401 clause 6.3.2): where a packet-mode component (SCId, the `type` of its FIG 0/2 TMId 3 entry) is carried.
+ * Current configuration only, in order of first appearance; an entry that would cross the end of its FIG is not read (the rest
+ * of that FIG is skipped). FIG 0/3 never restarts the parser and leaves the sub-channel and component lists alone. */
+typedef struct
+{
+  int32_t scid, sub_ch_id, packet_address, dscty, dg_flag;
+  int32_t ca_org; /* -1 if absent */
+} dabstar_packet_comp;
+int  dabstar_fib_parser_packet_components(const dabstar_fib_parser * p, dabstar_packet_comp * out, int cap);
 
 /* Cyclic-prefix correlation of DabProcessor::_process_ofdm_symbols_1_to_L (main/dab_processor.cpp:317-333): samples = n frames x
  * 75 x 2552 complex floats (data symbols 1..75 of a frame with their prefixes); out = n x (re, im) of
@@ -460,6 +518,26 @@ int     dabstar_decoder_mp2_frames(const dabstar_decoder * dec, int recording, i
 int64_t dabstar_decoder_mp2_payload(const dabstar_decoder * dec, int recording, int sub_ch_id, uint8_t * out, int64_t cap);
 /* device time of the last run's MP2 pass */
 double  dabstar_decoder_mp2_ms(const dabstar_decoder * dec);
+/* Packet-mode data groups inside the run (see dabstar_packet_groups) for the chosen (sub-channel, address) streams, on the device,
+ * on the run's own MSC payload; a sub-channel's packets are parsed once however many of its addresses are chosen. sub_ch_id -1:
+ * every packet-mode component of the recording's own FIC, that is every FIG 0/2 TMId 3 component whose SCId a FIG 0/3 entry
+ * resolves to a sub-channel, with that entry's packet address and DG flag (needs auto-config; `address` is ignored). An explicit
+ * id must name a sub-channel set with dabstar_decoder_set_subchannels whose bit rate is a multiple of 8 (with auto-config it is
+ * looked up in the run's own FIC), and address must be 1..1023. The DG flag of an explicit selection is the one the run's own
+ * FIG 0/3 gives that (sub-channel, address) with auto-config, and 0 (MSC data groups) otherwise. enable = 0 deselects it. scan_mode
+ * decodes no MSC and so no groups; streaming is not supported (DABSTAR_E_UNSUPPORTED: a data group can span two chunks). */
+int     dabstar_decoder_set_packet(dabstar_decoder * dec, int recording, int sub_ch_id, int address, int enable);
+/* records of the last run's data groups of one stream, exactly as dabstar_packet_groups returns them for dabstar_decoder_msc_copy's
+ * bits of that sub-channel; returns the count (E_INVALID: the stream was not packet-decoded in the last run) */
+int     dabstar_decoder_data_groups(const dabstar_decoder * dec, int recording, int sub_ch_id, int address, dabstar_data_group * out, int cap);
+/* their bytes in record order; returns bytes written (out NULL: the bytes there are) */
+int64_t dabstar_decoder_data_group_payload(const dabstar_decoder * dec, int recording, int sub_ch_id, int address, uint8_t * out, int64_t cap);
+int     dabstar_decoder_packet_stats(const dabstar_decoder * dec, int recording, int sub_ch_id, int address, dabstar_packet_stats * out);
+/* device time of the last run's packet pass */
+double  dabstar_decoder_packet_ms(const dabstar_decoder * dec);
+/* FIG 0/3 packet-mode components of a self-configured recording as the FIB parser holds them at the end of the run; returns the
+ * count (E_INVALID: not self-configured) */
+int     dabstar_decoder_packet_components(const dabstar_decoder * dec, int recording, dabstar_packet_comp * out, int cap);
 /* EtiGenerator (eti_handler/eti_generator.h:56-66: start_eti_generator before run / process_block per symbol): every
  * sub-channel set with dabstar_decoder_set_subchannels is decoded for every CIF through the generator's own whole-CIF
  * de-interleaver (first frame with its 17th CIF; its start-up bookkeeping, which loses the 16th CIF, is reproduced) and
