@@ -75,6 +75,15 @@ class PacketCompC(ctypes.Structure):
     _fields_ = [(n, ctypes.c_int32) for n in ("scid", "sub_ch_id", "packet_address", "dscty", "dg_flag", "ca_org")]
 
 
+class FecFrameC(ctypes.Structure):
+    _fields_ = [(n, ctypes.c_int32) for n in ("first_slot", "run_slot", "first_frame", "last_frame", "status", "rows_corrected", "rows_failed",
+                                              "bytes_corrected", "headers_matched", "reserved")]
+
+
+class FecSchemeC(ctypes.Structure):
+    _fields_ = [("sub_ch_id", ctypes.c_int32), ("scheme", ctypes.c_int32)]
+
+
 class EnsembleInfoC(ctypes.Structure):
     _fields_ = [(n, ctypes.c_int32) for n in ("eid", "change_flags", "alarm", "cif_count_hi", "cif_count_lo", "n_subch", "n_components", "restarts")]
 
@@ -128,6 +137,9 @@ EXPORTS = [
     ("dabstar_packet_groups", ctypes.c_int), ("dabstar_fib_parser_packet_components", ctypes.c_int), ("dabstar_decoder_set_packet", ctypes.c_int),
     ("dabstar_decoder_data_groups", ctypes.c_int), ("dabstar_decoder_data_group_payload", ctypes.c_int64), ("dabstar_decoder_packet_stats", ctypes.c_int),
     ("dabstar_decoder_packet_ms", ctypes.c_double), ("dabstar_decoder_packet_components", ctypes.c_int),
+    ("dabstar_packet_fec", ctypes.c_int), ("dabstar_packet_groups_fec", ctypes.c_int), ("dabstar_fib_parser_fec_schemes", ctypes.c_int),
+    ("dabstar_decoder_set_packet_fec", ctypes.c_int), ("dabstar_decoder_fec_frames", ctypes.c_int), ("dabstar_decoder_packet_fec_ms", ctypes.c_double),
+    ("dabstar_decoder_fec_schemes", ctypes.c_int),
 ]
 
 _lib = None

@@ -129,13 +129,18 @@ DG_OK, DG_NO_CRC, DG_CRC_ERROR, DG_MALFORMED, DG_RAW = 0, 1, 2, 3, 4
 class PacketProcessor:
     """Packet-mode data groups of one address of a run of logical frames of one packet-mode sub-channel: packets parsed and
     CRC-checked, data groups assembled and (DG flag 0) their MSC data group headers and CRCs checked on the GPU
-    (include/dabstar_b200.h, dabstar_packet_groups). MOT, EPG and the other data-service decoders stay CPU consumers of the groups."""
+    (include/dabstar_b200.h, dabstar_packet_groups). MOT, EPG and the other data-service decoders stay CPU consumers of the groups.
+    fec=True: the sub-channel carries packet-mode FEC (FIG 0/14 scheme 1); its FEC frames are corrected first and the FEC packets
+    skipped (dabstar_packet_groups_fec), and fec_frames / stats hold the last call's FEC frame records and counters."""
 
-    def __init__(self, bit_rate: int, address: int, ctx: "Context | None" = None, dg_flag: int = 0):
+    def __init__(self, bit_rate: int, address: int, ctx: "Context | None" = None, dg_flag: int = 0, fec: bool = False):
         self.ctx = ctx or default_context()
         self.bit_rate = int(bit_rate)
         self.address = int(address)
         self.dg_flag = int(dg_flag)
+        self.fec = bool(fec)
+        self.fec_frames: list = []
+        self.stats = None
 
     def add_frames(self, frame_bits: np.ndarray):
         """frame_bits: uint8[n_frames, 24*bit_rate] (one bit per byte). Returns (records, payload uint8[bytes]): one record per data
@@ -145,8 +150,18 @@ class PacketProcessor:
         cap = max(n * (self.bit_rate // 8), 1)
         rec = (_lib.DataGroupC * cap)()
         pay = np.zeros(max(n * 3 * self.bit_rate, 1), np.uint8)
-        m = self.ctx.check(self.ctx.lib.dabstar_packet_groups(self.ctx.h, _ptr(b), self.bit_rate, n, self.address, self.dg_flag, rec, cap, _ptr(pay), MEM_HOST),
-                           "dabstar_packet_groups")
+        if self.fec:
+            fcap = max(n * (self.bit_rate // 8) // 2 + 1, 1)
+            frames = (_lib.FecFrameC * fcap)()
+            st = _lib.PacketStatsC()
+            nf = ctypes.c_int(0)
+            m = self.ctx.check(self.ctx.lib.dabstar_packet_groups_fec(self.ctx.h, _ptr(b), self.bit_rate, n, self.address, self.dg_flag, rec, cap, _ptr(pay),
+                                                                      ctypes.byref(st), frames, fcap, ctypes.byref(nf), MEM_HOST), "dabstar_packet_groups_fec")
+            self.fec_frames = list(frames[:nf.value])
+            self.stats = st
+        else:
+            m = self.ctx.check(self.ctx.lib.dabstar_packet_groups(self.ctx.h, _ptr(b), self.bit_rate, n, self.address, self.dg_flag, rec, cap, _ptr(pay), MEM_HOST),
+                               "dabstar_packet_groups")
         recs = list(rec[:m])
         return recs, pay[:sum(r.length for r in recs)]
 
@@ -156,6 +171,32 @@ class PacketProcessor:
         for r in records:
             g = payload[r.offset:r.offset + r.length].tobytes()
             yield r, g, g[r.data_start:r.data_start + r.data_length]
+
+
+FEC_CLEAN, FEC_CORRECTED, FEC_PARTIAL, FEC_INCOMPLETE = 0, 1, 2, 3
+
+
+class PacketFec:
+    """Packet-mode FEC (EN 300 401 clause 5.3.5) of a run of logical frames of one packet-mode sub-channel, on the GPU
+    (include/dabstar_b200.h, dabstar_packet_fec): FEC frames located, their RS(204,188) rows corrected."""
+
+    def __init__(self, bit_rate: int, ctx: "Context | None" = None):
+        self.ctx = ctx or default_context()
+        self.bit_rate = int(bit_rate)
+
+    def correct(self, frame_bits: np.ndarray):
+        """frame_bits: uint8[n_frames, 24*bit_rate] (one bit per byte). Returns (corrected bits, same shape; FEC frame records)."""
+        b = _np(frame_bits, np.uint8).reshape(-1, 24 * self.bit_rate)
+        n = b.shape[0]
+        out = np.zeros_like(b)
+        cap = max(n * (self.bit_rate // 8) // 2 + 1, 1)
+        rec = (_lib.FecFrameC * cap)()
+        m = self.ctx.check(self.ctx.lib.dabstar_packet_fec(self.ctx.h, _ptr(b), self.bit_rate, n, _ptr(out), rec, cap, MEM_HOST), "dabstar_packet_fec")
+        return out, list(rec[:m])
+
+
+def _fec_schemes(arr, n) -> list[tuple[int, int]]:
+    return [(a.sub_ch_id, a.scheme) for a in arr[:n]]
 
 
 @dataclass
@@ -235,6 +276,13 @@ class FibParser:
         arr = (_lib.PacketCompC * max(n, 1))()
         self.lib.dabstar_fib_parser_packet_components(self.h, arr, n)
         return _packet_components(arr, n)
+
+    def fec_schemes(self) -> list[tuple[int, int]]:
+        """FIG 0/14: (sub_ch_id, FEC scheme) in order of first appearance (scheme 1: packet-mode FEC; 0, 2, 3: none)."""
+        n = self.lib.dabstar_fib_parser_fec_schemes(self.h, None, 0)
+        arr = (_lib.FecSchemeC * max(n, 1))()
+        self.lib.dabstar_fib_parser_fec_schemes(self.h, arr, n)
+        return _fec_schemes(arr, n)
 
 
 class Context:
@@ -784,6 +832,31 @@ class DabProcessor:
         arr = (_lib.PacketCompC * max(n, 1))()
         self.ctx.lib.dabstar_decoder_packet_components(self.h, recording, arr, n)
         return _packet_components(arr, n)
+
+    def set_packet_fec(self, recording: int, sub_ch_id: int = -1, enable: bool = True):
+        """Packet-mode FEC in front of the packet pass (off by default): sub_ch_id forces it on for that sub-channel; -1: every
+        sub-channel the recording's own FIG 0/14 gives scheme 1 (needs set_auto_config). Applies to sub-channels with a set_packet
+        stream."""
+        self.ctx.check(self.ctx.lib.dabstar_decoder_set_packet_fec(self.h, recording, int(sub_ch_id), int(enable)), "dabstar_decoder_set_packet_fec")
+
+    def fec_frames(self, recording: int, sub_ch_id: int) -> list:
+        """The FEC frame records of the sub-channel in the last run, as PacketFec.correct returns them for its logical frames."""
+        lib = self.ctx.lib
+        n = self.ctx.check(lib.dabstar_decoder_fec_frames(self.h, recording, int(sub_ch_id), None, 0), "dabstar_decoder_fec_frames")
+        arr = (_lib.FecFrameC * max(n, 1))()
+        lib.dabstar_decoder_fec_frames(self.h, recording, int(sub_ch_id), arr, n)
+        return list(arr[:n])
+
+    def packet_fec_ms(self) -> float:
+        """Device milliseconds of the last run's packet-mode FEC pass."""
+        return float(self.ctx.lib.dabstar_decoder_packet_fec_ms(self.h))
+
+    def fec_schemes(self, recording: int) -> list[tuple[int, int]]:
+        """FIG 0/14 (sub_ch_id, FEC scheme) pairs of a self-configured recording as the FIB parser holds them after the last run()."""
+        n = self.ctx.check(self.ctx.lib.dabstar_decoder_fec_schemes(self.h, recording, None, 0), "dabstar_decoder_fec_schemes")
+        arr = (_lib.FecSchemeC * max(n, 1))()
+        self.ctx.lib.dabstar_decoder_fec_schemes(self.h, recording, arr, n)
+        return _fec_schemes(arr, n)
 
     def start_eti_generator(self, recording: int, cif_count_hi: int = 0, cif_count_lo: int = 0):
         """DabProcessor::start_eti_generator (dab_processor.cpp:529-546): the next run also produces the ETI(NI) stream of

@@ -116,6 +116,29 @@ struct PacketPass
   }
 };
 
+// Packet-mode FEC over a table of streams (run_packet_fec): device work buffers, the corrected copies and the FEC mask the packet
+// pass reads, and the frame records in pinned host memory
+struct PfecPass
+{
+  std::vector<dab::PfecStream> streams; // the caller sets src (device, packed frames, all in one allocation), bit_rate and n_frames;
+                                        // the pass sets dst
+  // results of the last run_packet_fec: per stream its frame records, in stream order
+  std::vector<int> n_out;
+  const dab::PfecRec * rec = nullptr;   // sum(n_out) records (stream i's from streams[i].out0)
+  const uint8_t * mask = nullptr;       // device: one byte per slot (stream i's from streams[i].slot0), 1 on FEC packets
+  long long slots = 0;                  // 24-byte slots scanned
+  double ms = 0;                        // device time of the pass
+  std::vector<uint8_t> tables;          // GF(2^8) tables (pfec.cuh: PfecTables), uploaded once to d_tab
+  DevBuf d_streams, d_copy, d_code, d_start, d_mask, d_stage, d_cnt, d_rec, d_tab;
+  HostBuf h_cnt, h_rec;
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  ~PfecPass()
+  {
+    if (ev0) cudaEventDestroy(ev0);
+    if (ev1) cudaEventDestroy(ev1);
+  }
+};
+
 struct dabstar_ctx
 {
   int device = 0;
@@ -139,6 +162,7 @@ struct dabstar_ctx
   DabplusPass dabplus;   // dabstar_dabplus_decode's pass
   Mp2Pass mp2;           // dabstar_mp2_frames's pass
   PacketPass packet;     // dabstar_packet_groups's pass
+  PfecPass pfec;         // dabstar_packet_fec's and dabstar_packet_groups_fec's FEC pass
   HostBuf arena;        // pinned staging of small uploads; reused after every stream synchronisation
   size_t arena_off = 0;
   std::unique_ptr<dab::HostPool> pool; // host threads of the per-recording control loops (created by the first decoder run)
@@ -222,6 +246,18 @@ inline dabstar_mp2_frame mp2_public(const dab::Mp2Rec & r)
 // sub-channel, walk each stream (one read-back of the per-stream counters), then compact the records and group bytes in stream
 // order and copy them to p.h_out. Runs on `s`.
 int run_packet(dabstar_ctx * ctx, cudaStream_t s, PacketPass & p);
+// The FEC frames of every stream of p.streams, on the device (pfec_kernels.cu): copy the span of all streams' bytes to p.d_copy
+// (one cudaMemcpyAsync), locate the FEC-packet runs of every slot, list each stream's runs (one read-back of the per-stream counts), then
+// correct the rows of every complete frame in the copies and copy the records to p.h_rec. The packet pass then reads the copies
+// with p.mask (PacketSub::fec). Runs on `s`.
+int run_packet_fec(dabstar_ctx * ctx, cudaStream_t s, PfecPass & p);
+inline dabstar_fec_frame fec_frame_public(const dab::PfecRec & r)
+{
+  static_assert(sizeof(dab::PfecRec) == sizeof(dabstar_fec_frame), "PfecRec mirrors dabstar_fec_frame");
+  dabstar_fec_frame o;
+  memcpy(&o, &r, sizeof o);
+  return o;
+}
 inline dabstar_data_group data_group_public(const dab::DgRec & r)
 {
   static_assert(sizeof(dab::DgRec) == sizeof(dabstar_data_group), "DgRec mirrors dabstar_data_group");

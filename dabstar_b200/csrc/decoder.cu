@@ -57,6 +57,8 @@ struct Recording
     std::vector<PacketSel> packet_sel; // (sub-channel, address) streams whose data groups are assembled (dabstar_decoder_set_packet)
     bool packet_all = false;           // ... and every packet-mode component the recording's own FIG 0/2 and 0/3 describe
     bool packet() const { return packet_all || !packet_sel.empty(); }
+    std::vector<int> fec_ids; // sub-channels whose packets go through packet-mode FEC first (dabstar_decoder_set_packet_fec)
+    bool fec_all = false;     // ... and every sub-channel the recording's own FIG 0/14 gives scheme 1
   } cfg;
   // input
   const void * d_iq = nullptr;
@@ -104,6 +106,10 @@ struct Recording
   // a packet-decoded stream: its n records from rec0 and pay_bytes bytes from pay0 in dec->packet's result, and its counters
   struct PacketOut { int sub_ch_id, address, dg_flag, n; long long rec0, pay0, pay_bytes; dabstar_packet_stats stats; };
   std::vector<PacketOut> packet_out;
+  std::vector<dabstar_fec_scheme> fschemes; // auto_cfg: FIG 0/14 FEC schemes as the FIB parser holds them after the run
+  // a sub-channel through packet-mode FEC: its n frame records from rec0 in dec->pfec's result
+  struct FecOut { int sub_ch_id, n; long long rec0; };
+  std::vector<FecOut> fec_out;
   long long cnt_good_fibs = 0, cnt_sync_ok = 0, cnt_sync_fail = 0, cnt_windows = 0, cnt_cut = 0, cnt_heavy = 0, cnt_warmup = 0;
   // window scratch
   int w_first_desc = 0;
@@ -243,6 +249,7 @@ struct dabstar_decoder
   DabplusPass dabplus; // the DAB+ outer code of the last run (Recording::dabplus_out)
   Mp2Pass mp2;         // the MPEG layer II frames of the last run (Recording::mp2_out)
   PacketPass packet;   // the packet-mode data groups of the last run (Recording::packet_out)
+  PfecPass pfec;       // the packet-mode FEC frames of the last run (Recording::fec_out)
   double stage_ms[10] = { 0 };   // [8], [9]: the MSC pass split into its gather and trellis kernels (VitSpanHook)
   long long stage_launches[10] = { 0 };
   cudaEvent_t ev_get()
@@ -434,6 +441,35 @@ extern "C" int dabstar_decoder_set_packet(dabstar_decoder * dec, int recording, 
     if (m->sc.bit_rate < 8 || m->sc.bit_rate % 8) return ctx->fail(DABSTAR_E_INVALID, "packet mode: sub-channel %d has %d kbit/s, not a multiple of 8", sub_ch_id, m->sc.bit_rate);
   }
   if (std::find_if(c.packet_sel.begin(), c.packet_sel.end(), same) == c.packet_sel.end()) c.packet_sel.push_back({ sub_ch_id, address });
+  return 0;
+}
+extern "C" int dabstar_decoder_set_packet_fec(dabstar_decoder * dec, int recording, int sub_ch_id, int enable)
+{
+  if (!dec || recording < 0 || recording >= (int)dec->recs.size()) return DABSTAR_E_INVALID;
+  dabstar_ctx * ctx = dec->ctx;
+  Recording::Cfg & c = dec->recs[recording].cfg;
+  if (sub_ch_id < -1 || sub_ch_id > 63) return ctx->fail(DABSTAR_E_INVALID, "packet-mode FEC: sub-channel id %d", sub_ch_id);
+  if (enable && dec->streaming) return ctx->fail(DABSTAR_E_UNSUPPORTED, "packet-mode FEC across stream chunks is not supported");
+  if (!enable)
+  {
+    if (sub_ch_id == -1) c.fec_all = false;
+    else c.fec_ids.erase(std::remove(c.fec_ids.begin(), c.fec_ids.end(), sub_ch_id), c.fec_ids.end());
+    return 0;
+  }
+  if (sub_ch_id == -1)
+  {
+    if (!c.auto_cfg) return ctx->fail(DABSTAR_E_INVALID, "packet-mode FEC: sub-channel -1 (the recording's own FIG 0/14) needs self-configuration");
+    c.fec_all = true;
+    return 0;
+  }
+  if (!c.auto_cfg) // with self-configuration the sub-channel is looked up in the run's FIC
+  {
+    const MscOut * m = nullptr;
+    for (const MscOut & x : c.msc) if (x.sc.sub_ch_id == sub_ch_id) m = &x;
+    if (!m) return ctx->fail(DABSTAR_E_INVALID, "packet-mode FEC: recording %d has no sub-channel %d", recording, sub_ch_id);
+    if (m->sc.bit_rate < 8 || m->sc.bit_rate % 8) return ctx->fail(DABSTAR_E_INVALID, "packet-mode FEC: sub-channel %d has %d kbit/s, not a multiple of 8", sub_ch_id, m->sc.bit_rate);
+  }
+  if (std::find(c.fec_ids.begin(), c.fec_ids.end(), sub_ch_id) == c.fec_ids.end()) c.fec_ids.push_back(sub_ch_id);
   return 0;
 }
 extern "C" int dabstar_decoder_enable_eti(dabstar_decoder * dec, int recording, int enable, int cif_count_hi, int cif_count_lo)
@@ -1495,6 +1531,8 @@ struct Run
       dabstar_fib_parser_components(fp, R.comps.data(), (int)R.comps.size());
       R.pcomps.resize((size_t)std::max(0, dabstar_fib_parser_packet_components(fp, nullptr, 0)));
       dabstar_fib_parser_packet_components(fp, R.pcomps.data(), (int)R.pcomps.size());
+      R.fschemes.resize((size_t)std::max(0, dabstar_fib_parser_fec_schemes(fp, nullptr, 0)));
+      dabstar_fib_parser_fec_schemes(fp, R.fschemes.data(), (int)R.fschemes.size());
       dabstar_fib_parser_destroy(fp);
     }
     return sync_profiles(ctx);
@@ -1809,17 +1847,23 @@ struct Run
 
 // ---- packet mode: the data groups of every selected (sub-channel, address) stream on the same packed MSC payload (run_packet).
 // Each selected sub-channel's packets are parsed once; first_frame / last_frame count its logical frames as msc_copy lists them.
+// Sub-channels with packet-mode FEC go through run_packet_fec first; their packets are then parsed from the corrected copies.
 static int packet_phase(dabstar_decoder * dec)
 {
   dabstar_ctx * ctx = dec->ctx;
   PacketPass & pp = dec->packet;
+  PfecPass & pf = dec->pfec;
   pp.subs.clear();
   pp.streams.clear();
+  pf.streams.clear();
   std::vector<std::pair<int, int>> owner; // (recording, sub-channel) of every stream
+  std::vector<std::pair<int, int>> fec_owner; // (recording, sub-channel) of every FEC stream
+  std::vector<int> fec_sub;                   // ... and its index in pp.subs
   for (int r = 0; r < (int)dec->recs.size(); r++)
   {
     Recording & R = dec->recs[r];
     R.packet_out.clear();
+    R.fec_out.clear();
     if (!R.cfg.packet()) continue;
     for (const MscOut & m : R.cfg.msc)
     {
@@ -1846,6 +1890,15 @@ static int packet_phase(dabstar_decoder * dec)
       if (sel.empty()) continue;
       const int sub = (int)pp.subs.size();
       pp.subs.push_back(PacketSub{ dec->d_mscpacked.as<uint8_t>() + m.out_off / 8, br, (int)(m.out_len / (24 * br)), 0, 0 });
+      bool fec = std::find(R.cfg.fec_ids.begin(), R.cfg.fec_ids.end(), id) != R.cfg.fec_ids.end();
+      if (R.cfg.fec_all && R.cfg.auto_cfg)
+        for (const dabstar_fec_scheme & x : R.fschemes) fec = fec || (x.sub_ch_id == id && x.scheme == 1);
+      if (fec)
+      {
+        pf.streams.push_back(PfecStream{ pp.subs.back().src, nullptr, br, pp.subs.back().n_frames, 0, 0, 0 });
+        fec_owner.push_back({ r, id });
+        fec_sub.push_back(sub);
+      }
       for (const auto & x : sel)
       {
         pp.streams.push_back(PacketStream{ sub, x.first, x.second, 0, 0, 0 });
@@ -1854,6 +1907,17 @@ static int packet_phase(dabstar_decoder * dec)
     }
   }
   if (pp.streams.empty()) return 0;
+  if (!pf.streams.empty())
+  {
+    if (int e = run_packet_fec(ctx, ctx->stream, pf)) return e;
+    for (size_t i = 0; i < pf.streams.size(); i++)
+    {
+      PacketSub & sb = pp.subs[(size_t)fec_sub[i]];
+      sb.src = pf.streams[i].dst;
+      sb.fec = pf.mask + pf.streams[i].slot0;
+      dec->recs[fec_owner[i].first].fec_out.push_back({ fec_owner[i].second, pf.n_out[i], pf.streams[i].out0 });
+    }
+  }
   if (int e = run_packet(ctx, ctx->stream, pp)) return e;
   for (size_t i = 0; i < pp.streams.size(); i++)
   {
@@ -1981,7 +2045,7 @@ static int decoder_run_pass(dabstar_decoder * dec, const void * const * iq, cons
 extern "C" int dabstar_decoder_run(dabstar_decoder * dec, const void * const * iq, const int64_t * n_samples, int mem)
 {
   if (!dec || !iq || !n_samples) return DABSTAR_E_INVALID;
-  for (auto & R : dec->recs) { R.cfg.tii_flags.clear(); R.dabplus_out.clear(); R.mp2_out.clear(); R.packet_out.clear(); }
+  for (auto & R : dec->recs) { R.cfg.tii_flags.clear(); R.dabplus_out.clear(); R.mp2_out.clear(); R.packet_out.clear(); R.fec_out.clear(); }
   dec->dabplus.ms = 0;
   dec->dabplus.rounds = 0;
   dec->dabplus.scanned = dec->dabplus.decoded = 0;
@@ -1989,6 +2053,8 @@ extern "C" int dabstar_decoder_run(dabstar_decoder * dec, const void * const * i
   dec->mp2.slots = 0;
   dec->packet.ms = 0;
   dec->packet.slots = 0;
+  dec->pfec.ms = 0;
+  dec->pfec.slots = 0;
   int rc = decoder_run_pass(dec, iq, n_samples, mem);
   double total_ms = dec->last_ms;
   for (int pass = 1; rc == 0 && pass <= 3; pass++)
@@ -2016,7 +2082,7 @@ extern "C" int dabstar_decoder_run(dabstar_decoder * dec, const void * const * i
   if (rc == 0 && !dec->cfg.scan_mode && audio_after_passes(dec))
   {
     rc = audio_phase(dec);
-    total_ms += dec->dabplus.ms + dec->mp2.ms + dec->packet.ms;
+    total_ms += dec->dabplus.ms + dec->mp2.ms + dec->pfec.ms + dec->packet.ms;
   }
   dec->last_ms = total_ms;
   return rc;
@@ -2185,6 +2251,29 @@ extern "C" int dabstar_decoder_packet_stats(const dabstar_decoder * dec, int rec
 extern "C" double dabstar_decoder_packet_ms(const dabstar_decoder * dec)
 {
   return dec ? dec->packet.ms : 0.0;
+}
+extern "C" int dabstar_decoder_fec_frames(const dabstar_decoder * dec, int recording, int sub_ch_id, dabstar_fec_frame * out, int cap)
+{
+  if (!dec || cap < 0 || (!out && cap > 0) || recording < 0 || recording >= (int)dec->recs.size()) return DABSTAR_E_INVALID;
+  for (const auto & d : dec->recs[recording].fec_out)
+    if (d.sub_ch_id == sub_ch_id)
+    {
+      for (int i = 0; i < d.n && i < cap; i++) out[i] = fec_frame_public(dec->pfec.rec[d.rec0 + i]);
+      return d.n;
+    }
+  return dec->ctx->fail(DABSTAR_E_INVALID, "fec_frames: recording %d sub-channel %d had no FEC pass in the last run", recording, sub_ch_id);
+}
+extern "C" double dabstar_decoder_packet_fec_ms(const dabstar_decoder * dec)
+{
+  return dec ? dec->pfec.ms : 0.0;
+}
+extern "C" int dabstar_decoder_fec_schemes(const dabstar_decoder * dec, int recording, dabstar_fec_scheme * out, int cap)
+{
+  if (!dec || recording < 0 || recording >= (int)dec->recs.size() || cap < 0 || (!out && cap > 0)) return DABSTAR_E_INVALID;
+  const Recording & R = dec->recs[recording];
+  if (!R.cfg.auto_cfg) return dec->ctx->fail(DABSTAR_E_INVALID, "fec_schemes: recording %d is not self-configured", recording);
+  for (int i = 0; i < (int)R.fschemes.size() && i < cap; i++) out[i] = R.fschemes[i];
+  return (int)R.fschemes.size();
 }
 extern "C" int dabstar_decoder_packet_components(const dabstar_decoder * dec, int recording, dabstar_packet_comp * out, int cap)
 {

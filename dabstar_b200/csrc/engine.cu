@@ -794,21 +794,105 @@ int run_packet(dabstar_ctx * ctx, cudaStream_t s, PacketPass & p)
   return 0;
 }
 
-extern "C" int dabstar_packet_groups(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, int address, int dg_flag, dabstar_data_group * out,
-                                     int cap, uint8_t * payload, int mem)
+int run_packet_fec(dabstar_ctx * ctx, cudaStream_t s, PfecPass & p)
 {
-  if (!ctx || (!frame_bits && n_frames > 0) || n_frames < 0 || cap < 0 || (cap > 0 && !out)) return DABSTAR_E_INVALID;
-  if (bit_rate < 8 || bit_rate % 8) return ctx->fail(DABSTAR_E_INVALID, "packet mode: bit rate %d is not a multiple of 8", bit_rate);
-  if (address < 1 || address > 1023) return ctx->fail(DABSTAR_E_INVALID, "packet mode: address %d is not 1..1023", address);
-  if (n_frames == 0) return 0;
+  if (!p.ev0) { CK(cudaEventCreate(&p.ev0)); CK(cudaEventCreate(&p.ev1)); }
+  const int ns = (int)p.streams.size();
+  long long n_slots = 0, n_stage = 0;
+  for (PfecStream & st : p.streams)
+  {
+    st.slot0 = n_slots;
+    st.stage0 = n_stage;
+    const long long n = (long long)st.n_frames * (st.bit_rate / 8);
+    n_slots += n;
+    n_stage += n / 2 + 1; // two run starts are at least two slots apart
+  }
+  p.n_out.assign((size_t)ns, 0);
+  p.slots = n_slots;
+  p.ms = 0;
+  p.rec = nullptr;
+  p.mask = nullptr;
+  if (n_slots == 0) return 0;
+  CK(cudaEventRecord(p.ev0, s));
+  if (p.tables.empty())
+  {
+    pfec_host_tables(p.tables);
+    CK(p.d_tab.reserve(p.tables.size()));
+    CK(cudaMemcpyAsync(p.d_tab.p, p.tables.data(), p.tables.size(), cudaMemcpyHostToDevice, s));
+  }
+  // one copy of the span of every stream's bytes (they lie in one allocation); the corrections go into it
+  const uint8_t * lo = p.streams[0].src, * hi = lo;
+  for (const PfecStream & st : p.streams)
+  {
+    lo = std::min(lo, st.src);
+    hi = std::max(hi, st.src + (size_t)st.n_frames * 3 * st.bit_rate);
+  }
+  CK(p.d_streams.reserve(sizeof(PfecStream) * (size_t)ns));
+  CK(p.d_copy.reserve((size_t)(hi - lo)));
+  CK(p.d_code.reserve((size_t)n_slots));
+  CK(p.d_start.reserve((size_t)n_slots));
+  CK(p.d_mask.reserve((size_t)n_slots));
+  CK(p.d_stage.reserve(sizeof(PfecStage) * (size_t)n_stage));
+  CK(p.d_cnt.reserve(sizeof(int) * (size_t)ns));
+  CK(p.h_cnt.reserve(sizeof(int) * (size_t)ns));
+  CK(cudaMemcpyAsync(p.d_copy.p, lo, (size_t)(hi - lo), cudaMemcpyDeviceToDevice, s));
+  for (PfecStream & st : p.streams) st.dst = p.d_copy.as<uint8_t>() + (st.src - lo);
+  PfecStream * d_st = p.d_streams.as<PfecStream>();
+  CK(cudaMemcpyAsync(d_st, p.streams.data(), sizeof(PfecStream) * (size_t)ns, cudaMemcpyHostToDevice, s));
+  CK(cudaMemsetAsync(p.d_mask.p, 0, (size_t)n_slots, s));
+  CK(launch_pfec_locate(s, d_st, ns, n_slots, p.d_code.as<uint8_t>(), p.d_start.as<uint8_t>(), &ctx->launches));
+  CK(launch_pfec_list(s, d_st, ns, p.d_code.as<uint8_t>(), p.d_start.as<uint8_t>(), p.d_stage.as<PfecStage>(), p.d_cnt.as<int>(), p.d_mask.as<uint8_t>(),
+                      &ctx->launches));
+  CK(cudaMemcpyAsync(p.h_cnt.p, p.d_cnt.p, sizeof(int) * (size_t)ns, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  long long n_rec = 0;
+  for (int i = 0; i < ns; i++)
+  {
+    p.n_out[(size_t)i] = p.h_cnt.as<int>()[i];
+    p.streams[(size_t)i].out0 = n_rec;
+    n_rec += p.n_out[(size_t)i];
+  }
+  CK(p.d_rec.reserve(sizeof(PfecRec) * (size_t)std::max(n_rec, 1LL)));
+  CK(p.h_rec.reserve(sizeof(PfecRec) * (size_t)std::max(n_rec, 1LL)));
+  CK(cudaMemcpyAsync(d_st, p.streams.data(), sizeof(PfecStream) * (size_t)ns, cudaMemcpyHostToDevice, s));
+  CK(launch_pfec_correct(s, d_st, ns, n_rec, p.d_tab.p, p.d_stage.as<PfecStage>(), p.d_rec.as<PfecRec>(), &ctx->launches));
+  if (n_rec > 0) CK(cudaMemcpyAsync(p.h_rec.p, p.d_rec.p, sizeof(PfecRec) * (size_t)n_rec, cudaMemcpyDeviceToHost, s));
+  p.rec = p.h_rec.as<PfecRec>();
+  p.mask = p.d_mask.as<uint8_t>();
+  CK(cudaEventRecord(p.ev1, s));
+  CK(cudaStreamSynchronize(s));
+  float ms = 0;
+  CK(cudaEventElapsedTime(&ms, p.ev0, p.ev1));
+  p.ms = ms;
+  return 0;
+}
+
+// The packed frames of a stage tap in ctx->scratch[1], and the FEC pass run on them when fec is set
+static int packet_tap_in(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, int mem, bool fec)
+{
   CK(cudaSetDevice(ctx->device));
   const size_t n_bits = (size_t)n_frames * 24 * bit_rate;
   const void * dbits;
   if (int r = stage_in(ctx, ctx->scratch[0], frame_bits, n_bits, mem, &dbits)) return r;
   CK(ctx->scratch[1].reserve(n_bits / 8)); // packed frames
   CK(launch_pack_bits(ctx->stream, (const uint8_t *)dbits, ctx->scratch[1].as<uint8_t>(), (long long)(n_bits / 8), &ctx->launches));
+  if (!fec) return 0;
+  PfecPass & f = ctx->pfec;
+  f.streams.assign(1, PfecStream{ ctx->scratch[1].as<uint8_t>(), nullptr, bit_rate, n_frames, 0, 0, 0 });
+  return run_packet_fec(ctx, ctx->stream, f);
+}
+
+static int packet_groups_tap(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, int address, int dg_flag, dabstar_data_group * out, int cap,
+                             uint8_t * payload, int mem, bool fec)
+{
+  if (!ctx || (!frame_bits && n_frames > 0) || n_frames < 0 || cap < 0 || (cap > 0 && !out)) return DABSTAR_E_INVALID;
+  if (bit_rate < 8 || bit_rate % 8) return ctx->fail(DABSTAR_E_INVALID, "packet mode: bit rate %d is not a multiple of 8", bit_rate);
+  if (address < 1 || address > 1023) return ctx->fail(DABSTAR_E_INVALID, "packet mode: address %d is not 1..1023", address);
+  if (n_frames == 0) return 0;
+  if (int r = packet_tap_in(ctx, frame_bits, bit_rate, n_frames, mem, fec)) return r;
   PacketPass & p = ctx->packet;
-  p.subs.assign(1, PacketSub{ ctx->scratch[1].as<uint8_t>(), bit_rate, n_frames, 0, 0 });
+  if (fec) p.subs.assign(1, PacketSub{ ctx->pfec.streams[0].dst, bit_rate, n_frames, 0, 0, ctx->pfec.mask });
+  else p.subs.assign(1, PacketSub{ ctx->scratch[1].as<uint8_t>(), bit_rate, n_frames, 0, 0 });
   p.streams.assign(1, PacketStream{ 0, address, dg_flag ? 1 : 0, 0, 0, 0 });
   if (int r = run_packet(ctx, ctx->stream, p)) return r;
   ctx->arena_off = 0;
@@ -823,6 +907,56 @@ extern "C" int dabstar_packet_groups(dabstar_ctx * ctx, const uint8_t * frame_bi
   {
     if (mem == DABSTAR_MEM_HOST) memcpy(payload, p.payload, bytes);
     else CK(cudaMemcpy(payload, p.payload, bytes, cudaMemcpyHostToDevice));
+  }
+  return n_out;
+}
+
+extern "C" int dabstar_packet_groups(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, int address, int dg_flag, dabstar_data_group * out,
+                                     int cap, uint8_t * payload, int mem)
+{
+  return packet_groups_tap(ctx, frame_bits, bit_rate, n_frames, address, dg_flag, out, cap, payload, mem, false);
+}
+
+extern "C" int dabstar_packet_groups_fec(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, int address, int dg_flag,
+                                         dabstar_data_group * out, int cap, uint8_t * payload, dabstar_packet_stats * stats, dabstar_fec_frame * fec_out,
+                                         int fec_cap, int * n_fec, int mem)
+{
+  if (!ctx || fec_cap < 0 || (fec_cap > 0 && !fec_out)) return DABSTAR_E_INVALID;
+  const int n = packet_groups_tap(ctx, frame_bits, bit_rate, n_frames, address, dg_flag, out, cap, payload, mem, n_frames > 0);
+  if (n < 0) return n;
+  const bool ran = n_frames > 0;
+  const int nf = ran ? ctx->pfec.n_out[0] : 0;
+  for (int i = 0; i < nf && i < fec_cap; i++) fec_out[i] = fec_frame_public(ctx->pfec.rec[i]);
+  if (n_fec) *n_fec = nf;
+  if (stats)
+  {
+    const PacketPass & p = ctx->packet;
+    *stats = ran && !p.n_out.empty() ? packet_stats_public(p.n_out[0], p.rec, p.n_out[0].groups) : dabstar_packet_stats{};
+  }
+  return n;
+}
+
+extern "C" int dabstar_packet_fec(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, uint8_t * corrected_bits, dabstar_fec_frame * out,
+                                  int cap, int mem)
+{
+  if (!ctx || (!frame_bits && n_frames > 0) || n_frames < 0 || cap < 0 || (cap > 0 && !out)) return DABSTAR_E_INVALID;
+  if (bit_rate < 8 || bit_rate % 8) return ctx->fail(DABSTAR_E_INVALID, "packet mode: bit rate %d is not a multiple of 8", bit_rate);
+  if (n_frames == 0) return 0;
+  if (int r = packet_tap_in(ctx, frame_bits, bit_rate, n_frames, mem, true)) return r;
+  ctx->arena_off = 0;
+  const PfecPass & f = ctx->pfec;
+  const int n_out = f.n_out[0];
+  for (int i = 0; i < n_out && i < cap; i++) out[i] = fec_frame_public(f.rec[i]);
+  if (corrected_bits)
+  {
+    const size_t n_bytes = (size_t)n_frames * 3 * bit_rate;
+    std::vector<uint8_t> packed(n_bytes), bits(n_bytes * 8);
+    CK(cudaMemcpyAsync(packed.data(), f.streams[0].dst, n_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    for (size_t i = 0; i < n_bytes; i++)
+      for (int b = 0; b < 8; b++) bits[8 * i + b] = (uint8_t)((packed[i] >> (7 - b)) & 1u);
+    if (mem == DABSTAR_MEM_HOST) memcpy(corrected_bits, bits.data(), bits.size());
+    else CK(cudaMemcpy(corrected_bits, bits.data(), bits.size(), cudaMemcpyHostToDevice));
   }
   return n_out;
 }

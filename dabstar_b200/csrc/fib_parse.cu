@@ -7,8 +7,9 @@
 //   FibDecoder::_subprocess_Fig0s2     decoder/fib_decoder_fig0.cpp:229-290 service -> sub-channel binding
 //   cProtLevelTable                    decoder/fib_table.h:51               EN 300 401 table 8 (short-form index)
 // It feeds MscHandler::set_channel (which sub-channels exist, where, how protected) and EtiGenerator (CIF counter,
-// sub-channel list). FIG 0/3 (EN 300 401 clause 6.3.2: where a packet-mode component is carried) is read from the standard; it
-// feeds the packet pass's self-configuration only and never restarts the parser. Labels, announcements, the "next
+// sub-channel list). FIG 0/3 (EN 300 401 clause 6.3.2: where a packet-mode component is carried) and FIG 0/14 (clause 6.2.2: the
+// FEC scheme of a packet-mode sub-channel) are read from the standard; they feed the packet pass's self-configuration only and
+// never restart the parser. Labels, announcements, the "next
 // configuration" database and the GUI timers of the reference's decoder are not part of it. Only the current configuration
 // (C/N = 0) is collected.
 // Plain host C++ (no device code); lives in a .cu file so that the one nvcc command of build.py picks it up.
@@ -58,10 +59,11 @@ struct dabstar_fib_parser
   std::vector<dabstar_subch> subch;          // in order of first appearance (FibConfigFig0::Fig0s1_BasicSubChannelOrganizationVec)
   std::vector<dabstar_service_comp> comps;   // (SId, component index) in order of first appearance
   std::vector<dabstar_packet_comp> pcomps;   // FIG 0/3, by SCId in order of first appearance
+  std::vector<dabstar_fec_scheme> fec;       // FIG 0/14, by SubChId in order of first appearance
   int prev_change = 0;
   int restarts = 0;
 
-  void restart() { subch.clear(); comps.clear(); pcomps.clear(); restarts++; }   // FibDecoder::_restart_fib_decoding: collected content is untrustworthy
+  void restart() { subch.clear(); comps.clear(); pcomps.clear(); fec.clear(); restarts++; }   // FibDecoder::_restart_fib_decoding: collected content is untrustworthy
 
   // returns bytes used, -1 to abandon the FIB, or -2 to abandon this FIG: an entry that would cross the end of the FIG
   // (fig_bits = its length in bits) is not read - a CRC-good but malformed FIG must not make the parser read past the FIB
@@ -153,6 +155,18 @@ struct dabstar_fib_parser
     return (o + len) / 8;
   }
 
+  // FIG 0/14: SubChId (6), FEC scheme (2)
+  int fig0s14(const uint8_t * d, int off_bytes, int fig_bits)
+  {
+    const int o = off_bytes * 8;
+    if (o + 8 > fig_bits) return -2;
+    const dabstar_fec_scheme e{ (int)bits(d, o, 6), (int)bits(d, o + 6, 2) };
+    bool known = false;
+    for (const dabstar_fec_scheme & x : fec) if (x.sub_ch_id == e.sub_ch_id) known = true;
+    if (!known) fec.push_back(e);
+    return (o + 8) / 8;
+  }
+
   void push(const uint8_t * fib) // 256 bits, one per byte; the caller has checked the CRC
   {
     int processed = 0;
@@ -179,6 +193,11 @@ struct dabstar_fib_parser
         {
           int used = 2;
           while (used < len + 1 && (used = fig0s3(d, used, 8 * (len + 1))) >= 0) {}
+        }
+        else if (cn == 0 && ext == 14)
+        {
+          int used = 2;
+          while (used < len + 1 && (used = fig0s14(d, used, 8 * (len + 1))) >= 0) {}
         }
         else if (cn == 0 && (ext == 1 || ext == 2))
         {
@@ -240,4 +259,11 @@ extern "C" int dabstar_fib_parser_packet_components(const dabstar_fib_parser * p
   const int n = (int)p->pcomps.size() < cap ? (int)p->pcomps.size() : cap;
   for (int i = 0; i < n; i++) out[i] = p->pcomps[i];
   return (int)p->pcomps.size();
+}
+extern "C" int dabstar_fib_parser_fec_schemes(const dabstar_fib_parser * p, dabstar_fec_scheme * out, int cap)
+{
+  if (!p || (!out && cap > 0)) return DABSTAR_E_INVALID;
+  const int n = (int)p->fec.size() < cap ? (int)p->fec.size() : cap;
+  for (int i = 0; i < n; i++) out[i] = p->fec[i];
+  return (int)p->fec.size();
 }

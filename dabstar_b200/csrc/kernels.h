@@ -4,6 +4,7 @@
 #include "viterbi.cuh"
 #include "mp2.cuh"
 #include "packet.cuh"
+#include "pfec.cuh"
 
 #include <vector>
 
@@ -177,6 +178,7 @@ struct PacketSub
   int bit_rate, n_frames;
   long long frame0;        // first of its logical frames in the pass's frame index space
   long long slot0;         // first of its n_frames * bit_rate / 8 packet slots
+  const uint8_t * fec = nullptr; // packet-mode FEC: one byte per 24-byte slot, non-zero on FEC packets (src is then the corrected copy)
 };
 struct PacketStream
 {
@@ -214,6 +216,37 @@ cudaError_t launch_packet_walk(cudaStream_t s, const PacketSub * sub, const Pack
 // the groups' records and useful data, n_out of them, in stream order from out_rec0 / out_pay0; the MSC data group headers parsed
 cudaError_t launch_packet_compact(cudaStream_t s, const PacketSub * sub, const PacketStream * st, int n_streams, long long n_out, const PacketSlot * slots,
                                   const PacketStage * stage, DgRec * out_rec, uint8_t * out_pay, unsigned long long * lc);
+
+// pfec_kernels.cu: packet-mode FEC over a table of streams (one FEC sub-channel of one recording each; pfec.cuh). A stream's
+// slots are its 24-byte slots, n_frames * bit_rate / 8 of them.
+struct PfecStream
+{
+  const uint8_t * src;     // n_frames logical frames of 3 * bit_rate packed bytes, as received
+  uint8_t * dst;           // the same bytes, copied before the pass; the corrections go here
+  int bit_rate, n_frames;
+  long long slot0;         // first of its slots in the pass's per-slot arrays (fit codes, run starts, FEC mask)
+  long long stage0;        // first of its located runs (room for one per two slots)
+  long long out0;          // first output record (set from the locate counts)
+};
+struct PfecStage           // a located run: its slot, its score, whether its frame is INCOMPLETE
+{
+  int run, score, incomplete;
+};
+struct PfecRec             // layout of dabstar_fec_frame
+{
+  int32_t first_slot, run_slot, first_frame, last_frame, status;
+  int32_t rows_corrected, rows_failed, bytes_corrected, headers_matched, reserved;
+};
+void pfec_host_tables(std::vector<uint8_t> & blob);
+// code[slot] = pfec_slot_code, then start[slot] = pfec_run_start, for every slot of every stream
+cudaError_t launch_pfec_locate(cudaStream_t s, const PfecStream * st, int n_streams, long long n_slots, uint8_t * code, uint8_t * start, unsigned long long * lc);
+// per stream (a block each): its runs in stream order at stage[stage0 ..], their count in cnt, and mask[slot0 + i] = 1 on the
+// slots of its runs (mask zeroed by the caller)
+cudaError_t launch_pfec_list(cudaStream_t s, const PfecStream * st, int n_streams, const uint8_t * code, const uint8_t * start, PfecStage * stage, int * cnt,
+                             uint8_t * mask, unsigned long long * lc);
+// the n_out frames (stream order from out0): rows decoded, corrections into dst, records into rec
+cudaError_t launch_pfec_correct(cudaStream_t s, const PfecStream * st, int n_streams, long long n_out, const void * tables, const PfecStage * stage, PfecRec * rec,
+                                unsigned long long * lc);
 
 // ofdm_kernels.cu
 cudaError_t launch_init_ref_arg(cudaStream_t s, const DeviceTables & t, unsigned long long * lc);

@@ -4,8 +4,9 @@
 //
 // Source: ETSI EN 300 401 clause 5.3.2 (packet structure: 24 / 48 / 72 / 96-byte packets, 24-bit header, CRC-16) and clause
 // 5.3.3 (MSC data group: header, session header, data field, CRC-16). Both CRCs are the FIB CRC of clause 5.2.1:
-// x^16 + x^12 + x^5 + 1, preset 0xFFFF, complemented, transmitted most significant bit first. Packet-mode FEC (FIG 0/14, the
-// RS(204,188) outer code of clause 5.3.5) is not part of this pass.
+// x^16 + x^12 + x^5 + 1, preset 0xFFFF, complemented, transmitted most significant bit first. On a sub-channel with packet-mode
+// FEC (FIG 0/14, the RS(204,188) outer code of clause 5.3.5, pfec.cuh) the frames are walked after correction, and a packet that
+// starts on a slot of an FEC-packet run is skipped (PKT_FEC).
 #pragma once
 #include <cstdint>
 
@@ -19,6 +20,7 @@ enum : int
   PKT_BAD_LENGTH = 2, // CRC good, useful data length > packet length - 5
   PKT_CUT = 3,        // the packet would run past the end of the logical frame; the frame's walk ends there
   PKT_EMPTY = 4,      // no packet starts in this slot (the frame's packets ended before it)
+  PKT_FEC = 5,        // an FEC packet (24 bytes) of packet-mode FEC: skipped, counted in the FEC frame records only
 };
 // status of a data group
 enum : int
@@ -70,14 +72,21 @@ __host__ __device__ inline int packet_classify(const uint8_t * p, int avail, uin
 }
 
 // The packets of one logical frame of fb bytes: slot k gets the k-th packet (fb / 24 slots; the rest PKT_EMPTY). Returns the
-// number of packets found (a PKT_CUT one included).
-__host__ __device__ inline int packet_frame(const uint8_t * f, int fb, PacketSlot * slots)
+// number of packets found (a PKT_CUT one included). fec (packet-mode FEC only): one byte per 24-byte slot of the frame, non-zero
+// where an FEC packet lies.
+__host__ __device__ inline int packet_frame(const uint8_t * f, int fb, PacketSlot * slots, const uint8_t * fec = nullptr)
 {
   const int n_slots = fb / 24;
   int pos = 0, k = 0;
   while (pos < fb && k < n_slots)
   {
     uint32_t h;
+    if (fec && fec[pos / 24])
+    {
+      slots[k++] = PacketSlot{ ((uint32_t)f[pos] << 16) | ((uint32_t)f[pos + 1] << 8) | f[pos + 2], (uint16_t)pos, (uint8_t)PKT_FEC, 0 };
+      pos += 24;
+      continue;
+    }
     const int c = packet_classify(f + pos, fb - pos, &h);
     slots[k++] = PacketSlot{ h, (uint16_t)pos, (uint8_t)c, 0 };
     if (c == PKT_CUT) break;

@@ -16,7 +16,8 @@ namespace dab
 {
 namespace
 {
-// thread = logical frame of any sub-channel: its packets into the frame's slots
+// thread = logical frame of any sub-channel: its packets into the frame's slots (with packet-mode FEC: of its corrected bytes, the
+// FEC packets skipped)
 __global__ void __launch_bounds__(128) k_packet_scan(const PacketSub * __restrict__ sub, int n_subs, long long n_frames, PacketSlot * __restrict__ slots)
 {
   const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -24,7 +25,7 @@ __global__ void __launch_bounds__(128) k_packet_scan(const PacketSub * __restric
   const PacketSub & s = sub[find_stream(sub, n_subs, g, [](const PacketSub & x) { return x.frame0; })];
   const long long f = g - s.frame0;
   const int fb = 3 * s.bit_rate, spf = s.bit_rate / 8;
-  packet_frame(s.src + f * fb, fb, slots + s.slot0 + f * spf);
+  packet_frame(s.src + f * fb, fb, slots + s.slot0 + f * spf, s.fec ? s.fec + f * spf : nullptr);
 }
 
 // What the walk carries from chunk to chunk. Scan 1: the CI of the last packet of the address (0 none, 4 | CI), and the count

@@ -19,6 +19,9 @@
 //     -p  all|id:address[,id:address...]: packet-mode data groups of those (sub-channel, address) streams (all: every packet-mode
 //         component of the recording's FIG 0/2 and 0/3, needs -a), packets and groups checked on the GPU; prints per stream the
 //         packet and group counters; with -o, <prefix><n>.subch<id>.addr<address>.dg holds the groups' bytes in order
+//     -F  all|id[,id...]: packet-mode FEC (RS(204,188) FEC frames located and corrected on the GPU) in front of -p on those
+//         sub-channels (all: every sub-channel the recording's FIG 0/14 gives FEC scheme 1, needs -a); prints per FEC sub-channel
+//         its FEC frames per status and the rows corrected / failed
 //     -q  signal quality of every frame as CSV: frame,sym0_pos,mer_db,snr_db,noise_power,fbb_hz (fbb_hz: the baseband frequency
 //         correction of the frame's data symbols); with several files, file n's lines go to <path>.<n>
 //
@@ -51,7 +54,7 @@ int main(int argc, char ** argv)
   int fmt = DABSTAR_FMT_U8;
   bool autoCfg = false, eti = false, xml = false, containers = false, tii = false;
   dabstar_sample_format sf{};
-  std::string prefix = "dab_out_", qualPath, dabplus, mp2, packet;
+  std::string prefix = "dab_out_", qualPath, dabplus, mp2, packet, fec;
   bool prefixSet = false;
   std::vector<dabstar_subch> subch;
   std::vector<const char *> files;
@@ -63,6 +66,7 @@ int main(int argc, char ** argv)
     else if (a == "-d" && i + 1 < argc) dabplus = argv[++i];
     else if (a == "-m" && i + 1 < argc) mp2 = argv[++i];
     else if (a == "-p" && i + 1 < argc) packet = argv[++i];
+    else if (a == "-F" && i + 1 < argc) fec = argv[++i];
     else if (a == "-a") autoCfg = true;
     else if (a == "-t") tii = true;
     else if (a == "-c") { containers = true; fmt = DABSTAR_FMT_CF32; }
@@ -147,10 +151,19 @@ int main(int argc, char ** argv)
       streams.push_back({ atoi(item.substr(0, c).c_str()), atoi(item.substr(c + 1).c_str()) });
       p = q + 1;
     }
+    std::vector<int> fecIds; // -F id list
+    for (size_t p = 0; fec != "all" && p < fec.size();)
+    {
+      const size_t q = std::min(fec.find(',', p), fec.size());
+      fecIds.push_back(atoi(fec.substr(p, q - p).c_str()));
+      p = q + 1;
+    }
     for (size_t r = 0; r < files.size(); r++)
     {
       if (packet == "all") proc.set_packet((int)r, -1);
       for (const auto & x : streams) proc.set_packet((int)r, x.first, x.second);
+      if (fec == "all") proc.set_packet_fec((int)r, -1);
+      for (int id : fecIds) proc.set_packet_fec((int)r, id);
     }
     if (!qualPath.empty()) proc.set_frame_quality(true);
     if (xml && !containers) proc.run_files(ptrs, ns, sf);
@@ -244,6 +257,19 @@ int main(int argc, char ** argv)
                files[r], id, addr, gr.size(), (long long)st.groups[0], (long long)st.groups[1], (long long)st.groups[2], (long long)st.groups[3], (long long)st.groups[4],
                (long long)st.packets, (long long)st.crc_errors, (long long)st.bad_length, (long long)st.cut, (long long)st.padding, (long long)st.command,
                (long long)st.other_address, (long long)st.continuity_breaks, (long long)st.abandoned, (long long)st.dropped);
+      }
+      for (int id = 0; !fec.empty() && id < 64; id++)
+      {
+        if (!proc.fec_decoded((int)r, id)) continue;
+        long cnt[4] = { 0 }, fixed = 0, failed = 0, bytes = 0;
+        const std::vector<dabstar_fec_frame> fr = proc.fec_frames((int)r, id);
+        for (const auto & x : fr)
+        {
+          if (x.status >= 0 && x.status < 4) cnt[x.status]++;
+          fixed += x.rows_corrected; failed += x.rows_failed; bytes += x.bytes_corrected;
+        }
+        printf("%s: FEC sub-channel %d: %zu FEC frames, %ld clean, %ld corrected, %ld partial, %ld incomplete; %ld rows corrected (%ld bytes), %ld rows failed\n",
+               files[r], id, fr.size(), cnt[0], cnt[1], cnt[2], cnt[3], fixed, bytes, failed);
       }
       if (autoCfg && tii)
         for (const auto & ev : proc.tii_events((int)r))

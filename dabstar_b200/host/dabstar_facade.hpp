@@ -519,6 +519,11 @@ public:
   {
     mC.check(dabstar_decoder_set_packet(mDec, recording, subChId, address, on ? 1 : 0), "dabstar_decoder_set_packet");
   }
+  // packet-mode FEC in front of the packet pass: subChId forces it on; -1 every sub-channel the recording's FIG 0/14 flags
+  void set_packet_fec(int recording, int subChId = -1, bool on = true)
+  {
+    mC.check(dabstar_decoder_set_packet_fec(mDec, recording, subChId, on ? 1 : 0), "dabstar_decoder_set_packet_fec");
+  }
   bool packet_decoded(int recording, int subChId, int address) const { return dabstar_decoder_data_groups(mDec, recording, subChId, address, nullptr, 0) >= 0; }
   // the last run's data groups of the stream; every group goes to sink, in order
   std::vector<dabstar_data_group> data_groups(int recording, int subChId, int address, const PacketProcessor::GroupSink & sink = nullptr) const
@@ -539,6 +544,14 @@ public:
     dabstar_packet_stats st{};
     mC.check(dabstar_decoder_packet_stats(mDec, recording, subChId, address, &st), "dabstar_decoder_packet_stats");
     return st;
+  }
+  bool fec_decoded(int recording, int subChId) const { return dabstar_decoder_fec_frames(mDec, recording, subChId, nullptr, 0) >= 0; }
+  // the last run's FEC frame records of a sub-channel with packet-mode FEC
+  std::vector<dabstar_fec_frame> fec_frames(int recording, int subChId) const
+  {
+    std::vector<dabstar_fec_frame> v((size_t)mC.check(dabstar_decoder_fec_frames(mDec, recording, subChId, nullptr, 0), "dabstar_decoder_fec_frames"));
+    if (!v.empty()) dabstar_decoder_fec_frames(mDec, recording, subChId, v.data(), (int)v.size());
+    return v;
   }
   // FIG 0/3 packet-mode components of a self-configured recording after the last run
   std::vector<dabstar_packet_comp> packet_components(int recording) const

@@ -39,7 +39,8 @@ class _Cfg(ctypes.Structure):
                 ("snr_db", ctypes.c_float), ("cfo_hz", ctypes.c_float), ("rms", ctypes.c_float),
                 ("lead_samples", ctypes.c_int32), ("tail_samples", ctypes.c_int32), ("n_subch", ctypes.c_int32),
                 ("subch", ctypes.c_void_p), ("fig_mode", ctypes.c_int32), ("eid", ctypes.c_int32), ("tii_main", ctypes.c_int32), ("tii_sub", ctypes.c_int32),
-                ("msc_payload", ctypes.c_void_p), ("n_packet", ctypes.c_int32), ("packet", ctypes.c_void_p)]
+                ("msc_payload", ctypes.c_void_p), ("n_packet", ctypes.c_int32), ("packet", ctypes.c_void_p),
+                ("n_fec", ctypes.c_int32), ("fec", ctypes.c_void_p)]
 
 
 @dataclass
@@ -68,7 +69,7 @@ def _load():
 def generate(n_frames: int, seed: int = 1, snr_db: float = 20.0, cfo_hz: float = 0.0, subch: list[SubChannel] | None = None,
              fmt: int = FMT_U8, rms: float = 0.25, lead_samples: int = 60000, tail_samples: int = 4096, out: np.ndarray | None = None,
              fig_mode: int = 0, eid: int = 0x1234, tii: tuple[int, int] | None = None, msc_payload: list | None = None,
-             packet: list | None = None) -> Recording:
+             packet: list | None = None, fec: list | None = None) -> Recording:
     """Synthesise `n_frames` Mode-I transmission frames. `lead_samples` of noise-like filler precede the first
     null symbol (the reference spends 40 960 samples on its level estimate before it searches the null).
     fig_mode 1: the FIC carries the ensemble's multiplex configuration (FIG 0/0 with a running CIF counter, FIG 0/1, FIG 0/2)
@@ -78,7 +79,9 @@ def generate(n_frames: int, seed: int = 1, snr_db: float = 20.0, cfo_hz: float =
     (e.g. DAB+ super-frames from tests/helpers.dabplus_superframe); the other sub-channels draw what they draw without it.
     packet: with fig_mode 1, [(sub_ch_id, scid, address, dscty, dg_flag), ...]: each listed sub-channel carries no programme service;
     each entry becomes a data service with one packet-mode (TMId 3) component in FIG 0/2 and a FIG 0/3 entry. Without it every
-    output is what it is without the argument."""
+    output is what it is without the argument.
+    fec: with fig_mode 1, [sub_ch_id, ...]: each is sent as a FIG 0/14 entry with FEC scheme 1 (packet-mode FEC); the payload itself
+    is whatever msc_payload carries. Without it every output is what it is without the argument."""
     lib = _load()
     subch = subch or []
     tab = subch_table(subch)
@@ -90,8 +93,10 @@ def generate(n_frames: int, seed: int = 1, snr_db: float = 20.0, cfo_hz: float =
             keep.append(None if p is None else np.ascontiguousarray(p, np.uint8).reshape(4 * n_frames, 24 * s.bit_rate))
         pay = (ctypes.c_void_p * max(len(subch), 1))(*[None if k is None else k.ctypes.data for k in keep])
     ptab = np.ascontiguousarray(np.array(packet or [], np.int32).reshape(-1, 5))
+    ftab = np.ascontiguousarray(np.array(fec or [], np.int32).reshape(-1))
     cfg = _Cfg(n_frames, fmt, seed, snr_db, cfo_hz, rms, lead_samples, tail_samples, len(subch), tab.ctypes.data, fig_mode, eid, tii[0] if tii else -1, tii[1] if tii else -1,
-               ctypes.cast(pay, ctypes.c_void_p) if pay is not None else None, len(ptab), ptab.ctypes.data if len(ptab) else None)
+               ctypes.cast(pay, ctypes.c_void_p) if pay is not None else None, len(ptab), ptab.ctypes.data if len(ptab) else None,
+               len(ftab), ftab.ctypes.data if len(ftab) else None)
     n = lib.dabsynth_num_samples(ctypes.byref(cfg))
     if out is None:
         out = np.empty(n, np.complex64) if fmt == FMT_CF32 else np.empty((n, 2), np.uint8 if fmt == FMT_U8 else np.int16)

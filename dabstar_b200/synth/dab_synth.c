@@ -44,6 +44,8 @@ typedef struct
   int32_t  n_packet;      /* fig_mode 1: packet-mode components (0: none, and the FIC is what it is without them) */
   const int32_t * packet; /*   n_packet x 5: subChId, SCId, packet address, DSCTy, DG flag. A listed sub-channel carries no programme
                                service; each entry becomes a data service with one TMId 3 component (FIG 0/2, P/D 1) and a FIG 0/3 entry */
+  int32_t  n_fec;         /* fig_mode 1: sub-channels flagged with packet-mode FEC (0: none, and the FIC is what it is without them) */
+  const int32_t * fec;    /*   n_fec subChIds, each sent as a FIG 0/14 entry with FEC scheme 1 (EN 300 401 clause 6.2.2) */
 } dabsynth_cfg;
 
 /* ---------------------------------------------------------------------------------------------- rng */
@@ -423,6 +425,20 @@ static int build_mci(const dabsynth_cfg * c, int f, fic_writer * w)
         }
       }
     }
+  }
+  /* FIG 0/14: SubChId (6 bits), FEC scheme (2 bits) */
+  i = 0;
+  while (i < c->n_fec)
+  {
+    int room = 30 - w->used;
+    if (room < 2 + 1) room = 30;
+    int n = room - 2;
+    if (n > c->n_fec - i) n = c->n_fec - i;
+    p = ficw_reserve(w, 2 + n);
+    if (!p || n == 0) return -1;
+    p[0] = (uint8_t)((0 << 5) | (1 + n));
+    p[1] = 14;                                          /* C/N 0, OE 0, P/D 0, extension 14 */
+    for (int k = 0; k < n; k++, i++) p[2 + k] = (uint8_t)(((c->fec[i] & 63) << 2) | 1);
   }
   ficw_finish(w);
   return 0;

@@ -313,8 +313,9 @@ int dabstar_mp2_frames(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_ra
  * continuity index is the previous one's plus 1 (mod 4); first opens a group (abandoning an open one), single is a group of its
  * own, intermediate keeps an open group only if it continues it, last closes an open group it continues into a record. Any
  * other packet abandons the open group or, without one, is dropped. With DG flag 0 the group is an MSC data group: its header,
- * session header and CRC are parsed and checked (status below); with DG flag 1 it is a RAW record. Packet-mode FEC (FIG 0/14,
- * RS(204,188)) is not applied: sub-channels that use it are decoded without the outer code. */
+ * session header and CRC are parsed and checked (status below); with DG flag 1 it is a RAW record. Sub-channels with packet-mode
+ * FEC (FIG 0/14 scheme 1, the RS(204,188) outer code of clause 5.3.5) are decoded with dabstar_packet_groups_fec: their FEC
+ * frames are located and corrected first (see dabstar_packet_fec), and the FEC packets are skipped. */
 enum { DABSTAR_DG_OK = 0, DABSTAR_DG_NO_CRC = 1, DABSTAR_DG_CRC_ERROR = 2, DABSTAR_DG_MALFORMED = 3, DABSTAR_DG_RAW = 4 };
 typedef struct
 {
@@ -350,6 +351,35 @@ typedef struct
   int64_t dropped;            /* intermediate / last packets without an open group */
   int64_t groups[5];          /* groups by status (DABSTAR_DG_*) */
 } dabstar_packet_stats;
+
+/* Packet-mode FEC (EN 300 401 clause 5.3.5), on the device. An FEC frame is an Application Data Table of 2256 bytes (94 slots of 24
+ * bytes holding whole packets) followed by 9 FEC packets of 24 bytes (2-byte header: length 00, continuity index, first / last
+ * flags, address 1022; 22 bytes of RS data), 103 slots that start on any 24-byte slot boundary of the stream. ADT and RS data form
+ * a 12 x 204 table filled column by column; each row is an RS(204,188) code word (shortened RS(255,239), field
+ * x^8 + x^4 + x^3 + x^2 + 1, roots alpha^0..alpha^15) that corrects up to 8 byte errors. The runs of FEC packets are located slot
+ * by slot (dabstar_b200/csrc/pfec.cuh states the rule: at least 6 of the 9 headers must fit, with their first / last flags); a
+ * row with more than 8 errors is left as received. */
+enum { DABSTAR_FEC_CLEAN = 0, DABSTAR_FEC_CORRECTED = 1, DABSTAR_FEC_PARTIAL = 2, DABSTAR_FEC_INCOMPLETE = 3 };
+typedef struct
+{
+  int32_t first_slot;          /* first 24-byte slot of the frame's ADT in the stream (< 0: the frame is cut by the stream start) */
+  int32_t run_slot;            /* first slot of its 9 FEC packets */
+  int32_t first_frame, last_frame; /* logical frames of its first and last slot inside the stream */
+  int32_t status;              /* DABSTAR_FEC_*: CLEAN, CORRECTED, PARTIAL (some rows failed), INCOMPLETE (cut by the stream's start
+                                  or end, or the previous run lies inside its ADT: not corrected) */
+  int32_t rows_corrected, rows_failed, bytes_corrected;
+  int32_t headers_matched;     /* FEC packet headers of the run that fit (of 9) */
+  int32_t reserved;
+} dabstar_fec_frame;
+/* The FEC pass alone: frame_bits as for dabstar_packet_groups; corrected_bits (may be NULL): the same bits after correction, in the
+ * same layout; out: one record per located FEC frame, in stream order (at most cap are written). Returns the number of frames or <0. */
+int dabstar_packet_fec(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, uint8_t * corrected_bits, dabstar_fec_frame * out,
+                       int cap, int mem);
+/* dabstar_packet_groups with the FEC pass in front: the packets are walked on the corrected bytes, and a packet that starts on a
+ * slot of a located FEC-packet run is skipped (it counts in no dabstar_packet_stats field). stats (may be NULL): the stream's
+ * counters; fec_out: the FEC frame records (at most fec_cap), *n_fec (may be NULL): their number. Returns the number of groups or <0. */
+int dabstar_packet_groups_fec(dabstar_ctx * ctx, const uint8_t * frame_bits, int bit_rate, int n_frames, int address, int dg_flag, dabstar_data_group * out,
+                              int cap, uint8_t * payload, dabstar_packet_stats * stats, dabstar_fec_frame * fec_out, int fec_cap, int * n_fec, int mem);
 
 /* ------------------------------------------------------------------------------------------------ multiplex configuration (FIG 0/0, 0/1, 0/2) */
 /* The part of FibDecoder the decode path depends on (decoder/fib_decoder.cpp:59-106 process_FIB,
@@ -391,6 +421,14 @@ typedef struct
   int32_t ca_org; /* -1 if absent */
 } dabstar_packet_comp;
 int  dabstar_fib_parser_packet_components(const dabstar_fib_parser * p, dabstar_packet_comp * out, int cap);
+/* FIG 0/14 (EN 300 401 clause 6.2.2): the FEC scheme of a packet-mode sub-channel: 0 none, 1 the FEC of clause 5.3.5, 2 and 3
+ * reserved (treated as none). Current configuration only, first appearance of each SubChId kept; an entry that would cross the end
+ * of its FIG is not read. FIG 0/14 never restarts the parser and leaves the other lists alone. */
+typedef struct
+{
+  int32_t sub_ch_id, scheme;
+} dabstar_fec_scheme;
+int  dabstar_fib_parser_fec_schemes(const dabstar_fib_parser * p, dabstar_fec_scheme * out, int cap);
 
 /* Cyclic-prefix correlation of DabProcessor::_process_ofdm_symbols_1_to_L (main/dab_processor.cpp:317-333): samples = n frames x
  * 75 x 2552 complex floats (data symbols 1..75 of a frame with their prefixes); out = n x (re, im) of
@@ -538,6 +576,21 @@ double  dabstar_decoder_packet_ms(const dabstar_decoder * dec);
 /* FIG 0/3 packet-mode components of a self-configured recording as the FIB parser holds them at the end of the run; returns the
  * count (E_INVALID: not self-configured) */
 int     dabstar_decoder_packet_components(const dabstar_decoder * dec, int recording, dabstar_packet_comp * out, int cap);
+/* Packet-mode FEC (see dabstar_packet_fec) in front of the packet pass for a sub-channel, off by default. An explicit sub_ch_id
+ * forces it on for that sub-channel (its bit rate must be a multiple of 8; with auto-config it is looked up in the run's own FIC);
+ * -1: every sub-channel the recording's own FIG 0/14 gives scheme 1 (needs auto-config). It applies to sub-channels that also have
+ * a dabstar_decoder_set_packet stream; their data groups are then those of dabstar_packet_groups_fec. The run's MSC payload
+ * (dabstar_decoder_msc_copy / _packed) stays as received. enable = 0 deselects it. scan_mode decodes nothing; streaming is not
+ * supported (DABSTAR_E_UNSUPPORTED). */
+int     dabstar_decoder_set_packet_fec(dabstar_decoder * dec, int recording, int sub_ch_id, int enable);
+/* the FEC frame records of one sub-channel in the last run, exactly as dabstar_packet_fec returns them for dabstar_decoder_msc_copy's
+ * bits of that sub-channel; returns the count (E_INVALID: no FEC pass on it in the last run) */
+int     dabstar_decoder_fec_frames(const dabstar_decoder * dec, int recording, int sub_ch_id, dabstar_fec_frame * out, int cap);
+/* device time of the last run's FEC pass */
+double  dabstar_decoder_packet_fec_ms(const dabstar_decoder * dec);
+/* FIG 0/14 FEC schemes of a self-configured recording as the FIB parser holds them at the end of the run; returns the count
+ * (E_INVALID: not self-configured) */
+int     dabstar_decoder_fec_schemes(const dabstar_decoder * dec, int recording, dabstar_fec_scheme * out, int cap);
 /* EtiGenerator (eti_handler/eti_generator.h:56-66: start_eti_generator before run / process_block per symbol): every
  * sub-channel set with dabstar_decoder_set_subchannels is decoded for every CIF through the generator's own whole-CIF
  * de-interleaver (first frame with its 17th CIF; its start-up bookkeeping, which loses the 16th CIF, is reproduced) and
